@@ -23,6 +23,7 @@ import time
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from untouched (it may be read-only)
 sys.path.insert(0, ROOT)
 from grapes_b200.synth import SHAPES  # noqa: E402
 
@@ -48,7 +49,15 @@ def parse_args():
     ap.add_argument("--full-eval", action="store_true",
                     help="also run scripts/bench_full_eval.py (full-graph evaluation forward on the opt-in tensor-core path, NOT yet "
                          "verified on a GPU) in a process of its own and attach its line as `full_graph_eval`")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (losses, sampler statistics, sampled "
+                         "nodes, classifier logits, updated parameters) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "grapes_b200":
+        ap.error("--dump-outputs writes the outputs of the grapes_b200 arm")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
@@ -231,6 +240,41 @@ def load_peaks():
     return 6650.0, 1400.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(eng, out_dir: str):
+    """Writes what the engine's last step handed back to its caller as ``out_dir/<name>.npy``: the losses and the per-hop
+    sampler statistics main.py logs, the nodes sampled at each hop, the batch's nodes with the classifier's logits over
+    them, the three networks' parameters after the optimiser update and the two optimisers' step counts (every step the
+    engine ran, untimed ones included).  Floats stay float32; node ids are stored as
+    float64 (exact).  The workload and every random draw are functions of the command-line seed, so two builds run with
+    the same arguments can be compared file by file."""
+    import numpy as np
+    from grapes_b200.engine import SCAL
+    torch.cuda.synchronize()
+    scal = eng.scal.cpu().double()
+    out = {k: scal[SCAL[k]:SCAL[k] + 1] for k in ("loss_c", "loss_gfn", "log_z", "tot_log_prob")}
+    out["sampler_stats"] = eng.stats.cpu()
+    for h, sz in enumerate(eng.hop_sizes()):
+        out[f"sampled_hop{h}"] = eng.prev[h + 1][eng.bsz:eng.bsz + sz["s"]].cpu().double()
+    A = eng.count("A")
+    out["all_nodes"] = eng.all_nodes[:A].cpu().double()
+    out["logits_c"] = eng.logits_c[:A].cpu()
+    out["adam_steps"] = eng.adam_steps.cpu()
+    for net, params in eng.state_dicts().items():
+        for name, t in params.items():
+            out[f"{net}.{name}"] = t.cpu()
+    arrays = {k: v.numpy() for k, v in out.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (k, a.dtype)
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------
 def cpu_reference_run(cfg, indptr, indices, x, y, train_idx, steps, warmup, budget_s, rank_offset=0):
     """Times the reference's CPU path (oracle port of main.py:161-291 + restated PyG GCNConv, torch CPU
@@ -384,6 +428,8 @@ def main():
     clocks = sampler.stop()
     ms = ev[0].elapsed_time(ev[K])
     eng.check_overflow()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)         # before the e2e and profiling steps below overwrite them
     if use_graph:
         # kernels recorded into the graph once, replayed K times (the NCCL exchange adds its own all-reduce kernel)
         per_step = eng.launches_per_graph + (1 if exchange_used == "nccl" else 0)

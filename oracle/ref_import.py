@@ -1,7 +1,10 @@
-"""TEST INFRASTRUCTURE ONLY.  Imports the reference's own ``modules/utils.py`` from
-/root/reference (present in the build container, absent on the GPU box) so the
-restatement in oracle/reference_port.py can be validated against it and golden vectors
-can be generated from it.  Nothing under tests -m gpu, smoke() or bench.py may use this.
+"""TEST INFRASTRUCTURE ONLY.  Imports the reference's own ``modules/utils.py`` from the
+checkout of the reference GRAPES project that ``GRAPES_REFERENCE_ROOT`` names (it is not
+part of this repository) so the restatement in oracle/reference_port.py can be validated
+against it and golden vectors can be generated from it.  Without it the live comparisons
+skip; the committed golden vectors hold the reference's outputs only for the cases
+tests/golden/make_golden.py records.  Nothing under tests -m gpu, smoke() or bench.py may
+use this.
 
 The reference pins scipy 1.13.1 (environment.yml:95); on scipy 1.18 indexing a CSR matrix
 with a ``torch.Tensor`` raises, so :class:`TensorIndexCSR` converts tensor indices to numpy
@@ -17,15 +20,15 @@ import numpy as np
 import scipy.sparse as sp
 import torch
 
-REFERENCE_ROOT = os.environ.get("GRAPES_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("GRAPES_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "modules", "utils.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "modules", "utils.py"))
 
 
 def load_reference_utils():
-    """Import /root/reference/modules/utils.py as a stand-alone module (it only needs
+    """Import the reference's modules/utils.py (under ``REFERENCE_ROOT``) as a stand-alone module (it only needs
     logging/os/numpy/psutil/scipy/torch, utils.py:1-10)."""
     path = os.path.join(REFERENCE_ROOT, "modules", "utils.py")
     spec = importlib.util.spec_from_file_location("grapes_reference_utils", path)
@@ -68,7 +71,7 @@ def reference_adjacency(edge_index: torch.Tensor, num_nodes: int) -> TensorIndex
 
 
 def load_reference_eval():
-    """Import /root/reference/eval.py (``evaluate``, eval.py:11-165) as a stand-alone module.  It imports
+    """Import the reference's eval.py (``evaluate``, eval.py:11-165) as a stand-alone module.  It imports
     ``torch_geometric`` for ONE type annotation (eval.py:4,14: absent here) and ``modules.utils`` (the reference's own,
     loaded by :func:`load_reference_utils`); both names are bound for the duration of the import only.  Everything the
     function then executes is the reference's own code."""
@@ -97,7 +100,7 @@ def load_reference_eval():
 
 
 def load_reference_gcn(conv_factory):
-    """Import /root/reference/modules/gcn.py with ``torch_geometric.nn.GCNConv`` bound to ``conv_factory`` (PyG is absent;
+    """Import the reference's modules/gcn.py with ``torch_geometric.nn.GCNConv`` bound to ``conv_factory`` (PyG is absent;
     the other convolutions it imports are never instantiated on this path).  The returned module's ``GCN`` is the
     reference's own class -- layer list, which edge list feeds which layer, relu / dropout placement, ``(logits,
     memory_alloc)`` return (gcn.py:9-42) -- over the oracle's restatement of the one GCNConv layer."""
@@ -167,7 +170,7 @@ class WandbStub:
 def load_reference_train(get_data, gcn_factory, utils_overrides=None):
     """The reference's own ``train(args)`` (main.py:57-340) as a callable.  main.py trains at import time (main.py:342-364),
     so only its import statements, the ``device`` assignment and the ``train`` FunctionDef are executed, verbatim from the AST
-    of /root/reference/main.py.  Bound while its imports run (none of them installed here or usable offline):
+    of the reference's main.py.  Bound while its imports run (none of them installed here or usable offline):
       wandb -> :class:`WandbStub` (returned);  tap.Tap -> object;  modules.data.get_data -> ``get_data`` (synthetic data);
       modules.gcn.GCN -> ``gcn_factory`` (the oracle's GCN restatement: PyG is absent);  modules.utils, eval -> the
       reference's own modules;  sp.csr_matrix -> :class:`_SparseShim` (index-type shim only).

@@ -20,19 +20,19 @@ reference's own call sites (gcn.py:18,21,32,36) plus a dense
 Pinning status (SURVEY.md section 8c):
   * integer path (get_neighborhoods, slice_adjacency, TensorMap, mask dedup) and
     sample_neighborhoods_from_probs: PINNED against the reference's own
-    ``modules/utils.py`` imported from /root/reference (oracle/ref_import.py,
+    ``modules/utils.py`` imported live (oracle/ref_import.py,
     tests/test_oracle.py::test_oracle_matches_live_reference) and against the committed fixtures in
     tests/golden/ produced by tests/golden/make_golden.py from that import, and
     against the only known-answer vector the reference holds (TensorMap
     docstring, utils.py:104-108).
   * evaluation (``reference_evaluate``, eval.py:11-165, full-batch and mini-batch): PINNED against the reference's
-    own ``evaluate`` imported live from /root/reference/eval.py (oracle/ref_import.py::load_reference_eval;
+    own ``evaluate`` imported live from the reference's eval.py (oracle/ref_import.py::load_reference_eval;
     tests/test_oracle.py::test_oracle_evaluate_matches_live_reference_eval: scores equal, logits of every ``gcn_c`` call
     equal bit for bit) and against the committed tests/golden/eval_*.npz produced by that function (evaluation blocks
     bit-exact, logits, scores).  The models inside are this file's GCN restatement, so this pins the evaluation LOOP
     (deterministic top-k, evaluation-direction slice, relabelling, batching, scores), not GCNConv.
   * the batch loop as a whole (``reference_step``, main.py:161-291: hop loop, both losses, autograd backward, both Adam
-    optimisers): PINNED against the reference's own ``train(args)`` executed live from /root/reference/main.py
+    optimisers): PINNED against the reference's own ``train(args)`` executed live from the reference's main.py
     (oracle/ref_import.py::load_reference_train runs the file's import statements and its ``train`` FunctionDef verbatim;
     wandb / tap / the dataset loader are stand-ins; the GCN class is the reference's own modules/gcn.py over this file's
     one-layer GCNConv restatement) --

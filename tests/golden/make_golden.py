@@ -1,11 +1,11 @@
-"""Generates the golden fixtures in this directory FROM THE REFERENCE ITSELF: imports
-/root/reference/modules/utils.py (through the scipy tensor-index shim of oracle/ref_import.py) and runs
+"""Generates the golden fixtures in this directory FROM THE REFERENCE ITSELF: imports the reference's
+modules/utils.py (through the scipy tensor-index shim of oracle/ref_import.py) and runs
 its own get_neighborhoods / slice_adjacency / TensorMap / sample_neighborhoods_from_probs and the mask
-dedup statements of main.py:183-195 on seeded synthetic graphs; and /root/reference/eval.py's own ``evaluate``
-(full-batch and mini-batch) for the eval_*.npz fixtures and /root/reference/main.py's own ``train`` for train_*.npz.  Run in the build container only
-(the GPU box has no /root/reference); the .npz outputs are committed.
+dedup statements of main.py:183-195 on seeded synthetic graphs; and the reference's eval.py ``evaluate``
+(full-batch and mini-batch) for the eval_*.npz fixtures and its main.py ``train`` for train_*.npz.  Needs a checkout of
+the reference GRAPES project, which this repository does not contain; the .npz outputs are committed.
 
-    python tests/golden/make_golden.py
+    GRAPES_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 """
 import os
 import sys
@@ -166,6 +166,8 @@ def main_train():
 
 
 if __name__ == "__main__":
+    if not ref_import.reference_available():
+        sys.exit("make_golden.py: set GRAPES_REFERENCE_ROOT to a checkout of the reference GRAPES project")
     main()
     main_eval()
     main_train()

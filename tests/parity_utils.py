@@ -1,5 +1,5 @@
 """Shared checker of the whole-step parity tests: the device engine against the CPU oracle's restatement of
-/root/reference/main.py:161-291 on the same graph, weights and injected Gumbel noise.
+the reference's main.py:161-291 on the same graph, weights and injected Gumbel noise.
 
 Bars (BASELINE.json north_star): frontier sets / dedup / relabel / blocks and sampled sets BIT-EXACT; logits,
 aggregated features, losses and gradients within 1e-5 relative (fp32), measured against the oracle run in float64

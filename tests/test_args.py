@@ -1,13 +1,16 @@
 """CPU tests: the Tap-compatible ``Arguments`` parser accepts every config file of the reference
-(read from /root/reference when present) and the spellings those files use."""
+(read from the checkout GRAPES_REFERENCE_ROOT names, when it is set) and the spellings those files use."""
 import glob
 import os
 
 import pytest
 
 from grapes_b200.args import Arguments, parse_cli
+from oracle.ref_import import REFERENCE_ROOT, reference_available
 
-REF_CONFIGS = sorted(glob.glob("/root/reference/configs/*/*.txt"))
+REF_CONFIGS = sorted(glob.glob(os.path.join(REFERENCE_ROOT, "configs", "*", "*.txt"))) if REFERENCE_ROOT else []
+needs_reference = pytest.mark.skipif(not reference_available(),
+                                     reason="needs GRAPES_REFERENCE_ROOT: a checkout of the reference GRAPES project")
 
 
 def test_defaults_match_reference_main_py():
@@ -36,7 +39,7 @@ def test_unknown_flag_and_bad_bool_are_errors():
         Arguments.parse_args(["--use_indicators", "maybe"])
 
 
-@pytest.mark.skipif(not REF_CONFIGS, reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_every_reference_config_file_parses():
     bad = []
     for path in REF_CONFIGS:
@@ -44,26 +47,26 @@ def test_every_reference_config_file_parses():
             a = parse_cli(["--config_file", path])
             assert a.hidden_dim > 0 and a.num_samples > 0
         except SystemExit:
-            bad.append(os.path.relpath(path, "/root/reference"))
+            bad.append(os.path.relpath(path, REFERENCE_ROOT))
     # configs/rl/flickr.txt:15 is malformed in the reference itself ("--runs=1 0", SURVEY.md section 5)
     assert bad == ["configs/rl/flickr.txt"], bad
     assert len(REF_CONFIGS) == 32
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/main.py"), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_fields_and_defaults_match_the_live_reference_class():
     """main.py:23-54 read from the reference's own source (AST of ``class Arguments(Tap)``): same field names in the same
     order, same defaults."""
     import ast
     import dataclasses
-    tree = ast.parse(open("/root/reference/main.py").read())
+    tree = ast.parse(open(os.path.join(REFERENCE_ROOT, "main.py")).read())
     cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "Arguments")
     ref = [(n.target.id, ast.literal_eval(n.value)) for n in cls.body if isinstance(n, ast.AnnAssign)]
     mine = [(f.name, f.default) for f in dataclasses.fields(Arguments)]
     assert mine == ref and len(ref) == 27
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/main.py"), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_arguments_object_drives_the_live_reference_train():
     """The drop-in ``Arguments`` is accepted by the reference's OWN ``train(args)`` (main.py:57-340 executed live, see
     oracle/ref_import.py::load_reference_train): every attribute the loop reads, and ``as_dict()`` (main.py:61)."""

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
              "vs_baseline", "dtype", "data", "config", "e2e", "gpu_launches", "cpu_baseline")
@@ -25,6 +27,61 @@ def test_reference_arm_prints_one_json_line_on_the_host():
     assert d["e2e"] == {"value": d["value"], "unit": "nodes/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["gpu_launches"] == 0 and d["higher_is_better"] is True and d["vs_baseline"] is None
+
+
+def test_bench_rejects_zero_steps_and_dumps_of_the_reference_arm(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny"] + extra,
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert res.returncode == 2 and not res.stdout.strip(), res.stderr[-2000:]
+    assert not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_last_timed_step_repeat_across_runs(cuda_device, tmp_path):
+    """`--dump-outputs DIR`: the last timed step's losses, sampler statistics, sampled nodes, logits and updated parameters
+    as float32 / float64 .npy files.  The optimisers counted prime + warm-up + `--steps` steps, the dumped batch holds the
+    targets of the batch the last timed step ran (not those of the prefetched next one), and two runs with the same
+    arguments dump the same numbers."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from grapes_b200.dist import shard_batches
+    prime, warmup, steps = 2, 3, 4
+    dumps = []
+    for run in ("a", "b"):
+        out = tmp_path / run
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--workload", "small",
+                              "--steps", str(steps), "--warmup", str(warmup), "--prime", str(prime), "--no-cpu-baseline",
+                              "--no-spmm", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert res.returncode == 0, res.stderr[-4000:]
+        d = json.loads(res.stdout.strip().splitlines()[-1])
+        assert d["steps"] == steps and d["warmup"] == warmup and d["prime_steps"] == prime
+        arrays = {p.stem: np.load(p) for p in sorted(out.glob("*.npy"))}
+        assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+        assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+        dumps.append(arrays)
+    a, b = dumps
+    assert a.keys() == b.keys()
+    for key in ("loss_c", "loss_gfn", "log_z", "tot_log_prob", "sampler_stats", "all_nodes", "logits_c", "adam_steps",
+                "gcn_c.gcn_layers.0.lin.weight", "gcn_gf.gcn_layers.1.bias", "gcn_z.gcn_layers.1.lin.weight"):
+        assert key in a, key
+    assert a["adam_steps"].tolist() == [prime + warmup + steps] * 2
+    # the batches in the order bench.py runs them (same seeded workload, warm-up and timed steps only)
+    cfg, _, _, _, _, train_idx = bench.build_workload("small", 0, cuda_device)
+    B = cfg["batch_size"]
+    mine = shard_batches(train_idx.numel() // B, 0, 1)
+    batch = lambda j: set(train_idx[mine[j % len(mine)] * B:(mine[j % len(mine)] + 1) * B].tolist())
+    last = warmup + steps - 1
+    dumped = set(a["all_nodes"].astype(np.int64).tolist())
+    assert batch(last) <= dumped and not batch(last + 1) <= dumped and not batch(last - 1) <= dumped
+    assert a["sampler_stats"].shape == (cfg["sampling_hops"], 4) and a["logits_c"].shape == (len(dumped), cfg["C"])
+    for h in range(cfg["sampling_hops"]):
+        s = a[f"sampled_hop{h}"]
+        assert 0 < s.size <= cfg["num_samples"] and np.array_equal(s, np.round(s)) and set(s.astype(np.int64).tolist()) <= dumped
+    assert np.isfinite(a["loss_c"]).all() and np.isfinite(a["logits_c"]).all()
+    for key in a:
+        assert np.array_equal(a[key], b[key]), key
 
 
 def test_committed_bench_line_carries_the_contract():

@@ -1,6 +1,6 @@
 """The CUDA path against the committed golden fixtures (tests/golden/*.npz), i.e. against outputs of the reference's OWN code
-(tests/golden/make_golden.py ran /root/reference/modules/utils.py, the mask statements of main.py:183-195 and eval.py's
-``evaluate`` in the build container; the GPU box has no /root/reference).  The other GPU tests compare with the oracle, which
+(tests/golden/make_golden.py ran the reference's modules/utils.py, the mask statements of main.py:183-195 and eval.py's
+``evaluate`` from a checkout of the reference project, which this repository does not contain).  The other GPU tests compare with the oracle, which
 tests/test_oracle.py holds to the same fixtures; here the fixtures are the checker directly.
 
 hoploop_*.npz  one batch of the hop loop through the drop-in callables (grapes_b200.utils): CSR, get_neighborhoods, mask dedup,

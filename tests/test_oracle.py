@@ -1,5 +1,5 @@
 """CPU tests (no GPU): the oracle against the golden vectors generated from the reference's own code
-(tests/golden/make_golden.py), against the reference imported live when /root/reference is present,
+(tests/golden/make_golden.py), against the reference imported live when GRAPES_REFERENCE_ROOT names a checkout of it,
 and against closed forms for the un-vendored PyG GCNConv arithmetic."""
 import glob
 import os
@@ -13,6 +13,8 @@ from oracle import ref_import
 from oracle import reference_port as rp
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+needs_reference = pytest.mark.skipif(not ref_import.reference_available(),
+                                     reason="needs GRAPES_REFERENCE_ROOT: a checkout of the reference GRAPES project")
 
 
 def _t(a):
@@ -83,7 +85,7 @@ def test_oracle_matches_reference_golden(path):
     assert torch.equal(node_map.map(target), _t(z["local_target_ids"]))
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 @pytest.mark.parametrize("name,seed", [("tiny", 3), ("cora", 1), ("small", 0)])
 def test_oracle_matches_live_reference(name, seed):
     ru = ref_import.load_reference_utils()
@@ -268,7 +270,7 @@ def test_oracle_evaluate_matches_reference_golden(path):
     assert mini["f1"] == pytest.approx(float(z["mini_f1"]), abs=1e-12)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 @pytest.mark.parametrize("name,seed,B,k,hops", [("tiny", 3, 32, 8, 2), ("small", 0, 200, 32, 3), ("cora", 1, 512, 16, 2)])
 def test_oracle_evaluate_matches_live_reference_eval(single_thread, name, seed, B, k, hops):
     """The reference's own ``evaluate`` imported live (oracle/ref_import.py::load_reference_eval), full-batch and mini-batch,
@@ -324,11 +326,11 @@ def _flat_weights(nets):
             for n, p in net.named_parameters()}
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 @pytest.mark.parametrize("case", sorted(TRAIN_CASES))
 def test_oracle_step_matches_live_reference_train(single_thread, case):
     """The reference's OWN ``train(args)`` (main.py:57-340: batch loop, hop loop, both losses, autograd backward, both Adam
-    optimisers, final evaluation) executed live from /root/reference/main.py (oracle/ref_import.py::load_reference_train)
+    optimisers, final evaluation) executed live from the reference's main.py (oracle/ref_import.py::load_reference_train)
     against the oracle's ``reference_step`` on the same data, initial weights and RNG stream: every batch's loss_c / loss_gfn /
     log_z / sum of log-probs and sampler statistics equal BIT FOR BIT, the weights of all three networks after the epoch equal
     to 1e-7 (autograd accumulates two of them in another order), the test score equal.  Pins SURVEY.md section 8 rows a2-a13
@@ -382,7 +384,7 @@ def test_oracle_step_matches_reference_train_golden(single_thread, path):
     assert o["f1"] == pytest.approx(float(z["test_f1"]), abs=1e-12)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_oracle_multi_epoch_and_minibatch_eval_match_live_reference_train(single_thread):
     """Four epochs of the reference's own ``train`` with its mid-training validation (main.py:313-326: epoch 4 with
     eval_frequency 5) and the final test evaluation both in MINI-BATCH mode (eval_full_batch=False): the TensorMap and the
@@ -402,7 +404,7 @@ def test_oracle_multi_epoch_and_minibatch_eval_match_live_reference_train(single
     assert o["f1"] == pytest.approx(test_f1, abs=1e-12)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_oracle_embed_nodes_matches_live_reference_train(single_thread):
     """--embed_nodes (main.py:89-100,116; SURVEY.md section 8 row f4): the reference draws the table with nn.init.normal_
     from the global RNG, makes it an nn.Parameter inside optimizer_c and trains it.  Live ``train`` against the oracle with
@@ -438,7 +440,7 @@ def test_oracle_embed_nodes_matches_live_reference_train(single_thread):
         assert torch.allclose(got_w[key], ref_w[key], rtol=0, atol=1e-7 * float(ref_w[key].abs().max())), key
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_oracle_gcn_wiring_matches_live_reference_gcn_class(single_thread):
     """modules/gcn.py:9-42 imported live (oracle/ref_import.py::load_reference_gcn; GCNConv bound to the oracle's layer):
     the reference's own ``GCN`` -- layer list, ``edge_index[-i]`` for hidden layer i and ``edge_index[0]`` for the output
@@ -466,7 +468,7 @@ def test_oracle_gcn_wiring_matches_live_reference_gcn_class(single_thread):
                 assert torch.equal(a, b) and isinstance(mem, float)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_oracle_edge_cases_match_live_reference_utils():
     """Edge cases the domain has (SURVEY.md section 4): empty row lists, rows without neighbours, a self-loop, an empty
     column set, duplicated ids in the row list, one candidate, k = 1, k >= n -- the reference's own functions against the
@@ -502,7 +504,7 @@ def test_oracle_edge_cases_match_live_reference_utils():
         assert torch.equal(tm_a.values, tm_b.values)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present (GPU box)")
+@needs_reference
 def test_host_side_dropins_inside_the_live_reference_loop(single_thread):
     """INTEGRATION.md section 1 (import-level drop-in), the part that needs no GPU: this repo's ``TensorMap`` and
     ``get_logger`` (grapes_b200/utils.py, pure torch / logging) bound in place of the reference's inside the reference's OWN
