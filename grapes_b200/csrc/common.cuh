@@ -111,6 +111,14 @@ static inline int grapes_max_i(int a, int b) { return a > b ? a : b; }
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 
+// device state words of one data-parallel exchange endpoint (peer_comm.cu; read by grapes_embed_merge_adam)
+#define PS_SEQ 0        // steps completed
+#define PS_TICKET_A 1   // push ticket
+#define PS_TICKET_C 2   // reduce ticket
+#define PS_FAILED 3     // sticky failure
+#define PS_GO 4         // go word of the current step: seq (arrived) or seq | GO_FAIL
+#define GO_FAIL 0x80000000u
+
 // fp32 -> tf32 (10-bit mantissa), round to nearest, ties away from zero: the value cvt.rna.tf32.f32 returns for every
 // finite input, in TWO integer instructions (add half an ulp to the magnitude bits, clear the 13 low bits).  ptxas expands
 // the cvt into ~6 instructions with NaN / Inf handling; the 3xTF32 operand split calls this twice per element and was

@@ -292,17 +292,20 @@ __global__ void __launch_bounds__(256) k_gfn_finalize_scale(float* scal, float l
 // every row's moments decay and every row whose moments are non-zero keeps moving, not only the rows of this batch.  The
 // gradient is sparse -- d loss_c / d x is non-zero only on the batch's all_nodes rows -- so it is read through the
 // all_nodes bitmap (local row = rank of the bit) instead of being scattered into a dense [N, F] buffer first.  Rows that
-// were never touched (m = v = 0, no gradient) are left alone: their update is exactly 0.  `step` = optimizer_c's count
-// BEFORE this update (grapes_adam_step2, launched afterwards, increments it).
+// were never touched (m = v = 0, no gradient) are left alone: their update is exactly 0.  The bias correction uses
+// t = *step + t_add: t_add = 1 when `step` is optimizer_c's count BEFORE this update (grapes_adam_embed: the parameter
+// Adam launched afterwards increments it), 0 when that launch already ran (grapes_embed_merge_adam).  go != NULL: the
+// go word of a data-parallel exchange; a failed exchange (GO_FAIL) makes the launch a no-op.
 __global__ void __launch_bounds__(256) k_adam_embed(float* __restrict__ x, float* __restrict__ m, float* __restrict__ v,
                                                     int64_t N, int F4, const uint32_t* __restrict__ bm,
                                                     const int* __restrict__ pref, const float* __restrict__ grows,
                                                     int ldg4, float lr, float beta1, float beta2, float eps,
-                                                    const float* __restrict__ step) {
+                                                    const float* __restrict__ step, const unsigned int* go, float t_add) {
     pdl_begin();
+    if (go && (*(volatile const unsigned int*)go & GO_FAIL)) return;
     __shared__ float s_step_size, s_bc2_sqrt;
     if (threadIdx.x == 0) {
-        const double t = (double)(*step) + 1.0;
+        const double t = (double)(*step) + (double)t_add;
         const double bc1 = 1.0 - pow((double)beta1, t), bc2 = 1.0 - pow((double)beta2, t);
         s_step_size = (float)((double)lr / bc1);
         s_bc2_sqrt = (float)sqrt(bc2);
@@ -331,6 +334,81 @@ __global__ void __launch_bounds__(256) k_adam_embed(float* __restrict__ x, float
         GRAPES_ADAM1(x) GRAPES_ADAM1(y) GRAPES_ADAM1(z) GRAPES_ADAM1(w)
 #undef GRAPES_ADAM1
         m4[i] = mi; v4[i] = vi; x4[i] = p;
+    }
+}
+
+// ---- data-parallel learned table: merge of the ranks' row-sparse gradients (grapes_embed_merge_adam) ----
+// world slots of grapes_embed_slot_floats floats, each [A, 3 pad | ids, cap rounded up to 4 | rows, cap x F]
+// (peer_comm.cu).  state != NULL: `slots` is this rank's second symmetric buffer (both parities) and the go word of the
+// step's exchange picks the parity, or makes every launch a no-op when the peers did not arrive.
+#define EMBED_MAX_WORLD 8
+
+__device__ __forceinline__ const float* embed_slots(const float* slots, long long slot, int world,
+                                                    const unsigned int* state, bool* skip) {
+    *skip = false;
+    if (!state) return slots;
+    const unsigned int go = *(volatile const unsigned int*)(state + PS_GO);
+    *skip = (go & GO_FAIL) != 0u;
+    return slots + (size_t)(go & 1u) * world * slot;
+}
+
+__global__ void __launch_bounds__(256) k_embed_union(const float* slots, long long slot, int world, int cap,
+                                                     const unsigned int* state, uint32_t* bm) {
+    pdl_begin();
+    bool skip;
+    const float* base = embed_slots(slots, slot, world, state, &skip);
+    if (skip) return;
+    const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
+    for (int r = 0; r < world; ++r) {
+        const int* s = reinterpret_cast<const int*>(base + (size_t)r * slot);
+        const int A = min(__ldcg(s), cap);
+        for (int i = gtid; i < A; i += gsz) bitmap_set(bm, __ldcg(s + 4 + i));
+    }
+}
+
+// one warp per union row v: lane r < world finds v in slot r's ascending id list (binary search), then the lanes walk
+// the row's float4 columns and add the ranks' rows in rank order (identical bits on every rank), times 1 / world
+__global__ void __launch_bounds__(256) k_embed_mean_rows(const float* slots, long long slot, int world, int cap, int F4,
+                                                         const unsigned int* state, const int* __restrict__ ids,
+                                                         const int* __restrict__ U_dev, int cap_U, float* __restrict__ mean,
+                                                         float inv_w) {
+    pdl_begin();
+    bool skip;
+    const float* base = embed_slots(slots, slot, world, state, &skip);
+    if (skip) return;
+    const int lane = threadIdx.x & 31;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
+    const int U = min(*U_dev, cap_U);
+    const int cap4 = (cap + 3) & ~3;
+    for (int row = warp; row < U; row += nwarps) {
+        const int v = ids[row];
+        int pos = -1;
+        if (lane < world) {
+            const int* s = reinterpret_cast<const int*>(base + (size_t)lane * slot);
+            const int A = min(__ldcg(s), cap);
+            int lo = 0, hi = A;
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (__ldcg(s + 4 + mid) < v) lo = mid + 1; else hi = mid;
+            }
+            if (lo < A && __ldcg(s + 4 + lo) == v) pos = lo;
+        }
+        int p[EMBED_MAX_WORLD];
+#pragma unroll
+        for (int r = 0; r < EMBED_MAX_WORLD; ++r) p[r] = __shfl_sync(0xffffffffu, pos, r);
+        for (int c = lane; c < F4; c += 32) {
+            float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+            for (int r = 0; r < EMBED_MAX_WORLD; ++r) {
+                if (r < world && p[r] >= 0) {
+                    const float4* rows = reinterpret_cast<const float4*>(base + (size_t)r * slot + 4 + cap4);
+                    const float4 g = __ldcg(rows + (size_t)p[r] * F4 + c);
+                    acc.x += g.x; acc.y += g.y; acc.z += g.z; acc.w += g.w;
+                }
+            }
+            acc.x *= inv_w; acc.y *= inv_w; acc.z *= inv_w; acc.w *= inv_w;
+            reinterpret_cast<float4*>(mean)[(size_t)row * F4 + c] = acc;
+        }
     }
 }
 
@@ -517,7 +595,42 @@ int grapes_adam_embed(grapes_ctx* ctx, float* table, float* exp_avg, float* exp_
     if (blocks > cap) blocks = cap;
     pdl((k_adam_embed), (int)blocks, 256, 0, (cudaStream_t)stream)(table, exp_avg, exp_avg_sq, num_nodes, F / 4, bm_rows,
                                                                   pref_rows, grad_rows, ldg / 4, lr, beta1, beta2, eps,
-                                                                  step_dev);
+                                                                  step_dev, nullptr, 1.0f);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_embed_merge_adam(grapes_ctx* ctx, const float* slots, int world, int cap_rows, int F,
+                            const unsigned int* state, uint32_t* bm_union, int* pref_union, int* union_ids, int cap_union,
+                            int* union_count, float* mean_rows, float* table, float* exp_avg, float* exp_avg_sq,
+                            int64_t num_nodes, float lr, float beta1, float beta2, float eps, const float* step_dev,
+                            int* overflow, void* stream) {
+    GRAPES_REQUIRE(ctx && slots && bm_union && pref_union && union_ids && union_count && mean_rows && table && exp_avg &&
+                       exp_avg_sq && step_dev && overflow, "null argument");
+    GRAPES_REQUIRE(world >= 1 && world <= EMBED_MAX_WORLD, "1 <= world <= 8");
+    GRAPES_REQUIRE(F > 0 && F % 4 == 0 && cap_rows > 0 && cap_union > 0, "table width must be a multiple of 4");
+    GRAPES_REQUIRE(num_nodes == ctx->num_nodes, "table rows != graph nodes");
+    cudaStream_t s = (cudaStream_t)stream;
+    const long long slot = grapes_embed_slot_floats(cap_rows, F);
+    pdl((k_embed_union), grid_for(ctx, (long long)cap_rows, 256), 256, 0, s)(slots, slot, world, cap_rows, state, bm_union);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    // popcount-prefix rank of the union bitmap: ascending union ids and the local row of every id
+    const int rc = grapes_rank_nodes(ctx, bm_union, nullptr, pref_union, nullptr, union_ids, nullptr, nullptr, nullptr,
+                                     nullptr, nullptr, 0, 0, cap_union, union_count, nullptr, overflow, stream);
+    if (rc != GRAPES_OK) return rc;
+    pdl((k_embed_mean_rows), grid_for(ctx, (long long)cap_union * 32, 256), 256, 0, s)(
+        slots, slot, world, cap_rows, F / 4, state, union_ids, union_count, cap_union, mean_rows, 1.0f / (float)world);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    const long long total = (long long)num_nodes * (F / 4);
+    long long blocks = (total + 255) / 256;
+    const long long bcap = (long long)ctx->sm_count * 8;
+    if (blocks > bcap) blocks = bcap;
+    pdl((k_adam_embed), (int)blocks, 256, 0, s)(table, exp_avg, exp_avg_sq, num_nodes, F / 4, bm_union, pref_union,
+                                               mean_rows, F / 4, lr, beta1, beta2, eps, step_dev,
+                                               state ? state + PS_GO : nullptr, 0.0f);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;

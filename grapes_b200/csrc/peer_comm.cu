@@ -16,6 +16,16 @@
 // A peer that never arrives (timeout) raises GRAPES_OVF_PEER_TIMEOUT, and the step is a NO-OP on this rank: parameters,
 // moments, step counts and the sequence number stay untouched, and the failure is sticky (every later launch is a
 // no-op too) until the host sees the flag.  No per-step host argument: the launch is captured into the step's CUDA graph.
+//
+// Learned node features (grapes_step_tail_embed): the table gradient is non-zero only on the step's all_nodes rows, so
+// each rank also pushes (A, all_nodes[:A], dXc[:A, :F]) into slot[rank] of a SECOND symmetric buffer
+// [parity 0: world slots | parity 1: world slots] of every rank (grapes_embed_slot_floats per slot).  Those stores sit
+// before the block's __threadfence_system() and ticket, so the one per-step flag of the first buffer covers both
+// payloads: no second flag, wait or timeout.  grapes_embed_merge_adam then reads this rank's own second buffer in a
+// LATER launch of the same stream (union of the id lists, rank-order mean rows, dense table Adam).  Two parities still
+// suffice, but only because that merge launch sits between this rank's tails of steps s and s + 1 on one stream: a rank
+// can push step s + 2 into slot parity s & 1 of peer p only after its tail of s + 1 saw p's flag of s + 1, which p's
+// tail of s + 1 releases after (stream order) p's merge of step s has finished reading parity s & 1.
 #define GRAPES_PDL_GROUP 8
 #include "common.cuh"
 
@@ -41,14 +51,6 @@ __device__ __forceinline__ unsigned int ld_acquire_gpu_u32(const unsigned int* p
     return v;
 }
 
-// device state words of one exchange endpoint
-#define PS_SEQ 0        // steps completed
-#define PS_TICKET_A 1   // push ticket
-#define PS_TICKET_C 2   // reduce ticket
-#define PS_FAILED 3     // sticky failure
-#define PS_GO 4         // go word of the current step: seq (arrived) or seq | GO_FAIL
-#define GO_FAIL 0x80000000u
-
 struct TailArgs {
     // exchange
     PeerTable pt; int rank, world, n, n_pad;
@@ -61,12 +63,23 @@ struct TailArgs {
     float beta1, beta2, eps; float* steps;
 };
 
-template <bool PEER>
-__global__ void __launch_bounds__(256) k_step_tail(const TailArgs a) {
+// table payload of the learned node features (k_step_tail_embed)
+struct EmbedPush {
+    float* buf[PEER_MAX];              // base of every rank's second symmetric buffer
+    const int* count;                  // A: rows of this step (device)
+    const int* ids;                    // all_nodes[:A], ascending
+    const float* rows; int ldg;        // dXc[:A, :F], pitch ldg floats
+    int F, cap;                        // row width (multiple of 4), rows per slot (cap_A)
+    long long slot;                    // floats per slot (grapes_embed_slot_floats)
+};
+
+template <bool PEER, bool EMBED>
+__device__ __forceinline__ void step_tail(const TailArgs& a, const EmbedPush* e) {
     pdl_begin();
     __shared__ float s_step_size[2], s_bc2_sqrt[2];
     __shared__ int s_last, s_go;
     const int tid = threadIdx.x;
+    __builtin_assume(tid < 256);                           // __launch_bounds__(256) of both kernels below
     const int gtid = blockIdx.x * blockDim.x + tid, gsz = gridDim.x * blockDim.x;
     // ---- loss_gfn and the scale of the accumulated gradient directions (every thread, from read-only inputs) ----
     float g_gf = 0.f, g_z = 0.f;
@@ -113,6 +126,31 @@ __global__ void __launch_bounds__(256) k_step_tail(const TailArgs a) {
 #pragma unroll
                 for (int r = 0; r < PEER_MAX; ++r)
                     if (r < a.world) a.pt.buf[r][my_slot + i] = gi;
+            }
+            if (EMBED) {
+                // slot: [A, 3 pad | ids, cap rounded up to 4 | rows, cap x F]
+                const int A = min(*e->count, e->cap), F4 = e->F >> 2, cap4 = (e->cap + 3) & ~3;
+                const size_t es = (size_t)(seq & 1u) * a.world * e->slot + (size_t)a.rank * e->slot;
+                for (int i = gtid; i < A; i += gsz) {
+                    const int v = e->ids[i];
+#pragma unroll
+                    for (int r = 0; r < PEER_MAX; ++r)
+                        if (r < a.world) reinterpret_cast<int*>(e->buf[r] + es)[4 + i] = v;
+                }
+                if (gtid == 0) {
+#pragma unroll
+                    for (int r = 0; r < PEER_MAX; ++r)
+                        if (r < a.world) reinterpret_cast<int*>(e->buf[r] + es)[0] = A;
+                }
+                const float4* g4 = reinterpret_cast<const float4*>(e->rows);
+                const int ldg4 = e->ldg >> 2;
+                for (int i = gtid; i < A * F4; i += gsz) {
+                    const int row = i / F4, c = i - row * F4;
+                    const float4 gv = g4[(size_t)row * ldg4 + c];
+#pragma unroll
+                    for (int r = 0; r < PEER_MAX; ++r)
+                        if (r < a.world) reinterpret_cast<float4*>(e->buf[r] + es + 4 + cap4)[i] = gv;
+                }
             }
         }
         __threadfence_system();
@@ -205,7 +243,17 @@ __global__ void __launch_bounds__(256) k_step_tail(const TailArgs a) {
     }
 }
 
-static int launch_tail(grapes_ctx* ctx, TailArgs& a, void* const* peer_bufs, void* stream) {
+template <bool PEER>
+__global__ void __launch_bounds__(256) k_step_tail(const TailArgs a) {
+    step_tail<PEER, false>(a, nullptr);
+}
+
+__global__ void __launch_bounds__(256) k_step_tail_embed(const TailArgs a, const EmbedPush e) {
+    step_tail<true, true>(a, &e);
+}
+
+static int launch_tail(grapes_ctx* ctx, TailArgs& a, void* const* peer_bufs, void* stream,
+                       const EmbedPush* embed = nullptr) {
     for (int r = 0; r < PEER_MAX; ++r)
         a.pt.buf[r] = (peer_bufs && r < a.world) ? reinterpret_cast<float*>(peer_bufs[r]) : nullptr;
     a.n_pad = (a.n + 63) / 64 * 64;
@@ -216,7 +264,8 @@ static int launch_tail(grapes_ctx* ctx, TailArgs& a, void* const* peer_bufs, voi
     // every block spins on the go word while the push of the others is in flight: the grid must be co-resident
     if (blocks > ctx->sm_count * 2) blocks = ctx->sm_count * 2;
     cudaStream_t s = (cudaStream_t)stream;
-    if (peer_bufs && a.world > 1) pdl((k_step_tail<true>), blocks, 256, 0, s)(a);
+    if (embed) pdl((k_step_tail_embed), blocks, 256, 0, s)(a, *embed);
+    else if (peer_bufs && a.world > 1) pdl((k_step_tail<true>), blocks, 256, 0, s)(a);
     else pdl((k_step_tail<false>), blocks, 256, 0, s)(a);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
@@ -276,6 +325,48 @@ int grapes_step_tail(grapes_ctx* ctx, float* scal, int do_scale, float loss_coef
     a.off0 = off0; a.n0 = n0; a.lr0 = lr0; a.off1 = off1; a.n1 = n1; a.lr1 = lr1;
     a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.steps = steps_dev;
     return launch_tail(ctx, a, peer_bufs, stream);
+}
+
+int64_t grapes_embed_slot_floats(int cap_rows, int F) {
+    return 4 + ((int64_t)cap_rows + 3) / 4 * 4 + (int64_t)cap_rows * F;
+}
+
+int64_t grapes_embed_peer_buffer_floats(int cap_rows, int F, int world) {
+    return 2 * (int64_t)(world < 1 ? 1 : world) * grapes_embed_slot_floats(cap_rows, F);
+}
+
+// grapes_step_tail with peers, plus the learned table's payload of this step (A = *count_dev rows: ids[:A] ascending,
+// rows[:A, :F] at pitch ldg) pushed into slot[rank] of every rank's second symmetric buffer (embed_bufs, each of
+// grapes_embed_peer_buffer_floats(cap_rows, F, world) floats) under the same per-step flag.
+int grapes_step_tail_embed(grapes_ctx* ctx, float* scal, int do_scale, float loss_coef, float log_z_init, int reinforce,
+                           int have_log_z, const float* dir, int gf_off, int n_gf, int z_off, int n_z,
+                           void* const* peer_bufs, void* const* embed_bufs, int rank, int world, int n, float* params,
+                           float* grads, float* exp_avg, float* exp_avg_sq, int off0, int n0, float lr0, int off1, int n1,
+                           float lr1, float beta1, float beta2, float eps, float* steps_dev, unsigned int* state,
+                           int* err_flag, const int* count_dev, const int* ids, const float* rows, int ldg, int F,
+                           int cap_rows, void* stream) {
+    GRAPES_REQUIRE(ctx && params && grads && exp_avg && exp_avg_sq && steps_dev && state && err_flag && peer_bufs &&
+                       embed_bufs && count_dev && ids && rows, "null argument");
+    GRAPES_REQUIRE(!do_scale || (scal && dir), "a gradient scale needs the scalar block and the direction buffer");
+    GRAPES_REQUIRE(world >= 1 && world <= PEER_MAX && rank >= 0 && rank < world, "1 <= world <= 8");
+    GRAPES_REQUIRE(n > 0 && n0 >= 0 && n1 >= 0, "empty gradient");
+    GRAPES_REQUIRE(F > 0 && F % 4 == 0 && ldg % 4 == 0 && ldg >= F && cap_rows > 0,
+                   "table width and row pitch must be multiples of 4");
+    GRAPES_REQUIRE((reinterpret_cast<uintptr_t>(rows) & 15) == 0, "rows must be 16-byte aligned");
+    TailArgs a;
+    memset(&a, 0, sizeof(a));
+    a.rank = rank; a.world = world; a.n = n; a.state = state; a.err_flag = err_flag;
+    a.scal = scal; a.do_scale = do_scale; a.loss_coef = loss_coef; a.log_z_init = log_z_init; a.reinforce = reinforce; a.have_log_z = have_log_z;
+    a.dir = dir; a.gf_off = gf_off; a.n_gf = n_gf; a.z_off = z_off; a.n_z = n_z;
+    a.p = params; a.g = grads; a.m = exp_avg; a.v = exp_avg_sq;
+    a.off0 = off0; a.n0 = n0; a.lr0 = lr0; a.off1 = off1; a.n1 = n1; a.lr1 = lr1;
+    a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.steps = steps_dev;
+    EmbedPush e;
+    memset(&e, 0, sizeof(e));
+    for (int r = 0; r < PEER_MAX; ++r) e.buf[r] = r < world ? reinterpret_cast<float*>(embed_bufs[r]) : nullptr;
+    e.count = count_dev; e.ids = ids; e.rows = rows; e.ldg = ldg; e.F = F; e.cap = cap_rows;
+    e.slot = grapes_embed_slot_floats(cap_rows, F);
+    return launch_tail(ctx, a, peer_bufs, stream, &e);
 }
 
 }  // extern "C"

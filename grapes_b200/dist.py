@@ -49,9 +49,10 @@ class PeerGradExchange:
     """Symmetric (peer-mapped) gradient buffers for ``grapes_step_tail`` / ``grapes_allreduce_adam_peer``: every rank
     allocates the same buffer with ``torch.distributed._symmetric_memory`` and receives the peers' device pointers, so the
     mean all-reduce and both Adam updates run as ONE kernel over NVLink inside the step's CUDA graph (no host-side
-    collective call)."""
+    collective call).  ``embed_floats`` > 0 adds a second symmetric buffer of that many floats (``ebuf``, peers'
+    pointers in ``embed_ptrs``): the payload of a learned node-feature table (``grapes_step_tail_embed``)."""
 
-    def __init__(self, n_floats: int, device: torch.device, group=None):
+    def __init__(self, n_floats: int, device: torch.device, group=None, embed_floats: int = 0):
         import ctypes
         import torch.distributed._symmetric_memory as symm_mem
         from ._lib import lib
@@ -66,6 +67,14 @@ class PeerGradExchange:
         ptrs = [int(p) for p in self.hdl.buffer_ptrs]
         assert ptrs[self.rank] == self.buf.data_ptr()
         self.peer_ptrs = (ctypes.c_void_p * self.world)(*ptrs)              # HOST array handed to the C ABI
+        self.ebuf, self.embed_ptrs = None, None
+        if embed_floats > 0:
+            self.ebuf = symm_mem.empty(int(embed_floats), dtype=torch.float32, device=device)
+            self.ebuf.zero_()
+            self.ehdl = symm_mem.rendezvous(self.ebuf, group.group_name if hasattr(group, "group_name") else group)
+            eptrs = [int(p) for p in self.ehdl.buffer_ptrs]
+            assert eptrs[self.rank] == self.ebuf.data_ptr()
+            self.embed_ptrs = (ctypes.c_void_p * self.world)(*eptrs)
         self.state = torch.zeros(int(lib().cdll.grapes_peer_state_words()), dtype=torch.int32, device=device)
         torch.cuda.synchronize(device)
         # NOTE: no collective here.  The caller must synchronise the ranks once before the first exchange (every buffer is

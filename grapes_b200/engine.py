@@ -300,15 +300,19 @@ class GrapesEngine:
         # ---- ONE pool that is cleared by ONE memset at the start of every step:
         #   bitmaps (int32 words): all_nodes | indicator rows | prev rows of hop 0..H-1 | batch rows of hop 0..H-1 | prev rows H
         #   floats: scalars | per-hop stats | gradient direction of the sampler nets
+        #   (+ with a learned table: the union of the ranks' rows of a data-parallel step, grapes_embed_merge_adam)
         n_bm = 1 + max(self.num_ind, 1) + 2 * H + 1
         n_fl = 16 + 4 * H + n_par
-        self.step_pool = z(n_bm * W + n_fl, **i32)
+        n_un = 1 if self.embed_nodes else 0
+        self.step_pool = z((n_bm + n_un) * W + n_fl, **i32)
         bm = self.step_pool[:n_bm * W].view(n_bm, W)
+        if self.embed_nodes:
+            self.bm_union = self.step_pool[n_bm * W:(n_bm + 1) * W]
         self.bm_all = bm[0]
         self.bm_ind = bm[1:1 + max(self.num_ind, 1)]
         self.bm_prev = [bm[1 + max(self.num_ind, 1) + h] for h in range(H)] + [bm[n_bm - 1]]   # [H]: rows of the last block (evaluation)
         self.bm_batch = [bm[1 + max(self.num_ind, 1) + H + h] for h in range(H)]
-        fl = self.step_pool[n_bm * W:].view(torch.float32)
+        fl = self.step_pool[(n_bm + n_un) * W:].view(torch.float32)
         self.zero_pool = fl
         self.scal = fl[:16]
         self.stats = fl[16:16 + 4 * H].view(H, 4)
@@ -357,10 +361,10 @@ class GrapesEngine:
         self.par = p
 
     # ------------------------------------------------------------------ helpers
-    _CNT = dict(B=0, A=1, cl_nnz=2)
+    _CNT = dict(B=0, A=1, cl_nnz=2, U=6)
 
     def _cnt(self, name: str, idx: int = 0) -> int:
-        """device address of a global size (B, A, cl_nnz[0..2])"""
+        """device address of a global size (B, A, cl_nnz[0..3], U: union rows of a data-parallel table step)"""
         return self.counts.data_ptr() + 4 * (self._CNT[name] + idx)
 
     def _hc(self, h: int, name: str) -> int:
@@ -842,15 +846,31 @@ class GrapesEngine:
           "peer"  one launch over NVLink peer memory (``grapes_step_tail``: gradient scale + push all-reduce + Adam),
                   captured with the rest of the step -- the N-rank step is ONE graph launch;
           "nccl"  ``ncclAllReduce(AVG)`` on the flat buffer between the scale and the Adam launch (captured into the step
-                  graph as well when the step is replayed from a graph)."""
+                  graph as well when the step is replayed from a graph).
+        With learned node features (``embed_nodes``) the table is replicated like ``x``: rank 0's table is broadcast once
+        here (the moments start at zero), every step ships its row-sparse table gradient (at most cap_A rows) to every
+        rank -- inside the peer tail, or by one ``all_gather`` -- and every rank applies the same dense Adam to the mean
+        of the ranks' gradients (``grapes_embed_merge_adam``), so the tables stay bit-identical."""
         import torch.distributed as dist
-        if self.embed_nodes:
-            raise GrapesError("embed_nodes is single-GPU (SURVEY.md section 8e): the table gradient is not exchanged")
         if exchange not in ("peer", "nccl"):
             raise ValueError("exchange must be 'peer' or 'nccl'")
         group = group or dist.group.WORLD
         self.dp_world, self.dp_rank = dist.get_world_size(group), dist.get_rank(group)
         self.peer, self.dp_group = None, None
+        if self.embed_nodes and self.dp_world > 8:
+            raise GrapesError("learned node features are exchanged among at most 8 ranks (one NVLink box)")
+        embed_floats = 0
+        if self.embed_nodes and self.dp_world > 1:
+            self.emb_slot = int(self.L.cdll.grapes_embed_slot_floats(self.cap_A, self.F))
+            embed_floats = int(self.L.cdll.grapes_embed_peer_buffer_floats(self.cap_A, self.F, self.dp_world))
+            # union of the ranks' rows: at most world * cap_A distinct ids
+            self.cap_U = min(self.N, self.dp_world * self.cap_A)
+            self.pref_union = torch.zeros(self.W + 1, dtype=torch.int32, device=self.device)
+            self.union_ids = torch.zeros(self.cap_U, dtype=torch.int32, device=self.device)
+            self.mean_rows = torch.zeros((self.cap_U, self.F), dtype=torch.float32, device=self.device)
+            dist.broadcast(self.x, src=dist.get_global_rank(group, 0), group=group)
+            self.emb_exp_avg.zero_()
+            self.emb_exp_avg_sq.zero_()
         if self.dp_world > 1:
             if exchange == "peer":
                 # symmetric (peer-mapped) buffers need P2P access between every pair of GPUs of the group.  Every rank tries,
@@ -859,7 +879,7 @@ class GrapesEngine:
                 from .dist import PeerGradExchange, ranks_agree
                 ok, why = True, ""
                 try:
-                    self.peer = PeerGradExchange(self.n_par, self.device, group)
+                    self.peer = PeerGradExchange(self.n_par, self.device, group, embed_floats=embed_floats)
                 except Exception as exc:                      # noqa: BLE001 -- reported below, never silent
                     ok, why, self.peer = False, f"{type(exc).__name__}: {exc}", None
                 if not ranks_agree(ok, self.device, group):
@@ -874,6 +894,12 @@ class GrapesEngine:
                 warm = torch.zeros_like(self.grads)
                 for _ in range(24):
                     dist.all_reduce(warm, op=dist.ReduceOp.AVG, group=group)
+                if self.embed_nodes:
+                    # fixed-size payload of this rank (one slot) and the world slots it is gathered into
+                    self.emb_payload = torch.zeros(self.emb_slot, dtype=torch.float32, device=self.device)
+                    self.emb_gathered = torch.zeros(self.dp_world * self.emb_slot, dtype=torch.float32, device=self.device)
+                    for _ in range(24):
+                        dist.all_gather_into_tensor(self.emb_gathered, self.emb_payload, group=group)
                 torch.cuda.synchronize(self.device)
         self._graphs.clear()
 
@@ -889,7 +915,8 @@ class GrapesEngine:
         scale = not self.random_sampling
         n_z = 0 if self.reinforce else nz.size                       # gcn_z has no grad under REINFORCE (main.py:279)
         n1 = (gf.size + n_z) if scale else 0
-        if self.embed_nodes:
+        embed_dp = self.embed_nodes and self.dp_world > 1
+        if self.embed_nodes and not embed_dp:
             L.grapes_adam_embed(ctx, ptr(self.x), ptr(self.emb_exp_avg), ptr(self.emb_exp_avg_sq), self.N, self.F,
                                 ptr(self.bm_all), ptr(self.pref_all), ptr(self.dXc), self.dXc.shape[1], self.lr_gc,
                                 0.9, 0.999, 1e-8, ptr(self.adam_steps), st)
@@ -903,8 +930,28 @@ class GrapesEngine:
             L.grapes_adam_step2(ctx, ptr(self.params), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq),
                                 nc.base, nc.size, self.lr_gc, gf.base, n1, self.lr_gf, 0.9, 0.999, 1e-8,
                                 ptr(self.adam_steps), st)
+            if embed_dp:
+                # this rank's slot (A | all_nodes | dXc rows): three device copies, then one all-gather of the fixed slot
+                pi, A = self.emb_payload.view(torch.int32), self.cap_A
+                rows_at = 4 + _round_up(A, 4)
+                pi[0:1].copy_(self.counts[self._CNT["A"]:self._CNT["A"] + 1])
+                pi[4:4 + A].copy_(self.all_nodes)
+                self.emb_payload[rows_at:rows_at + A * self.F].view(A, self.F).copy_(self.dXc[:, :self.F])
+                dist.all_gather_into_tensor(self.emb_gathered, self.emb_payload, group=self.dp_group)
+                self._enqueue_embed_merge(ptr(self.emb_gathered), None, st)
             return
         pe = self.peer
+        if embed_dp:
+            L.grapes_step_tail_embed(ctx, ptr(self.scal), int(scale), self.loss_coef, self.log_z_init, int(self.reinforce),
+                                     1, ptr(self.gdir), gf.base, gf.size if scale else 0, nz.base, n_z if scale else 0,
+                                     pe.peer_ptrs, pe.embed_ptrs, pe.rank, pe.world, self.n_par, ptr(self.params),
+                                     ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), nc.base, nc.size,
+                                     self.lr_gc, gf.base, n1, self.lr_gf, 0.9, 0.999, 1e-8, ptr(self.adam_steps),
+                                     ptr(pe.state), ptr(self.overflow), self._cnt("A"), ptr(self.all_nodes),
+                                     ptr(self.dXc), self.dXc.shape[1], self.F, self.cap_A, st)
+            # same stream, before the next tail: the parity argument of csrc/peer_comm.cu needs it there
+            self._enqueue_embed_merge(ptr(pe.ebuf), ptr(pe.state), st)
+            return
         L.grapes_step_tail(ctx, ptr(self.scal), int(scale), self.loss_coef, self.log_z_init, int(self.reinforce), 1,
                            ptr(self.gdir), gf.base, gf.size if scale else 0, nz.base, n_z if scale else 0,
                            pe.peer_ptrs if pe is not None else None, pe.rank if pe is not None else 0,
@@ -912,6 +959,14 @@ class GrapesEngine:
                            ptr(self.exp_avg), ptr(self.exp_avg_sq), nc.base, nc.size, self.lr_gc, gf.base, n1, self.lr_gf,
                            0.9, 0.999, 1e-8, ptr(self.adam_steps), ptr(pe.state if pe is not None else self.tail_state),
                            ptr(self.overflow), st)
+
+    def _enqueue_embed_merge(self, slots, state, st):
+        """optimizer_c's step of the table on the mean of the ranks' row-sparse gradients (after the parameter Adam, so
+        the step count it reads already includes this step)."""
+        self.L.grapes_embed_merge_adam(self.g.ctx, slots, self.dp_world, self.cap_A, self.F, state, ptr(self.bm_union),
+                                       ptr(self.pref_union), ptr(self.union_ids), self.cap_U, self._cnt("U"),
+                                       ptr(self.mean_rows), ptr(self.x), ptr(self.emb_exp_avg), ptr(self.emb_exp_avg_sq),
+                                       self.N, self.lr_gc, 0.9, 0.999, 1e-8, ptr(self.adam_steps), ptr(self.overflow), st)
 
     # ------------------------------------------------------------------ public API
     def set_targets(self, target_nodes: torch.Tensor, state: Optional[int] = None):
@@ -1055,6 +1110,10 @@ class GrapesEngine:
         out["grads"] = {k: {n: t.clone() for n, t in v.items()} for k, v in self.grad_dicts().items()}
         if self.embed_nodes:
             out["grad_x_rows"] = self.dXc[:A, :self.F].clone()       # d loss_c / d x[all_nodes]
+            if self.dp_world > 1:                                     # the rows the data-parallel table step applied
+                U = self.count("U")
+                out["embed_union"] = self.union_ids[:U].clone()
+                out["embed_mean_rows"] = self.mean_rows[:U].clone()
         out["cl_edges"] = []
         for slot, hop in ((0, H - 1), (1, 0)):
             e = sizes[hop]["blk"]

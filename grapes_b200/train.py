@@ -72,7 +72,8 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
             raise ValueError('Dataset does not contain node features, and embed_nodes is False. '
                              'Did you mean to run with --embed_nodes=True?')          # main.py:91-94
         # main.py:95-100: embeddings = nn.Parameter(FloatTensor(N, node_emb_dim).normal_()), appended to optimizer_c.
-        # Here the table lives in HBM and the engine's optimiser launch updates it in place (grapes_adam_embed).
+        # Here the table lives in HBM and the engine's optimiser launch updates it in place (grapes_adam_embed); under
+        # torchrun it is replicated and every rank applies the mean of the ranks' row-sparse gradients.
         logger.info('Using learned node embeddings for features')
         gen = torch.Generator().manual_seed(0 if args.seed is None else args.seed)
         data.x = torch.empty(data.num_nodes, args.node_emb_dim).normal_(generator=gen).to(device)

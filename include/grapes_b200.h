@@ -367,6 +367,39 @@ int grapes_step_tail(grapes_ctx* ctx, float* scal, int do_scale, float loss_coef
                      int n0, float lr0, int off1, int n1, float lr1, float beta1, float beta2, float eps, float* steps_dev,
                      unsigned int* state, int* err_flag, void* stream);
 
+/* ---- data parallelism with learned node features (main.py:89-100,116: the table inside optimizer_c) ---------------
+ * The table is replicated like x; its gradient is row-sparse (the step's all_nodes rows, at most cap_rows = B + H*k),
+ * so every rank ships only (A, all_nodes[:A], d loss_c / d x[all_nodes[:A], :F]).  One slot holds that payload:
+ * [A, 3 pad | cap_rows ids rounded up to 4 | cap_rows x F floats]; the second symmetric buffer of the peer exchange is
+ * 2 parities x world slots.                                                                                         */
+int64_t grapes_embed_slot_floats(int cap_rows, int F);
+int64_t grapes_embed_peer_buffer_floats(int cap_rows, int F, int world);
+/* grapes_step_tail with peers (world <= 8) that also pushes this step's table payload -- A = *count_dev rows, ids[:A]
+ * ascending, rows[:A, :F] at pitch ldg (16-byte aligned) -- into slot[rank] of parity (step & 1) of every rank's
+ * second buffer (embed_bufs: HOST array of `world` peer-mapped pointers, grapes_embed_peer_buffer_floats each).  The
+ * step's one flag covers both payloads; on a failed exchange nothing is pushed.  Follow it, on the same stream and before
+ * the next tail, with grapes_embed_merge_adam(state = the same state): its read of this step's slots must finish before
+ * any peer can push two steps later.                                                                                  */
+int grapes_step_tail_embed(grapes_ctx* ctx, float* scal, int do_scale, float loss_coef, float log_z_init, int reinforce,
+                           int have_log_z, const float* dir, int gf_off, int n_gf, int z_off, int n_z,
+                           void* const* peer_bufs, void* const* embed_bufs, int rank, int world, int n, float* params,
+                           float* grads, float* exp_avg, float* exp_avg_sq, int off0, int n0, float lr0, int off1, int n1,
+                           float lr1, float beta1, float beta2, float eps, float* steps_dev, unsigned int* state,
+                           int* err_flag, const int* count_dev, const int* ids, const float* rows, int ldg, int F,
+                           int cap_rows, void* stream);
+/* optimizer_c's step of the table on the mean over ranks of the row-sparse gradients, g(v) = (1/world) sum_r G_r(v)
+ * added in rank order (identical bits on every rank): union bitmap of the world id lists (bm_union: num_words uint32,
+ * zero on entry), its popcount-prefix rank (pref_union: num_words + 1; union_ids[:*union_count], cap_union >= the union
+ * size), the mean rows (mean_rows [cap_union, F]), then grapes_adam_embed's dense table walk with step_dev = optimizer_c's
+ * count AFTER this step's parameter Adam (the bias correction uses *step_dev as is).  state != NULL: `slots` is this
+ * rank's second peer buffer and the exchange's go word picks the parity; a failed exchange makes all of it a no-op
+ * (table, moments untouched).  state == NULL: `slots` holds the world slots contiguously (an all-gather).             */
+int grapes_embed_merge_adam(grapes_ctx* ctx, const float* slots, int world, int cap_rows, int F,
+                            const unsigned int* state, uint32_t* bm_union, int* pref_union, int* union_ids, int cap_union,
+                            int* union_count, float* mean_rows, float* table, float* exp_avg, float* exp_avg_sq,
+                            int64_t num_nodes, float lr, float beta1, float beta2, float eps, const float* step_dev,
+                            int* overflow, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
