@@ -111,6 +111,55 @@ static inline int grapes_max_i(int a, int b) { return a > b ? a : b; }
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 
+// Philox4x32-10 (Salmon et al. 2011): counter-based, one call = 4 uniforms
+__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
+    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(M0, ctr.x), lo0 = M0 * ctr.x;
+        const uint32_t hi1 = __umulhi(M1, ctr.z), lo1 = M1 * ctr.z;
+        ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
+        key.x += W0; key.y += W1;
+    }
+    return ctr;
+}
+// the selection's Gumbel stream: counter (i / 4, 0, offset): word y is always 0
+__device__ __forceinline__ float philox_uniform(unsigned long long seed, unsigned long long offset, int i) {
+    uint4 ctr = make_uint4((uint32_t)(i >> 2), 0u, (uint32_t)offset, (uint32_t)(offset >> 32));
+    const uint4 r = philox4x32_10(ctr, make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+    const uint32_t x = (i & 3) == 0 ? r.x : (i & 3) == 1 ? r.y : (i & 3) == 2 ? r.z : r.w;
+    return (float)(x & 0xffffffu) * (1.0f / 16777216.0f);   // 24-bit mantissa in [0,1), as torch.rand
+}
+
+// Inverted dropout of the classifier GCN (modules/gcn.py:33,37).  The keep bit of entry i = row * width + col of site
+// `tag` (= 1 + site + 2 * rank; site 0 = hidden layer, 1 = logits) is a pure function of (seed, step, tag, i): Philox
+// counter (i / 4, tag, step), key = the seed's two words, keep iff the 24 low bits of word i % 4 are < threshold
+// (= llrint((1 - p) * 2^24), computed on the host).  tag >= 1 keeps it apart from the selection stream (y = 0).
+// drop_state = {seed, step} in device memory; the step's last reader advances `step` (grapes_classifier_loss_dropout).
+struct DropParams {
+    unsigned long long* state;          // {seed, step}
+    uint32_t tag, threshold;
+    float scale;                        // 1 / (1 - p); 0 when p == 1 (nothing is kept)
+};
+__device__ __forceinline__ uint4 dropout_words(unsigned long long seed, unsigned long long step, uint32_t tag,
+                                               unsigned long long i) {
+    return philox4x32_10(make_uint4((uint32_t)(i >> 2), tag, (uint32_t)step, (uint32_t)(step >> 32)),
+                         make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+}
+__device__ __forceinline__ bool dropout_keep(unsigned long long seed, unsigned long long step, uint32_t tag,
+                                             uint32_t threshold, unsigned long long i) {
+    const uint4 r = dropout_words(seed, step, tag, i);
+    const uint32_t x = (i & 3) == 0 ? r.x : (i & 3) == 1 ? r.y : (i & 3) == 2 ? r.z : r.w;
+    return (x & 0xffffffu) < threshold;
+}
+// keep bits of entries i0 .. i0 + 3 (bit j = entry i0 + j); i0 % 4 == 0: one Philox call
+__device__ __forceinline__ uint32_t dropout_keep4(unsigned long long seed, unsigned long long step, uint32_t tag,
+                                                  uint32_t threshold, unsigned long long i0) {
+    const uint4 r = dropout_words(seed, step, tag, i0);
+    return ((r.x & 0xffffffu) < threshold ? 1u : 0u) | ((r.y & 0xffffffu) < threshold ? 2u : 0u) |
+           ((r.z & 0xffffffu) < threshold ? 4u : 0u) | ((r.w & 0xffffffu) < threshold ? 8u : 0u);
+}
+
 // device state words of one data-parallel exchange endpoint (peer_comm.cu; read by grapes_embed_merge_adam)
 #define PS_SEQ 0        // steps completed
 #define PS_TICKET_A 1   // push ticket

@@ -584,6 +584,67 @@ __global__ void __launch_bounds__(G_THREADS) k_gemm(const float* __restrict__ A,
     }
 }
 
+// keep bits of the 4 consecutive entries i0 .. i0 + 3 of a dropout site (one Philox call when i0 is a multiple of 4)
+__device__ __forceinline__ uint32_t drop_bits4(unsigned long long seed, unsigned long long step, const DropParams& dp,
+                                               unsigned long long i0) {
+    if ((i0 & 3) == 0) return dropout_keep4(seed, step, dp.tag, dp.threshold, i0);
+    uint32_t b = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) b |= dropout_keep(seed, step, dp.tag, dp.threshold, i0 + j) ? (1u << j) : 0u;
+    return b;
+}
+
+// Dropout forms of the classifier's hidden layer (modules/gcn.py:33), kept apart from k_gemm / k_gemm_s so the plain
+// products carry no dropout branch.  FWD: C = dropout(relu(A W^T + b)), A [M x K] and W [N x K] K-contiguous (layout 3),
+// keep bit of entry (row, col) at i = row * N + col.  !FWD: C = (G > 0) ? s * (A B) : 0, A [M x K] K-contiguous, B [K x N]
+// (layout 1): the backward of dropout(relu(.)) when G holds the dropped activations (zero wherever the unit was dropped
+// or inactive).
+template <bool FWD>
+__global__ void __launch_bounds__(G_THREADS) k_gemm_dropout(const float* __restrict__ A, int lda,
+                                                            const float* __restrict__ B, int ldb, float* __restrict__ C,
+                                                            int ldc, const int* __restrict__ M_dev, int M_cap, int N,
+                                                            int K, const float* __restrict__ bias,
+                                                            const float* __restrict__ relu_gate, int ldg, DropParams dp) {
+    pdl_begin();
+    __shared__ __align__(16) float As[GB_K][GB_M + G_PAD];
+    __shared__ __align__(16) float Bs[GB_K][GB_N + G_PAD];
+    const int M = M_dev ? min(*M_dev, M_cap) : M_cap;
+    const int n0 = blockIdx.x * GB_N;
+    const unsigned long long seed = FWD ? dp.state[0] : 0ull, step = FWD ? dp.state[1] : 0ull;
+    for (int m0 = blockIdx.y * GB_M; m0 < M; m0 += gridDim.y * GB_M) {
+        float acc[8][8];
+#pragma unroll
+        for (int r = 0; r < 8; ++r)
+#pragma unroll
+            for (int c = 0; c < 8; ++c) acc[r][c] = 0.f;
+        gemm_mainloop<true, FWD>(A, lda, m0, M, B, ldb, n0, N, 0, K, As, Bs, acc);
+        const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {
+            const int row = m0 + g_row(ty, r);
+            if (row >= M) continue;
+            uint32_t keep = 0u;
+            if (FWD) {
+                const unsigned long long i0 = (unsigned long long)row * N + n0 + tx * 4;
+                keep = drop_bits4(seed, step, dp, i0) | (drop_bits4(seed, step, dp, i0 + 64) << 4);
+            }
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                const int col = n0 + g_col(tx, c);
+                if (col >= N) continue;
+                float v = acc[r][c];
+                if (FWD) {
+                    v = fmaxf(v + bias[col], 0.f);
+                    v = ((keep >> c) & 1u) ? v * dp.scale : 0.f;
+                } else {
+                    v = (relu_gate[(size_t)row * ldg + col] > 0.f) ? v * dp.scale : 0.f;
+                }
+                C[(size_t)row * ldc + col] = v;
+            }
+        }
+    }
+}
+
 // Split-K "TN" product for weight gradients:  P[slab][M x N] = sum_{r in slab} A[r, m] * B[r, n]
 // (A: R x M row-major, B: R x N row-major, R = rows from the device).  grid = (tiles_n, tiles_m, slabs).
 // Slab boundaries are multiples of GB_K so the summation order does not depend on the grid.
@@ -741,6 +802,51 @@ __global__ void __launch_bounds__(G_THREADS) k_gemm_s(const float* __restrict__ 
                 if (bias) v += bias[col];
                 if (relu) v = fmaxf(v, 0.f);
                 if (relu_gate) v = (relu_gate[(size_t)row * ldg + col] > 0.f) ? v : 0.f;
+                C[(size_t)row * ldc + col] = v;
+            }
+        }
+    }
+}
+
+// small-tile form of k_gemm_dropout (classifier-sized products)
+template <bool FWD>
+__global__ void __launch_bounds__(G_THREADS) k_gemm_s_dropout(const float* __restrict__ A, int lda,
+                                                              const float* __restrict__ B, int ldb,
+                                                              float* __restrict__ C, int ldc,
+                                                              const int* __restrict__ M_dev, int M_cap, int N, int K,
+                                                              const float* __restrict__ bias,
+                                                              const float* __restrict__ relu_gate, int ldg,
+                                                              DropParams dp) {
+    pdl_begin();
+    __shared__ __align__(16) float As[GB_K][GS_M + GS_PAD];
+    __shared__ __align__(16) float Bs[GB_K][GS_N + GS_PAD];
+    const int M = M_dev ? min(*M_dev, M_cap) : M_cap;
+    const int n0 = blockIdx.x * GS_N;
+    const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
+    const unsigned long long seed = FWD ? dp.state[0] : 0ull, step = FWD ? dp.state[1] : 0ull;
+    for (int m0 = blockIdx.y * GS_M; m0 < M; m0 += gridDim.y * GS_M) {
+        float acc[4][4];
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+#pragma unroll
+            for (int c = 0; c < 4; ++c) acc[r][c] = 0.f;
+        gemm_mainloop_s<true, FWD>(A, lda, m0, M, B, ldb, n0, N, 0, K, As, Bs, acc);
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+            const int row = m0 + ty * 4 + r;
+            if (row >= M) continue;
+            const uint32_t keep = FWD ? drop_bits4(seed, step, dp, (unsigned long long)row * N + n0 + tx * 4) : 0u;
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                const int col = n0 + tx * 4 + c;
+                if (col >= N) continue;
+                float v = acc[r][c];
+                if (FWD) {
+                    v = fmaxf(v + bias[col], 0.f);
+                    v = ((keep >> c) & 1u) ? v * dp.scale : 0.f;
+                } else {
+                    v = (relu_gate[(size_t)row * ldg + col] > 0.f) ? v * dp.scale : 0.f;
+                }
                 C[(size_t)row * ldc + col] = v;
             }
         }
@@ -908,6 +1014,27 @@ static inline int grid_for(const grapes_ctx* ctx, long long work, int threads, i
     long long cap = (long long)ctx->sm_count * per_sm;
     if (b < 1) b = 1;
     return (int)(b < cap ? b : cap);
+}
+
+// the two dropout forms of the classifier's hidden layer; same tile choice as grapes_gemm
+template <bool FWD>
+static int launch_gemm_dropout(grapes_ctx* ctx, const float* A, int lda, const float* B, int ldb, float* C, int ldc,
+                               const int* M_dev, int M_cap, int N, int K, const float* bias, const float* relu_gate,
+                               int ldg, DropParams dp, cudaStream_t s) {
+    if (M_cap == 0) return GRAPES_OK;
+    grapes_count_launches(1);
+    if ((long long)grapes_div_up(N, GB_N) * grapes_div_up(M_cap, GB_M) < ctx->sm_count) {
+        dim3 grid(grapes_div_up(N, GS_N), grapes_min_i(grapes_div_up(M_cap, GS_M), 65535));
+        pdl((k_gemm_s_dropout<FWD>), grid, G_THREADS, 0, s)(A, lda, B, ldb, C, ldc, M_dev, M_cap, N, K, bias, relu_gate,
+                                                          ldg, dp);
+    } else {
+        const int tiles_n = grapes_div_up(N, GB_N);
+        const int tiles_m = grapes_min_i(grapes_div_up(M_cap, GB_M), grapes_max_i(1, (ctx->sm_count * 4) / tiles_n));
+        pdl((k_gemm_dropout<FWD>), dim3(tiles_n, tiles_m), G_THREADS, 0, s)(A, lda, B, ldb, C, ldc, M_dev, M_cap, N, K,
+                                                                           bias, relu_gate, ldg, dp);
+    }
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
 }
 
 static int g_agg_variant = 0;
@@ -1118,6 +1245,27 @@ int grapes_gemm(grapes_ctx* ctx, int layout, const float* A, int lda, const floa
     }
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
+}
+
+int grapes_gemm_bias_relu_dropout(grapes_ctx* ctx, const float* A, int lda, const float* W, int ldw, float* H, int ldh,
+                                  const int* M_dev, int M_cap, int N, int K, const float* bias,
+                                  unsigned long long* drop_state, uint32_t tag, uint32_t threshold, float scale,
+                                  void* stream) {
+    GRAPES_REQUIRE(ctx && A && W && H && bias && drop_state, "null argument");
+    GRAPES_REQUIRE(M_cap >= 0 && N > 0 && K > 0 && tag >= 1u && threshold <= (1u << 24), "bad shape or dropout parameters");
+    DropParams dp = {drop_state, tag, threshold, scale};
+    return launch_gemm_dropout<true>(ctx, A, lda, W, ldw, H, ldh, M_dev, M_cap, N, K, bias, nullptr, 0, dp,
+                                     (cudaStream_t)stream);
+}
+
+int grapes_gemm_gated_scaled(grapes_ctx* ctx, const float* A, int lda, const float* B, int ldb, float* C, int ldc,
+                             const int* M_dev, int M_cap, int N, int K, const float* gate, int ldg, float scale,
+                             void* stream) {
+    GRAPES_REQUIRE(ctx && A && B && C && gate, "null argument");
+    GRAPES_REQUIRE(M_cap >= 0 && N > 0 && K > 0, "bad shape");
+    DropParams dp = {nullptr, 0u, 0u, scale};
+    return launch_gemm_dropout<false>(ctx, A, lda, B, ldb, C, ldc, M_dev, M_cap, N, K, nullptr, gate, ldg, dp,
+                                      (cudaStream_t)stream);
 }
 
 // out[M x N] (+)= scale * A[R x M]^T B[R x N]   (weight gradients; deterministic split over rows)

@@ -172,11 +172,9 @@ __global__ void __launch_bounds__(LR2_WARPS * 32) k_loss_rows2(
     }
 }
 
-__global__ void __launch_bounds__(LOSS_THREADS) k_loss_final2(const int* __restrict__ A_dev, int A_cap, int C,
-                                                              const float* __restrict__ row_loss,
-                                                              const float* __restrict__ colpart, int nblocks,
-                                                              float* loss_out, float* __restrict__ colsum_out) {
-    pdl_begin();
+__device__ __forceinline__ void loss_final2_body(const int* __restrict__ A_dev, int A_cap, int C,
+                                                 const float* __restrict__ row_loss, const float* __restrict__ colpart,
+                                                 int nblocks, float* loss_out, float* __restrict__ colsum_out) {
     __shared__ float s[32];
     __shared__ float s_col[LOSS_THREADS];
     const int A = min(*A_dev, A_cap);
@@ -205,6 +203,215 @@ __global__ void __launch_bounds__(LOSS_THREADS) k_loss_final2(const int* __restr
         for (int gg = 0; gg < groups; ++gg) t += s_col[gg * C + threadIdx.x];
         colsum_out[threadIdx.x] = t;
     }
+}
+
+__global__ void __launch_bounds__(LOSS_THREADS) k_loss_final2(const int* __restrict__ A_dev, int A_cap, int C,
+                                                              const float* __restrict__ row_loss,
+                                                              const float* __restrict__ colpart, int nblocks,
+                                                              float* loss_out, float* __restrict__ colsum_out) {
+    pdl_begin();
+    loss_final2_body(A_dev, A_cap, C, row_loss, colpart, nblocks, loss_out, colsum_out);
+}
+
+// ---------------------------------------------------------------------------------------
+// Dropout forms of the classifier loss (modules/gcn.py:37: logits = dropout(A_hat_2 (h W2^T) + b2), the loss on the
+// dropped logits).  `logits` holds the pre-dropout values the +b2 aggregation wrote; the dropped logits are written back
+// in place and the gradient leaves as d logits_pre = d logits (.) keep * s, the input of dZ and of the b2 column sums.
+// The keep bit of (row, c) is entry row * C + c of the logits site.  The loss-final kernel is the last reader of the
+// step's drop_state and advances its step word.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(LR2_WARPS * 32) k_loss_rows2_dropout(
+    float* __restrict__ logits, int ldl, int C, const int* __restrict__ A_dev, int A_cap,
+    const int* __restrict__ tgt_of_row, const int* __restrict__ targets, int B,
+    const int64_t* __restrict__ labels_i64, const float* __restrict__ labels_f32, float reg_param,
+    float* __restrict__ dlogits, float* __restrict__ row_loss, float* __restrict__ colpart, DropParams dp) {
+    pdl_begin();
+    extern __shared__ float s_cols[];                    // [LR2_WARPS][C]
+    const int A = min(*A_dev, A_cap);
+    const int lane = lane_id(), warp = threadIdx.x >> 5;
+    const int row = blockIdx.x * LR2_WARPS + warp;
+    float* mycols = s_cols + warp * C;
+    for (int c = lane; c < C; c += 32) mycols[c] = 0.f;
+    if (row < A) {
+        float* lr = logits + (size_t)row * ldl;
+        float* dr = dlogits + (size_t)row * ldl;
+        const unsigned long long seed = dp.state[0], step = dp.state[1];
+        uint32_t keep = 0u;                              // bit j: column lane + 32 j (C <= LOSS_THREADS)
+        for (int c = lane, j = 0; c < C; c += 32, ++j) {
+            const bool k = dropout_keep(seed, step, dp.tag, dp.threshold, (unsigned long long)row * C + c);
+            keep |= k ? (1u << j) : 0u;
+            lr[c] = k ? lr[c] * dp.scale : 0.f;
+        }
+        __syncwarp();
+        const int r = tgt_of_row[row];
+        float loss = 0.f;
+        if (r >= 0 && labels_i64) {
+            const float invB = 1.0f / (float)B;
+            const int y = (int)labels_i64[targets[r]];
+            float mx = -INFINITY;
+            for (int c = lane; c < C; c += 32) mx = fmaxf(mx, lr[c]);
+            mx = warp_max(mx);
+            float se = 0.f;
+            for (int c = lane; c < C; c += 32) se += expf(lr[c] - mx);
+            se = warp_sum(se);
+            const float lse = mx + logf(se);
+            for (int c = lane; c < C; c += 32) mycols[c] = (expf(lr[c] - lse) - (c == y ? 1.f : 0.f)) * invB;
+            loss = (lse - lr[y]) * invB;
+        } else if (r >= 0) {
+            const float inv = 1.0f / ((float)B * (float)C);
+            const float* yr = labels_f32 + (size_t)targets[r] * C;
+            float a = 0.f;
+            for (int c = lane; c < C; c += 32) {
+                const float l = lr[c], y = yr[c];
+                a += (1.0f - y) * l + fmaxf(-l, 0.f) + log1pf(expf(-fabsf(l)));
+                mycols[c] = (1.0f / (1.0f + expf(-l)) - y) * inv;
+            }
+            loss = warp_sum(a) * inv;
+        }
+        if (reg_param != 0.f && C > 1) {                 // reg_param * var(logits[row], unbiased)
+            const float invc1 = 1.0f / (float)(C - 1);
+            float sm = 0.f;
+            for (int c = lane; c < C; c += 32) sm += lr[c];
+            const float mean = warp_sum(sm) / (float)C;
+            float sq = 0.f;
+            for (int c = lane; c < C; c += 32) {
+                const float d = lr[c] - mean;
+                sq = fmaf(d, d, sq);
+                mycols[c] += reg_param * 2.0f * d * invc1;
+            }
+            loss += reg_param * warp_sum(sq) * invc1;
+        }
+        __syncwarp();
+        for (int c = lane, j = 0; c < C; c += 32, ++j) {
+            const float g = ((keep >> j) & 1u) ? mycols[c] * dp.scale : 0.f;
+            mycols[c] = g;
+            dr[c] = g;
+        }
+        if (lane == 0) row_loss[row] = loss;
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+        float a = 0.f;
+#pragma unroll
+        for (int w = 0; w < LR2_WARPS; ++w) a += s_cols[w * C + c];
+        colpart[(size_t)blockIdx.x * C + c] = a;
+    }
+}
+
+__global__ void __launch_bounds__(LOSS_THREADS) k_loss_final2_dropout(const int* __restrict__ A_dev, int A_cap, int C,
+                                                                      const float* __restrict__ row_loss,
+                                                                      const float* __restrict__ colpart, int nblocks,
+                                                                      float* loss_out, float* __restrict__ colsum_out,
+                                                                      DropParams dp) {
+    pdl_begin();
+    if (threadIdx.x == 0) dp.state[1] += 1ull;         // every reader of this step's masks has completed
+    loss_final2_body(A_dev, A_cap, C, row_loss, colpart, nblocks, loss_out, colsum_out);
+}
+
+// dropped value of logits[row, c] (the k_loss_rows form reads the pre-dropout logits; k_loss_final_dropout writes them)
+__device__ __forceinline__ float dropped_logit(const float* lr, int c, unsigned long long i, unsigned long long seed,
+                                               unsigned long long step, const DropParams& dp) {
+    return dropout_keep(seed, step, dp.tag, dp.threshold, i) ? lr[c] * dp.scale : 0.f;
+}
+
+__global__ void __launch_bounds__(256) k_loss_rows_dropout(const float* __restrict__ logits, int ldl, int C,
+                                                           const int* __restrict__ row_ids,
+                                                           const int* __restrict__ targets, int B,
+                                                           const int64_t* __restrict__ labels_i64,
+                                                           const float* __restrict__ labels_f32,
+                                                           float* __restrict__ dlogits, float* __restrict__ row_loss,
+                                                           DropParams dp) {
+    pdl_begin();
+    const int lane = lane_id();
+    const int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (r >= B) return;
+    const int row = row_ids[r];
+    const float* lr = logits + (size_t)row * ldl;
+    const unsigned long long seed = dp.state[0], step = dp.state[1], i0 = (unsigned long long)row * C;
+    if (labels_i64) {
+        const float invB = 1.0f / (float)B;
+        const int y = (int)labels_i64[targets[r]];
+        float mx = -INFINITY;
+        for (int c = lane; c < C; c += 32) mx = fmaxf(mx, dropped_logit(lr, c, i0 + c, seed, step, dp));
+        mx = warp_max(mx);
+        float se = 0.f;
+        for (int c = lane; c < C; c += 32) se += expf(dropped_logit(lr, c, i0 + c, seed, step, dp) - mx);
+        se = warp_sum(se);
+        const float lse = mx + logf(se);
+        for (int c = lane; c < C; c += 32) {
+            const float pr = expf(dropped_logit(lr, c, i0 + c, seed, step, dp) - lse);
+            dlogits[(size_t)row * ldl + c] = (pr - (c == y ? 1.f : 0.f)) * invB;
+        }
+        if (lane == 0) row_loss[r] = (lse - dropped_logit(lr, y, i0 + y, seed, step, dp)) * invB;
+    } else {
+        const float inv = 1.0f / ((float)B * (float)C);
+        const float* yr = labels_f32 + (size_t)targets[r] * C;
+        float a = 0.f;
+        for (int c = lane; c < C; c += 32) {
+            const float l = dropped_logit(lr, c, i0 + c, seed, step, dp), y = yr[c];
+            a += (1.0f - y) * l + fmaxf(-l, 0.f) + log1pf(expf(-fabsf(l)));
+            dlogits[(size_t)row * ldl + c] = (1.0f / (1.0f + expf(-l)) - y) * inv;
+        }
+        a = warp_sum(a);
+        if (lane == 0) row_loss[r] = a * inv;
+    }
+}
+
+// one CTA: drops every row of the logits in place, adds the reg_param term on the dropped logits, masks the whole
+// gradient, then advances the step word
+__global__ void __launch_bounds__(LOSS_THREADS) k_loss_final_dropout(float* __restrict__ logits, int ldl, int C,
+                                                                     const int* __restrict__ A_dev, int A_cap, int B,
+                                                                     const float* __restrict__ row_loss,
+                                                                     float reg_param, float* __restrict__ dlogits,
+                                                                     float* loss_out, DropParams dp) {
+    pdl_begin();
+    __shared__ float s[32];
+    const int A = min(*A_dev, A_cap);
+    const int lane = lane_id(), warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const unsigned long long seed = dp.state[0], step = dp.state[1];
+    float part = 0.f;
+    for (int r = threadIdx.x; r < B; r += blockDim.x) part += row_loss[r];
+    float loss = block_sum_1024(part, s);
+    const bool reg = reg_param != 0.f && C > 1;
+    float rp = 0.f;
+    for (int row = warp; row < A; row += nwarps) {
+        float* lr = logits + (size_t)row * ldl;
+        float* dr = dlogits + (size_t)row * ldl;
+        const unsigned long long i0 = (unsigned long long)row * C;
+        for (int c = lane; c < C; c += 32) lr[c] = dropped_logit(lr, c, i0 + c, seed, step, dp);
+        if (reg) {                                       // reg_param * sum_rows var(logits, dim=1), unbiased
+            const float invc1 = 1.0f / (float)(C - 1);
+            float sm = 0.f;
+            for (int c = lane; c < C; c += 32) sm += lr[c];
+            const float mean = warp_sum(sm) / (float)C;
+            float sq = 0.f;
+            for (int c = lane; c < C; c += 32) {
+                const float d = lr[c] - mean;
+                sq = fmaf(d, d, sq);
+                dr[c] += reg_param * 2.0f * d * invc1;
+            }
+            sq = warp_sum(sq);
+            if (lane == 0) rp += sq * invc1;
+        }
+        for (int c = lane; c < C; c += 32)
+            dr[c] = dropout_keep(seed, step, dp.tag, dp.threshold, i0 + c) ? dr[c] * dp.scale : 0.f;
+    }
+    if (reg) loss += reg_param * block_sum_1024(rp, s);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        *loss_out = loss;
+        dp.state[1] = step + 1ull;
+    }
+}
+
+// keep[r * width + c] = keep bit of entry (r, c) of a dropout site, r < *rows_dev (the step's masks, for inspection)
+__global__ void __launch_bounds__(256) k_dropout_mask(unsigned long long seed, unsigned long long step, uint32_t tag,
+                                                      uint32_t threshold, const int* __restrict__ rows_dev, int cap_rows,
+                                                      int width, uint8_t* __restrict__ keep) {
+    pdl_begin();
+    const long long n = (long long)min(*rows_dev, cap_rows) * width;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        keep[i] = dropout_keep(seed, step, tag, threshold, (unsigned long long)i) ? 1 : 0;
 }
 
 // scal layout (float): see GRAPES_SCAL_* in the header.
@@ -524,6 +731,57 @@ int grapes_classifier_loss(grapes_ctx* ctx, const float* logits, int ldl, int C,
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     if (colsum_out) return grapes_colsum(ctx, dlogits, A_dev, A_cap, ldl, C, 1.0f, 0, colsum_out, stream);
+    return GRAPES_OK;
+}
+
+int grapes_classifier_loss_dropout(grapes_ctx* ctx, float* logits, int ldl, int C, const int* A_dev, int A_cap,
+                                   const int* row_ids, const int* tgt_of_row, const int* targets, int B,
+                                   const int64_t* labels_i64, const float* labels_f32, float reg_param, float* dlogits,
+                                   float* loss_out, float* colsum_out, unsigned long long* drop_state, uint32_t tag,
+                                   uint32_t threshold, float scale, void* stream) {
+    GRAPES_REQUIRE(ctx && logits && A_dev && row_ids && targets && dlogits && loss_out && drop_state, "null argument");
+    GRAPES_REQUIRE((labels_i64 != nullptr) != (labels_f32 != nullptr), "exactly one label array");
+    GRAPES_REQUIRE(B > 0 && C > 0, "bad shape");
+    GRAPES_REQUIRE(tag >= 1u && threshold <= (1u << 24), "bad dropout parameters");
+    cudaStream_t s = (cudaStream_t)stream;
+    const DropParams dp = {drop_state, tag, threshold, scale};
+    if (tgt_of_row && C <= LOSS_THREADS) {
+        const int nblocks = grapes_div_up(A_cap, LR2_WARPS);
+        GRAPES_REQUIRE(((size_t)A_cap + (size_t)nblocks * C) * sizeof(float) <= ctx->partials_bytes, "partial buffer too small");
+        float* row_loss = ctx->partials;
+        float* colpart = ctx->partials + A_cap;
+        pdl((k_loss_rows2_dropout), nblocks, LR2_WARPS * 32, LR2_WARPS * C * sizeof(float), s)(
+            logits, ldl, C, A_dev, A_cap, tgt_of_row, targets, B, labels_i64, labels_f32, reg_param, dlogits, row_loss,
+            colpart, dp);
+        grapes_count_launches(1);
+        pdl((k_loss_final2_dropout), 1, LOSS_THREADS, 0, s)(A_dev, A_cap, C, row_loss, colpart, nblocks, loss_out,
+                                                            colsum_out, dp);
+        grapes_count_launches(1);
+        GRAPES_LAUNCH_OK();
+        return GRAPES_OK;
+    }
+    GRAPES_CUDA_OK(cudaMemsetAsync(dlogits, 0, sizeof(float) * (size_t)A_cap * ldl, s));
+    GRAPES_REQUIRE((size_t)B * sizeof(float) <= ctx->partials_bytes, "partial buffer too small");
+    pdl((k_loss_rows_dropout), grapes_div_up((long long)B * 32, 256), 256, 0, s)(logits, ldl, C, row_ids, targets, B,
+                                                                              labels_i64, labels_f32, dlogits,
+                                                                              ctx->partials, dp);
+    grapes_count_launches(1);
+    pdl((k_loss_final_dropout), 1, LOSS_THREADS, 0, s)(logits, ldl, C, A_dev, A_cap, B, ctx->partials, reg_param,
+                                                       dlogits, loss_out, dp);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    if (colsum_out) return grapes_colsum(ctx, dlogits, A_dev, A_cap, ldl, C, 1.0f, 0, colsum_out, stream);
+    return GRAPES_OK;
+}
+
+int grapes_dropout_mask(grapes_ctx* ctx, int64_t seed, int64_t step, uint32_t tag, uint32_t threshold,
+                        const int* rows_dev, int cap_rows, int width, uint8_t* keep, void* stream) {
+    GRAPES_REQUIRE(ctx && rows_dev && keep, "null argument");
+    GRAPES_REQUIRE(cap_rows >= 0 && width > 0, "bad shape");
+    pdl((k_dropout_mask), grid_for(ctx, (long long)cap_rows * width, 256), 256, 0, (cudaStream_t)stream)(
+        (unsigned long long)seed, (unsigned long long)step, tag, threshold, rows_dev, cap_rows, width, keep);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
     return GRAPES_OK;
 }
 

@@ -47,25 +47,6 @@ __device__ __forceinline__ unsigned long long composite(uint32_t ukey, int idx) 
     return ((unsigned long long)ukey << 32) | (unsigned long long)(0xffffffffu - (uint32_t)idx);
 }
 
-// Philox4x32-10 (Salmon et al. 2011): counter-based, one call = 4 uniforms
-__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
-    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(M0, ctr.x), lo0 = M0 * ctr.x;
-        const uint32_t hi1 = __umulhi(M1, ctr.z), lo1 = M1 * ctr.z;
-        ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-        key.x += W0; key.y += W1;
-    }
-    return ctr;
-}
-__device__ __forceinline__ float philox_uniform(unsigned long long seed, unsigned long long offset, int i) {
-    uint4 ctr = make_uint4((uint32_t)(i >> 2), 0u, (uint32_t)offset, (uint32_t)(offset >> 32));
-    const uint4 r = philox4x32_10(ctr, make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-    const uint32_t x = (i & 3) == 0 ? r.x : (i & 3) == 1 ? r.y : (i & 3) == 2 ? r.z : r.w;
-    return (float)(x & 0xffffffu) * (1.0f / 16777216.0f);   // 24-bit mantissa in [0,1), as torch.rand
-}
-
 __device__ __forceinline__ float sigmoidf_(float l) { return 1.0f / (1.0f + expf(-l)); }
 // Bernoulli(logits=l).log_prob(y) = -BCEWithLogits(l, y)  (utils.py:71)
 __device__ __forceinline__ float bern_log_prob(float l, float y) {

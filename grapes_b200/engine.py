@@ -84,7 +84,11 @@ class GrapesEngine:
                  log_z_init: float = 0., reg_param: float = 0., random_sampling: bool = False,
                  reinforce_baseline: bool = False, seed: int = 0, cap_edges: Optional[int] = None,
                  cap_nodes: Optional[int] = None, cap_block: Optional[int] = None,
-                 use_tensor_cores: bool = True, multi_stream: bool = True, embed_nodes: bool = False):
+                 use_tensor_cores: bool = True, multi_stream: bool = True, embed_nodes: bool = False,
+                 dropout: float = 0.):
+        dropout = float(dropout)
+        if not 0. <= dropout <= 1.:
+            raise ValueError(f"dropout probability has to be between 0 and 1, but got {dropout}")
         self.g = graph
         self.L = lib()
         dev = graph.device
@@ -196,6 +200,14 @@ class GrapesEngine:
         self.sel_work = z(int(self.L.cdll.grapes_select_work_floats(graph.ctx, cap_n)), **f32)   # zero once: the library keeps its histogram clean
         self.overflow = z(1, **i32)
         self.rng_state = torch.tensor([seed & 0x7fffffffffffffff, 0], dtype=torch.int64, device=dev)
+        # inverted dropout of gcn_c (modules/gcn.py:33,37): keep with probability 1 - p, as an integer threshold on 24 random
+        # bits (llrint, so a host mirror reproduces the masks exactly); kept entries are scaled by 1 / (1 - p).  The masks
+        # come from their own counter pair {seed, step}, advanced once per training step inside the step, so the sampler's
+        # Philox stream (rng_state) is the same with and without dropout.
+        self.dropout = dropout
+        self.drop_threshold = int(round((1. - dropout) * (1 << 24)))
+        self.drop_scale = 1. / (1. - dropout) if dropout < 1. else 0.
+        self.drop_state = torch.tensor([seed & 0x7fffffffffffffff, 0], dtype=torch.int64, device=dev)
         # ---- two step states (see _alloc_step_state); self.<buffer> always refers to the ACTIVE one ----
         base_names = set(self.__dict__)
         self._states = []
@@ -383,6 +395,11 @@ class GrapesEngine:
     def _scal(self, name: str) -> int:
         return self.scal.data_ptr() + 4 * SCAL[name]
 
+    def _drop_tag(self, site: int) -> int:
+        """Philox counter word of a dropout site (0: hidden layer, 1: logits) on this rank: data-parallel ranks draw
+        independent masks, and rank 0 of any world draws what one GPU draws"""
+        return 1 + site + 2 * self.dp_rank
+
     def state_dicts(self) -> Dict[str, Dict[str, torch.Tensor]]:
         return {"gcn_c": self.net_c.views(self.params), "gcn_gf": self.net_gf.views(self.params),
                 "gcn_z": self.net_z.views(self.params)}
@@ -523,16 +540,22 @@ class GrapesEngine:
             join(sA)
             join(sP)
             return
-        self._enqueue_classifier_forward(ctx, st)
+        self._enqueue_classifier_forward(ctx, st, training=True)
         L.tag = "[cls]"
         nc = self.net_c
         ldYc = self.Yc.shape[1]
         A_dev, cap_A = self._cnt("A"), self.cap_A
         # loss + d loss / d logits + d loss / d b2 (column sums) in one launch (main.py:260-261)
-        L.grapes_classifier_loss(ctx, ptr(self.logits_c), C, C, A_dev, cap_A, ptr(self.target_local),
-                                 ptr(self.tgt_of_row) if self.cap_A <= 4096 else None, ptr(self.targets), B, None if self.multilabel else ptr(self.y),
-                                 ptr(self.y) if self.multilabel else None, self.reg_param, ptr(self.dlogits),
-                                 self._scal("loss_c"), self._grd(nc.b2), st)
+        loss_args = (ctx, ptr(self.logits_c), C, C, A_dev, cap_A, ptr(self.target_local),
+                     ptr(self.tgt_of_row) if self.cap_A <= 4096 else None, ptr(self.targets), B,
+                     None if self.multilabel else ptr(self.y), ptr(self.y) if self.multilabel else None, self.reg_param,
+                     ptr(self.dlogits), self._scal("loss_c"), self._grd(nc.b2))
+        if self.dropout > 0:
+            # on dropout(logits) (modules/gcn.py:37); the last launch advances drop_state (every reader has run)
+            L.grapes_classifier_loss_dropout(*loss_args, ptr(self.drop_state), self._drop_tag(1), self.drop_threshold,
+                                             self.drop_scale, st)
+        else:
+            L.grapes_classifier_loss(*loss_args, st)
         # backward of the classifier (loss_c.backward(), main.py:267); the two weight-gradient products that nothing
         # else waits for run on side B next to the chain dZ -> dpre1 -> dW1
         L.grapes_aggregate(ctx, ptr(self.dlogits), C, C, None, A_dev, cap_A, ptr(self.cl_out_off),
@@ -540,8 +563,13 @@ class GrapesEngine:
         fork(sB)
         with on(sB):
             L.grapes_gemm_tn(ctx_b, ptr(self.dZ), C, ptr(self.out1), D, A_dev, cap_A, C, D, 1.0, 0, self._grd(nc.W2), stB)
-        L.grapes_gemm(ctx, 1, ptr(self.dZ), C, self._par(nc.W2), D, ptr(self.dpre1), D, A_dev, cap_A, D, C, None, 0,
-                      ptr(self.out1), D, st)
+        if self.dropout > 0:
+            # out1 holds dropout(relu(pre1)): zero wherever the unit is inactive or dropped, so the gate is relu' * keep
+            L.grapes_gemm_gated_scaled(ctx, ptr(self.dZ), C, self._par(nc.W2), D, ptr(self.dpre1), D, A_dev, cap_A, D, C,
+                                       ptr(self.out1), D, self.drop_scale, st)
+        else:
+            L.grapes_gemm(ctx, 1, ptr(self.dZ), C, self._par(nc.W2), D, ptr(self.dpre1), D, A_dev, cap_A, D, C, None, 0,
+                          ptr(self.out1), D, st)
         fork(sB)
         with on(sB):
             L.grapes_colsum(ctx_b, ptr(self.dpre1), A_dev, cap_A, D, D, 1.0, 0, self._grd(nc.b1), stB)
@@ -567,9 +595,10 @@ class GrapesEngine:
                                         self._dir(gf.base), gf.size, self._grd(gf.base),
                                         self._dir(nz.base), n_z, self._grd(nz.base), st)
 
-    def _enqueue_classifier_forward(self, ctx, st):
+    def _enqueue_classifier_forward(self, ctx, st, training: bool):
         """all_nodes + relabel of the per-hop blocks + gcn_norm structure of the classifier's two layers, then
-        logits = gcn_c(x[all_nodes], [block_0 .. block_{H-1}]) (main.py:252-257, eval.py:147-151)."""
+        logits = gcn_c(x[all_nodes], [block_0 .. block_{H-1}]) (main.py:252-257, eval.py:147-151).  ``training``: the
+        hidden layer is dropped (modules/gcn.py:33); the logits are dropped by the training step's loss launch."""
         L = self.L
         H, F, D, C, B = self.H, self.F, self.D, self.C, self.bsz
         ovf = ptr(self.overflow)
@@ -616,8 +645,13 @@ class GrapesEngine:
         (L.grapes_aggregate_bf16 if self.x_bf16 else L.grapes_aggregate)(
                            ctx, X, F, self.ldx, ptr(self.all_nodes), A_dev, cap_A, ptr(self.cl_in_off[0]),
                            ptr(self.cl_in_src[0]), ptr(self.cl_dinv[0]), None, 0, None, 0, ptr(self.Yc), ldYc, None, None, -1, st)
-        L.grapes_gemm(ctx, 3, ptr(self.Yc), ldYc, self._par(nc.W1), F, ptr(self.out1), D, A_dev, cap_A, D, F,
-                      self._par(nc.b1), 1, None, 0, st)
+        if training and self.dropout > 0:
+            L.grapes_gemm_bias_relu_dropout(ctx, ptr(self.Yc), ldYc, self._par(nc.W1), F, ptr(self.out1), D, A_dev, cap_A,
+                                            D, F, self._par(nc.b1), ptr(self.drop_state), self._drop_tag(0),
+                                            self.drop_threshold, self.drop_scale, st)
+        else:
+            L.grapes_gemm(ctx, 3, ptr(self.Yc), ldYc, self._par(nc.W1), F, ptr(self.out1), D, A_dev, cap_A, D, F,
+                          self._par(nc.b1), 1, None, 0, st)
         L.grapes_gemm(ctx, 3, ptr(self.out1), D, self._par(nc.W2), D, ptr(self.Zc), C, A_dev, cap_A, C, D, None, 0,
                       None, 0, st)
         L.grapes_aggregate(ctx, ptr(self.Zc), C, C, None, A_dev, cap_A, ptr(self.cl_in_off[1]),
@@ -670,7 +704,7 @@ class GrapesEngine:
             L.grapes_bitmap_set(ctx, ptr(self.prev[h + 1]), self._hc(h + 1, "P"), cap_P, ptr(self.bm_prev[h + 1]), st)
             L.grapes_slice_block(ctx, rows, ptr(hw.e_row), ptr(hw.e_col), m_dev, cap_m, ptr(self.bm_prev[h + 1]),
                                  ptr(hw.blk_src), ptr(hw.blk_dst), self.cap_blk, self._hc(h, "blk"), ovf, st)
-        self._enqueue_classifier_forward(ctx, st)
+        self._enqueue_classifier_forward(ctx, st, training=False)          # evaluation never drops
         # predictions = argmax(logits)[node_map.map(target_nodes)]   (eval.py:152-153)
         L.grapes_argmax_rows(ctx, ptr(self.logits_c), self.C, self.C, ptr(self.target_local), self._cnt("B"), self.B,
                              pred_ptr, st)
@@ -1020,10 +1054,12 @@ class GrapesEngine:
                     # re-run: its reset already happened; every kernel has been launched by an earlier variant then)
                     flags, pf = list(self._front_ready), self._prefetch_next
                     rng = self.rng_state.clone()             # the warm-up must not consume the Philox stream
+                    drop = self.drop_state.clone()           # ... nor a dropout step
                     self._prefetch_next = False
                     self._enqueue(None, False)
                     torch.cuda.synchronize()
                     self.rng_state.copy_(rng)
+                    self.drop_state.copy_(drop)
                     self._front_ready, self._prefetch_next = flags, pf
                 gr = torch.cuda.CUDAGraph()
                 n0 = self.L.grapes_kernel_launches()
@@ -1105,7 +1141,20 @@ class GrapesEngine:
         A = self.count("A")
         out["all_nodes"] = self.all_nodes[:A].clone()
         out["target_local"] = self.target_local[:self.bsz].clone()
-        out["logits_c"] = self.logits_c[:A].clone()
+        out["logits_c"] = self.logits_c[:A].clone()          # after dropout (modules/gcn.py:37)
+        if self.dropout > 0:
+            # the step's masks, evaluated by the kernels' keep function at the step value the step used
+            seed, step = (int(v) for v in self.drop_state.tolist())
+            step -= 1
+            keep = []
+            for site, width in ((0, self.D), (1, self.C)):
+                k = torch.zeros((A, width), dtype=torch.uint8, device=self.device)
+                if A > 0:
+                    self.L.grapes_dropout_mask(self.g.ctx, seed, step, self._drop_tag(site), self.drop_threshold,
+                                               self._cnt("A"), A, width, ptr(k), torch.cuda.current_stream().cuda_stream)
+                keep.append(k.bool())
+            out["dropout_keep"], out["dropout_step"] = tuple(keep), step
+            out["hidden_c"] = self.out1[:A].clone()              # dropout(relu(layer 1))
         out["scalars"] = self.scalars()
         out["grads"] = {k: {n: t.clone() for n, t in v.items()} for k, v in self.grad_dicts().items()}
         if self.embed_nodes:

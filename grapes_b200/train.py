@@ -80,8 +80,6 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
         data.num_features = num_features = args.node_emb_dim
     if args.model_type != 'gcn':
         raise ValueError("only model_type='gcn' is wired in the reference's train() (main.py:109)")
-    if args.dropout != 0.:
-        raise NotImplementedError("dropout > 0 is not used by any reference config; use grapes_b200.gcn.GCN directly")
 
     # frontier capacity of the library context: a batch expands at most (B + k) rows of at most max_deg entries
     graph = DeviceGraph.from_edge_index(data.edge_index, data.num_nodes, device=device)
@@ -98,7 +96,8 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
                           use_indicators=args.use_indicators, hidden_dim=args.hidden_dim, lr_gc=args.lr_gc,
                           lr_gf=args.lr_gf, loss_coef=args.loss_coef, log_z_init=args.log_z_init,
                           reg_param=args.reg_param, random_sampling=args.random_sampling,
-                          reinforce_baseline=args.reinforce_baseline, seed=0 if args.seed is None else args.seed)
+                          reinforce_baseline=args.reinforce_baseline, seed=0 if args.seed is None else args.seed,
+                          dropout=args.dropout)                # gcn_c only (main.py:107-112); evaluation never drops
     if world > 1:
         engine.enable_data_parallel(exchange=exchange)
     train_idx = data.train_mask.nonzero().squeeze(1).to(device)

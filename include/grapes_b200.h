@@ -225,6 +225,21 @@ int grapes_vec_sum(grapes_ctx* ctx, const float* v, const int* n_dev, int cap_n,
 int grapes_gemm(grapes_ctx* ctx, int layout, const float* A, int lda, const float* B, int ldb, float* C, int ldc,
                 const int* M_dev, int M_cap, int N, int K, const float* bias, int relu, const float* relu_gate,
                 int ldg, void* stream);
+/* Dropout of the classifier's hidden layer, h = dropout(relu(A_hat_1 (x W1^T) + b1)) (modules/gcn.py:33).  Masks: the keep
+ * bit of entry (row, col) of a site of width w is a pure function of (seed, step, tag, row * w + col) -- Philox4x32-10 with
+ * counter (i / 4, tag, step), key = seed, keep iff the low 24 bits of word i % 4 are < threshold -- where
+ * drop_state = {seed, step} (device, 2 x uint64), tag = 1 + site + 2 * rank (site 0: hidden, 1: logits) and
+ * threshold = llrint((1 - p) * 2^24); kept entries are multiplied by scale = 1 / (1 - p) (0 when p == 1).
+ * H[M x N] = dropout(relu(A W^T + b)): A [M x K] and W [N x K] K-contiguous (grapes_gemm layout 3).                    */
+int grapes_gemm_bias_relu_dropout(grapes_ctx* ctx, const float* A, int lda, const float* W, int ldw, float* H, int ldh,
+                                  const int* M_dev, int M_cap, int N, int K, const float* bias,
+                                  unsigned long long* drop_state, uint32_t tag, uint32_t threshold, float scale,
+                                  void* stream);
+/* its backward (modules/gcn.py:33): C = (gate > 0) ? scale * (A B) : 0, A [M x K] K-contiguous, B [K x N] (layout 1); with
+ * gate = the dropped activations H this is d pre = (dZ W2) (.) relu' (.) keep * scale                                  */
+int grapes_gemm_gated_scaled(grapes_ctx* ctx, const float* A, int lda, const float* B, int ldb, float* C, int ldc,
+                             const int* M_dev, int M_cap, int N, int K, const float* gate, int ldg, float scale,
+                             void* stream);
 /* out[M x N] (+)= scale * A[R x M]^T B[R x N]  (weight gradients; deterministic split over rows)     */
 int grapes_gemm_tn(grapes_ctx* ctx, const float* A, int lda, const float* B, int ldb, const int* R_dev, int R_cap,
                    int M, int N, float scale, int accumulate, float* out, void* stream);
@@ -310,6 +325,19 @@ int grapes_classifier_loss(grapes_ctx* ctx, const float* logits, int ldl, int C,
                            const float* labels_f32, float reg_param, float* dlogits, float* loss_out,
                            float* colsum_out /* optional: column sums of dlogits = d loss / d last bias */,
                            void* stream);
+/* the same loss on dropout(logits) (modules/gcn.py:37; masks as grapes_gemm_bias_relu_dropout, site width C): `logits`
+ * holds the pre-dropout logits and receives the dropped ones in place; dlogits = d loss / d (pre-dropout logits), i.e.
+ * the gradient at the dropped logits times keep * scale; colsum_out its column sums.  Its last launch advances
+ * drop_state's step word by one: call it once per training step, after every other reader of the step's masks.   */
+int grapes_classifier_loss_dropout(grapes_ctx* ctx, float* logits, int ldl, int C, const int* A_dev, int A_cap,
+                                   const int* row_ids, const int* tgt_of_row, const int* targets, int B,
+                                   const int64_t* labels_i64, const float* labels_f32, float reg_param, float* dlogits,
+                                   float* loss_out, float* colsum_out, unsigned long long* drop_state, uint32_t tag,
+                                   uint32_t threshold, float scale, void* stream);
+/* keep[r * width + c] (0 / 1) = keep bit of entry (r, c) of a dropout site at (seed, step), r < *rows_dev
+ * (modules/gcn.py:33,37): the masks a training step drew, for inspection and replay                               */
+int grapes_dropout_mask(grapes_ctx* ctx, int64_t seed, int64_t step, uint32_t tag, uint32_t threshold,
+                        const int* rows_dev, int cap_rows, int width, uint8_t* keep, void* stream);
 /* out[i] = argmax_c logits[row_ids[i], c], i < *B_dev: predictions of the target rows (eval.py:152-153); ties -> lowest c */
 int grapes_argmax_rows(grapes_ctx* ctx, const float* logits, int ldl, int C, const int* row_ids, const int* B_dev,
                        int cap_B, int* out, void* stream);
