@@ -18,7 +18,6 @@ struct grapes_ctx {
     unsigned long long* scan_status;     // [scan_cap_tiles]
     unsigned int* scan_counters;         // [0] ticket, [1] done
     int scan_cap_tiles;
-    unsigned long long* hs_status;       // [2 * scan_cap_tiles] look-back words of the fused hop-structure kernel (rank | scan)
     // hub-row worklist for the per-row sort
     int* hub_rows;                       // [hub_cap]
     int* hub_count;                      // [1]

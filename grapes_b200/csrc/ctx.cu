@@ -63,7 +63,6 @@ int grapes_ctx_create(int device, int64_t num_nodes, int64_t max_frontier, int64
     c->partials_bytes = (size_t)(partials_bytes > (1 << 20) ? partials_bytes : (1 << 20));
     cudaError_t e;
     if ((e = cudaMalloc(&c->scan_status, sizeof(unsigned long long) * c->scan_cap_tiles)) != cudaSuccess ||
-        (e = cudaMalloc(&c->hs_status, sizeof(unsigned long long) * 2 * c->scan_cap_tiles)) != cudaSuccess ||
         (e = cudaMalloc(&c->scan_counters, sizeof(unsigned int) * 4)) != cudaSuccess ||
         (e = cudaMalloc(&c->hub_rows, sizeof(int) * c->hub_cap)) != cudaSuccess ||
         (e = cudaMalloc(&c->hub_count, sizeof(int))) != cudaSuccess ||
@@ -73,7 +72,6 @@ int grapes_ctx_create(int device, int64_t num_nodes, int64_t max_frontier, int64
         return GRAPES_ERR_NOMEM;
     }
     GRAPES_CUDA_OK(cudaMemset(c->scan_status, 0, sizeof(unsigned long long) * c->scan_cap_tiles));
-    GRAPES_CUDA_OK(cudaMemset(c->hs_status, 0, sizeof(unsigned long long) * 2 * c->scan_cap_tiles));
     GRAPES_CUDA_OK(cudaMemset(c->scan_counters, 0, sizeof(unsigned int) * 4));
     GRAPES_CUDA_OK(cudaMemset(c->hub_count, 0, sizeof(int)));
     *out = c;
@@ -83,7 +81,6 @@ int grapes_ctx_create(int device, int64_t num_nodes, int64_t max_frontier, int64
 int grapes_ctx_destroy(grapes_ctx* c) {
     if (!c) return GRAPES_OK;
     cudaFree(c->scan_status);
-    cudaFree(c->hs_status);
     cudaFree(c->scan_counters);
     cudaFree(c->hub_rows);
     cudaFree(c->hub_count);

@@ -7,11 +7,8 @@
 //   TensorMap.update / .map     /root/reference/modules/utils.py:98-120
 //   slice_adjacency             /root/reference/modules/utils.py:85-95
 // All outputs are bit-exact with those (ordering contracts in DESIGN.md section 3).
-#include <cooperative_groups.h>
-#include <cstdlib>
 #define GRAPES_PDL_GROUP 1
 #include "common.cuh"
-namespace cg = cooperative_groups;
 
 // ---------------------------------------------------------------------------------------
 // k_row_offsets: one block.  rows[P] -> row_off[P+1] (exclusive scan of CSR degrees), m.
@@ -418,221 +415,6 @@ __global__ void __launch_bounds__(256) k_sort_rows(const int* __restrict__ off, 
 }
 
 // ---------------------------------------------------------------------------------------
-// k_hop_structure: everything between the row expansion and the feature aggregation of a hop in ONE cooperative launch
-// (k_rank_scan -> k_edge_local -> k_scan_i32 -> k_fill -> k_sort_rows, same arithmetic, same outputs):
-//   phase 1  rank: single-pass scan over the node bitmap, id lists, indicator bits          (main.py:183-195)
-//   phase 2  relabel of the expanded edges + in-degree histogram                            (TensorMap.map, main.py:195)
-//   phase 3  exclusive scan of the histogram -> in_off, deg^-1/2                             (gcn_norm)
-//   phase 4  slot claim (dst-sorted CSR)          phase 5  ascending sources inside each row
-// Five dependent launches of ~1 us of work each cost ~5 us apiece (launch ramp + drain); a grid barrier costs ~1.5 us.
-// Tiles are assigned round-robin (tile = block, block + grid, ...): every block walks its tiles in increasing order and
-// all blocks are co-resident (cooperative launch), so the decoupled look-back never waits on an unscheduled tile.
-// Nothing produced inside the kernel is read through the read-only cache (no const __restrict__ on those arrays).
-// ---------------------------------------------------------------------------------------
-#define HS_THREADS 256
-struct HopStructArgs {
-    const uint32_t* bm_batch; const uint32_t* bm_prev; int W;
-    int* pref_batch; int* pref_nb; int* batch_nodes; int* nb_nodes; int* nb_local; int* nb_index;
-    uint32_t* ind_bits; uint32_t* bm_ind; int ind_rows; int hop; int cap_n; int* n_out; int* c_out; int* overflow;
-    const int* rows; const int* e_row; const int* e_col; const int* m_dev; int cap_m;
-    int* e_src; int* e_dst; int* cnt; int* in_off; int* in_src; int* tmp; float* dinv; int* nnz_out;
-    unsigned long long* status_a; unsigned long long* status_b;
-};
-
-__global__ void __launch_bounds__(HS_THREADS, 2) k_hop_structure(const HopStructArgs a) {
-    cg::grid_group grid = cg::this_grid();
-    __shared__ unsigned long long s_scan[HS_THREADS / 32 + 2];
-    __shared__ unsigned long long s_excl;
-    const int tid = threadIdx.x;
-    const int W = a.W, cap_n = a.cap_n, hop = a.hop, ind_rows = a.ind_rows;
-    const int gthreads = gridDim.x * HS_THREADS, gtid = blockIdx.x * HS_THREADS + tid;
-
-    // ---------------- phase 1: rank (k_rank_scan) ----------------
-    const int nt1 = (W + RANK_TILE - 1) / RANK_TILE;
-    for (int tile = blockIdx.x; tile < nt1; tile += gridDim.x) {
-        const int w0 = tile * RANK_TILE + tid * RANK_WPT;
-        uint32_t b[RANK_WPT], p[RANK_WPT];
-        unsigned long long mine = 0ull;
-#pragma unroll
-        for (int i = 0; i < RANK_WPT; ++i) {
-            const int w = w0 + i;
-            b[i] = (w < W) ? a.bm_batch[w] : 0u;
-            p[i] = (w < W && a.bm_prev) ? a.bm_prev[w] : 0u;
-            mine += ((unsigned long long)__popc(b[i]) << 31) | (unsigned long long)__popc(b[i] & ~p[i]);
-        }
-        uint32_t iw[RANK_WPT][8];
-        if (a.ind_bits) {
-#pragma unroll
-            for (int i = 0; i < RANK_WPT; ++i) {
-                const int w = w0 + i;
-#pragma unroll
-                for (int h = 0; h < 8; ++h) {
-                    iw[i][h] = 0u;
-                    if (b[i] && ((h < ind_rows - 1 && h < hop) || h == ind_rows - 1)) iw[i][h] = a.bm_ind[(size_t)h * W + w];
-                }
-            }
-        }
-        unsigned long long total;
-        const unsigned long long excl_in_tile = block_scan_excl<unsigned long long>(mine, s_scan, &total);
-        if (tid < 32) {
-            const unsigned long long ex = lb_exclusive(a.status_a, tile, total);
-            if (tid == 0) s_excl = ex;
-        }
-        __syncthreads();
-        const unsigned long long pre = s_excl + excl_in_tile;
-        int rb = (int)(pre >> 31), rn = (int)(pre & 0x7fffffffull);
-#pragma unroll
-        for (int i = 0; i < RANK_WPT; ++i) {
-            const int w = w0 + i;
-            if (w >= W) break;
-            a.pref_batch[w] = rb;
-            if (a.pref_nb) a.pref_nb[w] = rn;
-            uint32_t bits = b[i];
-            const uint32_t nbits = bits & ~p[i];
-            if (a.bm_ind) a.bm_ind[(size_t)hop * W + w] = nbits;
-            uint32_t ind_w[8];
-            if (a.ind_bits && bits) {
-#pragma unroll
-                for (int h = 0; h < 8; ++h) {
-                    ind_w[h] = iw[i][h];
-                    if (h == hop && h < ind_rows - 1) ind_w[h] = nbits;
-                }
-            }
-            while (bits) {
-                const int t = __ffs(bits) - 1;
-                bits &= bits - 1u;
-                const int v = (w << 5) + t;
-                const int j = rb++;
-                if (j < cap_n) {
-                    a.batch_nodes[j] = v;
-                    if (a.ind_bits) {
-                        uint32_t ib = 0u;
-#pragma unroll
-                        for (int h = 0; h < 8; ++h) ib |= ((ind_w[h] >> t) & 1u) << h;
-                        a.ind_bits[j] = ib;
-                    }
-                }
-                if ((nbits >> t) & 1u) {
-                    const int q = rn++;
-                    if (q < cap_n && a.nb_nodes) { a.nb_nodes[q] = v; a.nb_local[q] = min(j, cap_n - 1); }
-                    if (a.nb_index && j < cap_n) a.nb_index[j] = q < cap_n ? q : -1;
-                } else if (a.nb_index && j < cap_n) a.nb_index[j] = -1;
-            }
-        }
-        if (tile == nt1 - 1 && tid == HS_THREADS - 1) {
-            const unsigned long long tot = s_excl + total;
-            int n = (int)(tot >> 31), c = (int)(tot & 0x7fffffffull);
-            if (n > cap_n) { atomicOr(a.overflow, GRAPES_OVF_NODES); n = cap_n; if (c > cap_n) c = cap_n; }
-            *a.n_out = n;
-            if (a.c_out) *a.c_out = c;
-        }
-        __syncthreads();                                    // s_excl / s_scan are reused by the block's next tile
-    }
-    grid.sync();
-
-    // ---------------- phase 2: local ids of the expanded edges + in-degree histogram (k_edge_local) ----------------
-    const int m = *a.m_dev;
-    const int n = min(*(volatile int*)a.n_out, cap_n);
-    for (int e = gtid; e < m; e += gthreads) {
-        const int sg = a.rows[a.e_row[e]], dg = a.e_col[e];
-        int sl = a.pref_batch[sg >> 5] + __popc(a.bm_batch[sg >> 5] & ((1u << (sg & 31)) - 1u));
-        int dl = a.pref_batch[dg >> 5] + __popc(a.bm_batch[dg >> 5] & ((1u << (dg & 31)) - 1u));
-        if (sl >= cap_n || dl >= cap_n) sl = dl = 0;        // node capacity exceeded: dropped self-edge (see k_edge_local)
-        a.e_src[e] = sl;
-        a.e_dst[e] = dl;
-        if (sl != dl) atomicAdd(&a.cnt[dl], 1);
-    }
-    grid.sync();
-
-    // ---------------- phase 3: in_off = exclusive scan(cnt), deg^-1/2 (k_scan_i32) ----------------
-    const int nt3 = max((n + SCAN_TILE - 1) / SCAN_TILE, 1);
-    for (int tile = blockIdx.x; tile < nt3; tile += gridDim.x) {
-        const int i0 = tile * SCAN_TILE + tid * SCAN_IPT;
-        int v[SCAN_IPT];
-        unsigned long long mine = 0ull;
-#pragma unroll
-        for (int i = 0; i < SCAN_IPT; ++i) {
-            v[i] = (i0 + i < n) ? __ldcg(&a.cnt[i0 + i]) : 0;
-            mine += (unsigned long long)v[i];
-        }
-        unsigned long long total;
-        const unsigned long long excl_in_tile = block_scan_excl<unsigned long long>(mine, s_scan, &total);
-        if (tid < 32) {
-            const unsigned long long ex = lb_exclusive(a.status_b, tile, total);
-            if (tid == 0) s_excl = ex;
-        }
-        __syncthreads();
-        int run = (int)(s_excl + excl_in_tile);
-#pragma unroll
-        for (int i = 0; i < SCAN_IPT; ++i) {
-            const int idx = i0 + i;
-            if (idx < n) {
-                a.in_off[idx] = run;
-                a.dinv[idx] = 1.0f / sqrtf((float)(v[i] + 1));
-                run += v[i];
-            }
-        }
-        if (tile == nt3 - 1 && tid == HS_THREADS - 1) {
-            const int tot = (int)(s_excl + total);
-            a.in_off[n] = tot;
-            if (a.nnz_out) *a.nnz_out = tot;
-        }
-        __syncthreads();
-    }
-    grid.sync();
-
-    // ---------------- phase 4: slot claim, leaves cnt[] all-zero again (k_fill) ----------------
-    for (int e = gtid; e < m; e += gthreads) {
-        const int k = a.e_dst[e], v = a.e_src[e];
-        if (k != v) {
-            const int pos = __ldcg(&a.in_off[k]) + atomicSub(&a.cnt[k], 1) - 1;
-            a.in_src[pos] = v;
-        }
-    }
-    // look-back words back to zero for the next launch (every tile of both scans is long past its look-back)
-    for (int i = gtid; i < nt1; i += gthreads) a.status_a[i] = 0ull;
-    for (int i = gtid; i < nt3; i += gthreads) a.status_b[i] = 0ull;
-    grid.sync();
-
-    // ---------------- phase 5: ascending sources inside each row (k_sort_rows) ----------------
-    {
-        const int lane = lane_id();
-        const int warps = gthreads >> 5;
-        for (int j0 = (gtid >> 5) * 32; j0 < n; j0 += warps * 32) {
-            const int jr = j0 + lane;
-            const int len_l = (jr < n) ? __ldcg(&a.in_off[jr + 1]) - __ldcg(&a.in_off[jr]) : 0;
-            unsigned todo = __ballot_sync(GRAPES_FULL_MASK, len_l >= 2);
-            while (todo) {
-                const int t = __ffs(todo) - 1;
-                todo &= todo - 1u;
-                const int j = j0 + t;
-                const int beg = __ldcg(&a.in_off[j]), len = __ldcg(&a.in_off[j + 1]) - beg;
-                if (len <= 32) {
-                    const int x = (lane < len) ? __ldcg(&a.in_src[beg + lane]) : 0x7fffffff;
-                    int r = 0;
-                    for (int u = 0; u < len; ++u) {
-                        const int y = __shfl_sync(GRAPES_FULL_MASK, x, u);
-                        r += (y < x) || (y == x && u < lane);
-                    }
-                    __syncwarp();
-                    if (lane < len) a.in_src[beg + r] = x;
-                } else {
-                    for (int i = lane; i < len; i += 32) {
-                        const int x = __ldcg(&a.in_src[beg + i]);
-                        int r = 0;
-                        for (int u = 0; u < len; ++u) { const int y = __ldcg(&a.in_src[beg + u]); r += (y < x) || (y == x && u < i); }
-                        a.tmp[beg + r] = x;
-                    }
-                    __syncwarp();
-                    for (int i = lane; i < len; i += 32) a.in_src[beg + i] = __ldcg(&a.tmp[beg + i]);
-                }
-                __syncwarp();
-            }
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------
 // k_build_csr_small: the whole build (hist -> scan -> fill -> per-row sort -> deg^-1/2) in ONE 1024-thread CTA for
 // graphs with at most SMALL_N nodes (the classifier's sampled blocks: <= B + hops*k nodes, main.py:252-257).
 // ---------------------------------------------------------------------------------------
@@ -950,50 +732,6 @@ int grapes_rank_nodes(grapes_ctx* ctx, const uint32_t* bm_batch, const uint32_t*
         bm_ind, ind_rows, hop, cap_n, n_dev, c_dev, overflow, ctx->scan_status, ctx->scan_counters);
         grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
-    return GRAPES_OK;
-}
-
-int grapes_hop_structure(grapes_ctx* ctx, const uint32_t* bm_batch, const uint32_t* bm_prev, int* pref_batch, int* pref_nb,
-                         int* batch_nodes, int* nb_nodes, int* nb_local, int* nb_index, uint32_t* ind_bits,
-                         uint32_t* bm_ind, int ind_rows, int hop, int cap_n, int* n_dev, int* c_dev, const int* rows,
-                         const int* e_row, const int* e_col, const int* m_dev, int cap_m, int* e_src, int* e_dst,
-                         int* cnt_scratch, int* in_off, int* in_src, int* tmp_val, float* dinv, int* nnz_dev,
-                         int* overflow, void* stream) {
-    GRAPES_REQUIRE(ctx && bm_batch && pref_batch && batch_nodes && n_dev && rows && e_row && e_col && m_dev && e_src &&
-                       e_dst && cnt_scratch && in_off && in_src && tmp_val && dinv && overflow,
-                   "null argument");
-    GRAPES_REQUIRE(!nb_nodes || (nb_local && pref_nb && c_dev), "nb_nodes needs nb_local, pref_nb, c_dev");
-    GRAPES_REQUIRE(grapes_div_up(ctx->num_words, RANK_TILE) <= ctx->scan_cap_tiles &&
-                       grapes_div_up(cap_n, SCAN_TILE) + 1 <= ctx->scan_cap_tiles, "scan scratch too small");
-    HopStructArgs a;
-    a.bm_batch = bm_batch; a.bm_prev = bm_prev; a.W = ctx->num_words;
-    a.pref_batch = pref_batch; a.pref_nb = pref_nb; a.batch_nodes = batch_nodes; a.nb_nodes = nb_nodes;
-    a.nb_local = nb_local; a.nb_index = nb_index; a.ind_bits = ind_bits; a.bm_ind = bm_ind; a.ind_rows = ind_rows;
-    a.hop = hop; a.cap_n = cap_n; a.n_out = n_dev; a.c_out = c_dev; a.overflow = overflow;
-    a.rows = rows; a.e_row = e_row; a.e_col = e_col; a.m_dev = m_dev; a.cap_m = cap_m;
-    a.e_src = e_src; a.e_dst = e_dst; a.cnt = cnt_scratch; a.in_off = in_off; a.in_src = in_src; a.tmp = tmp_val;
-    a.dinv = dinv; a.nnz_out = nnz_dev;
-    a.status_a = ctx->hs_status; a.status_b = ctx->hs_status + ctx->scan_cap_tiles;
-    static int per_sm = -1;
-    if (per_sm < 0) {
-        int v = 0;
-        GRAPES_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, k_hop_structure, HS_THREADS, 0));
-        per_sm = v < 1 ? 1 : (v > 2 ? 2 : v);
-    }
-    cudaLaunchConfig_t cfg = {};
-    // a cooperative grid needs ALL its CTAs resident at once: a GPU-wide grid waits for every SM that a persistent tensor
-    // core kernel of a side branch holds, a small one slips in next to them (measured, DESIGN.md section 9)
-    static int want = -2;
-    if (want == -2) { const char* e = getenv("GRAPES_HS_CTAS"); want = e ? atoi(e) : 48; }
-    int nblk = ctx->sm_count * per_sm;
-    if (want > 0 && want < nblk) nblk = want;
-    cfg.gridDim = dim3((unsigned)nblk); cfg.blockDim = dim3(HS_THREADS);
-    cfg.dynamicSmemBytes = 0; cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeCooperative; at[0].val.cooperative = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    GRAPES_CUDA_OK(cudaLaunchKernelEx(&cfg, k_hop_structure, a));
-    grapes_count_launches(1);
     return GRAPES_OK;
 }
 

@@ -1038,12 +1038,17 @@ static int launch_gemm_dropout(grapes_ctx* ctx, const float* A, int lda, const f
 }
 
 static int g_agg_variant = 0;
-static int g_agg_min_rows = 4096;       // smallest row capacity that takes the multi-row / TMA-staged forms (aligned widths)
+#define AGG_MIN_ROWS 4096               // smallest row capacity that takes the multi-row / TMA-staged forms (aligned widths)
 
 extern "C" {
 
-int grapes_agg_variant(int v) { g_agg_variant = v; return 0; }
-int grapes_agg_tma_min_rows(int rows) { g_agg_min_rows = rows > 0 ? rows : 4096; return 0; }
+// 0 (default): the forms chosen by shape; 1: the register-staged kernels k_agg<4|2|1> only, the bit-exact reference
+// that the parity tests compare k_agg_tma with
+int grapes_agg_variant(int v) {
+    GRAPES_REQUIRE(v == 0 || v == 1, "aggregation variant is 0 (default) or 1 (register-staged)");
+    g_agg_variant = v;
+    return GRAPES_OK;
+}
 
 static int aggregate_impl(grapes_ctx* ctx, const void* Xv, int x_bf16, int F, int ldx, const int* nodes, const int* n_dev,
                           int cap_n, const int* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits,
@@ -1084,47 +1089,35 @@ static int aggregate_impl(grapes_ctx* ctx, const void* Xv, int x_bf16, int F, in
         GRAPES_LAUNCH_OK();
         return GRAPES_OK;
     }
-    if (a16 && (F % 4 != 0) && (ldx % 4 == 0) && ldx >= ((F + 3) & ~3) && (ldo % 4 == 0) && (ldo - F <= 32) && cap_n >= 256 &&
-        (g_agg_variant == 0 || g_agg_variant >= 100)) {
+    const bool shaped = g_agg_variant == 0;
+    const bool whole = cap_n > (1 << 19);
+    if (shaped && a16 && (F % 4 != 0) && (ldx % 4 == 0) && ldx >= ((F + 3) & ~3) && (ldo % 4 == 0) && (ldo - F <= 32) &&
+        cap_n >= 256) {
         // rows whose width is not a multiple of 4 (Reddit 602, Cora 1433) on a table with a padded row pitch: TMA-staged
-        // form with a partial last feature lane
-        const int v = g_agg_variant ? g_agg_variant : (cap_n > (1 << 19) ? 132 : 216);   // Reddit-shape hop: 2 CTAs/SM 0.236, 1 CTA/SM 0.272 ms/step
+        // form with a partial last feature lane.  Reddit-shape hop: 2 CTAs/SM 0.236, 1 CTA/SM 0.272 ms/step
         if (grapes_launch_agg_tma(ctx, X, 0, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias, relu,
-                                  out, ldo, out_hi, out_lo, ones_col, v % 100, v / 100, s) == 0) {
+                                  out, ldo, out_hi, out_lo, ones_col, whole ? 32 : 16, whole ? 1 : 2, s) == 0) {
             grapes_count_launches(1);
             GRAPES_LAUNCH_OK();
             return GRAPES_OK;
         }
     }
-    if (a16 && (F % 4 == 0) && (ldx % 4 == 0) && (ldo % 4 == 0) && (ldo - F <= 32) && cap_n >= g_agg_min_rows) {
-        // frontier-sized: R rows per warp with interleaved load chains (variant chosen by grapes_agg_variant, default 0)
-#define AGG_LAUNCH(RR, MB)                                                                                              \
-    pdl((k_agg_rows<RR, MB>), grid_for(ctx, (long long)grapes_div_up(cap_n, RR) * 32, 256, MB), 256, 0, s)(                 \
-        X, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias, relu, out, ldo, out_hi, out_lo,  \
-        ones_col)
-        // default: rows staged by TMA bulk copies (spmm_tma.cu).  Measured on B200 (scripts/bench_spmm.py): frontier-sized
-        // launches are best with 8-entry chunks and 3 CTAs/SM (ncu: 21.8 us against 23.3 at 2 CTAs/SM, 24.6 at 4), whole-graph launches
-        // with 32-entry chunks and 1 CTA/SM.
-        // grapes_agg_variant: 100 + ec / 200 + ec force a shape, 1..6 select the register-staged kernels.
-        if (g_agg_variant == 0 || g_agg_variant >= 100) {
-            const int v = g_agg_variant ? g_agg_variant : (cap_n > (1 << 19) ? 132 : (F > 256 ? 216 : 308));   // wide rows: 2 CTAs per SM
-            if (grapes_launch_agg_tma(ctx, X, 0, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias,
-                                      relu, out, ldo, out_hi, out_lo, ones_col, v % 100, v / 100, s) == 0) {
-                grapes_count_launches(1);
-                GRAPES_LAUNCH_OK();
-                return GRAPES_OK;
-            }
+    if (shaped && a16 && (F % 4 == 0) && (ldx % 4 == 0) && (ldo % 4 == 0) && (ldo - F <= 32) && cap_n >= AGG_MIN_ROWS) {
+        // rows staged by TMA bulk copies (spmm_tma.cu).  Measured on B200 (scripts/bench_spmm.py): frontier-sized
+        // launches are best with 8-entry chunks and 3 CTAs/SM (ncu: 21.8 us against 23.3 at 2 CTAs/SM, 24.6 at 4), wide
+        // rows with 2 CTAs/SM, whole-graph launches with 32-entry chunks and 1 CTA/SM.
+        const int ec = whole ? 32 : (F > 256 ? 16 : 8), cps = whole ? 1 : (F > 256 ? 2 : 3);
+        if (grapes_launch_agg_tma(ctx, X, 0, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias, relu,
+                                  out, ldo, out_hi, out_lo, ones_col, ec, cps, s) == 0) {
+            grapes_count_launches(1);
+            GRAPES_LAUNCH_OK();
+            return GRAPES_OK;
         }
-        switch (g_agg_variant) {
-            case 1: pdl((k_agg<4>), blocks, 256, 0, s)(X, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind,
-                                                    bias, relu, out, ldo, out_hi, out_lo, ones_col); break;
-            case 2: AGG_LAUNCH(2, 6); break;
-            case 3: AGG_LAUNCH(2, 4); break;
-            case 4: AGG_LAUNCH(4, 3); break;
-            case 5: AGG_LAUNCH(4, 2); break;
-            case 6: AGG_LAUNCH(4, 4); break;
-            default: AGG_LAUNCH(2, 4); break;      // best register-staged form (products-shaped hop, 65k rows): 2 rows per warp
-        }
+        // shapes k_agg_tma does not cover: 2 rows per warp with interleaved load chains, the best register-staged form
+        // (products-shaped hop, 65k rows)
+        pdl((k_agg_rows<2, 4>), grid_for(ctx, (long long)grapes_div_up(cap_n, 2) * 32, 256, 4), 256, 0, s)(
+            X, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias, relu, out, ldo, out_hi, out_lo,
+            ones_col);
     } else if (a16 && (F % 4 == 0) && (ldx % 4 == 0) && (ldo % 4 == 0))
         pdl((k_agg<4>), blocks, 256, 0, s)(X, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias,
                                         relu, out, ldo, out_hi, out_lo, ones_col);

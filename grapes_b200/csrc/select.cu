@@ -3,31 +3,17 @@
 // (/root/reference/modules/utils.py:13-71) and the deterministic top-k of the mini-batch evaluator
 // (/root/reference/eval.py:126-130), without the per-hop D2H of the mask (utils.py:60).
 //
-// Two kernels:
-//   k_logits_keys (GPU-wide)   layer-2 aggregation of the sampler net -> logits (main.py:210-213); for every
-//                 candidate the probability, Gumbel noise and perturbed key (utils.py:37-42) as an
-//                 order-preserving uint32, the log-probability / gradient of the UNSELECTED outcome, entropy
-//                 statistics (per-block partials, combined later in a fixed order), and a 2048-bucket histogram
-//                 of a monotone coarse image of the key (uniform 1/32-wide buckets on [-32, 32)).
-//   k_select      (one 8-CTA cluster)  exact k-th largest key: the bucket holding the threshold comes from the
-//                 histogram, its (few) members are gathered into CTA 0's shared memory through DSMEM and ranked
-//                 exactly on the composite (key, lowest index first); every CTA then marks its selected items,
-//                 fixes their log-probability / gradient, and writes them in ascending order.  If the bucket is too
-//                 crowded (massive ties) an MSB-first radix select on the 64-bit composite finds the same threshold.
+// One kernel, k_select_fused, does the whole hop on every SM: layer-2 aggregation of the sampler net -> logits
+// (main.py:210-213), the perturbed keys (utils.py:37-42) as order-preserving uint32, a 2048-bucket histogram of a
+// monotone coarse image of the keys, the exact k-th largest key, and the selected items in ascending order with their
+// log-probability / gradient and the entropy statistics.
 // Ties at the threshold go to the LOWEST candidate index (torch.topk leaves ties unspecified; the oracle uses
 // the same rule).  Integer counting only -> the selected set does not depend on scheduling.
-#include <cooperative_groups.h>
-
 #define GRAPES_PDL_GROUP 16
 #include "common.cuh"
-namespace cg = cooperative_groups;
 
-#define SEL_THREADS 1024
-#define SEL_WARPS (SEL_THREADS / 32)
-#define SEL_CTAS 8
 #define SEL_BUCKETS 2048
-#define SEL_MEMBER_CAP 2048
-#define SEL_STAT_FLOATS 8            // per-block partials of k_logits_keys: min p, max p, sum e, sum e^2, sum lp, sum dl
+#define SEL_STAT_FLOATS 8            // per-block partials: min p, max p, sum e, sum e^2, sum lp, sum dl
 
 __device__ __forceinline__ uint32_t float_to_ordered(float f) {
     if (f != f) return 0u;                                   // NaN ranks lowest
@@ -36,12 +22,6 @@ __device__ __forceinline__ uint32_t float_to_ordered(float f) {
 }
 __device__ __forceinline__ float ordered_to_float(uint32_t u) {
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
-}
-// monotone non-decreasing coarse image of a key: uniform buckets of width 1/32 on [-32, 32), clamped
-__device__ __forceinline__ int key_bucket(uint32_t ukey) {
-    if (ukey == 0u) return 0;                                // NaN
-    const float x = (ordered_to_float(ukey) + 32.0f) * 32.0f;
-    return (int)fminf(fmaxf(x, 0.f), (float)(SEL_BUCKETS - 1));
 }
 __device__ __forceinline__ unsigned long long composite(uint32_t ukey, int idx) {
     return ((unsigned long long)ukey << 32) | (unsigned long long)(0xffffffffu - (uint32_t)idx);
@@ -79,398 +59,7 @@ struct OpMin { __device__ float operator()(float a, float b) const { return fmin
 struct OpMax { __device__ float operator()(float a, float b) const { return fmaxf(a, b); } };
 
 // ---------------------------------------------------------------------------------------
-// k_logits_keys: one thread per frontier row j.
-//   aggregated mode (in_off != nullptr):  logit[j] = dinv[j]^2 z[j] + sum_s dinv[s] dinv[j] z[s] + bias
-//                                         (layer 2 of the sampler GCN at width 1; z may come as `nparts` partials)
-//   direct mode     (in_off == nullptr):  logit[j] = z[j]
-//   i = nb_index[j] (candidate index, -1 = not a candidate; nullptr = identity).  For candidates:
-//   lg_c[i] = logit, ukeys[i] = ordered(key), keys_out[i] = key, bucket histogram, statistics of p = sigmoid(logit),
-//   log_prob[i] / dl_all[j] / mask_out[i] of the UNSELECTED outcome (selected outcome when k >= c: everything is kept).
-// stat_part[block][8] = (min p, max p, sum entropy, sum entropy^2, sum log_prob, sum dl) of the block's candidates.
-// ---------------------------------------------------------------------------------------
-#define KEYS_THREADS 256
-__global__ void __launch_bounds__(KEYS_THREADS) k_logits_keys(
-    const float* __restrict__ z, int nparts, int part_stride, const int* __restrict__ n_dev, int cap_n,
-    const int* __restrict__ in_off, const int* __restrict__ in_src, const float* __restrict__ dinv,
-    const float* __restrict__ bias, const int* __restrict__ nb_index, const int* __restrict__ c_dev, int k, int mode,
-    const float* __restrict__ noise, const unsigned long long* __restrict__ rng_state,
-    float* __restrict__ logits_all, float* __restrict__ lg_c, uint32_t* __restrict__ ukeys,
-    float* __restrict__ keys_out, float* __restrict__ log_prob, float* __restrict__ dl_all,
-    uint8_t* __restrict__ mask_out, float* __restrict__ stat_part) {
-    pdl_begin();
-    __shared__ float s_red[KEYS_THREADS / 32];
-    const int n = min(*n_dev, cap_n);
-    const bool take_all = (k >= min(*c_dev, cap_n));          // utils.py:31-33: no noise is drawn
-    unsigned long long seed = 0ull, offset = 0ull;
-    if (mode == GRAPES_NOISE_PHILOX) { seed = rng_state[0]; offset = rng_state[1]; }
-    const float b = bias ? bias[0] : 0.f;
-    float pmin = INFINITY, pmax = -INFINITY, esum = 0.f, esq = 0.f, lpsum = 0.f, dlsum = 0.f;
-    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
-        float logit;
-        if (in_off) {
-            const float dj = dinv[j];
-            float zj = z[j];
-            for (int t = 1; t < nparts; ++t) zj += z[(size_t)t * part_stride + j];
-            float a = dj * dj * zj;
-            const int end = in_off[j + 1];
-            for (int p = in_off[j]; p < end; ++p) {
-                const int sl = in_src[p];
-                float zs = z[sl];
-                for (int t = 1; t < nparts; ++t) zs += z[(size_t)t * part_stride + sl];
-                a = fmaf(dinv[sl] * dj, zs, a);
-            }
-            logit = a + b;
-        } else {
-            logit = z[j];
-        }
-        if (logits_all) logits_all[j] = logit;
-        const int i = nb_index ? nb_index[j] : j;
-        if (i < 0) {
-            if (dl_all) dl_all[j] = 0.f;
-            continue;
-        }
-        lg_c[i] = logit;
-        const float p = sigmoidf_(logit);
-        const float y = take_all ? 1.f : 0.f;
-        const float lp = bern_log_prob(logit, y);
-        const float d = y - p;
-        if (log_prob) log_prob[i] = lp;
-        if (dl_all) dl_all[j] = d;
-        if (mask_out) mask_out[i] = take_all ? 1 : 0;
-        lpsum += lp; dlsum += d;
-        if (take_all) continue;
-        float key;
-        if (mode == GRAPES_NOISE_KEYS) key = noise[i];
-        else if (mode == GRAPES_NOISE_NONE_TOPK_PROBS) key = p;               // eval.py:126
-        else {
-            float g;
-            if (mode == GRAPES_NOISE_GUMBEL) g = noise[i];
-            else {
-                float u = (mode == GRAPES_NOISE_UNIFORM) ? noise[i] : philox_uniform(seed, offset, i);
-                if (mode == GRAPES_NOISE_PHILOX) u = u * ((1.0f - 1.1920929e-07f) - 1.17549435e-38f) + 1.17549435e-38f;
-                g = -logf(-logf(u));
-            }
-            key = logf(p) + g;                                                // utils.py:42
-        }
-        const uint32_t uk = float_to_ordered(key);
-        ukeys[i] = uk;
-        if (keys_out) keys_out[i] = key;
-        pmin = fminf(pmin, p); pmax = fmaxf(pmax, p);
-        const float e = entropy_bits(p);
-        esum += e; esq = fmaf(e, e, esq);
-    }
-    pmin = block_reduce<float, OpMin, KEYS_THREADS / 32>(pmin, s_red, OpMin(), INFINITY);
-    pmax = block_reduce<float, OpMax, KEYS_THREADS / 32>(pmax, s_red, OpMax(), -INFINITY);
-    esum = block_reduce<float, OpAdd, KEYS_THREADS / 32>(esum, s_red, OpAdd(), 0.f);
-    esq = block_reduce<float, OpAdd, KEYS_THREADS / 32>(esq, s_red, OpAdd(), 0.f);
-    lpsum = block_reduce<float, OpAdd, KEYS_THREADS / 32>(lpsum, s_red, OpAdd(), 0.f);
-    dlsum = block_reduce<float, OpAdd, KEYS_THREADS / 32>(dlsum, s_red, OpAdd(), 0.f);
-    if (threadIdx.x == 0) {
-        float* sp = stat_part + (size_t)blockIdx.x * SEL_STAT_FLOATS;
-        sp[0] = pmin; sp[1] = pmax; sp[2] = esum; sp[3] = esq; sp[4] = lpsum; sp[5] = dlsum; sp[6] = 0.f; sp[7] = 0.f;
-    }
-}
-
-// ---------------------------------------------------------------------------------------
-// k_select
-// ---------------------------------------------------------------------------------------
-// phase time stamps of the last k_select launch (globaltimer ns, CTA 0 thread 0) -- scripts/bench_select.py
-__device__ unsigned long long g_sel_stamps[16];
-__device__ __forceinline__ void sel_stamp(int slot, int rank) {
-    if (threadIdx.x == 0 && rank == 0) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        g_sel_stamps[slot] = t;
-    }
-}
-
-#define SEL_LOCAL_CAP 256            // members of the threshold bucket one CTA may hold before the radix fallback
-
-struct SelShared {
-    int hist[SEL_BUCKETS];                       // this CTA's bucket histogram
-    int coarse[64];                              // sums of 32 consecutive buckets
-    unsigned long long member[SEL_LOCAL_CAP];    // this CTA's members of the threshold bucket (composites)
-    int m_count;
-    // every CTA publishes its totals to all
-    int sel_count[SEL_CTAS];
-    float lp_delta[SEL_CTAS], dl_delta[SEL_CTAS];
-    // fallback radix select (CTA 0 holds the cluster-wide state)
-    int rhist[256];
-    unsigned long long prefix;
-    int kr;
-};
-
-__global__ void __cluster_dims__(SEL_CTAS, 1, 1) __launch_bounds__(SEL_THREADS, 1) k_select(
-    const uint32_t* __restrict__ ukeys, const float* __restrict__ lg_c, const int* __restrict__ nb_local,
-    const int* __restrict__ nb_nodes, const int* __restrict__ c_dev, int cap_c, int k, int mode,
-    unsigned long long* rng_state, const float* __restrict__ stat_part, int nstat, int staged,
-    int* __restrict__ sampled_out, int sampled_offset, int* __restrict__ s_dev, int* __restrict__ total_dev,
-    uint8_t* __restrict__ mask_out, float* __restrict__ log_prob, float* tot_log_prob, float* __restrict__ stats,
-    float* __restrict__ dl_all, float* sum_dl, uint32_t* bm_mark) {
-    pdl_begin();
-    cg::cluster_group cluster = cg::this_cluster();
-    const int rank = (int)cluster.block_rank();
-    __shared__ SelShared sh;
-    __shared__ float s_red[SEL_WARPS];
-    __shared__ long long s_scan[SEL_WARPS + 2];
-    __shared__ int s_wcnt[SEL_THREADS];              // per (round, warp) selected counts of one super-round
-    __shared__ int s_x[SEL_CTAS][64];                // exchanged coarse / fine counts
-    __shared__ unsigned long long s_all[SEL_CTAS * SEL_LOCAL_CAP];   // every CTA's members, gathered locally
-    __shared__ int s_lhist[256];
-    __shared__ int s_cb, s_above_c, s_bucket, s_above, s_fb;
-    __shared__ unsigned long long s_thr;
-    extern __shared__ uint32_t s_keys[];             // staged: this CTA's keys
-    SelShared* sh0 = cluster.map_shared_rank(&sh, 0);
-    const int c = min(*c_dev, cap_c);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const bool take_all = (k >= c);
-    const int chunk = (c + SEL_CTAS - 1) / SEL_CTAS;
-    const int cb = min(c, rank * chunk), ce = min(c, cb + chunk);
-    const int len = ce - cb;                         // CTA r owns the contiguous candidates [cb, ce)
-#define KEY(q) (staged ? s_keys[q] : ukeys[cb + (q)])
-    sel_stamp(0, rank);
-    if (tid == 0) { sh.m_count = 0; sh.kr = k; sh.prefix = 0ull; s_fb = 0; }
-    if (tid < 256) sh.rhist[tid] = 0;
-
-    unsigned long long thr_comp = 0ull;              // take_all: everything is selected
-    if (!take_all) {
-        // ---- 1. this CTA's bucket histogram (keys staged in shared memory on the way) ----
-        for (int b = tid; b < SEL_BUCKETS; b += SEL_THREADS) sh.hist[b] = 0;
-        __syncthreads();
-        for (int q0 = 0; q0 < len; q0 += 8 * SEL_THREADS) {
-            uint32_t v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) { const int q = q0 + u * SEL_THREADS + tid; v[u] = (q < len) ? ukeys[cb + q] : 0u; }
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int q = q0 + u * SEL_THREADS + tid;
-                if (q < len) { if (staged) s_keys[q] = v[u]; atomicAdd(&sh.hist[key_bucket(v[u])], 1); }
-            }
-        }
-        __syncthreads();
-        for (int cbn = warp; cbn < 64; cbn += SEL_WARPS) {
-            const int t = warp_sum(sh.hist[cbn * 32 + lane]);
-            if (lane == 0) sh.coarse[cbn] = t;
-        }
-        cluster.sync();                              // all 8 histograms complete and visible
-        sel_stamp(1, rank);
-        // ---- 2. threshold bucket: coarse level, then the 32 buckets inside it (every CTA, redundantly) ----
-        if (tid < SEL_CTAS * 64) s_x[tid >> 6][tid & 63] = cluster.map_shared_rank(sh.coarse, tid >> 6)[tid & 63];
-        __syncthreads();
-        if (warp == 0) {                             // lane l owns coarse bins 63-2l, 62-2l (descending)
-            int t0 = 0, t1 = 0;
-#pragma unroll
-            for (int r = 0; r < SEL_CTAS; ++r) { t0 += s_x[r][63 - 2 * lane]; t1 += s_x[r][62 - 2 * lane]; }
-            const int incl = warp_scan_incl(t0 + t1), excl = incl - (t0 + t1);
-            if (excl < k && excl + t0 >= k) { s_cb = 63 - 2 * lane; s_above_c = excl; }
-            else if (excl + t0 < k && incl >= k) { s_cb = 62 - 2 * lane; s_above_c = excl + t0; }
-        }
-        __syncthreads();
-        const int cbin = s_cb;
-        if (tid < SEL_CTAS * 32) s_x[tid >> 5][tid & 31] = cluster.map_shared_rank(sh.hist, tid >> 5)[cbin * 32 + (tid & 31)];
-        __syncthreads();
-        if (warp == 0) {                             // lane l owns bucket 31-l of the coarse bin (descending)
-            int t = 0;
-#pragma unroll
-            for (int r = 0; r < SEL_CTAS; ++r) t += s_x[r][31 - lane];
-            const int incl = warp_scan_incl(t), excl = incl - t;
-            const int krem = k - s_above_c;
-            if (excl < krem && incl >= krem) { s_bucket = cbin * 32 + 31 - lane; s_above = s_above_c + excl; }
-        }
-        __syncthreads();
-        const int bucket = s_bucket, above = s_above;
-        // ---- 3. members of the threshold bucket: local list, then every CTA gathers all 8 lists and ranks exactly
-        //         on the composite (key desc, index asc) ----
-        for (int q = tid; q < len; q += SEL_THREADS) {
-            const uint32_t u = KEY(q);
-            if (key_bucket(u) == bucket) {
-                const int pos = atomicAdd(&sh.m_count, 1);
-                if (pos < SEL_LOCAL_CAP) sh.member[pos] = composite(u, cb + q);
-            }
-        }
-        cluster.sync();
-        sel_stamp(2, rank);
-        int M = 0;
-        bool crowded = false;
-        int mbase[SEL_CTAS + 1];
-        mbase[0] = 0;
-#pragma unroll
-        for (int r = 0; r < SEL_CTAS; ++r) {
-            const int mr = cluster.map_shared_rank(&sh, r)->m_count;
-            crowded |= (mr > SEL_LOCAL_CAP);
-            mbase[r + 1] = mbase[r] + min(mr, SEL_LOCAL_CAP);
-        }
-        M = mbase[SEL_CTAS];
-        if (!crowded) {
-            for (int t = tid; t < M; t += SEL_THREADS) {
-                int r = 0;
-#pragma unroll
-                for (int rr = 1; rr < SEL_CTAS; ++rr) r += (t >= mbase[rr]);
-                s_all[t] = cluster.map_shared_rank(&sh, r)->member[t - mbase[r]];
-            }
-            __syncthreads();
-            const int want = k - above - 1;          // members that must rank above the threshold member
-            for (int t = tid; t < M; t += SEL_THREADS) {
-                const unsigned long long mine = s_all[t];
-                int r = 0;
-                for (int o = 0; o < M; ++o) r += (s_all[o] > mine);
-                if (r == want) s_thr = mine;
-            }
-            __syncthreads();
-            thr_comp = s_thr;
-        } else {
-            // ---- fallback (crowded bucket, e.g. massive ties): MSB-first radix select on the 64-bit composite,
-            //      8 passes of 8 bits over all candidates, histograms merged into CTA 0 with DSMEM atomics ----
-            for (int shift = 56; shift >= 0; shift -= 8) {
-                __syncthreads();
-                if (tid < 256) s_lhist[tid] = 0;
-                if (tid == 0) s_thr = sh0->prefix;
-                __syncthreads();
-                const unsigned long long prefix = s_thr;
-                const unsigned long long himask = (shift == 56) ? 0ull : (~0ull << (shift + 8));
-                for (int q = tid; q < len; q += SEL_THREADS) {
-                    const unsigned long long cm = composite(KEY(q), cb + q);
-                    if ((cm & himask) == prefix) atomicAdd(&s_lhist[(int)((cm >> shift) & 255ull)], 1);
-                }
-                __syncthreads();
-                if (tid < 256 && s_lhist[tid]) atomicAdd(&sh0->rhist[tid], s_lhist[tid]);
-                cluster.sync();
-                if (rank == 0 && tid == 0) {
-                    int cum = 0;
-                    const int krem = sh.kr;
-                    for (int bin = 255; bin >= 0; --bin) {
-                        const int hcount = sh.rhist[bin];
-                        if (cum + hcount >= krem) {
-                            sh.prefix = prefix | ((unsigned long long)bin << shift);
-                            sh.kr = krem - cum;
-                            break;
-                        }
-                        cum += hcount;
-                    }
-                    for (int bin = 0; bin < 256; ++bin) sh.rhist[bin] = 0;
-                }
-                cluster.sync();
-            }
-            if (tid == 0) s_thr = sh0->prefix;
-            __syncthreads();
-            thr_comp = s_thr;                        // the k-th largest composite itself (composites are distinct)
-        }
-    } else {
-        cluster.sync();                              // every CTA runs before the first remote access below
-    }
-    sel_stamp(3, rank);
-
-    // ---- 4. count the selected items of this CTA; fix their log-prob / gradient (k_logits_keys wrote the
-    //         unselected outcome) ----
-    int my_cnt = 0;
-    float lp_delta = 0.f, dl_delta = 0.f;
-    if (!take_all) {
-        for (int q = tid; q < len; q += SEL_THREADS) {
-            if (composite(KEY(q), cb + q) >= thr_comp) {
-                const int i = cb + q;
-                ++my_cnt;
-                const float l = lg_c[i];
-                const float lp1 = bern_log_prob(l, 1.f), lp0 = bern_log_prob(l, 0.f);
-                if (log_prob) log_prob[i] = lp1;
-                if (dl_all) dl_all[nb_local ? nb_local[i] : i] = 1.f - sigmoidf_(l);
-                if (mask_out) mask_out[i] = 1;
-                lp_delta += lp1 - lp0;
-                dl_delta += 1.f;
-            }
-        }
-    }
-    long long total;
-    block_scan_excl<long long>((long long)my_cnt, s_scan, &total);
-    lp_delta = block_reduce<float, OpAdd, SEL_WARPS>(lp_delta, s_red, OpAdd(), 0.f);
-    dl_delta = block_reduce<float, OpAdd, SEL_WARPS>(dl_delta, s_red, OpAdd(), 0.f);
-    if (tid < SEL_CTAS) {                            // publish to every CTA: after the barrier each reads only its own copy
-        SelShared* dst = cluster.map_shared_rank(&sh, tid);
-        dst->sel_count[rank] = take_all ? len : (int)total;
-        dst->lp_delta[rank] = lp_delta;
-        dst->dl_delta[rank] = dl_delta;
-    }
-    cluster.sync();                                  // after this nobody touches remote shared memory
-    sel_stamp(4, rank);
-    int carry = 0;                                   // selected items in lower-ranked CTAs
-    for (int r = 0; r < rank; ++r) carry += sh.sel_count[r];
-
-    // ---- 5. ordered output: position = #selected with a smaller index (ballot per 32 items + one scan per
-    //         super-round of 32 x 1024 items) ----
-    for (int sr = 0; sr < len; sr += 32 * SEL_THREADS) {
-        const int rounds = min(32, (len - sr + SEL_THREADS - 1) / SEL_THREADS);
-        for (int u = 0; u < rounds; ++u) {           // pass a: flags -> per (round, warp) counts
-            const int q = sr + u * SEL_THREADS + tid;
-            bool sel = false;
-            if (q < len) sel = take_all || composite(KEY(q), cb + q) >= thr_comp;
-            const uint32_t bal = __ballot_sync(GRAPES_FULL_MASK, sel);
-            if (lane == 0) s_wcnt[u * 32 + warp] = __popc(bal);
-        }
-        if (tid >= rounds * 32) s_wcnt[tid] = 0;
-        __syncthreads();
-        long long tot2;
-        const int base = (int)block_scan_excl<long long>((long long)s_wcnt[tid], s_scan, &tot2);
-        s_wcnt[tid] = base;                          // exclusive prefix of (round, warp) in index order
-        __syncthreads();
-        for (int u = 0; u < rounds; ++u) {           // pass b: positions
-            const int q = sr + u * SEL_THREADS + tid;
-            bool sel = false;
-            if (q < len) sel = take_all || composite(KEY(q), cb + q) >= thr_comp;
-            const uint32_t bal = __ballot_sync(GRAPES_FULL_MASK, sel);
-            if (sel) {
-                const int i = cb + q;
-                const int pos = carry + s_wcnt[u * 32 + warp] + __popc(bal & ((1u << lane) - 1u));
-                const int g = nb_nodes ? nb_nodes[i] : i;
-                if (sampled_out) sampled_out[sampled_offset + pos] = g;
-                if (bm_mark && nb_nodes) bitmap_set(bm_mark, g);
-            }
-        }
-        carry += (int)tot2;
-        __syncthreads();
-    }
-    sel_stamp(5, rank);
-    if (rank != 0) return;
-    if (tid < 32) {
-        // statistics / sums: per-block partials of k_logits_keys combined in a fixed order
-        float mn = INFINITY, mx = -INFINITY;
-        double es = 0.0, eq = 0.0, lp = 0.0, dl = 0.0;
-        for (int bq = tid; bq < nstat; bq += 32) {
-            const float* p = stat_part + (size_t)bq * SEL_STAT_FLOATS;
-            mn = fminf(mn, p[0]); mx = fmaxf(mx, p[1]); es += (double)p[2]; eq += (double)p[3];
-            lp += (double)p[4]; dl += (double)p[5];
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            mn = fminf(mn, __shfl_xor_sync(GRAPES_FULL_MASK, mn, o));
-            mx = fmaxf(mx, __shfl_xor_sync(GRAPES_FULL_MASK, mx, o));
-            es += __shfl_xor_sync(GRAPES_FULL_MASK, es, o);
-            eq += __shfl_xor_sync(GRAPES_FULL_MASK, eq, o);
-            lp += __shfl_xor_sync(GRAPES_FULL_MASK, lp, o);
-            dl += __shfl_xor_sync(GRAPES_FULL_MASK, dl, o);
-        }
-        if (tid == 0) {
-            for (int r = 0; r < SEL_CTAS; ++r) { lp += (double)sh.lp_delta[r]; dl += (double)sh.dl_delta[r]; }   // fixed order
-            const int s = take_all ? c : k;
-            if (s_dev) *s_dev = s;
-            if (total_dev) *total_dev = sampled_offset + s;
-            if (tot_log_prob) *tot_log_prob += (float)lp;
-            if (sum_dl) *sum_dl += (float)dl;
-            if (stats) {
-                if (take_all) { stats[0] = stats[1] = stats[2] = stats[3] = 0.f; }   // reference returns {}
-                else {
-                    const double mean = (c > 0) ? es / (double)c : 0.0;
-                    const double var = (c > 1) ? fmax(0.0, (eq - (double)c * mean * mean) / (double)(c - 1)) : 0.0;
-                    stats[0] = mn; stats[1] = mx; stats[2] = (float)mean; stats[3] = (float)sqrt(var);   // unbiased (utils.py:56)
-                }
-            }
-            if (mode == GRAPES_NOISE_PHILOX && !take_all) rng_state[1] += 1ull;
-            sel_stamp(6, 0);
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------
-// k_select_fused: the whole sampler head of a hop in ONE launch on every SM (replaces k_logits_keys + the one-cluster
-// k_select on the critical path of the step):
+// k_select_fused: the whole sampler head of a hop in ONE launch on every SM:
 //   phase A  (all blocks; block b owns a contiguous range of frontier rows, hence of candidates)  layer-2 aggregation
 //            -> logits, probabilities, noise, perturbed keys, log-prob / gradient of the UNSELECTED outcome, statistic
 //            partials; bucket histogram of the keys: shared memory per block, merged into ONE global histogram.
@@ -903,54 +492,26 @@ __global__ void __launch_bounds__(SF_THREADS, 1) k_select_fused(
     }
 }
 
-static inline int keys_grid(const grapes_ctx* ctx, int cap_n) {
-    long long b = ((long long)cap_n + KEYS_THREADS - 1) / KEYS_THREADS;
-    const long long cap = (long long)ctx->sm_count * 8;
-    if (b < 1) b = 1;
-    return (int)(b < cap ? b : cap);
-}
+// floats of scratch grapes_select_* needs in `work` (zeroed ONCE by the caller; every launch leaves the integer part clean):
+// per-block statistics | per-block deltas | candidate logits | integer words (barrier counters, global histogram,
+// per-block counts, member list)
+#define SEL_LG_OFFSET ((int64_t)(SEL_STAT_FLOATS + SF_DELTA_FLOATS) * SF_MAX_BLOCKS)
+static inline int64_t sel_int_offset(int cap_c) { return (SEL_LG_OFFSET + (int64_t)cap_c + 16 + 3) / 4 * 4; }
 
 extern "C" {
 
-// debugging aid: copies the 16 phase time stamps (ns) of the last selection launch to the host (synchronises)
-int grapes_debug_select_stamps(int64_t* out16) {
-    unsigned long long h[16];
-    if (cudaMemcpyFromSymbol(h, g_sel_stamps, sizeof(h)) != cudaSuccess) return GRAPES_ERR_CUDA;
-    for (int i = 0; i < 16; ++i) out16[i] = (int64_t)h[i];
-    return GRAPES_OK;
+int64_t grapes_select_work_floats(grapes_ctx* ctx, int cap_c) {
+    if (!ctx) return 0;
+    return sel_int_offset(cap_c) + SF_I_TOTAL + 16;
 }
 
 // debugging aid: phase time stamps (ns) of the last fused selection launch that used `work` (synchronises)
-int grapes_debug_select_fused_stamps(grapes_ctx* ctx, const float* work, int cap_c, int64_t* out8);
-
-// floats of scratch grapes_select_* needs in `work` (zeroed ONCE by the caller; every launch leaves the integer part clean):
-// per-block statistics | per-block deltas | candidate logits | integer words of the fused kernel (barrier counters,
-// global histogram, per-block counts, member list)
-static inline int64_t sel_stat_floats(const grapes_ctx* ctx, int cap_c) {
-    const int64_t a = (int64_t)SEL_STAT_FLOATS * keys_grid(ctx, cap_c), b = (int64_t)SEL_STAT_FLOATS * SF_MAX_BLOCKS;
-    return a > b ? a : b;
-}
-static inline int64_t sel_lg_offset(const grapes_ctx* ctx, int cap_c) {
-    return sel_stat_floats(ctx, cap_c) + (int64_t)SF_DELTA_FLOATS * SF_MAX_BLOCKS;
-}
-static inline int64_t sel_int_offset(const grapes_ctx* ctx, int cap_c) {
-    return (sel_lg_offset(ctx, cap_c) + (int64_t)cap_c + 16 + 3) / 4 * 4;
-}
-int64_t grapes_select_work_floats(grapes_ctx* ctx, int cap_c) {
-    if (!ctx) return 0;
-    return sel_int_offset(ctx, cap_c) + SF_I_TOTAL + 16;
-}
-
 int grapes_debug_select_fused_stamps(grapes_ctx* ctx, const float* work, int cap_c, int64_t* out8) {
     if (!ctx || !work || !out8) return GRAPES_ERR_ARG;
-    const int* iw = reinterpret_cast<const int*>(work + sel_int_offset(ctx, cap_c));
+    const int* iw = reinterpret_cast<const int*>(work + sel_int_offset(cap_c));
     if (cudaMemcpy(out8, iw + SF_I_STAMP, 8 * sizeof(int64_t), cudaMemcpyDeviceToHost) != cudaSuccess) return GRAPES_ERR_CUDA;
     return GRAPES_OK;
 }
-
-static int g_select_variant = 0;
-// 0 (default): k_select_fused, one launch on every SM; 1: k_logits_keys + the one-cluster k_select (A/B and fallback)
-int grapes_select_variant(int v) { g_select_variant = v; return 0; }
 
 // Sampler-net layer 2 + keys for one hop (main.py:210-213 + utils.py:37-42), then the selection (utils.py:43-71).
 //   z / nparts / part_stride, in_off / in_src / dinv / bias: as grapes_aggregate_scalar; in_off == NULL means
@@ -974,42 +535,16 @@ int grapes_select_hop(grapes_ctx* ctx, const float* z, int nparts, int part_stri
     GRAPES_REQUIRE(noise_mode != GRAPES_NOISE_PHILOX || rng_state, "rng_state required");
     GRAPES_REQUIRE((((size_t)work) & 15) == 0, "work must be 16-byte aligned");
     GRAPES_REQUIRE(!(nb_index && dl_all) || nb_local, "a frontier (nb_index) needs nb_local for the gradient scatter");
-    cudaStream_t s = (cudaStream_t)stream;
+    // one block per SM at most: every block must become resident for the two grid barriers
+    const int nb = grapes_min_i(grapes_min_i(ctx->sm_count, SF_MAX_BLOCKS), grapes_max_i(1, grapes_div_up(cap_n, SF_THREADS)));
     float* stat_part = work;
-    float* lg_c = work + sel_lg_offset(ctx, cap_n);
-    if (g_select_variant == 0) {
-        // one block per SM at most: every block must become resident for the two grid barriers
-        int nb = grapes_min_i(grapes_min_i(ctx->sm_count, SF_MAX_BLOCKS), grapes_max_i(1, grapes_div_up(cap_n, SF_THREADS)));
-        float* delta_part = work + sel_stat_floats(ctx, cap_n);
-        int* iw = reinterpret_cast<int*>(work + sel_int_offset(ctx, cap_n));
-        pdl((k_select_fused), nb, SF_THREADS, 0, s)(z, nparts, part_stride, n_dev, cap_n, in_off, in_src, dinv, bias,
-                                                   nb_index, nb_local, nb_nodes, c_dev, k, noise_mode, noise, rng_state,
-                                                   logits_all, lg_c, ukeys_scratch, keys_out, sampled_out, sampled_offset,
-                                                   s_dev, total_dev, mask_out, log_prob, tot_log_prob, stats, dl_all,
-                                                   sum_dl, bm_mark, stat_part, delta_part, iw);
-        grapes_count_launches(1);
-        GRAPES_LAUNCH_OK();
-        return GRAPES_OK;
-    }
-    const int nblk = keys_grid(ctx, cap_n);
-    pdl((k_logits_keys), nblk, KEYS_THREADS, 0, s)(z, nparts, part_stride, n_dev, cap_n, in_off, in_src, dinv, bias,
-                                                nb_index, c_dev, k, noise_mode, noise, rng_state, logits_all, lg_c,
-                                                ukeys_scratch, keys_out, log_prob, dl_all, mask_out, stat_part);
-    grapes_count_launches(1);
-    // keys of one CTA's chunk staged in shared memory when they fit next to the ~57 KB of static state
-    const size_t chunk_bytes = ((size_t)(cap_n + SEL_CTAS - 1) / SEL_CTAS) * sizeof(uint32_t);
-    const int staged = chunk_bytes <= 160 * 1024 ? 1 : 0;
-    const int smem = staged ? (int)chunk_bytes : 0;
-    static int attr[64] = {0};                       // per device: the attribute belongs to the device's copy of the function
-    int& have = attr[ctx->device & 63];
-    if (smem > have) {
-        GRAPES_CUDA_OK(cudaFuncSetAttribute(k_select, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        have = smem;
-    }
-    pdl((k_select), SEL_CTAS, SEL_THREADS, smem, s)(ukeys_scratch, lg_c, nb_local, nb_nodes, c_dev, cap_n, k, noise_mode,
-                                                 rng_state, stat_part, nblk, staged, sampled_out, sampled_offset,
-                                                 s_dev, total_dev, mask_out, log_prob, tot_log_prob, stats, dl_all,
-                                                 sum_dl, bm_mark);
+    float* delta_part = work + (int64_t)SEL_STAT_FLOATS * SF_MAX_BLOCKS;
+    float* lg_c = work + SEL_LG_OFFSET;
+    int* iw = reinterpret_cast<int*>(work + sel_int_offset(cap_n));
+    pdl((k_select_fused), nb, SF_THREADS, 0, (cudaStream_t)stream)(
+        z, nparts, part_stride, n_dev, cap_n, in_off, in_src, dinv, bias, nb_index, nb_local, nb_nodes, c_dev, k,
+        noise_mode, noise, rng_state, logits_all, lg_c, ukeys_scratch, keys_out, sampled_out, sampled_offset, s_dev,
+        total_dev, mask_out, log_prob, tot_log_prob, stats, dl_all, sum_dl, bm_mark, stat_part, delta_part, iw);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;

@@ -59,15 +59,7 @@ struct AtB { int g; float dsl, dj; uint32_t sb; int rk; };        // node id, de
 // metadata, one LDS.128 of the row per 128 columns, 4 FFMA, one branch.
 // XB16: the feature table holds bf16 (papers100M-shaped config: 128 bf16 features); rows are staged as stored (2F bytes)
 // and widened to fp32 when they are read from shared memory; all arithmetic and the output stay fp32.
-// VS ("virtual columns in the slot", fp32 tables): the columns [F, ldo) -- indicators | ones | zero pad -- are handled by the
-// SAME float4 lanes as the feature columns instead of one scalar lane each: the copy stage writes the entry's indicator
-// floats right behind its TMA-staged row, so the lane that owns columns F .. F+3 accumulates them with the ordinary
-// LDS.128 + 4 FFMA (same order, same values as the scalar form -> bitwise identical), and the row is written with float4
-// stores only.  Per output row this removes the shift/and/convert/fma chain of every entry and the scalar
-// convert + 2 stores per virtual column (15 % of the kernel's instructions at frontier size, ncu source view).  Measured
-// on B200: 2 us SLOWER per frontier-sized launch than the scalar form (the kernel waits on fixed-latency dependencies at
-// 23 % occupancy, it is not short of issue slots), so the launcher only uses it on request (grapes_agg_tma_virtual_slot).
-template <int NPASS, bool HAS_IND, int OUTMODE, bool XB16, bool VS>
+template <int NPASS, bool HAS_IND, int OUTMODE, bool XB16>
 __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
     const void* __restrict__ X, int F, int ldx, const int* __restrict__ nodes, const int* __restrict__ n_dev, int cap_n,
     const int* __restrict__ in_off, const int* __restrict__ in_src, const float* __restrict__ dinv,
@@ -81,9 +73,7 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
     // bytes staged per row: the row rounded up to a whole float4 (F % 4 != 0: the table's rows are padded, ldx >= round_up(F, 4);
     // the pad values are accumulated into the unused components of the last feature lane and never stored)
     const uint32_t rowbytes = XB16 ? (uint32_t)F * 2u : (uint32_t)((F + 3) & ~3) * 4u;
-    const int ni4 = (VS && HAS_IND) ? (num_ind + 3) >> 2 : 0;      // float4 groups of indicator columns behind each staged row
-    const uint32_t rowstride = rowbytes + 16u * (uint32_t)ni4;
-    const uint32_t slot_bytes = (uint32_t)ec * rowstride;
+    const uint32_t slot_bytes = (uint32_t)ec * rowbytes;
     unsigned char* wslots = at_smem + (size_t)warp * 2u * slot_bytes;
     unsigned char* tail = at_smem + (size_t)AT_WARPS * 2u * slot_bytes;
     int4* s_meta = reinterpret_cast<int4*>(tail) + warp * 64;                         // [2 slots][32 entries]
@@ -91,18 +81,13 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
     uint64_t* bars = reinterpret_cast<uint64_t*>(tail + (size_t)AT_WARPS * 64u * 16u +
                                                  (size_t)AT_WARPS * AT_POS_STRIDE * 4u) + warp * 2;
     const uint32_t bar0 = at_smem_u32(&bars[0]), bar1 = at_smem_u32(&bars[1]);
-    const uint32_t slot0 = at_smem_u32(wslots);
     if (lane == 0) { at_mbar_init(bar0, 1); at_mbar_init(bar1, 1); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncwarp();
     uint32_t ph = 0;                                              // phase parity of the two barriers (bits 0, 1)
-    bool act[NPASS];                                              // this lane accumulates columns p*128 + 4*lane .. +3
-    bool acto[NPASS];                                             // ... and stores them
+    bool act[NPASS];                                              // this lane accumulates and stores columns p*128 + 4*lane .. +3
 #pragma unroll
-    for (int p = 0; p < NPASS; ++p) {
-        act[p] = p * 128 + lane * 4 < F + 4 * ni4;
-        acto[p] = p * 128 + lane * 4 < (VS ? ldo : F);
-    }
+    for (int p = 0; p < NPASS; ++p) act[p] = p * 128 + lane * 4 < F;
     const int cv = F + lane;                                      // this lane's virtual column
     const float vconst = (cv == ones_col) ? 1.f : 0.f;
 
@@ -154,15 +139,9 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
                 const uint32_t bar = (c & 1) ? bar1 : bar0;
                 if (lane == 0) at_mbar_expect_tx(bar, (uint32_t)cnt * rowbytes);
                 s_meta[(c & 1) * 32 + lane] = make_int4(__float_as_int(b.dsl * b.dj), b.rk, (int)b.sb, 0);  // self: dj * dj
-                if (VS && HAS_IND && (b.rk & AT_VALID)) {           // indicator floats of the entry's source behind its row
-                    float4* ip = reinterpret_cast<float4*>(wslots + (size_t)(c & 1) * slot_bytes + (size_t)lane * rowstride + rowbytes);
-                    for (int q = 0; q < ni4; ++q)
-                        ip[q] = make_float4((float)((b.sb >> (4 * q)) & 1u), (float)((b.sb >> (4 * q + 1)) & 1u),
-                                            (float)((b.sb >> (4 * q + 2)) & 1u), (float)((b.sb >> (4 * q + 3)) & 1u));
-                }
                 __syncwarp();
                 if (b.rk & AT_VALID)
-                    at_bulk_row(slot0 + (uint32_t)(c & 1) * slot_bytes + (uint32_t)lane * rowstride,
+                    at_bulk_row(at_smem_u32(wslots) + (uint32_t)(c & 1) * slot_bytes + (uint32_t)lane * rowbytes,
                                 reinterpret_cast<const unsigned char*>(X) + (size_t)b.g * ldx * (XB16 ? 2u : 4u), rowbytes, bar);
             }
         };
@@ -195,7 +174,7 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
             // lane l owns columns 4l .. 4l+3 of every 128-column pass: a float4 (fp32 table) or a uint2 (bf16 table)
             const unsigned char* rp = wslots + (size_t)(c & 1) * slot_bytes + (size_t)lane * (XB16 ? 8u : 16u);
             const int4* mp = s_meta + (c & 1) * 32;
-            for (int t = 0; t < cnt; ++t, rp += rowstride) {
+            for (int t = 0; t < cnt; ++t, rp += rowbytes) {
                 const int4 m = mp[t];                                      // broadcast: weight | row + flags | indicator bits
                 const float wt = __int_as_float(m.x);
 #pragma unroll
@@ -213,25 +192,20 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
                         acc[p].z = fmaf(wt, v.z, acc[p].z); acc[p].w = fmaf(wt, v.w, acc[p].w);
                     }
                 }
-                if (HAS_IND && !VS) aind = fmaf(wt, (float)(((uint32_t)m.z >> lane) & 1u), aind);
+                if (HAS_IND) aind = fmaf(wt, (float)(((uint32_t)m.z >> lane) & 1u), aind);
                 if (m.y & AT_LAST) {                               // warp-uniform: the row is complete
                     const size_t orow = (size_t)(j0 + (m.y & 0x1ff)) * ldo;
 #pragma unroll
                     for (int p = 0; p < NPASS; ++p) {
-                        if (acto[p]) {
+                        if (act[p]) {
                             const int c0 = p * 128 + lane * 4;
-                            float4 a = act[p] ? acc[p] : make_float4(0.f, 0.f, 0.f, 0.f);
-                            if (!VS || c0 < F) {
-                                if (bias) {
-                                    if (c0 + 4 <= F) { a.x += bias[c0]; a.y += bias[c0 + 1]; a.z += bias[c0 + 2]; a.w += bias[c0 + 3]; }
-                                    else { a.x += bias[c0]; if (c0 + 1 < F) a.y += bias[c0 + 1]; if (c0 + 2 < F) a.z += bias[c0 + 2]; }
-                                }
-                                if (relu) { a.x = fmaxf(a.x, 0.f); a.y = fmaxf(a.y, 0.f); a.z = fmaxf(a.z, 0.f); a.w = fmaxf(a.w, 0.f); }
-                            } else {                               // virtual lane: indicators (accumulated) | ones | zero pad
-                                const int oc = ones_col - c0;
-                                if (oc == 0) a.x = 1.f; else if (oc == 1) a.y = 1.f; else if (oc == 2) a.z = 1.f; else if (oc == 3) a.w = 1.f;
+                            float4 a = acc[p];
+                            if (bias) {
+                                if (c0 + 4 <= F) { a.x += bias[c0]; a.y += bias[c0 + 1]; a.z += bias[c0 + 2]; a.w += bias[c0 + 3]; }
+                                else { a.x += bias[c0]; if (c0 + 1 < F) a.y += bias[c0 + 1]; if (c0 + 2 < F) a.z += bias[c0 + 2]; }
                             }
-                            if (!VS && c0 + 4 > F) {               // last feature lane of a row with F % 4 != 0: 1..3 valid columns
+                            if (relu) { a.x = fmaxf(a.x, 0.f); a.y = fmaxf(a.y, 0.f); a.z = fmaxf(a.z, 0.f); a.w = fmaxf(a.w, 0.f); }
+                            if (c0 + 4 > F) {                      // last feature lane of a row with F % 4 != 0: 1..3 valid columns
                                 const int nvv = F - c0;
                                 auto put = [&](int i, float val) {
                                     if (OUTMODE & 1) out[orow + c0 + i] = val;
@@ -257,7 +231,7 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
                         }
                         acc[p] = make_float4(0.f, 0.f, 0.f, 0.f);    // next row starts from fma(w_self, x, 0)
                     }
-                    if (!VS && cv < ldo) {                         // virtual columns, one scalar lane each
+                    if (cv < ldo) {                                // virtual columns, one scalar lane each
                         const float v = (HAS_IND && lane < num_ind) ? aind : vconst;
                         if (OUTMODE & 1) out[orow + cv] = v;
                         if (OUTMODE & 2) { const float h = at_tf32(v); out_hi[orow + cv] = h; out_lo[orow + cv] = at_tf32(v - h); }
@@ -272,12 +246,8 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
     }
 }
 
-int g_agg_tma_vs = 0;          // grapes_agg_tma_virtual_slot(1): pad columns through the float4 lanes -- bit-identical, fewer
-                               // instructions, and measured ~2 us SLOWER per frontier-sized launch on B200 -> opt-in (DESIGN.md section 9)
-extern "C" int grapes_agg_tma_virtual_slot(int on) { g_agg_tma_vs = on ? 1 : 0; return 0; }
-
-size_t grapes_agg_tma_smem(int F, int ec, int es = 4, int extra = 0) {
-    return (size_t)AT_WARPS * 2u * (size_t)ec * ((size_t)F * (size_t)es + (size_t)extra) + (size_t)AT_WARPS * 64u * 16u +
+size_t grapes_agg_tma_smem(int F, int ec, int es = 4) {
+    return (size_t)AT_WARPS * 2u * (size_t)ec * (size_t)F * (size_t)es + (size_t)AT_WARPS * 64u * 16u +
            (size_t)AT_WARPS * AT_POS_STRIDE * 4u + AT_WARPS * 16u;
 }
 
@@ -296,41 +266,34 @@ int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int
     const size_t budget = cps == 1 ? 226u * 1024u : (cps == 2 ? 113u * 1024u : (size_t)(227u * 1024u / cps - 1024u));
     const int npass = (F + 127) / 128;
     const bool has_ind = ind_bits != nullptr && num_ind > 0;
-    // virtual columns through the float4 lanes (VS): fp32 table, pad columns present and inside the last 128-column pass
-    const bool vs = !x_bf16 && F % 4 == 0 && ldo > F && ldo <= npass * 128 && g_agg_tma_vs;
-    const int extra = (vs && has_ind) ? 16 * ((num_ind + 3) / 4) : 0;
     const int Fs = x_bf16 ? F : ((F + 3) & ~3);                                       // staged row width
     int ec = ec_req > 0 ? ec_req : 32;
     if (ec > 32) ec = 32;
-    while (ec > 1 && grapes_agg_tma_smem(Fs, ec, es, extra) > budget) ec >>= 1;
-    const size_t smem = grapes_agg_tma_smem(Fs, ec, es, extra);
+    while (ec > 1 && grapes_agg_tma_smem(Fs, ec, es) > budget) ec >>= 1;
+    const size_t smem = grapes_agg_tma_smem(Fs, ec, es);
     if (smem > 226u * 1024u) return 1;
     const int rb_min = (size_t)Fs * es >= 2048 ? 2 : 8;      // wide rows (Reddit 2.4 KB, Cora 5.7 KB): spread a small frontier over every warp
     long long blocks = ((long long)cap_n + AT_WARPS * rb_min - 1) / (AT_WARPS * rb_min);
     const long long cap = (long long)ctx->sm_count * (smem > 113u * 1024u ? 1 : (cps >= 2 ? cps : 2));
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
-#define AT_LAUNCH5(NP, IND, OM, XB, VSF)                                                                                 \
+#define AT_LAUNCH_INST(NP, IND, OM, XB)                                                                                 \
     do {                                                                                                                \
         static bool configured = false;                                                                                 \
         if (!configured) {                                                                                              \
-            if (cudaFuncSetAttribute(k_agg_tma<NP, IND, OM, XB, VSF>, cudaFuncAttributeMaxDynamicSharedMemorySize,          \
+            if (cudaFuncSetAttribute(k_agg_tma<NP, IND, OM, XB>, cudaFuncAttributeMaxDynamicSharedMemorySize,           \
                                      (int)(226u * 1024u)) != cudaSuccess) return 1;                                     \
             configured = true;                                                                                          \
         }                                                                                                               \
-        pdl((k_agg_tma<NP, IND, OM, XB, VSF>), (int)blocks, AT_THREADS, smem, s)(X, F, ldx, nodes, n_dev, cap_n, in_off,   \
-                                                                               in_src, dinv, ind_bits, num_ind, bias, relu, \
-                                                                               out, ldo, out_hi, out_lo, ones_col, ec,     \
-                                                                               rb_min);                                    \
-    } while (0)
-#define AT_LAUNCH4(NP, IND, OM, XB)                                                                                     \
-    do {                                                                                                                \
-        if (!XB && vs) AT_LAUNCH5(NP, IND, OM, false, true); else AT_LAUNCH5(NP, IND, OM, XB, false);                   \
+        pdl((k_agg_tma<NP, IND, OM, XB>), (int)blocks, AT_THREADS, smem, s)(X, F, ldx, nodes, n_dev, cap_n, in_off,     \
+                                                                          in_src, dinv, ind_bits, num_ind, bias, relu,  \
+                                                                          out, ldo, out_hi, out_lo, ones_col, ec,       \
+                                                                          rb_min);                                      \
     } while (0)
 #define AT_LAUNCH2(NP, IND, XB)                                                                                         \
     do {                                                                                                                \
-        if (om == 1) AT_LAUNCH4(NP, IND, 1, XB); else if (om == 2) AT_LAUNCH4(NP, IND, 2, XB);                          \
-        else AT_LAUNCH4(NP, IND, 3, XB);                                                                                \
+        if (om == 1) AT_LAUNCH_INST(NP, IND, 1, XB); else if (om == 2) AT_LAUNCH_INST(NP, IND, 2, XB);                  \
+        else AT_LAUNCH_INST(NP, IND, 3, XB);                                                                            \
     } while (0)
 #define AT_LAUNCH(NP)                                                                                                   \
     do {                                                                                                                \
@@ -349,8 +312,7 @@ int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int
     else AT_LAUNCH(12);
 #undef AT_LAUNCH_B16
 #undef AT_LAUNCH2
-#undef AT_LAUNCH5
-#undef AT_LAUNCH4
+#undef AT_LAUNCH_INST
 #undef AT_LAUNCH
     return 0;
 }

@@ -18,7 +18,6 @@ from __future__ import annotations
 import contextlib
 import ctypes
 import math
-import os
 from typing import Dict, List, Optional, Sequence
 
 import torch
@@ -128,11 +127,11 @@ class GrapesEngine:
         # backward walks Y in chunks of 128 columns.
         self.use_tc = bool(use_tensor_cores) and (self.D % 128 == 0) and self.D <= 512
         self.use_tc_bwd = self.use_tc and self.D // 128 <= 2    # backward accumulators: halves x (hi | lo) x 128 columns of TMEM
-        # default (GRAPES_Y_SINGLE=0 restores the pre-split pair): the aggregation writes Y once as fp32 and the tcgen05 kernels split it into (hi, lo) themselves
+        # Fp <= 1024: the aggregation writes Y once as fp32 and the tcgen05 kernels split it into (hi, lo) themselves
         # (half the Y bytes written and read; the default forward k_l1_fwd_ts needs the raw fp32 Y: it splits it on the way into
         # tensor memory; products-shape: aggregation 73.8 -> 60.8,
         # forward 120 -> 136, backward 155 -> 149 us per step, step 0.512 -> 0.508 ms)
-        self.y_single = self.use_tc and os.environ.get("GRAPES_Y_SINGLE", "1" if self.Fp <= 1024 else "0") == "1"   # Cora-shape (K = 1436): the pair is 2 % faster
+        self.y_single = self.use_tc and self.Fp <= 1024    # Cora-shape (K = 1436): the (hi, lo) pair is 2 % faster
         if self.use_tc_bwd:
             self.ldY = _round_up(self.Fp + 1, 4)           # room for the column of ones (bias column)
         self.ldW = _round_up(self.Fp, 4)
@@ -147,9 +146,6 @@ class GrapesEngine:
         # chain, side B the induced-block slices.  Each stream has its own library context (scan / split-K scratch).
         self.multi_stream = bool(multi_stream)
         if self.multi_stream:
-            # the critical path (hop chain + classifier) runs at high priority so its kernels are scheduled ahead of the
-            # queued backward / slice kernels of the side streams
-            self.main_hp = torch.cuda.Stream(device=dev, priority=-1) if os.environ.get("GRAPES_HP", "0") == "1" else None
             self.side_a, self.side_b = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
             self.side_p = torch.cuda.Stream(device=dev)          # front end of the NEXT batch (cross-step prefetch)
             self.ctx_a, self.ctx_b, self.ctx_p = graph.new_ctx(), graph.new_ctx(16 << 20), graph.new_ctx(16 << 20)
@@ -157,11 +153,10 @@ class GrapesEngine:
             # so the hop chain's small kernels are not queued behind them (measured, DESIGN.md section 9)
             # products / arxiv shape (K ~ 100): 96 of 148 SMs -> 0.549 -> 0.533 / 0.251 -> 0.236 ms/step; with long K
             # (Reddit 602, Cora 1433 columns) the backward is heavy enough to become the critical path when limited
-            side_sms = int(os.environ.get("GRAPES_SIDE_SMS", "96" if (F + self.H + 1) <= 256 else "0"))
-            if side_sms > 0:
-                self.L.grapes_ctx_set_sm_limit(self.ctx_a, side_sms)
+            if (F + self.H + 1) <= 256:
+                self.L.grapes_ctx_set_sm_limit(self.ctx_a, 96)
         else:
-            self.side_a = self.side_b = self.side_p = self.main_hp = None
+            self.side_a = self.side_b = self.side_p = None
             self.ctx_a = self.ctx_b = self.ctx_p = graph.ctx
 
         # ---- capacities -------------------------------------------------------------------
@@ -280,22 +275,10 @@ class GrapesEngine:
         self.launches_per_graph = 0
         self.record: Optional[dict] = None
         # timing experiments only (scripts/ablate.py): leave out parts of the step to see what the rest costs
-        self.ablate = set(filter(None, os.environ.get("GRAPES_ABLATE", "").split(",")))
-        # rank + relabel + CSR build of a hop as ONE cooperative launch (grapes_hop_structure): bit-identical, 73 -> 61
-        # launches per step, but NOT faster (34 us per hop either way: the phases are memory-latency chains, and a
-        # cooperative grid has to wait for SMs held by the side branches) -> opt-in
-        self.fused_struct = os.environ.get("GRAPES_FUSED_STRUCT", "0") == "1"
+        self.ablate = set()
         # where the gcn_z chain sits on the backward branch: behind the LAST hop's backward it overlaps the classifier tail
         # (small kernels) instead of hop 1's aggregation + GEMM: products 0.533 -> 0.511 ms/step; neutral with long K
-        self.z_at = os.environ.get("GRAPES_Z_AT", "last" if (F + self.H + 1) <= 256 else "hop0")
-        if os.environ.get("GRAPES_AGG_VARIANT"):
-            self.L.cdll.grapes_agg_variant(int(os.environ["GRAPES_AGG_VARIANT"]))
-        if os.environ.get("GRAPES_AGG_MIN_ROWS"):
-            self.L.cdll.grapes_agg_tma_min_rows(int(os.environ["GRAPES_AGG_MIN_ROWS"]))
-        if os.environ.get("GRAPES_SELECT_VARIANT"):
-            self.L.cdll.grapes_select_variant(int(os.environ["GRAPES_SELECT_VARIANT"]))
-        if os.environ.get("GRAPES_TC_DEBUG"):
-            self.L.cdll.grapes_tc_debug(int(os.environ["GRAPES_TC_DEBUG"]))
+        self.z_at = "last" if (F + self.H + 1) <= 256 else "hop0"
 
     def _alloc_step_state(self):
         """Every buffer that belongs to ONE step in flight (bitmap / scalar pool, id lists, device-side sizes, per-hop
@@ -419,16 +402,6 @@ class GrapesEngine:
     # ------------------------------------------------------------------ the step
     def _enqueue(self, gumbel_noise: Optional[Sequence[Optional[torch.Tensor]]], apply_optim: bool,
                  noise_mode: int = NOISE_GUMBEL):
-        hp = self.main_hp if (self.multi_stream and self.side_a is not None) else None
-        if hp is None:
-            return self._enqueue_on(gumbel_noise, apply_optim, noise_mode)
-        caller = torch.cuda.current_stream()
-        hp.wait_stream(caller)
-        with torch.cuda.stream(hp):
-            self._enqueue_on(gumbel_noise, apply_optim, noise_mode)
-        caller.wait_stream(hp)
-
-    def _enqueue_on(self, gumbel_noise, apply_optim, noise_mode):
         L, g = self.L, self.g
         main = torch.cuda.current_stream()
         multi = self.multi_stream and self.side_a is not None
@@ -466,8 +439,7 @@ class GrapesEngine:
         else:
             self._enqueue_front0(ctx, st)
 
-        if os.environ.get("GRAPES_PREFETCH_AT", "start") == "start":
-            self._enqueue_prefetch(fork, on, sP, stP)
+        self._enqueue_prefetch(fork, on, sP, stP)
 
         for h in range(H):
             hw = self.hops[h]
@@ -484,7 +456,7 @@ class GrapesEngine:
                     L.grapes_slice_block(ctx_b, rows, ptr(hw.e_row), ptr(hw.e_col), m_dev, cap_m,
                                          ptr(self.bm_prev[h - 1]), ptr(pw.blk_src), ptr(pw.blk_dst), self.cap_blk,
                                          self._hc(h - 1, "blk"), ovf, stB)
-                self._enqueue_hop_structure(h, ctx, st)
+                self._enqueue_hop_graph(h, ctx, st)
             if need_Y:
                 if tc:
                     if h == 0:
@@ -522,9 +494,6 @@ class GrapesEngine:
                     self._enqueue_hop_backward(h, ctx_a, stA)
                     if h == H - 1 and self.z_at != "hop0":
                         self._enqueue_gcn_z(ctx_a, stA)
-
-        if os.environ.get("GRAPES_PREFETCH_AT", "start") == "tail":
-            self._enqueue_prefetch(fork, on, sP, stP)
 
         # ---- last block: slice_adjacency(rows = T u S_{H-1}, cols = prev_{H-1}) ----
         rows, P_dev, m_dev = ptr(self.prev[H]), self._hc(H, "P"), self._hc(H, "m")
@@ -683,7 +652,7 @@ class GrapesEngine:
                 L.grapes_expand_frontier(ctx, ptr(g.indptr), ptr(g.indices), rows, P_dev, cap_P, ptr(hw.row_off), m_dev,
                                          cap_m, ptr(hw.e_row), ptr(hw.e_col), ptr(self.bm_prev[h]), ptr(self.bm_batch[h]),
                                          ovf, st)
-                self._enqueue_hop_structure(h, ctx, st)
+                self._enqueue_hop_graph(h, ctx, st)
             if self.use_tc:
                 if h == 0:
                     self._split_weights(ctx, st)
@@ -749,7 +718,7 @@ class GrapesEngine:
             self._activate(cur)
         self._front_ready[1 - cur] = True
 
-    def _enqueue_hop_structure(self, h: int, ctx, st):
+    def _enqueue_hop_graph(self, h: int, ctx, st):
         """After the row expansion of hop h: mask dedup + id lists + indicator bits (main.py:183-195), local relabel,
         gcn_norm structure of the hop graph (dst-sorted CSR, deg^-1/2) and Y = A_hat [x | indicators] (feature gather
         fused, main.py:198-204 + GCNConv aggregation).  None of it depends on the weights."""
@@ -759,26 +728,16 @@ class GrapesEngine:
         rows = ptr(self.prev[h])
         m_dev, n_dev, c_dev = self._hc(h, "m"), self._hc(h, "n"), self._hc(h, "c")
         ovf = ptr(self.overflow)
-        if self.fused_struct:
-            # rank -> relabel + histogram -> scan -> fill -> per-row sort in ONE cooperative launch (grid barriers)
-            L.grapes_hop_structure(ctx, ptr(self.bm_batch[h]), ptr(self.bm_prev[h]), ptr(self.pref_batch),
-                                   ptr(self.pref_nb), ptr(hw.batch_nodes), ptr(hw.nb_nodes), ptr(hw.nb_local),
-                                   ptr(hw.nb_index), ptr(hw.ind_bits) if self.use_ind else None,
-                                   ptr(self.bm_ind) if self.use_ind else None, self.num_ind, h, cap_n, n_dev, c_dev,
-                                   rows, ptr(hw.e_row), ptr(hw.e_col), m_dev, cap_m, ptr(hw.e_src), ptr(hw.e_dst),
-                                   ptr(self.cnt_scratch), ptr(hw.in_off), ptr(hw.in_src), ptr(self.tmp_val),
-                                   ptr(hw.dinv), self._hc(h, "nnz"), ovf, st)
-        else:
-            L.grapes_rank_nodes(ctx, ptr(self.bm_batch[h]), ptr(self.bm_prev[h]), ptr(self.pref_batch),
-                                ptr(self.pref_nb), ptr(hw.batch_nodes), ptr(hw.nb_nodes), ptr(hw.nb_local),
-                                ptr(hw.nb_index), ptr(hw.ind_bits) if self.use_ind else None,
-                                ptr(self.bm_ind) if self.use_ind else None, self.num_ind, h, cap_n,
-                                n_dev, c_dev, ovf, st)
-            L.grapes_edges_to_local(ctx, rows, ptr(hw.e_row), ptr(hw.e_col), m_dev, cap_m, ptr(self.bm_batch[h]),
-                                    ptr(self.pref_batch), cap_n, ptr(hw.e_src), ptr(hw.e_dst), ptr(self.cnt_scratch), st)
-            L.grapes_build_csr(ctx, ptr(hw.e_dst), ptr(hw.e_src), m_dev, cap_m, n_dev, cap_n, ptr(self.cnt_scratch),
-                               1, ptr(hw.in_off), ptr(hw.in_src), ptr(self.tmp_val), ptr(hw.dinv),
-                               self._hc(h, "nnz"), ovf, st)
+        L.grapes_rank_nodes(ctx, ptr(self.bm_batch[h]), ptr(self.bm_prev[h]), ptr(self.pref_batch),
+                            ptr(self.pref_nb), ptr(hw.batch_nodes), ptr(hw.nb_nodes), ptr(hw.nb_local),
+                            ptr(hw.nb_index), ptr(hw.ind_bits) if self.use_ind else None,
+                            ptr(self.bm_ind) if self.use_ind else None, self.num_ind, h, cap_n,
+                            n_dev, c_dev, ovf, st)
+        L.grapes_edges_to_local(ctx, rows, ptr(hw.e_row), ptr(hw.e_col), m_dev, cap_m, ptr(self.bm_batch[h]),
+                                ptr(self.pref_batch), cap_n, ptr(hw.e_src), ptr(hw.e_dst), ptr(self.cnt_scratch), st)
+        L.grapes_build_csr(ctx, ptr(hw.e_dst), ptr(hw.e_src), m_dev, cap_m, n_dev, cap_n, ptr(self.cnt_scratch),
+                           1, ptr(hw.in_off), ptr(hw.in_src), ptr(self.tmp_val), ptr(hw.dinv),
+                           self._hc(h, "nnz"), ovf, st)
         if not self.random_sampling:
             tc = self.use_tc
             agg_x = L.grapes_aggregate_bf16 if self.x_bf16 else L.grapes_aggregate
@@ -800,7 +759,7 @@ class GrapesEngine:
         L.grapes_expand_frontier(ctx, ptr(g.indptr), ptr(g.indices), ptr(self.prev[0]), self._hc(0, "P"), self.cap_P,
                                  ptr(hw.row_off), self._hc(0, "m"), self.cap_m, ptr(hw.e_row), ptr(hw.e_col),
                                  ptr(self.bm_prev[0]), ptr(self.bm_batch[0]), ptr(self.overflow), st)
-        self._enqueue_hop_structure(0, ctx, st)
+        self._enqueue_hop_graph(0, ctx, st)
 
     def _enqueue_hop_backward(self, h: int, ctx, st):
         """Side stream A.  Gradient direction of sum(log_prob_h) w.r.t. gcn_gf (main.py:271-287 via

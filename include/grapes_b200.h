@@ -124,15 +124,6 @@ int grapes_rank_nodes(grapes_ctx* ctx, const uint32_t* bm_batch, const uint32_t*
                       int* pref_nb, int* batch_nodes, int* nb_nodes, int* nb_local, int* nb_index, uint32_t* ind_bits,
                       uint32_t* bm_ind, int ind_rows, int hop, int cap_n, int* n_dev, int* c_dev, int* overflow,
                       void* stream);
-/* grapes_rank_nodes + grapes_edges_to_local + grapes_build_csr (frontier-sized form) in ONE cooperative launch with
- * grid barriers between the five phases: same outputs bit for bit (main.py:183-195 + gcn_norm structure of the hop
- * graph); cnt_scratch all-zero on entry and on exit.                                                              */
-int grapes_hop_structure(grapes_ctx* ctx, const uint32_t* bm_batch, const uint32_t* bm_prev, int* pref_batch, int* pref_nb,
-                         int* batch_nodes, int* nb_nodes, int* nb_local, int* nb_index, uint32_t* ind_bits,
-                         uint32_t* bm_ind, int ind_rows, int hop, int cap_n, int* n_dev, int* c_dev, const int* rows,
-                         const int* e_row, const int* e_col, const int* m_dev, int cap_m, int* e_src, int* e_dst,
-                         int* cnt_scratch, int* in_off, int* in_src, int* tmp_val, float* dinv, int* nnz_dev,
-                         int* overflow, void* stream);
 /* node_map.map(neighborhoods) (main.py:195): local (src, dst) of every expanded edge.  cnt_hist
  * (optional, all-zero on entry) receives the in-degree histogram grapes_build_csr(hist_done=1) needs.
  * cap_n = capacity of every node-indexed buffer downstream (cnt_hist, in_off, dinv, Y ...): when the frontier holds
@@ -190,18 +181,11 @@ int grapes_aggregate(grapes_ctx* ctx, const float* X, int F, int ldx, const int*
                      const int* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits, int num_ind,
                      const float* bias, int relu, float* out, int ldo, float* out_hi, float* out_lo, int ones_col,
                      void* stream);
+/* 0 (default) = aggregation form chosen by shape; 1 = the register-staged kernels only, the bit-exact reference of the
+ * TMA-staged form (csrc/gcn.cu aggregate_impl).  Any other value is GRAPES_ERR_ARG.                                */
+int grapes_agg_variant(int v);
 /* the same with the feature table stored as bf16 (papers100M-shaped config: 128 bf16 features, BASELINE.json configs[4]);
  * rows are widened to fp32 as they are read, arithmetic and outputs stay fp32.  ldx in elements.                */
-/* TMA-staged aggregation: 1 = the pad columns [F, ldo) go through the float4 lanes (indicator floats staged behind each
- * row in shared memory), 0 (default) = one scalar lane per pad column.  Bitwise identical results; the float4 form
- * executes 15 % fewer instructions and measured slower on B200, so it is opt-in.                                  */
-int grapes_agg_tma_virtual_slot(int on);
-/* smallest row capacity (cap_n) whose aligned-width aggregation takes the TMA-staged form (default 4096; smaller launches
- * use one warp per row)                                                                                              */
-int grapes_agg_tma_min_rows(int rows);
-/* A/B knob of the measurement scripts: 0 (default) = shape chosen by the launcher; 1..6 = a register-staged kernel,
- * 100 + ec / 200 + ec = a forced TMA-staged shape (csrc/gcn.cu aggregate_impl).  Every variant is bitwise identical.   */
-int grapes_agg_variant(int v);
 int grapes_aggregate_bf16(grapes_ctx* ctx, const void* X_bf16, int F, int ldx, const int* nodes, const int* n_dev,
                           int cap_n, const int* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits,
                           int num_ind, const float* bias, int relu, float* out, int ldo, float* out_hi, float* out_lo,
@@ -285,15 +269,9 @@ int grapes_sampler_l1_bwd_tc(grapes_ctx* ctx, const float* Y, const float* Y_lo,
                              float* gw2, void* stream);
 
 /* ---- selection (utils.py:13-71; eval.py:126-130) --------------------------------------------- */
-/* debugging aid: phase time stamps (globaltimer ns) of the last on-chip selection launch, HOST array of 16 */
-int grapes_debug_select_stamps(int64_t* out16);
 /* floats of scratch (`work`, 16-byte aligned, ZEROED ONCE by the caller: every launch leaves its counters clean) the
  * two calls below need for cap_c candidates                                                              */
 int64_t grapes_select_work_floats(grapes_ctx* ctx, int cap_c);
-/* 0 (default): the whole head of a hop as ONE launch on every SM (k_select_fused: layer-2 aggregation, keys, global
- * bucket histogram, two software grid barriers, exact threshold, ordered output); 1: GPU-wide key pass + selection on
- * one 8-CTA cluster (the earlier form; kept for A/B measurements).  Same results bit for bit.                 */
-int grapes_select_variant(int v);
 /* debugging aid: globaltimer stamps (ns) of block 0 at the phase boundaries of the last fused selection launch that used
  * `work` (start, keys done, histogram merged, barrier 1, members listed, barrier 2, outputs done, last block done);
  * HOST array of 8, synchronises                                                                                      */

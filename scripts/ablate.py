@@ -1,5 +1,5 @@
 """Timing experiments on the products-shaped workload: the step graph with parts left out
-(GRAPES_ABLATE-style switches) or on one stream, to see what sits on the critical path.
+(`GrapesEngine.ablate`) or on one stream, to see what sits on the critical path.
 Not a benchmark: results of ablated steps are wrong by construction."""
 import os, sys, json, time
 import torch

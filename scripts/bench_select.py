@@ -1,6 +1,5 @@
 """Micro-benchmark of the selection head on products- / Reddit-sized candidate sets (k = 256): CUDA-event time of
-grapes_select_topk for the fused one-launch kernel (variant 0, default) and the earlier k_logits_keys + one-cluster
-k_select pair (variant 1, with its in-kernel phase stamps)."""
+grapes_select_topk (k_select_fused, one launch on every SM) with its in-kernel phase stamps."""
 import ctypes, os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -10,8 +9,7 @@ from grapes_b200.utils import _any_ctx
 def main():
     dev = torch.device("cuda", 0)
     L = lib(); ctx = _any_ctx(dev).ctx
-    for variant, c in ((v, c) for c in (8192, 65536, 150000) for v in (0, 1)):
-        L.cdll.grapes_select_variant(variant)
+    for c in (8192, 65536, 150000):
         k = 256
         logits = torch.randn(c, device=dev) * 2
         nb = torch.arange(c, device=dev, dtype=torch.int32)
@@ -34,23 +32,12 @@ def main():
         e0.record()
         for _ in range(20): run()
         e1.record(); torch.cuda.synchronize()
-        out = (ctypes.c_int64 * 16)()
-        L.cdll.grapes_debug_select_stamps(out)
-        t = list(out)
-        names = {0: "start", 1: "bucket found", 2: "members gathered", 3: "threshold", 4: "counts exchanged", 5: "outputs", 6: "end"}
-        rel = {names[i]: round((t[i] - t[0]) / 1e3, 2) for i in sorted(names) if t[i]}
-        torch.manual_seed(0)
-        ref = torch.sort(sampled[:k]).values.clone()
-        if variant == 0:
-            o8 = (ctypes.c_int64 * 8)()
-            L.cdll.grapes_debug_select_fused_stamps(ctx, ctypes.c_void_p(work.data_ptr()), c, o8)
-            t8 = list(o8)
-            n8 = ["start", "keys done", "hist merged", "barrier 1", "members listed", "barrier 2", "outputs done", "last block done"]
-            rel = {n8[i]: round((t8[i] - t8[0]) / 1e3, 2) for i in range(8)}
-        tag = "fused (one launch, every SM)" if variant == 0 else "k_logits_keys + one-cluster k_select"
-        print(f"c={c} variant {variant} [{tag}]: {e0.elapsed_time(e1) / 20 * 1e3:.1f} us per select"
-              + f"; stamps us: {rel}")
-    L.cdll.grapes_select_variant(0)
+        o8 = (ctypes.c_int64 * 8)()
+        L.cdll.grapes_debug_select_fused_stamps(ctx, ctypes.c_void_p(work.data_ptr()), c, o8)
+        t8 = list(o8)
+        n8 = ["start", "keys done", "hist merged", "barrier 1", "members listed", "barrier 2", "outputs done", "last block done"]
+        rel = {n8[i]: round((t8[i] - t8[0]) / 1e3, 2) for i in range(8)}
+        print(f"c={c}: {e0.elapsed_time(e1) / 20 * 1e3:.1f} us per select; stamps us: {rel}")
 
 if __name__ == "__main__":
     main()

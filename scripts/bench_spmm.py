@@ -1,6 +1,7 @@
 """Full-graph SpMM micro-benchmark (SURVEY.md section 8 f1: eval.py:47-70 aggregates over the WHOLE graph):
-Y = A_hat X on the products-shaped graph, every aggregation variant, bitwise compared with the register-staged
-kernel and timed with CUDA events.  Also the frontier-shaped gather (n rows, ~1 source each)."""
+Y = A_hat X on the products-shaped graph with the default aggregation (form chosen by shape) and with the register-staged
+kernels (grapes_agg_variant 1), bitwise compared and timed with CUDA events.  Also the frontier-shaped gather (n rows,
+~1 source each)."""
 import os, sys, json
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -37,7 +38,7 @@ def run(L, ctx, X, F, nodes, n, in_off, in_src, dinv, variant, reps=5, hi_lo=Fal
 
 def main():
     which = sys.argv[1] if len(sys.argv) > 1 else "products"
-    variants = [int(v) for v in (sys.argv[2].split(",") if len(sys.argv) > 2 else "0,132,216,208,116".split(","))]
+    variants = (0, 1)
     dev = torch.device("cuda", 0)
     cfg, indptr, indices, x, y, train_idx = build_workload(which, 0, dev)
     N, F = cfg["N"], cfg["F"]
@@ -82,21 +83,16 @@ def main():
         _, ms2 = run(L, g.ctx, x, F, nodes, n, off, src, dv, v, reps=9, hi_lo=False, ldo=ldo)
         _, ms3 = run(L, g.ctx, x, F, nodes, n, off, src, dv, v, reps=9, hi_lo=True, ldo=ldo, do_flush=False)
         print(f"hop-shaped v{v}: {ms*1e3:.2f} us  equal={same}  algorithmic {alg/ms/1e6:.0f} GB/s; single fp32 output {ms2*1e3:.2f} us; hi/lo warm L2 {ms3*1e3:.2f} us", flush=True)
-    # ---- the engine's hop aggregation itself: indicator columns + ones column, (hi, lo) output; pad columns through the
-    # float4 lanes (virtual slot, opt-in) against one scalar lane per pad column (default) ----
+    # ---- the engine's hop aggregation itself: indicator columns + ones column, (hi, lo) output ----
     bits = torch.randint(0, 16, (n,), generator=gen, device=dev, dtype=torch.int32)
     ldo2 = ((F + 4 + 1 + 3) // 4) * 4
     cnt = torch.tensor([n], dtype=torch.int32, device=dev)
     hi, lo = torch.zeros(n, ldo2, device=dev), torch.zeros(n, ldo2, device=dev)
     st = torch.cuda.current_stream().cuda_stream
-    L.cdll.grapes_agg_variant(0)
     flush = torch.zeros(256 << 20, dtype=torch.uint8, device=dev)
     keep = {}
-    vlist = [int(v) for v in os.environ.get("HOP_VARIANTS", "0").split(",")]
-    for vs in [(a, b) for b in vlist for a in (1, 0)]:
-        L.cdll.grapes_agg_variant(vs[1])
-        vs, vtag = vs[0], f"{vs[0]}_v{vs[1]}"
-        L.cdll.grapes_agg_tma_virtual_slot(vs)
+    for v in variants:
+        L.cdll.grapes_agg_variant(v)
         ts = []
         for it in range(12):
             flush.sum()
@@ -107,12 +103,10 @@ def main():
             e1.record(); torch.cuda.synchronize()
             if it: ts.append(e0.elapsed_time(e1))
         ts.sort()
-        keep[vs] = (hi.clone(), lo.clone())
-        vs = vtag
+        keep[v] = (hi.clone(), lo.clone())
         alg = 4.0 * n * (F + ldo2) + 12.0 * n + 4.0 * n
-        res[f"hop_ind_virtual_slot_{vs}"] = {"us": round(ts[len(ts) // 2] * 1e3, 2), "alg_GBps": round(alg / ts[len(ts) // 2] / 1e6, 1)}
-        print(f"hop aggregation with indicators, virtual_slot={vs}: {ts[len(ts)//2]*1e3:.2f} us", flush=True)
-    L.cdll.grapes_agg_tma_virtual_slot(0)
+        res[f"hop_ind_v{v}"] = {"us": round(ts[len(ts) // 2] * 1e3, 2), "alg_GBps": round(alg / ts[len(ts) // 2] / 1e6, 1)}
+        print(f"hop aggregation with indicators v{v}: {ts[len(ts)//2]*1e3:.2f} us", flush=True)
     L.cdll.grapes_agg_variant(0)
     res["hop_ind_bitwise_equal"] = bool(torch.equal(keep[0][0], keep[1][0]) and torch.equal(keep[0][1], keep[1][1]))
     print(json.dumps(res))

@@ -266,27 +266,6 @@ def test_step_parity_bf16_feature_table(cuda_device, name, seed, tc):
     _check_step(st, eng, train_idx[:B], cuda_device, apply_optim=False)
 
 
-def test_fused_hop_structure_kernel_is_bit_identical(cuda_device):
-    """grapes_hop_structure (one cooperative launch, grid barriers between rank / relabel / scan / fill / sort) against
-    the five separate launches: every integer output and the aggregated features bit for bit."""
-    d, st, eng, train_idx, B = _setup("small", 5, cuda_device, use_tensor_cores=True)
-    t = train_idx[:B].to(cuda_device)
-    noise = [torch.rand(eng.cap_n, device=cuda_device).clamp_(1e-6, 1 - 1e-6).log().neg().log().neg() for _ in range(eng.H)]
-    eng.fused_struct = False
-    r0 = eng.step(t, gumbel_noise=noise, apply_optim=False, record=True)
-    eng.fused_struct = True
-    r1 = eng.step(t, gumbel_noise=noise, apply_optim=False, record=True)
-    eng.check_overflow()
-    for a, b in zip(r0["hops"], r1["hops"]):
-        for key in ("batch_nodes", "neighbor_nodes", "nb_local", "ind_bits", "e_src", "e_dst", "in_off", "in_src", "dinv",
-                    "Y", "sampled", "block_edges", "logits_all", "log_prob"):
-            assert torch.equal(a[key], b[key]), key
-    assert torch.equal(r0["all_nodes"], r1["all_nodes"])
-    for net in r0["grads"]:
-        for name in r0["grads"][net]:
-            assert torch.equal(r0["grads"][net][name], r1["grads"][net][name]), (net, name)
-
-
 def test_node_capacity_overflow_is_flagged_and_memory_safe(cuda_device):
     """A caller-chosen cap_nodes smaller than the frontier: the step must raise GRAPES_OVF_NODES (in the overflow word and
     in the step's flag scalar) and stay inside every buffer -- checked under compute-sanitizer memcheck with GRAPES_SANITIZE=1."""

@@ -81,9 +81,8 @@ def test_gcn_input_gradient(cuda_device):
 
 @pytest.mark.parametrize("F,num_ind,ones", [(100, 4, True), (36, 4, True), (100, 3, False), (64, 8, True), (256, 3, True)])
 @pytest.mark.parametrize("hi_lo", [False, True])
-def test_agg_tma_virtual_columns_bit_identical(cuda_device, F, num_ind, ones, hi_lo):
-    """The TMA-staged aggregation with the pad columns (indicators | ones | zeros) carried by the float4 lanes
-    (grapes_agg_tma_virtual_slot 1, opt-in) == one scalar lane per pad column (0, default) == the register-staged kernel
+def test_agg_tma_pad_columns_bit_identical_to_register_staged(cuda_device, F, num_ind, ones, hi_lo):
+    """The TMA-staged aggregation with its pad columns (indicators | ones | zeros) == the register-staged kernel
     (grapes_agg_variant 1), bit for bit; the indicator columns equal the weighted sums of the source bits."""
     from grapes_b200._lib import lib, ptr
     from grapes_b200.graph import DeviceGraph
@@ -116,19 +115,15 @@ def test_agg_tma_virtual_columns_bit_identical(cuda_device, F, num_ind, ones, hi
         torch.cuda.synchronize()
         return (a, b) if hi_lo else (a,)
     try:
-        L.cdll.grapes_agg_tma_virtual_slot(1)
-        y_vs = run()
-        L.cdll.grapes_agg_tma_virtual_slot(0)
-        y_scalar = run()
+        y_tma = run()
         L.cdll.grapes_agg_variant(1)
         y_reg = run()
     finally:
         L.cdll.grapes_agg_variant(0)
-        L.cdll.grapes_agg_tma_virtual_slot(0)
-    for a, b, c in zip(y_vs, y_scalar, y_reg):
+    for a, b in zip(y_tma, y_reg):
         assert not torch.isnan(a).any()
-        assert torch.equal(a, b) and torch.equal(a, c)
-    y = y_vs[0] + y_vs[1] if hi_lo else y_vs[0]
+        assert torch.equal(a, b)
+    y = y_tma[0] + y_tma[1] if hi_lo else y_tma[0]
     # reference of the pad columns in float64
     w_self = dinv.double() ** 2
     bitf = torch.stack([((bits >> i) & 1).double() for i in range(num_ind)], 1)
