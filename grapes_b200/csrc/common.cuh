@@ -95,11 +95,12 @@ static inline PdlLaunch<K> pdl(K kernel, dim3 grid, dim3 block, size_t smem = 0,
 #endif
 
 #ifdef __CUDACC__
-// spmm_tma.cu: 0 = launched, 1 = shape not covered (the caller falls back to the register-staged kernels)
+// spmm_tma.cu: 0 = launched, 1 = shape not covered (the caller falls back to the register-staged kernels).  in_off is int
+// (off64 = 0) or the int64 offsets of a row slab (off64 = 1: n_dev = {R, r0}, out only, no indicator columns)
 int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int ldx, const int* nodes, const int* n_dev, int cap_n,
-                          const int* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits, int num_ind,
+                          const void* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits, int num_ind,
                           const float* bias, int relu, float* out, int ldo, float* out_hi, float* out_lo, int ones_col,
-                          int ec_req, int ctas_per_sm, cudaStream_t s);
+                          int ec_req, int ctas_per_sm, cudaStream_t s, int off64 = 0);
 #endif
 
 static inline int grapes_div_up(long long a, long long b) { return (int)((a + b - 1) / b); }
@@ -174,6 +175,11 @@ __device__ __forceinline__ uint32_t dropout_keep4(unsigned long long seed, unsig
 __device__ __forceinline__ float grapes_tf32_rna(float x) {
     return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u);
 }
+
+// element type of a CSR row-offset array: int for the sampled blocks and graphs below 2^31 entries, int64 (W64) for the
+// whole-graph structure of larger graphs (grapes_graph_norm_*)
+template <bool W64> struct GrapesOff { typedef int T; };
+template <> struct GrapesOff<true> { typedef long long T; };
 
 // local id of global node v: rank of bit v in the bitmap (pref = exclusive popcount prefix per word)
 __device__ __forceinline__ int bitmap_rank(const uint32_t* __restrict__ bm, const int* __restrict__ pref, int v) {

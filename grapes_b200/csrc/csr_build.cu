@@ -30,6 +30,8 @@
 #define CB_MED_THREADS 256
 #define CB_LONG_THREADS 1024
 
+static inline size_t cb_align(size_t x) { return (x + 255) & ~(size_t)255; }
+
 // ---------------------------------------------------------------------------------------------------------------------
 // 64-bit exclusive scan of int32 counts: tile sums -> one CTA scans the tile sums -> tiles rescan with their offset.
 // ---------------------------------------------------------------------------------------------------------------------
@@ -196,10 +198,7 @@ __global__ void __launch_bounds__(CB_THREADS) k_csr_scatter_part(const unsigned 
 // Sort + unique of a row of d <= 32 K entries held K per lane (entry i in register i / 32 of lane i % 32): the ascending-only
 // bitonic network with shuffles for strides < 32 and register-to-register exchanges above; +inf pads the tail.
 template <int K>
-__device__ __forceinline__ int cb_warp_sort_unique(int* __restrict__ row, int d, int lane) {
-    int v[K];
-#pragma unroll
-    for (int j = 0; j < K; ++j) v[j] = (j * 32 + lane < d) ? row[j * 32 + lane] : 0x7fffffff;
+__device__ __forceinline__ void cb_warp_bitonic(int (&v)[K], int lane) {
 #pragma unroll
     for (int size = 2; size <= 32 * K; size <<= 1) {
         if (size <= 32) {                                   // flip step inside a register: partner = lane ^ (size - 1)
@@ -243,6 +242,14 @@ __device__ __forceinline__ int cb_warp_sort_unique(int* __restrict__ row, int d,
             }
         }
     }
+}
+
+template <int K>
+__device__ __forceinline__ int cb_warp_sort_unique(int* __restrict__ row, int d, int lane) {
+    int v[K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) v[j] = (j * 32 + lane < d) ? row[j * 32 + lane] : 0x7fffffff;
+    cb_warp_bitonic<K>(v, lane);
     int base = 0;
 #pragma unroll
     for (int j = 0; j < K; ++j) {
@@ -258,6 +265,28 @@ __device__ __forceinline__ int cb_warp_sort_unique(int* __restrict__ row, int d,
         base += __popc(m);
     }
     return base;
+}
+
+// ascending-only bitonic network over a[0 .. d) in shared memory, one warp (rows of 129 .. CB_WARP_MAX entries)
+__device__ __forceinline__ void cb_warp_bitonic_smem(int* a, int d, int lane) {
+    int P = 64;
+    while (P < d) P <<= 1;
+    for (int size = 2; size <= P; size <<= 1) {
+        const int half = size >> 1;
+        for (int p = lane; p < (P >> 1); p += 32) {
+            const int blk = p / half, off = p - blk * half;
+            const int i = blk * size + off, j = blk * size + size - 1 - off;
+            if (j < d) { const int x = a[i], y = a[j]; if (x > y) { a[i] = y; a[j] = x; } }
+        }
+        __syncwarp();
+        for (int st = size >> 2; st > 0; st >>= 1) {
+            for (int p = lane; p < (P >> 1); p += 32) {
+                const int i = 2 * st * (p / st) + (p % st), j = i + st;
+                if (j < d) { const int x = a[i], y = a[j]; if (x > y) { a[i] = y; a[j] = x; } }
+            }
+            __syncwarp();
+        }
+    }
 }
 
 __global__ void __launch_bounds__(CB_THREADS) k_csr_sort_short(int64_t N, const long long* __restrict__ raw_off,
@@ -283,24 +312,7 @@ __global__ void __launch_bounds__(CB_THREADS) k_csr_sort_short(int64_t N, const 
             // network as cb_bitonic, __syncwarp between stages), then writes the unique values back in order
             for (int i = lane; i < d; i += 32) a[i] = tmp[o + i];
             __syncwarp();
-            int P = 64;
-            while (P < d) P <<= 1;
-            for (int size = 2; size <= P; size <<= 1) {
-                const int half = size >> 1;
-                for (int p = lane; p < (P >> 1); p += 32) {
-                    const int blk = p / half, off = p - blk * half;
-                    const int i = blk * size + off, j = blk * size + size - 1 - off;
-                    if (j < d) { const int x = a[i], y = a[j]; if (x > y) { a[i] = y; a[j] = x; } }
-                }
-                __syncwarp();
-                for (int st = size >> 2; st > 0; st >>= 1) {
-                    for (int p = lane; p < (P >> 1); p += 32) {
-                        const int i = 2 * st * (p / st) + (p % st), j = i + st;
-                        if (j < d) { const int x = a[i], y = a[j]; if (x > y) { a[i] = y; a[j] = x; } }
-                    }
-                    __syncwarp();
-                }
-            }
+            cb_warp_bitonic_smem(a, d, lane);
             int base = 0;
             for (int i0 = 0; i0 < d; i0 += 32) {
                 const int i = i0 + lane;
@@ -412,9 +424,154 @@ __global__ void __launch_bounds__(CB_THREADS) k_csr_compact(int64_t N, const lon
     }
 }
 
-int g_csr_direct_scatter = 0;      // 0 = by shape, 1 = single-pass random scatter, 2 = partition + windowed scatter (A/B)
+// ---------------------------------------------------------------------------------------------------------------------
+// Whole-graph gcn_norm structure with int64 offsets (grapes_graph_norm_*): the transposed adjacency, in_off [N+1] int64,
+// in_src int32 (sources ascending, stored self-loops dropped, duplicates kept), dinv = (indeg + 1)^-1/2.  A counting sort by
+// destination read straight from the input (CSR rows or int64 edge chunks, no expanded copy), then per-row sorts with the
+// tiers above, without the unique step.  Scratch: cnt int32 [N] (in-degree -> scatter cursor -> sort worklist), tile sums
+// of the 64-bit scan, 4 flags.
+// ---------------------------------------------------------------------------------------------------------------------
+#define GN_ERR_ID 1                  // an id outside [0, N): the edge is skipped, the caller raises
+#define GN_ERR_DEG 2                 // a node with >= 2^31 - 1 in-edges: not representable, the caller raises
 
-static inline size_t cb_align(size_t x) { return (x + 255) & ~(size_t)255; }
+template <bool SCATTER>
+__device__ __forceinline__ void gn_edge(int64_t r, int64_t c, int64_t N, int* __restrict__ cnt,
+                                        const long long* __restrict__ in_off, int* __restrict__ in_src, int* __restrict__ err) {
+    if (r < 0 || r >= N || c < 0 || c >= N) { if (!SCATTER) atomicOr(err, GN_ERR_ID); return; }
+    if (r == c) return;                                              // stored self-loop: dropped (one is added per node)
+    const int k = atomicAdd(&cnt[c], 1);
+    if (SCATTER) in_src[in_off[c] + k] = (int)r;
+    else if (k == 0x7ffffffe) atomicOr(err, GN_ERR_DEG);
+}
+
+// CSR rows [r0, r1): row r is the source, its indices the destinations; one warp per row
+template <bool SCATTER>
+__global__ void __launch_bounds__(CB_THREADS) k_gn_csr(const long long* __restrict__ indptr, const int* __restrict__ indices,
+                                                        int64_t r0, int64_t r1, int64_t N, int* __restrict__ cnt,
+                                                        const long long* __restrict__ in_off, int* __restrict__ in_src,
+                                                        int* __restrict__ err) {
+    const int lane = lane_id();
+    const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t r = r0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); r < r1; r += warps) {
+        const long long e1 = indptr[r + 1];
+        for (long long e = indptr[r] + lane; e < e1; e += 32) gn_edge<SCATTER>(r, indices[e], N, cnt, in_off, in_src, err);
+    }
+}
+
+// edge chunk: src[e] -> dst[e], e < n (a slice of the int64 rows of edge_index)
+template <bool SCATTER>
+__global__ void __launch_bounds__(CB_THREADS) k_gn_edges(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
+                                                          int64_t n, int64_t N, int* __restrict__ cnt,
+                                                          const long long* __restrict__ in_off, int* __restrict__ in_src,
+                                                          int* __restrict__ err) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += stride)
+        gn_edge<SCATTER>(src[e], dst[e], N, cnt, in_off, in_src, err);
+}
+
+// dinv = (indeg + 1)^-1/2 with correctly rounded sqrt and divide (torch's 1.0 / sqrt(float)); cnt becomes the cursor
+__global__ void __launch_bounds__(CB_THREADS) k_gn_dinv(int64_t N, int* __restrict__ cnt, float* __restrict__ dinv) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride) {
+        dinv[i] = __fdiv_rn(1.f, __fsqrt_rn((float)((long long)cnt[i] + 1)));
+        cnt[i] = 0;
+    }
+}
+
+// rows of <= CB_WARP_MAX entries: one warp each, in registers (<= 128) or a shared-memory strip; longer rows are listed
+// for k_gn_sort_rows (medium from the front of the worklist, long from the back)
+__global__ void __launch_bounds__(CB_THREADS) k_gn_sort_short(int64_t N, const long long* __restrict__ in_off,
+                                                               int* __restrict__ in_src, int* __restrict__ worklist,
+                                                               int* __restrict__ wl_count) {
+    __shared__ int s_rows[CB_THREADS / 32][CB_WARP_MAX];
+    const int lane = lane_id();
+    int* a = s_rows[threadIdx.x >> 5];
+    const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < N; r += warps) {
+        const long long o = in_off[r];
+        const int d = (int)(in_off[r + 1] - o);
+        int* row = in_src + o;
+        if (d <= 1) continue;
+        if (d > CB_WARP_MAX) {
+            if (lane == 0) {
+                if (d <= CB_MED_MAX) worklist[atomicAdd(&wl_count[0], 1)] = (int)r;
+                else worklist[N - 1 - atomicAdd(&wl_count[1], 1)] = (int)r;
+            }
+            continue;
+        }
+        if (d > 128) {
+            for (int i = lane; i < d; i += 32) a[i] = row[i];
+            __syncwarp();
+            cb_warp_bitonic_smem(a, d, lane);
+            for (int i = lane; i < d; i += 32) row[i] = a[i];
+            __syncwarp();
+            continue;
+        }
+        if (d <= 32) {
+            int v[1] = {lane < d ? row[lane] : 0x7fffffff};
+            cb_warp_bitonic<1>(v, lane);
+            if (lane < d) row[lane] = v[0];
+        } else if (d <= 64) {
+            int v[2];
+#pragma unroll
+            for (int j = 0; j < 2; ++j) v[j] = (j * 32 + lane < d) ? row[j * 32 + lane] : 0x7fffffff;
+            cb_warp_bitonic<2>(v, lane);
+#pragma unroll
+            for (int j = 0; j < 2; ++j) if (j * 32 + lane < d) row[j * 32 + lane] = v[j];
+        } else {
+            int v[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) v[j] = (j * 32 + lane < d) ? row[j * 32 + lane] : 0x7fffffff;
+            cb_warp_bitonic<4>(v, lane);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) if (j * 32 + lane < d) row[j * 32 + lane] = v[j];
+        }
+    }
+}
+
+template <int THREADS, int SMEM_INTS, bool LONG>
+__global__ void __launch_bounds__(THREADS) k_gn_sort_rows(int64_t N, const long long* __restrict__ in_off,
+                                                           int* __restrict__ in_src, const int* __restrict__ worklist,
+                                                           const int* __restrict__ wl_count) {
+    extern __shared__ int cb_sm[];
+    const int cnt = wl_count[LONG ? 1 : 0];
+    for (int w = blockIdx.x; w < cnt; w += gridDim.x) {
+        const int r = LONG ? worklist[N - 1 - w] : worklist[w];
+        const long long o = in_off[r];
+        const int d = (int)(in_off[r + 1] - o);
+        int* row = in_src + o;
+        if (d <= SMEM_INTS) {
+            for (int i = threadIdx.x; i < d; i += THREADS) cb_sm[i] = row[i];
+            __syncthreads();
+            cb_bitonic(cb_sm, d);
+            for (int i = threadIdx.x; i < d; i += THREADS) row[i] = cb_sm[i];
+        } else {
+            __syncthreads();
+            cb_bitonic(row, d);                           // hub row: in place in HBM
+        }
+        __syncthreads();
+    }
+}
+
+struct GnLayout { size_t cnt, tile_sum, flags, total; };
+static GnLayout gn_layout(int64_t N) {
+    GnLayout L;
+    size_t o = 0;
+    L.cnt = o; o += cb_align(sizeof(int) * (size_t)N);
+    L.tile_sum = o; o += cb_align(sizeof(long long) * ((size_t)((N + CB_SCAN_TILE - 1) / CB_SCAN_TILE) + 1));
+    L.flags = o; o += cb_align(sizeof(int) * 4);
+    L.total = o;
+    return L;
+}
+
+static int gn_sms(int* sms) {
+    int dev = 0;
+    GRAPES_CUDA_OK(cudaGetDevice(&dev));
+    GRAPES_CUDA_OK(cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev));
+    return GRAPES_OK;
+}
+
+int g_csr_direct_scatter = 0;      // 0 = by shape, 1 = single-pass random scatter, 2 = partition + windowed scatter (A/B)
 
 struct CbLayout {
     size_t deg, ucount, raw_off, tile_sum, worklist, flags, bucket_fill, tmp, pairs, total;
@@ -525,6 +682,118 @@ int grapes_csr_from_edges(const int64_t* src, const int64_t* dst, int64_t num_ed
     cb_scan64(ucount, N, tile_sum, (long long*)indptr, (long long*)nnz_dev, s);
     pdl(k_csr_compact, row_grid, CB_THREADS, 0, s)(N, raw_off, tmp, (const long long*)indptr, indices);
     grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+
+int64_t grapes_graph_norm_workspace_bytes(int64_t num_nodes) {
+    if (num_nodes <= 0) return 0;
+    return (int64_t)gn_layout(num_nodes).total;
+}
+
+int grapes_graph_norm_begin(int64_t num_nodes, void* workspace, int64_t workspace_bytes, int* err_dev, void* stream) {
+    GRAPES_REQUIRE(num_nodes > 0 && num_nodes < (1ll << 31), "num_nodes must fit int32");
+    GRAPES_REQUIRE(workspace && err_dev, "null argument");
+    const GnLayout L = gn_layout(num_nodes);
+    GRAPES_REQUIRE(workspace_bytes >= (int64_t)L.total, "workspace smaller than grapes_graph_norm_workspace_bytes()");
+    cudaStream_t s = (cudaStream_t)stream;
+    GRAPES_CUDA_OK(cudaMemsetAsync((unsigned char*)workspace + L.cnt, 0, sizeof(int) * (size_t)num_nodes, s));
+    GRAPES_CUDA_OK(cudaMemsetAsync((unsigned char*)workspace + L.flags, 0, sizeof(int) * 4, s));
+    GRAPES_CUDA_OK(cudaMemsetAsync(err_dev, 0, sizeof(int), s));
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_add_csr(int pass, int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0, int64_t r1,
+                              int64_t* in_off, int* in_src, void* workspace, int* err_dev, void* stream) {
+    GRAPES_REQUIRE(pass == 0 || pass == 1, "pass is 0 (count) or 1 (scatter)");
+    GRAPES_REQUIRE(indptr && workspace && err_dev && (pass == 0 || (in_off && in_src)), "null argument");
+    GRAPES_REQUIRE(0 <= r0 && r0 <= r1 && r1 <= num_nodes, "row range outside [0, N]");
+    if (r1 == r0) return GRAPES_OK;
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    int* cnt = (int*)((unsigned char*)workspace + gn_layout(num_nodes).cnt);
+    const int64_t ctas = ((r1 - r0) * 32 + CB_THREADS - 1) / CB_THREADS;
+    const int grid = (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (pass == 0)
+        pdl(k_gn_csr<false>, grid, CB_THREADS, 0, s)((const long long*)indptr, indices, r0, r1, num_nodes, cnt, nullptr,
+                                                      nullptr, err_dev);
+    else
+        pdl(k_gn_csr<true>, grid, CB_THREADS, 0, s)((const long long*)indptr, indices, r0, r1, num_nodes, cnt,
+                                                     (const long long*)in_off, in_src, err_dev);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_add_edges(int pass, int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                int64_t* in_off, int* in_src, void* workspace, int* err_dev, void* stream) {
+    GRAPES_REQUIRE(pass == 0 || pass == 1, "pass is 0 (count) or 1 (scatter)");
+    GRAPES_REQUIRE(num_edges >= 0, "negative edge count");
+    GRAPES_REQUIRE(workspace && err_dev && (num_edges == 0 || (src && dst)) && (pass == 0 || (in_off && in_src)),
+                   "null argument");
+    if (num_edges == 0) return GRAPES_OK;
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    int* cnt = (int*)((unsigned char*)workspace + gn_layout(num_nodes).cnt);
+    const int64_t ctas = (num_edges + CB_THREADS - 1) / CB_THREADS;
+    const int grid = (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (pass == 0)
+        pdl(k_gn_edges<false>, grid, CB_THREADS, 0, s)(src, dst, num_edges, num_nodes, cnt, nullptr, nullptr, err_dev);
+    else
+        pdl(k_gn_edges<true>, grid, CB_THREADS, 0, s)(src, dst, num_edges, num_nodes, cnt, (const long long*)in_off, in_src,
+                                                       err_dev);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_offsets(int64_t num_nodes, void* workspace, int64_t* in_off, float* dinv, int64_t* nnz_dev,
+                              void* stream) {
+    GRAPES_REQUIRE(workspace && in_off && dinv && nnz_dev, "null argument");
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    const GnLayout L = gn_layout(num_nodes);
+    unsigned char* ws = (unsigned char*)workspace;
+    int* cnt = (int*)(ws + L.cnt);
+    cudaStream_t s = (cudaStream_t)stream;
+    cb_scan64(cnt, num_nodes, (long long*)(ws + L.tile_sum), (long long*)in_off, (long long*)nnz_dev, s);
+    const int64_t ctas = (num_nodes + CB_THREADS - 1) / CB_THREADS;
+    pdl(k_gn_dinv, (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16), CB_THREADS, 0, s)(num_nodes, cnt, dinv);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_finish(int64_t num_nodes, const int64_t* in_off, int* in_src, void* workspace, void* stream) {
+    GRAPES_REQUIRE(in_off && in_src && workspace, "null argument");
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    const GnLayout L = gn_layout(num_nodes);
+    unsigned char* ws = (unsigned char*)workspace;
+    int* worklist = (int*)(ws + L.cnt);                   // the cursor is spent after the scatter pass
+    int* flags = (int*)(ws + L.flags);
+    const long long* off = (const long long*)in_off;
+    cudaStream_t s = (cudaStream_t)stream;
+    GRAPES_CUDA_OK(cudaMemsetAsync(flags, 0, sizeof(int) * 2, s));
+    const int64_t row_ctas = (num_nodes * 32 + CB_THREADS - 1) / CB_THREADS;
+    pdl(k_gn_sort_short, (int)(row_ctas < (int64_t)sms * 16 ? row_ctas : (int64_t)sms * 16), CB_THREADS, 0, s)(
+        num_nodes, off, in_src, worklist, flags);
+    {
+        static bool configured = false;
+        if (!configured) {
+            GRAPES_CUDA_OK(cudaFuncSetAttribute(k_gn_sort_rows<CB_LONG_THREADS, CB_LONG_SMEM, true>,
+                                                cudaFuncAttributeMaxDynamicSharedMemorySize, CB_LONG_SMEM * 4));
+            configured = true;
+        }
+    }
+    pdl((k_gn_sort_rows<CB_MED_THREADS, CB_MED_MAX, false>), sms * 8, CB_MED_THREADS, CB_MED_MAX * 4, s)(
+        num_nodes, off, in_src, worklist, flags);
+    pdl((k_gn_sort_rows<CB_LONG_THREADS, CB_LONG_SMEM, true>), sms, CB_LONG_THREADS, CB_LONG_SMEM * 4, s)(
+        num_nodes, off, in_src, worklist, flags);
+    grapes_count_launches(3);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
 }

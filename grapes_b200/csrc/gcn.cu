@@ -57,22 +57,28 @@ __device__ __forceinline__ void vec_fma_x(float (&acc)[VEC], float w, const void
 // Sources are preloaded 32 at a time and broadcast by shuffle so the dependent chain
 // in_src -> nodes -> X is paid once per 32 sources.
 // ---------------------------------------------------------------------------------------
-template <int VEC, bool XB16 = false>
+// W64: a row slab of the whole-graph structure past 2^31 entries, as in k_agg_tma (n_dev = {R, r0}, output row j is graph
+// row r0 + j, int64 in_off indexed by graph row, nodes null); the same fma chain as the int32 form.
+template <int VEC, bool XB16 = false, bool W64 = false>
 __global__ void __launch_bounds__(256) k_agg(const void* __restrict__ X, int F, int ldx,
                                              const int* __restrict__ nodes, const int* __restrict__ n_dev, int cap_n,
-                                             const int* __restrict__ in_off, const int* __restrict__ in_src,
+                                             const typename GrapesOff<W64>::T* __restrict__ in_off,
+                                             const int* __restrict__ in_src,
                                              const float* __restrict__ dinv, const uint32_t* __restrict__ ind_bits,
                                              int num_ind, const float* __restrict__ bias, int relu,
                                              float* __restrict__ out, int ldo, float* __restrict__ out_hi,
                                              float* __restrict__ out_lo, int ones_col) {
+    typedef typename GrapesOff<W64>::T OffT;
     pdl_begin();
     const int n = min(*n_dev, cap_n);
+    const int r0 = W64 ? n_dev[1] : 0;
     const int lane = lane_id();
     const int warps = (gridDim.x * blockDim.x) >> 5;
     for (int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += warps) {
-        const float dj = dinv[j];
-        const int beg = in_off[j], end = in_off[j + 1];
-        const size_t gj = nodes ? (size_t)nodes[j] : (size_t)j;
+        const int jr = r0 + j;                               // row of in_off / dinv / X
+        const float dj = dinv[jr];
+        const OffT beg = in_off[jr], end = in_off[jr + 1];
+        const size_t gj = nodes ? (size_t)nodes[j] : (size_t)jr;
         float* oj = out ? out + (size_t)j * ldo : nullptr;
         float* ohj = out_hi ? out_hi + (size_t)j * ldo : nullptr;
         float* olj = out_hi ? out_lo + (size_t)j * ldo : nullptr;
@@ -83,15 +89,15 @@ __global__ void __launch_bounds__(256) k_agg(const void* __restrict__ X, int F, 
 #pragma unroll
             for (int i = 0; i < VEC; ++i) acc[i] = 0.f;
             if (act) vec_fma_x<VEC, XB16>(acc, dj * dj, X, gj * ldx + c0);
-            for (int pb = beg; pb < end; pb += 32) {
-                const int p = pb + lane;
+            for (OffT pb = beg; pb < end; pb += 32) {
+                const OffT p = pb + lane;
                 float w = 0.f; unsigned long long sg = 0ull;
                 if (p < end) {
                     const int sl = in_src[p];
                     w = dinv[sl] * dj;
                     sg = nodes ? (unsigned long long)nodes[sl] : (unsigned long long)sl;
                 }
-                const int cnt = min(32, end - pb);
+                const int cnt = (int)min((OffT)32, end - pb);
                 for (int t = 0; t < cnt; ++t) {
                     const float wt = __shfl_sync(GRAPES_FULL_MASK, w, t);
                     const unsigned long long st = __shfl_sync(GRAPES_FULL_MASK, sg, t);
@@ -120,7 +126,7 @@ __global__ void __launch_bounds__(256) k_agg(const void* __restrict__ X, int F, 
             float a = 0.f;
             if (lane < num_ind) {
                 a = dj * dj * (float)((ind_bits[j] >> lane) & 1u);
-                for (int p = beg; p < end; ++p) {
+                for (OffT p = beg; p < end; ++p) {
                     const int sl = in_src[p];
                     a = fmaf(dinv[sl] * dj, (float)((ind_bits[sl] >> lane) & 1u), a);
                 }
@@ -1146,6 +1152,54 @@ int grapes_aggregate_bf16(grapes_ctx* ctx, const void* X_bf16, int F, int ldx, c
                           int ones_col, void* stream) {
     return aggregate_impl(ctx, X_bf16, 1, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias, relu,
                           out, ldo, out_hi, out_lo, ones_col, stream);
+}
+
+int grapes_aggregate_rows64(grapes_ctx* ctx, const void* X, int x_bf16, int F, int ldx, const int* slab_dev, int cap_r,
+                            const int64_t* in_off, const int* in_src, const float* dinv, const float* bias, float* out,
+                            int ldo, void* stream) {
+    GRAPES_REQUIRE(ctx && X && slab_dev && in_off && in_src && dinv && out, "null argument");
+    GRAPES_REQUIRE(F > 0 && ldx >= F && ldo >= F, "bad shape");
+    if (cap_r <= 0) return GRAPES_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    const long long* off = reinterpret_cast<const long long*>(in_off);
+    const bool shaped = g_agg_variant == 0;
+    const bool whole = cap_r > (1 << 19);
+    const size_t al = ((size_t)X) | ((size_t)out);
+    const bool a16 = (al & 15) == 0, a8 = (al & 7) == 0;
+    // the forms and launch shapes grapes_aggregate / grapes_aggregate_bf16 pick for a whole graph of cap_r rows
+    bool launched = false;
+    if (shaped && a16) {
+        if (x_bf16) {
+            if (cap_r >= 4096)
+                launched = grapes_launch_agg_tma(ctx, X, 1, F, ldx, nullptr, slab_dev, cap_r, off, in_src, dinv, nullptr, 0,
+                                                 bias, 0, out, ldo, nullptr, nullptr, -1, whole ? 32 : 16, whole ? 1 : 2, s,
+                                                 1) == 0;
+        } else if ((F % 4 != 0) && (ldx % 4 == 0) && ldx >= ((F + 3) & ~3) && (ldo % 4 == 0) && (ldo - F <= 32) &&
+                   cap_r >= 256) {
+            launched = grapes_launch_agg_tma(ctx, X, 0, F, ldx, nullptr, slab_dev, cap_r, off, in_src, dinv, nullptr, 0,
+                                             bias, 0, out, ldo, nullptr, nullptr, -1, whole ? 32 : 16, whole ? 1 : 2, s, 1) == 0;
+        } else if ((F % 4 == 0) && (ldx % 4 == 0) && (ldo % 4 == 0) && (ldo - F <= 32) && cap_r >= AGG_MIN_ROWS) {
+            const int ec = whole ? 32 : (F > 256 ? 16 : 8), cps = whole ? 1 : (F > 256 ? 2 : 3);
+            launched = grapes_launch_agg_tma(ctx, X, 0, F, ldx, nullptr, slab_dev, cap_r, off, in_src, dinv, nullptr, 0,
+                                             bias, 0, out, ldo, nullptr, nullptr, -1, ec, cps, s, 1) == 0;
+        }
+    }
+    if (!launched) {                       // register-staged: layouts the TMA form does not take, and agg variant 1
+        const int blocks = grid_for(ctx, (long long)cap_r * 32, 256, 8);
+#define AGG64(VEC, XB) pdl((k_agg<VEC, XB, true>), blocks, 256, 0, s)(X, F, ldx, nullptr, slab_dev, cap_r, off, in_src, dinv, \
+                                                                       nullptr, 0, bias, 0, out, ldo, nullptr, nullptr, -1)
+        const bool v4 = a16 && (F % 4 == 0) && (ldx % 4 == 0) && (ldo % 4 == 0);
+        const bool v2 = a8 && (F % 2 == 0) && (ldx % 2 == 0) && (ldo % 2 == 0);
+        if (x_bf16) {
+            if (v4) AGG64(4, true); else if (v2) AGG64(2, true); else AGG64(1, true);
+        } else {
+            if (v4) AGG64(4, false); else if (v2) AGG64(2, false); else AGG64(1, false);
+        }
+#undef AGG64
+    }
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
 }
 
 int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int part_stride, const int* n_dev, int cap_n, const int* in_off,

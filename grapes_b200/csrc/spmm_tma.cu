@@ -59,17 +59,22 @@ struct AtB { int g; float dsl, dj; uint32_t sb; int rk; };        // node id, de
 // metadata, one LDS.128 of the row per 128 columns, 4 FFMA, one branch.
 // XB16: the feature table holds bf16 (papers100M-shaped config: 128 bf16 features); rows are staged as stored (2F bytes)
 // and widened to fp32 when they are read from shared memory; all arithmetic and the output stay fp32.
-template <int NPASS, bool HAS_IND, int OUTMODE, bool XB16>
+// W64: a row slab of the whole-graph structure past 2^31 entries (grapes_aggregate_rows64).  n_dev = {R, r0}: output row j
+// (j < R) is graph row r0 + j; in_off is int64 and indexed by graph row; sources, dinv and X rows are graph ids (nodes is
+// null).  The summation order is that of the int32 form, so a slab's rows are bit-identical to the same rows of it.
+template <int NPASS, bool HAS_IND, int OUTMODE, bool XB16, bool W64 = false>
 __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
     const void* __restrict__ X, int F, int ldx, const int* __restrict__ nodes, const int* __restrict__ n_dev, int cap_n,
-    const int* __restrict__ in_off, const int* __restrict__ in_src, const float* __restrict__ dinv,
+    const typename GrapesOff<W64>::T* __restrict__ in_off, const int* __restrict__ in_src, const float* __restrict__ dinv,
     const uint32_t* __restrict__ ind_bits, int num_ind, const float* __restrict__ bias, int relu, float* __restrict__ out,
     int ldo, float* __restrict__ out_hi, float* __restrict__ out_lo, int ones_col, int ec, int rb_min) {
+    typedef typename GrapesOff<W64>::T OffT;
     pdl_begin();
     extern __shared__ __align__(128) unsigned char at_smem[];
     const int lane = lane_id();
     const int warp = threadIdx.x >> 5;
     const int n = min(*n_dev, cap_n);
+    const int r0 = W64 ? n_dev[1] : 0;
     // bytes staged per row: the row rounded up to a whole float4 (F % 4 != 0: the table's rows are padded, ldx >= round_up(F, 4);
     // the pad values are accumulated into the unused components of the last feature lane and never stored)
     const uint32_t rowbytes = XB16 ? (uint32_t)F * 2u : (uint32_t)((F + 3) & ~3) * 4u;
@@ -98,8 +103,9 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
     while (top < RB) top <<= 1;                                   // binary-search span (power of two >= RB)
     for (int j0 = (blockIdx.x * AT_WARPS + warp) * RB; j0 < n; j0 += total_warps * RB) {
         const int nr = min(RB, n - j0);
-        const int base_off = in_off[j0];
-        for (int u = lane; u <= nr; u += 32) s_pos[u] = u + in_off[j0 + u] - base_off;   // first entry of row u
+        const OffT base_off = in_off[r0 + j0];
+        for (int u = lane; u <= nr; u += 32)                                         // first entry of row u
+            s_pos[u] = W64 ? u + (int)(in_off[r0 + j0 + u] - base_off) : u + (int)in_off[j0 + u] - (int)base_off;
         __syncwarp();
         const int T = s_pos[nr];
         const int nchunks = (T + ec - 1) / ec;
@@ -123,7 +129,7 @@ __global__ void __launch_bounds__(AT_THREADS) k_agg_tma(
         auto stageB = [&](const AtA& a) -> AtB {
             AtB b; b.g = 0; b.dsl = 0.f; b.dj = 0.f; b.sb = 0u; b.rk = a.rk;
             if (a.rk & AT_VALID) {
-                const int j = j0 + (a.rk & 0x1ff);
+                const int j = r0 + j0 + (a.rk & 0x1ff);
                 const int sl = (a.rk & AT_SELF) ? j : a.sl;
                 b.g = nodes ? nodes[sl] : sl;
                 b.dsl = dinv[sl];
@@ -253,9 +259,9 @@ size_t grapes_agg_tma_smem(int F, int ec, int es = 4) {
 
 // Returns 0 when the kernel was launched, 1 when the shape is not covered (caller falls back to k_agg_rows / k_agg).
 int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int ldx, const int* nodes, const int* n_dev, int cap_n,
-                          const int* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits, int num_ind,
+                          const void* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits, int num_ind,
                           const float* bias, int relu, float* out, int ldo, float* out_hi, float* out_lo, int ones_col,
-                          int ec_req, int ctas_per_sm, cudaStream_t s) {
+                          int ec_req, int ctas_per_sm, cudaStream_t s, int off64) {
     // fp32 rows must start 16-byte aligned and be readable up to a whole float4: ldx % 4 == 0 and ldx >= round_up(F, 4)
     // (F itself may be any width: Reddit 602, Cora 1433 -- the caller pads the table's row pitch, engine.py)
     if (ldx % 4 != 0 || ldx < ((F + 3) & ~3) || ldo % 4 != 0 || ldo - F > 32 || F > 128 * 12 || F < 4) return 1;
@@ -277,19 +283,19 @@ int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int
     const long long cap = (long long)ctx->sm_count * (smem > 113u * 1024u ? 1 : (cps >= 2 ? cps : 2));
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
-#define AT_LAUNCH_INST(NP, IND, OM, XB)                                                                                 \
+#define AT_LAUNCH_W(NP, IND, OM, XB, W)                                                                                 \
     do {                                                                                                                \
         static bool configured = false;                                                                                 \
         if (!configured) {                                                                                              \
-            if (cudaFuncSetAttribute(k_agg_tma<NP, IND, OM, XB>, cudaFuncAttributeMaxDynamicSharedMemorySize,           \
+            if (cudaFuncSetAttribute(k_agg_tma<NP, IND, OM, XB, W>, cudaFuncAttributeMaxDynamicSharedMemorySize,        \
                                      (int)(226u * 1024u)) != cudaSuccess) return 1;                                     \
             configured = true;                                                                                          \
         }                                                                                                               \
-        pdl((k_agg_tma<NP, IND, OM, XB>), (int)blocks, AT_THREADS, smem, s)(X, F, ldx, nodes, n_dev, cap_n, in_off,     \
-                                                                          in_src, dinv, ind_bits, num_ind, bias, relu,  \
-                                                                          out, ldo, out_hi, out_lo, ones_col, ec,       \
-                                                                          rb_min);                                      \
+        pdl((k_agg_tma<NP, IND, OM, XB, W>), (int)blocks, AT_THREADS, smem, s)(                                         \
+            X, F, ldx, nodes, n_dev, cap_n, (const typename GrapesOff<W>::T*)in_off, in_src, dinv, ind_bits, num_ind,    \
+            bias, relu, out, ldo, out_hi, out_lo, ones_col, ec, rb_min);                                                \
     } while (0)
+#define AT_LAUNCH_INST(NP, IND, OM, XB) AT_LAUNCH_W(NP, IND, OM, XB, false)
 #define AT_LAUNCH2(NP, IND, XB)                                                                                         \
     do {                                                                                                                \
         if (om == 1) AT_LAUNCH_INST(NP, IND, 1, XB); else if (om == 2) AT_LAUNCH_INST(NP, IND, 2, XB);                  \
@@ -304,7 +310,15 @@ int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int
         if (has_ind) AT_LAUNCH2(NP, true, true); else AT_LAUNCH2(NP, false, true);                                      \
     } while (0)
     const int om = (out ? 1 : 0) | (out_hi ? 2 : 0);
-    if (x_bf16) {
+    if (off64) {                                   // whole-graph row slab: plain output, no indicator columns
+        if (om != 1 || has_ind) return 1;
+        if (x_bf16) {
+            if (npass == 1) AT_LAUNCH_W(1, false, 1, true, true); else AT_LAUNCH_W(2, false, 1, true, true);
+        } else if (npass == 1) AT_LAUNCH_W(1, false, 1, false, true);
+        else if (npass == 2) AT_LAUNCH_W(2, false, 1, false, true);
+        else if (npass <= 5) AT_LAUNCH_W(5, false, 1, false, true);
+        else AT_LAUNCH_W(12, false, 1, false, true);
+    } else if (x_bf16) {
         if (npass == 1) AT_LAUNCH_B16(1); else AT_LAUNCH_B16(2);
     } else if (npass == 1) AT_LAUNCH(1);
     else if (npass == 2) AT_LAUNCH(2);
@@ -313,6 +327,7 @@ int grapes_launch_agg_tma(grapes_ctx* ctx, const void* X, int x_bf16, int F, int
 #undef AT_LAUNCH_B16
 #undef AT_LAUNCH2
 #undef AT_LAUNCH_INST
+#undef AT_LAUNCH_W
 #undef AT_LAUNCH
     return 0;
 }

@@ -4,7 +4,9 @@ same two modes, same return ``(accuracy, f1)``.
 * ``full_batch=True`` (the default of every reference config, eval.py:47-70): ONE forward of the classifier over the
   whole graph.  The reference moves the model to the CPU for this (``eval_on_cpu=True``, main.py:43); here it stays
   on the B200 -- the whole-graph aggregation is ``grapes_aggregate`` (TMA-staged SpMM, csrc/spmm_tma.cu) on the
-  gcn_norm structure of the full CSR (:class:`grapes_b200.gcn.GraphNorm`, built once and cached on the graph).
+  gcn_norm structure of the full CSR (:class:`grapes_b200.gcn.GraphNorm`, built once and cached on the graph).  From
+  ``WIDE_MIN_EDGES`` edges on, the structure has int64 offsets (:class:`grapes_b200.gcn.WideGraphNorm`) and the forward
+  runs over row slabs (:func:`grapes_b200.gcn.full_graph_forward_streamed`): same logits, bounded memory.
 * ``full_batch=False`` (eval.py:71-163): every batch runs on the training engine's kernels, forward only
   (``GrapesEngine.predict``): frontier expansion, bitmap dedup / relabel, fused gather + aggregation, the sampler GCN's
   tcgen05 forward, DETERMINISTIC top-k on the probabilities (eval.py:126-130, ``GRAPES_NOISE_NONE_TOPK_PROBS``), the
@@ -24,18 +26,23 @@ from typing import Optional, Tuple
 import torch
 
 from ._lib import GrapesError
-from .gcn import GCN, GraphNorm, full_graph_forward
+from .gcn import GCN, GraphNorm, WideGraphNorm, full_graph_forward, full_graph_forward_streamed
 from .graph import DeviceGraph
 from .utils import TensorMap, get_logger
 
+# Edge count from which the full-batch evaluation runs on the int64 structure (WideGraphNorm) and the row-slab forward
+# (full_graph_forward_streamed): the int32 offsets of GraphNorm and grapes_aggregate hold fewer entries.
+WIDE_MIN_EDGES = (1 << 31) - 1
 
-def _graph_norm(adjacency: DeviceGraph, data) -> GraphNorm:
+
+def _graph_norm(adjacency: DeviceGraph, data, wide: bool = False):
     """gcn_norm structure of ``data.edge_index`` (what eval.py:50 feeds GCNConv), cached on the graph object."""
     ei = getattr(data, "edge_index", None)
-    key = None if ei is None else (ei.data_ptr(), tuple(ei.shape))
+    key = (None if ei is None else (ei.data_ptr(), tuple(ei.shape)), wide)
     cached = getattr(adjacency, "_graph_norm", None)
     if cached is None or cached[0] != key:
-        cached = (key, GraphNorm(adjacency, edge_index=ei))
+        adjacency._graph_norm = None                                  # the previous structure goes before the new one is built
+        cached = (key, (WideGraphNorm if wide else GraphNorm)(adjacency, edge_index=ei))
         adjacency._graph_norm = cached
     return cached[1]
 
@@ -81,6 +88,12 @@ def evaluate(gcn_c: GCN,
     mask_d = mask.to(device) if mask is not None else torch.ones(data.num_nodes, dtype=torch.bool, device=device)
 
     if full_batch:
+        ei = getattr(data, "edge_index", None)
+        if (int(ei.shape[1]) if ei is not None else adjacency.nnz) >= WIDE_MIN_EDGES:
+            # past 2^31 edges: int64 structure, row slabs, masked scores reduced per slab; [N, C] logits only on request
+            logits_total, res = full_graph_forward_streamed(gcn_c, x, _graph_norm(adjacency, data, wide=True), y=y,
+                                                            mask=mask_d, return_logits=return_predictions)
+            return (res + (logits_total,)) if return_predictions else res
         # eval.py:50.  GRAPES_EVAL_TC=1: the fused whole-graph forward with its hidden layer on the tensor cores
         # (gcn.full_graph_forward; written after this round's GPU budget was spent, measured by bench.py's full_graph_eval leg)
         if os.environ.get("GRAPES_EVAL_TC", "0") == "1":

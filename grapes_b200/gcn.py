@@ -71,7 +71,7 @@ class GraphNorm(NormAdj):
     library's own kernels -- ``grapes_row_offsets`` + ``grapes_expand_rows`` turn the CSR back into its edge list,
     ``grapes_build_csr`` (counting sort by destination, per-row sort, self-loops dropped, deg^-1/2) is the routine that
     builds every hop's structure.  One-off, cached on the graph; the aggregation itself is ``grapes_aggregate``
-    (TMA-staged SpMM) straight on these arrays.  nnz must fit int32 offsets (papers100M-shape needs sharding)."""
+    (TMA-staged SpMM) straight on these arrays.  nnz must fit int32 offsets; larger graphs use :class:`WideGraphNorm`."""
 
     def __init__(self, graph, edge_index=None, builder=None):
         """``builder``: "torch" (default; GPU-verified in round 1 and 2) sorts the (destination, source) keys with
@@ -193,6 +193,200 @@ class GraphNorm(NormAdj):
         if transpose:
             raise GrapesError("GraphNorm is forward-only (evaluation); training uses the sampled blocks")
         return super().aggregate(x, False, bias)
+
+
+class WideGraphNorm:
+    """The same gcn_norm structure as :class:`GraphNorm` with int64 row offsets, for graphs of any edge count
+    (``grapes_graph_norm_*``): ``in_off`` int64 [N+1], ``in_src`` int32 [nnz'], ``dinv`` fp32 [N], equal bit for bit to
+    the torch-sort builder.  Built on the device by a counting sort by destination that reads the input where it lies:
+    the graph's CSR, or ``edge_index`` (host or device, int64 [2, E]; duplicates kept and counted) in chunks of
+    ``chunk_edges`` columns, so a host edge list never has to be on the device at once.  Device memory beyond the
+    outputs: ``grapes_graph_norm_workspace_bytes(N)`` (~4 N bytes) plus one chunk of a host edge list (16 bytes per edge).
+    Forward only: its aggregation is ``aggregate_rows`` over row slabs (:func:`full_graph_forward_streamed`)."""
+
+    def __init__(self, graph, edge_index=None, chunk_edges: int = 1 << 27):
+        dev = graph.device
+        N = graph.num_nodes
+        L, st = lib(), _stream()
+        self.graph = graph
+        self.holder = _any_ctx(dev)
+        ws = torch.empty(max(int(L.cdll.grapes_graph_norm_workspace_bytes(N)), 1), dtype=torch.uint8, device=dev)
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        nnz = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.in_off = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        self.dinv = torch.empty(N, dtype=torch.float32, device=dev)
+
+        def run(pass_, in_src):
+            if edge_index is None:
+                L.grapes_graph_norm_add_csr(pass_, N, ptr(graph.indptr), ptr(graph.indices), 0, N, ptr(self.in_off),
+                                            ptr(in_src), ptr(ws), ptr(err), st)
+                return
+            E = int(edge_index.shape[1])
+            for a in range(0, E, chunk_edges):
+                src = edge_index[0, a:a + chunk_edges].to(device=dev, dtype=torch.int64).contiguous()
+                dst = edge_index[1, a:a + chunk_edges].to(device=dev, dtype=torch.int64).contiguous()
+                L.grapes_graph_norm_add_edges(pass_, N, ptr(src), ptr(dst), int(src.numel()), ptr(self.in_off),
+                                              ptr(in_src), ptr(ws), ptr(err), st)
+
+        L.grapes_graph_norm_begin(N, ptr(ws), ws.numel(), ptr(err), st)
+        run(0, None)
+        L.grapes_graph_norm_offsets(N, ptr(ws), ptr(self.in_off), ptr(self.dinv), ptr(nnz), st)
+        self._check(err)
+        self.n, self.E = N, int(nnz.item())                      # one-off read-back: the size of in_src
+        self.in_src = torch.empty(max(self.E, 1), dtype=torch.int32, device=dev)
+        run(1, self.in_src)
+        L.grapes_graph_norm_finish(N, ptr(self.in_off), ptr(self.in_src), ptr(ws), st)
+        del ws
+        if self.E == 0:
+            self.in_src = self.in_src[:0]
+
+    @staticmethod
+    def _check(err):
+        e = int(err.item())
+        if e & 1:
+            raise GrapesError("edge_index holds node ids outside [0, num_nodes)")
+        if e & 2:
+            raise GrapesError("a node has 2^31 - 1 or more in-edges")
+
+    def aggregate_rows(self, x: torch.Tensor, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None) -> torch.Tensor:
+        """out[j] = (A_hat x)[r0 + j] (+ bias) for j < R, slab = int32 {R, r0} on the device; x fp32 or bf16 rows
+        (widened on read), out fp32 [>= R, >= F] with a unit column stride."""
+        F = x.shape[1]
+        lib().grapes_aggregate_rows64(self.holder.ctx, ptr(x), int(x.dtype == torch.bfloat16), F, x.stride(0), ptr(slab),
+                                      R, ptr(self.in_off), ptr(self.in_src), ptr(self.dinv), ptr(bias), ptr(out),
+                                      out.stride(0), _stream())
+        return out
+
+
+def _gemm_into(A, lda, W, ldw, C, ldc, M, N, K, bias=None):
+    """C[:M, :N] = A W^T (+ bias) on the same SIMT ``grapes_gemm`` call as :func:`_gemm` (layout 3), into a caller view."""
+    if M > 0:
+        lib().grapes_gemm(_any_ctx(A.device).ctx, 3, ptr(A), lda, ptr(W), ldw, ptr(C), ldc, None, M, N, K, ptr(bias), 0,
+                          None, 0, _stream())
+
+
+def slab_rows_for(n: int, per_row_bytes: int, resident_bytes: int, device, mem_budget=None, max_rows: int = 1 << 20) -> int:
+    """Rows per slab that fit ``mem_budget`` bytes (default: free device memory, counting the blocks torch's allocator
+    holds unused, less a margin of 5 % of the device and at least 2 GiB) after ``resident_bytes`` more are allocated, at
+    most ``max_rows``: 2^20 rows already take the whole-graph launch shape of the aggregation (one CTA per SM, 32-entry
+    chunks), and the slab temporaries stay ~1-2 GB."""
+    if mem_budget is None:
+        free, total = torch.cuda.mem_get_info(device)
+        free += torch.cuda.memory_reserved(device) - torch.cuda.memory_allocated(device)
+        mem_budget = free - max(total // 20, 2 << 30)
+    rows = (int(mem_budget) - int(resident_bytes)) // max(int(per_row_bytes), 1)
+    if rows < 1:
+        raise GrapesError(f"streamed full-graph forward: {resident_bytes / 2**30:.1f} GiB resident leave no room for a slab "
+                          f"within the memory budget of {mem_budget / 2**30:.1f} GiB")
+    return int(min(rows, max_rows, max(n, 1)))
+
+
+@torch.no_grad()
+def full_graph_forward_streamed(gcn: "GCN", x: torch.Tensor, gn: WideGraphNorm, slab_rows=None, mem_budget=None,
+                                y=None, mask=None, return_logits: bool = True):
+    """``gcn_c(x, edge_index)`` over the whole graph (eval.py:50) for the two-layer classifier ``GCN(F, [D, C])``, one row
+    slab at a time, on a :class:`WideGraphNorm`.  The products are those of ``gcn(x, GraphNorm)`` in the same order and on
+    the same kernels, so the logits are bit-identical to it:
+
+    * layer 1, F <= D: per slab Y = A_hat X (``aggregate_rows`` on the fp32 or bf16 rows as stored), H = relu(Y W1^T + b1);
+      F > D: per slab P = X W1^T into a resident [N, D] array, then per slab H = relu(A_hat P + b1);
+    * Z[slab] = H W2^T into ONE resident [N, round_up(C, 4)] array (zero pad columns); H never exists for all N;
+    * per slab logits = A_hat Z + b2.
+
+    ``slab_rows`` (default: what ``mem_budget`` allows, see :func:`slab_rows_for`) bounds the slab temporaries.  With ``y``
+    (and ``mask``, default all rows) the scores of ``eval._scores`` are reduced per slab on the device.  Returns
+    (logits [N, C] or None when ``return_logits`` is False, (accuracy, f1) or None).  Other depths, a layer 2 that would
+    aggregate first (D <= C), other table dtypes and dropout in training mode raise ``GrapesError``."""
+    layers = list(gcn.gcn_layers)
+    if len(layers) != 2:
+        raise GrapesError(f"streamed full-graph forward covers the two-layer classifier, not {len(layers)} layers")
+    if gcn.training and gcn.dropout > 0:
+        raise GrapesError("streamed full-graph forward is evaluation only: dropout in training mode")
+    if x.dtype not in (torch.float32, torch.bfloat16) or x.dim() != 2 or x.stride(1) != 1:
+        raise GrapesError("streamed full-graph forward reads fp32 or bf16 rows with a unit column stride")
+    dev = x.device
+    N, F = x.shape                                    # (shadows torch.nn.functional inside this function)
+    w1 = layers[0].lin.weight.detach().float().contiguous()
+    b1 = layers[0].bias.detach().float().contiguous()
+    w2 = layers[1].lin.weight.detach().float().contiguous()
+    D, C = w1.shape[0], w2.shape[0]
+    if D <= C:
+        raise GrapesError("streamed full-graph forward needs hidden width D > classes C (layer 2 transforms first)")
+    C4 = (C + 3) // 4 * 4
+    b2 = F_pad(layers[1].bias.detach().float(), C4 - C).contiguous()
+    agg_first = F <= D
+    resident = N * C4 * 4 + (0 if agg_first else N * D * 4) + (N * C4 * 4 if return_logits else 0)
+    per_row = 4 * ((F if agg_first else 0) + (F if (not agg_first and x.dtype != torch.float32) else 0) + D + C4)
+    R = int(slab_rows) if slab_rows else slab_rows_for(N, per_row, resident, dev, mem_budget)
+    R = max(1, min(R, max(N, 1)))
+    starts = list(range(0, N, R))
+    slabs = torch.tensor([[min(R, N - r0), r0] for r0 in starts] or [[0, 0]], dtype=torch.int32, device=dev)
+
+    Z = torch.zeros((N, C4), dtype=torch.float32, device=dev)
+    H = torch.empty((R, D), dtype=torch.float32, device=dev)
+    if agg_first:
+        Y = torch.empty((R, F), dtype=torch.float32, device=dev)
+        for i, r0 in enumerate(starts):
+            n = min(R, N - r0)
+            gn.aggregate_rows(x, slabs[i], n, Y)
+            _gemm_into(Y, F, w1, F, H, D, n, D, F, bias=b1)
+            torch.relu_(H[:n])
+            _gemm_into(H, D, w2, D, Z[r0:], C4, n, C, D)
+        del Y
+    else:
+        P = torch.empty((N, D), dtype=torch.float32, device=dev)
+        for r0 in starts:
+            n = min(R, N - r0)
+            xs = x[r0:r0 + n] if x.dtype == torch.float32 else x[r0:r0 + n].float()
+            _gemm_into(xs, xs.stride(0), w1, F, P[r0:], D, n, D, F)
+        for i, r0 in enumerate(starts):
+            n = min(R, N - r0)
+            gn.aggregate_rows(P, slabs[i], n, H, bias=b1)
+            torch.relu_(H[:n])
+            _gemm_into(H, D, w2, D, Z[r0:], C4, n, C, D)
+        del P
+    del H
+
+    logits = torch.empty((N, C4), dtype=torch.float32, device=dev) if return_logits else None
+    out = None if return_logits else torch.empty((R, C4), dtype=torch.float32, device=dev)
+    counts = torch.zeros(3, dtype=torch.int64, device=dev) if y is not None else None
+    for i, r0 in enumerate(starts):
+        n = min(R, N - r0)
+        o = logits[r0:r0 + n] if return_logits else out
+        gn.aggregate_rows(Z, slabs[i], n, o, bias=b2)
+        if counts is not None:
+            lg, ys = o[:n, :C], y[r0:r0 + n]
+            if mask is not None:
+                m = mask[r0:r0 + n]
+                lg, ys = lg[m], ys[m]
+            counts += _slab_counts(lg, ys)
+    scores = None if counts is None else _scores_from_counts(counts, y.dim() == 1)
+    return (logits[:, :C] if return_logits else None), scores
+
+
+def _slab_counts(logits_masked: torch.Tensor, y_masked: torch.Tensor) -> torch.Tensor:
+    """(argmax hits, rows, 0) single-label or (tp, fp, fn) multi-label of one slab's masked rows, on the device."""
+    if y_masked.dim() == 1:
+        hits = (torch.argmax(logits_masked, dim=1) == y_masked).sum()
+        return torch.stack([hits, hits.new_tensor(y_masked.shape[0]), hits.new_zeros(())])
+    y_pred = logits_masked > 0
+    y_true = y_masked > 0.5
+    return torch.stack([(y_true & y_pred).sum(), (~y_true & y_pred).sum(), (y_true & ~y_pred).sum()])
+
+
+def _scores_from_counts(counts: torch.Tensor, single_label: bool):
+    """(accuracy, f1) from the summed slab counts, with the arithmetic of ``eval._scores``."""
+    a, b, c = (int(v) for v in counts.tolist())
+    if single_label:
+        acc = (torch.tensor(a, dtype=torch.float32) / b).item()      # float32 mean of the hit vector
+        return acc, acc
+    tp, fp, fn = a, b, c
+    try:
+        precision, recall = tp / (tp + fp), tp / (tp + fn)
+        f1 = 2 * (precision * recall) / (precision + recall)
+    except ZeroDivisionError:
+        f1 = 0.
+    return f1, f1
 
 
 def dense_bias_relu_tc(Y: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:

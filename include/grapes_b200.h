@@ -100,6 +100,29 @@ int grapes_csr_from_edges(const int64_t* src, const int64_t* dst, int64_t num_ed
                           int* indices, int64_t* nnz_dev, int* err_dev, void* workspace, int64_t workspace_bytes,
                           void* stream);
 
+/* ---- whole-graph gcn_norm structure with int64 offsets (replaces PyG gcn_norm at modules/gcn.py:18,21 for full-batch
+ * evaluation of graphs of any edge count): in_off int64 [N+1], in_src int32 [nnz'] (the in-neighbours of each destination,
+ * sources ascending, stored self-loops dropped, duplicates of an edge list kept and counted), dinv fp32 [N] =
+ * (indeg + 1)^-1/2.  Equal, bit for bit, to sorting the (destination, source) keys.  Sequence, all on `stream`, no host
+ * synchronisation inside:
+ *   begin -> add_*(pass 0) over the whole input -> offsets (in_off, dinv, *nnz_dev = nnz') -> add_*(pass 1) over the
+ *   same input in the same chunks or others -> finish (per-row sorts).
+ * The input is the graph's CSR (rows [r0, r1) of indptr / indices; row = source, index = destination) or chunks of an
+ * int64 edge list (src[e] -> dst[e], e.g. the rows of a slice of edge_index), read in place.  in_src needs nnz' entries,
+ * which the caller reads back after `offsets`.  *err_dev |= 1: an id outside [0, N) (the edge is skipped; the caller
+ * raises), |= 2: a node with 2^31 - 1 or more in-edges.
+ * Device scratch beyond the outputs: the caller's workspace, grapes_graph_norm_workspace_bytes(N) = 4 N bytes + 8 bytes
+ * per 8192 nodes + 1 KB of alignment, and nothing else (no chunk copies: the input is read where it lies).            */
+int64_t grapes_graph_norm_workspace_bytes(int64_t num_nodes);
+int grapes_graph_norm_begin(int64_t num_nodes, void* workspace, int64_t workspace_bytes, int* err_dev, void* stream);
+int grapes_graph_norm_add_csr(int pass, int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0, int64_t r1,
+                              int64_t* in_off, int* in_src, void* workspace, int* err_dev, void* stream);
+int grapes_graph_norm_add_edges(int pass, int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                int64_t* in_off, int* in_src, void* workspace, int* err_dev, void* stream);
+int grapes_graph_norm_offsets(int64_t num_nodes, void* workspace, int64_t* in_off, float* dinv, int64_t* nnz_dev,
+                              void* stream);
+int grapes_graph_norm_finish(int64_t num_nodes, const int64_t* in_off, int* in_src, void* workspace, void* stream);
+
 /* ---- frontier expansion / dedup / relabel  (utils.py:74-82, main.py:183-195, utils.py:98-120) */
 /* rows[P] -> row_off[P+1] = exclusive scan of CSR degrees, *m_dev = total.  Sets the bit of every
  * row in bm_rows (prev_nodes_mask, main.py:185) and of rows with degree > 0 in bm_batch.          */
@@ -190,6 +213,16 @@ int grapes_aggregate_bf16(grapes_ctx* ctx, const void* X_bf16, int F, int ldx, c
                           int cap_n, const int* in_off, const int* in_src, const float* dinv, const uint32_t* ind_bits,
                           int num_ind, const float* bias, int relu, float* out, int ldo, float* out_hi, float* out_lo,
                           int ones_col, void* stream);
+/* Whole-graph aggregation over one row slab of the int64 structure above (grapes_graph_norm_*), for graphs past 2^31
+ * entries.  slab_dev = {R, r0} on the device, R <= cap_r:
+ *   out[j, :F] = dinv[r0+j]^2 X[r0+j] + sum_{s in in(r0+j)} dinv[s] dinv[r0+j] X[s]  (+ bias),  j < R;  out[j, F:ldo) = 0.
+ * in_off is read at r0 + j, sources / dinv / X rows are graph ids.  X is fp32 or bf16 (x_bf16 = 1, widened on read); fp32
+ * arithmetic in the summation order of grapes_aggregate, so on a graph below 2^31 the rows are bit-identical to those of
+ * grapes_aggregate / grapes_aggregate_bf16 on the int32 structure.  TMA-staged where that kernel takes the layout,
+ * register-staged otherwise and under grapes_agg_variant(1).                                                           */
+int grapes_aggregate_rows64(grapes_ctx* ctx, const void* X, int x_bf16, int F, int ldx, const int* slab_dev, int cap_r,
+                            const int64_t* in_off, const int* in_src, const float* dinv, const float* bias, float* out,
+                            int ldo, void* stream);
 /* z may be given as `nparts` partial vectors `part_stride` floats apart (summed on the fly)           */
 int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int part_stride, const int* n_dev, int cap_n, const int* in_off,
                             const int* in_src, const float* dinv, const float* bias, float* out, float* zero_out,
