@@ -25,6 +25,9 @@ __device__ __forceinline__ float block_sum_1024(float v, float* s) {
 // dlogits must be zeroed by the caller (grapes_classifier_loss does it).
 // Stage 1 (one warp per target row): per-row loss term -> row_loss[r], gradient rows.  Stage 2 (one block): fixed-order
 // sum of the B terms (+ the reg_param * sum_rows var(logits) term and its gradient) -> *loss_out.
+// CE_LSE_NOTE: the cross-entropy terms keep log-sum-exp relative to the row maximum, p = exp((l - mx) - ls) and
+// loss = (mx - l_y) + ls with ls = log sum exp(l - mx).  Forming lse = mx + ls first rounds it to the ulp of |mx|
+// (3e-5 at |mx| ~ 500, 5e-4 at 5000), an error every probability of the row would inherit.
 __global__ void __launch_bounds__(256) k_loss_rows(const float* __restrict__ logits, int ldl, int C,
                                                    const int* __restrict__ row_ids, const int* __restrict__ targets,
                                                    int B, const int64_t* __restrict__ labels_i64,
@@ -45,12 +48,12 @@ __global__ void __launch_bounds__(256) k_loss_rows(const float* __restrict__ log
         float se = 0.f;
         for (int c = lane; c < C; c += 32) se += expf(lr[c] - mx);
         se = warp_sum(se);
-        const float lse = mx + logf(se);
+        const float ls = logf(se);                       // log-sum-exp - mx (see CE_LSE_NOTE)
         for (int c = lane; c < C; c += 32) {
-            const float pr = expf(lr[c] - lse);
+            const float pr = expf((lr[c] - mx) - ls);
             dlogits[(size_t)row * ldl + c] = (pr - (c == y ? 1.f : 0.f)) * invB;
         }
-        if (lane == 0) row_loss[r] = (lse - lr[y]) * invB;
+        if (lane == 0) row_loss[r] = ((mx - lr[y]) + ls) * invB;
     } else {
         const float inv = 1.0f / ((float)B * (float)C);
         const float* yr = labels_f32 + (size_t)targets[r] * C;
@@ -132,9 +135,9 @@ __global__ void __launch_bounds__(LR2_WARPS * 32) k_loss_rows2(
             float se = 0.f;
             for (int c = lane; c < C; c += 32) se += expf(lr[c] - mx);
             se = warp_sum(se);
-            const float lse = mx + logf(se);
-            for (int c = lane; c < C; c += 32) mycols[c] = (expf(lr[c] - lse) - (c == y ? 1.f : 0.f)) * invB;
-            loss = (lse - lr[y]) * invB;
+            const float ls = logf(se);                   // log-sum-exp - mx (see CE_LSE_NOTE)
+            for (int c = lane; c < C; c += 32) mycols[c] = (expf((lr[c] - mx) - ls) - (c == y ? 1.f : 0.f)) * invB;
+            loss = ((mx - lr[y]) + ls) * invB;
         } else if (r >= 0) {
             const float inv = 1.0f / ((float)B * (float)C);
             const float* yr = labels_f32 + (size_t)targets[r] * C;
@@ -254,9 +257,9 @@ __global__ void __launch_bounds__(LR2_WARPS * 32) k_loss_rows2_dropout(
             float se = 0.f;
             for (int c = lane; c < C; c += 32) se += expf(lr[c] - mx);
             se = warp_sum(se);
-            const float lse = mx + logf(se);
-            for (int c = lane; c < C; c += 32) mycols[c] = (expf(lr[c] - lse) - (c == y ? 1.f : 0.f)) * invB;
-            loss = (lse - lr[y]) * invB;
+            const float ls = logf(se);                   // log-sum-exp - mx (see CE_LSE_NOTE)
+            for (int c = lane; c < C; c += 32) mycols[c] = (expf((lr[c] - mx) - ls) - (c == y ? 1.f : 0.f)) * invB;
+            loss = ((mx - lr[y]) + ls) * invB;
         } else if (r >= 0) {
             const float inv = 1.0f / ((float)B * (float)C);
             const float* yr = labels_f32 + (size_t)targets[r] * C;
@@ -337,12 +340,12 @@ __global__ void __launch_bounds__(256) k_loss_rows_dropout(const float* __restri
         float se = 0.f;
         for (int c = lane; c < C; c += 32) se += expf(dropped_logit(lr, c, i0 + c, seed, step, dp) - mx);
         se = warp_sum(se);
-        const float lse = mx + logf(se);
+        const float ls = logf(se);                       // log-sum-exp - mx (see CE_LSE_NOTE)
         for (int c = lane; c < C; c += 32) {
-            const float pr = expf(dropped_logit(lr, c, i0 + c, seed, step, dp) - lse);
+            const float pr = expf((dropped_logit(lr, c, i0 + c, seed, step, dp) - mx) - ls);
             dlogits[(size_t)row * ldl + c] = (pr - (c == y ? 1.f : 0.f)) * invB;
         }
-        if (lane == 0) row_loss[r] = (lse - dropped_logit(lr, y, i0 + y, seed, step, dp)) * invB;
+        if (lane == 0) row_loss[r] = ((mx - dropped_logit(lr, y, i0 + y, seed, step, dp)) + ls) * invB;
     } else {
         const float inv = 1.0f / ((float)B * (float)C);
         const float* yr = labels_f32 + (size_t)targets[r] * C;

@@ -77,6 +77,12 @@ class _Hop:
 
 
 class GrapesEngine:
+    # largest cap_A = B + H * k whose classifier takes the "prep" form (one grapes_classifier_prep launch and the
+    # row-parallel loss); above it the step relabels with grapes_relabel, builds the CSRs with grapes_build_csr and takes
+    # the target-row loss.  It may be lowered (the two forms compute the same step) but never raised:
+    # grapes_classifier_prep refuses cap_A > SMALL_N (4096, csrc/frontier.cu).
+    PREP_MAX_ROWS = 4096
+
     def __init__(self, graph: DeviceGraph, x: torch.Tensor, y: torch.Tensor, *, num_classes: int,
                  batch_size: int, num_samples: int, sampling_hops: int, use_indicators: bool = True,
                  hidden_dim: int = 256, lr_gc: float = 1e-3, lr_gf: float = 1e-4, loss_coef: float = 1e4,
@@ -516,7 +522,7 @@ class GrapesEngine:
         A_dev, cap_A = self._cnt("A"), self.cap_A
         # loss + d loss / d logits + d loss / d b2 (column sums) in one launch (main.py:260-261)
         loss_args = (ctx, ptr(self.logits_c), C, C, A_dev, cap_A, ptr(self.target_local),
-                     ptr(self.tgt_of_row) if self.cap_A <= 4096 else None, ptr(self.targets), B,
+                     ptr(self.tgt_of_row) if self.cap_A <= self.PREP_MAX_ROWS else None, ptr(self.targets), B,
                      None if self.multilabel else ptr(self.y), ptr(self.y) if self.multilabel else None, self.reg_param,
                      ptr(self.dlogits), self._scal("loss_c"), self._grd(nc.b2))
         if self.dropout > 0:
@@ -578,7 +584,7 @@ class GrapesEngine:
                             None, None, None, 0, 0, self.cap_A, self._cnt("A"), None, ovf, st)
         # GCN.forward with a per-layer list: hidden layer <- edge_indices[-1], last layer <- edge_indices[0] (gcn.py:30-36)
         b0, b1 = self.hops[H - 1], self.hops[0]
-        if self.cap_A <= 4096:
+        if self.cap_A <= self.PREP_MAX_ROWS:
             L.grapes_classifier_prep(ctx, ptr(self.bm_all), ptr(self.pref_all), self._cnt("A"), self.cap_A,
                                      ptr(self.targets), self._cnt("B"), B, ptr(self.target_local),
                                      ptr(b0.blk_src), ptr(b0.blk_dst), self._hc(H - 1, "blk"),

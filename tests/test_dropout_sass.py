@@ -2,7 +2,9 @@
 the machine code of the existing classifier GEMMs (k_gemm<*,*>, k_gemm_s<*,*>), classifier loss kernels and the fused
 selection kernel unchanged.  tests/golden/dropout_sass.json holds the sha256 of their SASS (instructions and encodings,
 addresses stripped) as the recorded nvcc release compiles them with the library's flags; another nvcc release may
-schedule differently, so the test skips there."""
+schedule differently, so the test skips there.  The digests of k_loss_rows and k_loss_rows2 were re-recorded once, when
+their cross-entropy terms changed to keep log-sum-exp relative to the row maximum (csrc/loss_optim.cu CE_LSE_NOTE);
+every other function keeps the digest recorded before the dropout forms were added."""
 import json
 import os
 import subprocess
@@ -26,7 +28,7 @@ def _demangle(names):
     return {n: d.split("(")[0].replace("void ", "") for n, d in zip(names, out)}
 
 
-def test_existing_classifier_and_selection_kernels_keep_their_sass(tmp_path):
+def test_classifier_and_selection_kernels_keep_their_recorded_sass(tmp_path):
     nvcc, cuobjdump = _tool("nvcc"), _tool("cuobjdump")
     if not nvcc or not cuobjdump:
         pytest.skip("nvcc / cuobjdump not available")
