@@ -469,6 +469,50 @@ __global__ void __launch_bounds__(CB_THREADS) k_gn_edges(const int64_t* __restri
         gn_edge<SCATTER>(src[e], dst[e], N, cnt, in_off, in_src, err);
 }
 
+// Destination window [lo, hi) of the structure (grapes_graph_norm_window_*): pass 1 scatters only the edges into the window,
+// at win_off[c - lo] (offsets local to the window).  Ids were checked by pass 0 over the same input.
+__device__ __forceinline__ void gnw_edge(int64_t r, int64_t c, int64_t N, int64_t lo, int64_t hi, int* __restrict__ cnt,
+                                         const long long* __restrict__ win_off, int* __restrict__ in_src) {
+    if (r < 0 || r >= N || c < lo || c >= hi || r == c) return;
+    const int k = atomicAdd(&cnt[c], 1);
+    in_src[win_off[c - lo] + k] = (int)r;
+}
+
+__global__ void __launch_bounds__(CB_THREADS) k_gnw_csr(const long long* __restrict__ indptr, const int* __restrict__ indices,
+                                                         int64_t r0, int64_t r1, int64_t N, int64_t lo, int64_t hi,
+                                                         int* __restrict__ cnt, const long long* __restrict__ win_off,
+                                                         int* __restrict__ in_src) {
+    const int lane = lane_id();
+    const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t r = r0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); r < r1; r += warps) {
+        const long long e1 = indptr[r + 1];
+        for (long long e = indptr[r] + lane; e < e1; e += 32) gnw_edge(r, indices[e], N, lo, hi, cnt, win_off, in_src);
+    }
+}
+
+__global__ void __launch_bounds__(CB_THREADS) k_gnw_edges(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
+                                                           int64_t n, int64_t N, int64_t lo, int64_t hi, int* __restrict__ cnt,
+                                                           const long long* __restrict__ win_off, int* __restrict__ in_src) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += stride)
+        gnw_edge(src[e], dst[e], N, lo, hi, cnt, win_off, in_src);
+}
+
+// bounds[k] = the least i in [0, N] with (in_off[i] + i) * W >= k * T, T = in_off[N] + N: the prefix of indeg + 1 cut into
+// W parts, so every window holds T / W of it to within one row's indeg + 1.  bounds[0] = 0, bounds[W] = N.
+__global__ void k_gn_bounds(int64_t N, const long long* __restrict__ in_off, int W, long long* __restrict__ bounds) {
+    const long long T = in_off[N] + N;
+    for (int k = threadIdx.x; k <= W; k += blockDim.x) {
+        const long long target = (long long)k * T;
+        long long a = 0, b = N;                                      // invariant: answer in [a, b]
+        while (a < b) {
+            const long long m = a + ((b - a) >> 1);
+            if ((in_off[m] + m) * W >= target) b = m; else a = m + 1;
+        }
+        bounds[k] = a;
+    }
+}
+
 // dinv = (indeg + 1)^-1/2 with correctly rounded sqrt and divide (torch's 1.0 / sqrt(float)); cnt becomes the cursor
 __global__ void __launch_bounds__(CB_THREADS) k_gn_dinv(int64_t N, int* __restrict__ cnt, float* __restrict__ dinv) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -794,6 +838,54 @@ int grapes_graph_norm_finish(int64_t num_nodes, const int64_t* in_off, int* in_s
     pdl((k_gn_sort_rows<CB_LONG_THREADS, CB_LONG_SMEM, true>), sms, CB_LONG_THREADS, CB_LONG_SMEM * 4, s)(
         num_nodes, off, in_src, worklist, flags);
     grapes_count_launches(3);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_window_bounds(int64_t num_nodes, const int64_t* in_off, int world, int64_t* bounds_dev,
+                                    void* stream) {
+    GRAPES_REQUIRE(in_off && bounds_dev, "null argument");
+    GRAPES_REQUIRE(num_nodes > 0 && num_nodes < (1ll << 31), "num_nodes must fit int32");
+    GRAPES_REQUIRE(world >= 1 && world <= 1024, "world must be in [1, 1024]");
+    pdl(k_gn_bounds, 1, 128, 0, (cudaStream_t)stream)(num_nodes, (const long long*)in_off, world,
+                                                                         (long long*)bounds_dev);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_window_add_csr(int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0, int64_t r1,
+                                     int64_t lo, int64_t hi, const int64_t* win_off, int* in_src, void* workspace,
+                                     void* stream) {
+    GRAPES_REQUIRE(indptr && workspace && win_off && in_src, "null argument");
+    GRAPES_REQUIRE(0 <= r0 && r0 <= r1 && r1 <= num_nodes, "row range outside [0, N]");
+    GRAPES_REQUIRE(0 <= lo && lo <= hi && hi <= num_nodes, "window outside [0, N]");
+    if (r1 == r0 || hi == lo) return GRAPES_OK;
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    int* cnt = (int*)((unsigned char*)workspace + gn_layout(num_nodes).cnt);
+    const int64_t ctas = ((r1 - r0) * 32 + CB_THREADS - 1) / CB_THREADS;
+    pdl(k_gnw_csr, (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16), CB_THREADS, 0, (cudaStream_t)stream)(
+        (const long long*)indptr, indices, r0, r1, num_nodes, lo, hi, cnt, (const long long*)win_off, in_src);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_window_add_edges(int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                       int64_t lo, int64_t hi, const int64_t* win_off, int* in_src, void* workspace,
+                                       void* stream) {
+    GRAPES_REQUIRE(num_edges >= 0, "negative edge count");
+    GRAPES_REQUIRE(workspace && win_off && in_src && (num_edges == 0 || (src && dst)), "null argument");
+    GRAPES_REQUIRE(0 <= lo && lo <= hi && hi <= num_nodes, "window outside [0, N]");
+    if (num_edges == 0 || hi == lo) return GRAPES_OK;
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    int* cnt = (int*)((unsigned char*)workspace + gn_layout(num_nodes).cnt);
+    const int64_t ctas = (num_edges + CB_THREADS - 1) / CB_THREADS;
+    pdl(k_gnw_edges, (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16), CB_THREADS, 0, (cudaStream_t)stream)(
+        src, dst, num_edges, num_nodes, lo, hi, cnt, (const long long*)win_off, in_src);
+    grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
 }

@@ -141,6 +141,80 @@ __global__ void __launch_bounds__(256) k_agg(const void* __restrict__ X, int F, 
 }
 
 // ---------------------------------------------------------------------------------------
+// k_agg_peer: k_agg<VEC, false, true> over an fp32 operand whose rows are partitioned between `world` owners (the layer 2
+// of the sharded whole-graph forward, grapes_aggregate_rows64_peer): row s lives at base[o] + (s - bound[o]) * ldx for the
+// owner o with bound[o] <= s < bound[o + 1], in this rank's memory or a peer's (NVLink).  The loading lane resolves the
+// owner and broadcasts the row address instead of the row id; the fma chain (self term, then sources ascending, bias last)
+// is k_agg's, so the rows are bit-identical to grapes_aggregate_rows64 over the unpartitioned operand.  A kernel of its own
+// rather than a template parameter of k_agg, which would rename every existing k_agg instantiation.
+// ---------------------------------------------------------------------------------------
+#define GRAPES_PEER_MAX 8
+struct PeerRows {
+    const float* base[GRAPES_PEER_MAX];
+    int bound[GRAPES_PEER_MAX + 1];
+    int world;
+};
+
+__device__ __forceinline__ const float* peer_row(const PeerRows& P, int s, int ldx) {
+    // selects with constant indices (bounds do not decrease: the last window starting at or before s owns it); an index
+    // computed at run time would copy the parameter struct to the stack
+    const float* b = P.base[0];
+    int lo = 0;
+#pragma unroll
+    for (int k = 1; k < GRAPES_PEER_MAX; ++k)
+        if (k < P.world && s >= P.bound[k]) { b = P.base[k]; lo = P.bound[k]; }
+    return b + (size_t)(s - lo) * ldx;
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(256) k_agg_peer(const PeerRows P, int F, int ldx, const int* __restrict__ n_dev, int cap_n,
+                                                  const long long* __restrict__ in_off, const int* __restrict__ in_src,
+                                                  const float* __restrict__ dinv, const float* __restrict__ bias,
+                                                  float* __restrict__ out, int ldo) {
+    pdl_begin();
+    const int n = min(*n_dev, cap_n);
+    const int r0 = n_dev[1];
+    const int lane = lane_id();
+    const int warps = (gridDim.x * blockDim.x) >> 5;
+    for (int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += warps) {
+        const int jr = r0 + j;
+        const float dj = dinv[jr];
+        const long long beg = in_off[jr], end = in_off[jr + 1];
+        const float* xj = peer_row(P, jr, ldx);
+        float* oj = out + (size_t)j * ldo;
+        for (int cb = 0; cb < F; cb += 32 * VEC) {
+            const int c0 = cb + lane * VEC;
+            const bool act = c0 < F;
+            float acc[VEC];
+#pragma unroll
+            for (int i = 0; i < VEC; ++i) acc[i] = 0.f;
+            if (act) vec_fma<VEC>(acc, dj * dj, xj + c0);
+            for (long long pb = beg; pb < end; pb += 32) {
+                const long long p = pb + lane;
+                float w = 0.f; unsigned long long sa = 0ull;
+                if (p < end) {
+                    const int sl = in_src[p];
+                    w = dinv[sl] * dj;
+                    sa = (unsigned long long)peer_row(P, sl, ldx);
+                }
+                const int cnt = (int)min(32ll, end - pb);
+                for (int t = 0; t < cnt; ++t) {
+                    const float wt = __shfl_sync(GRAPES_FULL_MASK, w, t);
+                    const unsigned long long st = __shfl_sync(GRAPES_FULL_MASK, sa, t);
+                    if (act) vec_fma<VEC>(acc, wt, reinterpret_cast<const float*>(st) + c0);
+                }
+            }
+            if (act) {
+#pragma unroll
+                for (int i = 0; i < VEC; ++i) if (bias) acc[i] += bias[c0 + i];
+                *reinterpret_cast<typename VecT<VEC>::T*>(oj + c0) = *reinterpret_cast<typename VecT<VEC>::T*>(acc);
+            }
+        }
+        for (int c = F + lane; c < ldo; c += 32) oj[c] = 0.f;
+    }
+}
+
+// ---------------------------------------------------------------------------------------
 // k_agg_rows: the same aggregation with R destination rows per warp, their dependent load chains interleaved
 // (row offsets -> source ids -> source node ids / weights -> feature rows): the chain is 4 memory latencies deep and
 // one-row-per-warp pays it once per row and wave; R rows in flight per warp cut the number of waves R-fold.  Same
@@ -1197,6 +1271,39 @@ int grapes_aggregate_rows64(grapes_ctx* ctx, const void* X, int x_bf16, int F, i
         }
 #undef AGG64
     }
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_aggregate_rows64_peer(grapes_ctx* ctx, const void* const* z_rows, const int64_t* bounds, int world, int F,
+                                 int ldz, const int* slab_dev, int cap_r, const int64_t* in_off, const int* in_src,
+                                 const float* dinv, const float* bias, float* out, int ldo, void* stream) {
+    if (cap_r <= 0) return GRAPES_OK;                    // an empty window: nothing to read or write
+    GRAPES_REQUIRE(ctx && z_rows && bounds && slab_dev && in_off && in_src && dinv && out, "null argument");
+    GRAPES_REQUIRE(world >= 1 && world <= GRAPES_PEER_MAX, "1 to 8 row owners");
+    GRAPES_REQUIRE(F > 0 && ldz >= F && ldo >= F, "bad shape");
+    PeerRows P = {};
+    size_t al = (size_t)out;
+    GRAPES_REQUIRE(bounds[0] == 0 && bounds[world] < (1ll << 31), "bounds[0] must be 0 and bounds[world] fit int32");
+    for (int o = 0; o < world; ++o) {
+        GRAPES_REQUIRE(bounds[o] <= bounds[o + 1], "bounds must not decrease");
+        GRAPES_REQUIRE(z_rows[o] || bounds[o] == bounds[o + 1], "null row base of a non-empty window");
+        P.base[o] = reinterpret_cast<const float*>(z_rows[o]);
+        P.bound[o] = (int)bounds[o];
+        al |= (size_t)z_rows[o];
+    }
+    P.bound[world] = (int)bounds[world];
+    P.world = world;
+    cudaStream_t s = (cudaStream_t)stream;
+    const long long* off = reinterpret_cast<const long long*>(in_off);
+    const int blocks = grid_for(ctx, (long long)cap_r * 32, 256, 8);
+    if ((al & 15) == 0 && F % 4 == 0 && ldz % 4 == 0 && ldo % 4 == 0)
+        pdl((k_agg_peer<4>), blocks, 256, 0, s)(P, F, ldz, slab_dev, cap_r, off, in_src, dinv, bias, out, ldo);
+    else if ((al & 7) == 0 && F % 2 == 0 && ldz % 2 == 0 && ldo % 2 == 0)
+        pdl((k_agg_peer<2>), blocks, 256, 0, s)(P, F, ldz, slab_dev, cap_r, off, in_src, dinv, bias, out, ldo);
+    else
+        pdl((k_agg_peer<1>), blocks, 256, 0, s)(P, F, ldz, slab_dev, cap_r, off, in_src, dinv, bias, out, ldo);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;

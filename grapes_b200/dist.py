@@ -80,3 +80,71 @@ class PeerGradExchange:
         # NOTE: no collective here.  The caller must synchronise the ranks once before the first exchange (every buffer is
         # zeroed before anyone publishes): GrapesEngine.enable_data_parallel does it with the all-reduce that also makes
         # the ranks agree on whether the peer mapping worked everywhere.
+
+
+def eval_batches(num_batches: int, rank: int, world: int) -> List[int]:
+    """Batches of the evaluation split that rank ``rank`` runs: every i with i mod W == rank, the tail round included
+    (unlike :func:`shard_batches`, nothing waits on a per-batch collective here, so no batch is dropped)."""
+    return list(range(rank, num_batches, world))
+
+
+def allreduce_counts_(counts: torch.Tensor, group=None) -> torch.Tensor:
+    """In-place integer sum over the ranks of ``group`` (hits / rows / tp / fp / fn): exact, so the scores computed from it
+    are those of one process over all rows."""
+    dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=group)
+    return counts
+
+
+def gather_batch_predictions(local: torch.Tensor, batch_sizes: List[int], group=None) -> torch.Tensor:
+    """The predictions of every batch in batch order, on every rank.  ``local`` holds this rank's batches
+    (:func:`eval_batches`) back to back; ``batch_sizes`` lists the size of every batch of the split."""
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    per_rank = [sum(batch_sizes[i] for i in eval_batches(len(batch_sizes), r, world)) for r in range(world)]
+    if local.numel() != per_rank[rank]:
+        raise ValueError(f"rank {rank} holds {local.numel()} predictions, its batches have {per_rank[rank]}")
+    width = max(per_rank + [1])
+    padded = torch.zeros(width, dtype=local.dtype, device=local.device)
+    padded[:local.numel()] = local
+    parts = [torch.empty_like(padded) for _ in range(world)]
+    dist.all_gather(parts, padded, group=group)
+    out, cursor = [], [0] * world
+    for i, n in enumerate(batch_sizes):
+        r = i % world
+        out.append(parts[r][cursor[r]:cursor[r] + n])
+        cursor[r] += n
+    return torch.cat(out) if out else local[:0]
+
+
+class PeerRowTable:
+    """The layer-2 operand table of :func:`grapes_b200.gcn.full_graph_forward_sharded` across the ranks of ``group``: one
+    ``torch.distributed._symmetric_memory`` buffer of ``rows`` x ``ld`` floats per rank (this rank's window of Z, zero pad
+    columns), ``ptrs`` = the HOST array of every rank's buffer address (own at ``rank``), and ``barrier()`` = the
+    stream-ordered barrier of the symmetric-memory handle (no host synchronisation).  Construction only allocates (rank
+    local); :meth:`rendezvous` maps the peers and is collective.  Built once per graph and classifier width and cached
+    with the window structure (``eval._sharded_eval``)."""
+
+    def __init__(self, rows: int, ld: int, device: torch.device, group=None):
+        import torch.distributed._symmetric_memory as symm_mem
+        self.group = group or dist.group.WORLD
+        self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
+        if self.world > 8:
+            raise RuntimeError("the peer row table is built for one NVSwitch box (<= 8 ranks)")
+        self.ld = int(ld)
+        self.buf = symm_mem.empty(max(int(rows), 1) * self.ld, dtype=torch.float32, device=device)
+        self.buf.zero_()
+        self.rows = self.buf.view(max(int(rows), 1), self.ld)
+        self.hdl, self.ptrs = None, None
+
+    def rendezvous(self):
+        import ctypes
+        import torch.distributed._symmetric_memory as symm_mem
+        g = self.group
+        self.hdl = symm_mem.rendezvous(self.buf, g.group_name if hasattr(g, "group_name") else g)
+        ptrs = [int(p) for p in self.hdl.buffer_ptrs]
+        assert ptrs[self.rank] == self.buf.data_ptr()
+        self.ptrs = (ctypes.c_void_p * self.world)(*ptrs)
+        torch.cuda.synchronize(self.buf.device)
+        return self
+
+    def barrier(self):
+        self.hdl.barrier(channel=0)

@@ -23,10 +23,15 @@ from __future__ import annotations
 import os
 from typing import Optional, Tuple
 
+import warnings
+
+import numpy as np
 import torch
+import torch.distributed as dist
 
 from ._lib import GrapesError
-from .gcn import GCN, GraphNorm, WideGraphNorm, full_graph_forward, full_graph_forward_streamed
+from .gcn import (GCN, GraphNorm, ShardedGraphNorm, WideGraphNorm, _scores_from_counts, full_graph_forward,
+                  full_graph_forward_sharded, full_graph_forward_streamed, row_slab_refusal)
 from .graph import DeviceGraph
 from .utils import TensorMap, get_logger
 
@@ -77,7 +82,10 @@ def evaluate(gcn_c: GCN,
              full_batch: bool = False,
              return_predictions: bool = False,
              engine=None,
+             group=None,
              ):
+    """``group``: a ``torch.distributed`` process group of more than one rank makes the evaluation data parallel, with
+    the scores of one process (see :func:`_evaluate_sharded`); None or a one-rank group runs the single-process code."""
     get_logger().info('Evaluating')
     device = torch.device(device)
     if device.type != "cuda":
@@ -86,6 +94,11 @@ def evaluate(gcn_c: GCN,
     y = data.y.to(device)
     gcn_c = gcn_c.to(device).eval()
     mask_d = mask.to(device) if mask is not None else torch.ones(data.num_nodes, dtype=torch.bool, device=device)
+    if group is not None and dist.is_initialized() and dist.get_world_size(group) > 1:
+        res = _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, device, x, y, mask_d, loader,
+                                full_batch, return_predictions, engine, group)
+        if res is not None:
+            return res
 
     if full_batch:
         ei = getattr(data, "edge_index", None)
@@ -120,6 +133,112 @@ def evaluate(gcn_c: GCN,
     targets = y[mask_d]
     acc = (all_predictions == targets).float().mean().item()          # accuracy_score == micro f1_score here
     return (acc, acc, all_predictions) if return_predictions else (acc, acc)
+
+
+def _mean_of_hits(hits: int, rows: int) -> float:
+    """``(pred == y).float().mean().item()`` on the device from the integer count: CUDA's mean is the float32 sum times
+    float32(1 / rows).  The float32 sum of a 0/1 vector is exact below 2^24 rows, so below that the result is bit for bit
+    the one-process score; past it the one-process sum may round and the two can differ in the last place (the integer
+    count here is the exact one)."""
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return float(np.float32(hits) * (np.float32(1) / np.float32(rows)))
+
+
+def _sharded_eval(adjacency: DeviceGraph, data, group, C4: int, device):
+    """(window structure, peer row table or None) of this rank, cached on the graph object like ``_graph_norm``.  The
+    table is None when the symmetric mapping failed on any rank (every rank agrees, so none of them waits on a peer)."""
+    from .dist import PeerRowTable, ranks_agree
+    ei = getattr(data, "edge_index", None)
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    key = (None if ei is None else (ei.data_ptr(), tuple(ei.shape)), world, rank, C4)
+    cached = getattr(adjacency, "_sharded_eval", None)
+    if cached is None or cached[0] != key:
+        adjacency._sharded_eval = None
+        sgn, table, why = None, None, ""
+        try:                                           # rank-local failures (memory, ids, mapping) become the fall-back
+            sgn = ShardedGraphNorm(adjacency, world, rank, edge_index=ei)
+            rows = max(sgn.bounds[r + 1] - sgn.bounds[r] for r in range(world))
+            table = PeerRowTable(rows, C4, device, group)
+        except Exception as exc:                       # noqa: BLE001 -- reported below, never silent
+            why = f"{type(exc).__name__}: {exc}"
+        if ranks_agree(table is not None, device, group):
+            try:
+                table.rendezvous()
+            except Exception as exc:                   # noqa: BLE001
+                why, table = f"{type(exc).__name__}: {exc}", None
+            if not ranks_agree(table is not None, device, group):
+                table = None
+        else:
+            table = None
+        if table is None:
+            sgn = None                                 # the replicated evaluation builds the whole structure instead
+            warnings.warn("grapes_b200: sharded full-batch structure or peer-mapped row table unavailable" +
+                          (f" ({why})" if why else
+                          " on another rank") + "; every rank runs the replicated full-batch evaluation")
+        cached = (key, sgn, table)
+        adjacency._sharded_eval = cached
+    return cached[1], cached[2]
+
+
+def _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, device, x, y, mask_d, loader, full_batch,
+                      return_predictions, engine, group):
+    """Data-parallel evaluation over the ranks of ``group``, with the scores one process computes:
+
+    * full batch: every rank builds its destination window of the structure (:class:`ShardedGraphNorm`) and runs
+      :func:`full_graph_forward_sharded` (layer 2 reads Z over peer memory); the integer counts are summed over the ranks.
+      ``return_predictions`` raises ``GrapesError`` (gathering [N, C] on every rank is the memory this path saves), and
+      ``GRAPES_EVAL_TC`` has no effect.  Returns None -- the caller then runs the replicated evaluation -- when the
+      row-slab forward does not cover the classifier (:func:`grapes_b200.gcn.row_slab_refusal`; weights and features are
+      replicated, so every rank decides alike) or when the window structure or the peer mapping failed on any rank.
+    * mini batch: rank r runs the batches i = r mod W of the split, all of them; hits and rows are summed as integers, and
+      ``return_predictions`` gathers every rank's predictions back into batch order."""
+    from .dist import allreduce_counts_, eval_batches, gather_batch_predictions, ranks_agree
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    if full_batch:
+        if return_predictions:
+            raise GrapesError("data-parallel full-batch evaluation returns scores only: gathering the [N, C] logits on "
+                              "every rank is the memory it avoids (evaluate without a group for the logits)")
+        if row_slab_refusal(gcn_c, x) is not None:
+            return None               # a classifier the row-slab forward does not cover: the same on every rank
+        C = int(gcn_c.gcn_layers[-1].lin.weight.shape[0])
+        sgn, table = _sharded_eval(adjacency, data, group, (C + 3) // 4 * 4, device)
+        if table is None:
+            return None
+        _, counts = full_graph_forward_sharded(gcn_c, x, sgn, table, y=y, mask=mask_d)
+        allreduce_counts_(counts, group)
+        ei = getattr(data, "edge_index", None)
+        if y.dim() == 1 and (int(ei.shape[1]) if ei is not None else adjacency.nnz) < WIDE_MIN_EDGES:
+            acc = _mean_of_hits(int(counts[0]), int(counts[1]))       # what _scores computes on one GPU
+            return acc, acc
+        return _scores_from_counts(counts, y.dim() == 1)
+
+    assert loader is not None, 'loader must be provided if full_batch is False'
+    batches = [b[0] if isinstance(b, (tuple, list)) else b for b in loader]
+    sizes = [int(b.numel()) for b in batches]
+    mine = eval_batches(len(batches), rank, world)
+    eng = engine if engine is not None else _eval_engine(adjacency, data, args, gcn_c, gcn_gf, num_indicators, device,
+                                                         max(sizes + [1]))
+    total = sum(sizes[i] for i in mine)
+    preds = torch.zeros(max(total, 1), dtype=torch.int32, device=device)
+    off = 0
+    for i in mine:
+        eng.predict(batches[i].to(device), preds[off:off + sizes[i]])
+        off += sizes[i]
+    failure = None
+    try:
+        eng.check_overflow()
+    except GrapesError as exc:                         # raised on every rank, so none of them waits in the all-reduce
+        failure = exc
+    if not ranks_agree(failure is None, device, group):
+        raise failure or GrapesError("data-parallel mini-batch evaluation: another rank's batches overflowed")
+    local = preds[:total].to(torch.int64)
+    targets = y[torch.cat([batches[i].to(device).long() for i in mine])] if mine else local
+    counts = torch.stack([(local == targets).sum(), local.new_tensor(total)])
+    allreduce_counts_(counts, group)
+    acc = _mean_of_hits(int(counts[0]), int(counts[1]))
+    if return_predictions:
+        return acc, acc, gather_batch_predictions(local, sizes, group)
+    return acc, acc
 
 
 def _eval_engine(adjacency: DeviceGraph, data, args, gcn_c: GCN, gcn_gf: GCN, num_indicators: int, device, batch_size: int):

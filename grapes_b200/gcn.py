@@ -221,10 +221,7 @@ class WideGraphNorm:
                 L.grapes_graph_norm_add_csr(pass_, N, ptr(graph.indptr), ptr(graph.indices), 0, N, ptr(self.in_off),
                                             ptr(in_src), ptr(ws), ptr(err), st)
                 return
-            E = int(edge_index.shape[1])
-            for a in range(0, E, chunk_edges):
-                src = edge_index[0, a:a + chunk_edges].to(device=dev, dtype=torch.int64).contiguous()
-                dst = edge_index[1, a:a + chunk_edges].to(device=dev, dtype=torch.int64).contiguous()
+            for src, dst in _edge_chunks(edge_index, chunk_edges, dev):
                 L.grapes_graph_norm_add_edges(pass_, N, ptr(src), ptr(dst), int(src.numel()), ptr(self.in_off),
                                               ptr(in_src), ptr(ws), ptr(err), st)
 
@@ -255,6 +252,94 @@ class WideGraphNorm:
         lib().grapes_aggregate_rows64(self.holder.ctx, ptr(x), int(x.dtype == torch.bfloat16), F, x.stride(0), ptr(slab),
                                       R, ptr(self.in_off), ptr(self.in_src), ptr(self.dinv), ptr(bias), ptr(out),
                                       out.stride(0), _stream())
+        return out
+
+
+def _edge_chunks(edge_index, chunk_edges, dev):
+    """(src, dst) int64 device slices of ``edge_index`` [2, E] (host or device), ``chunk_edges`` columns at a time."""
+    for a in range(0, int(edge_index.shape[1]), chunk_edges):
+        yield (edge_index[0, a:a + chunk_edges].to(device=dev, dtype=torch.int64).contiguous(),
+               edge_index[1, a:a + chunk_edges].to(device=dev, dtype=torch.int64).contiguous())
+
+
+class ShardedGraphNorm:
+    """One rank's destination window of the :class:`WideGraphNorm` structure, for the data-parallel full-batch evaluation
+    (:func:`full_graph_forward_sharded`).  The rows are cut into ``world`` contiguous windows ``bounds[r] .. bounds[r+1]``
+    balanced by the prefix of indeg + 1 (``grapes_graph_norm_window_bounds``; every rank computes the same bounds, windows
+    are empty when N < world).  Holds ``in_off`` int64 [rows + 1] local to the window, ``in_src`` int32 of the window's rows
+    only (~1/world of the whole) and ``dinv`` fp32 for all N nodes (the source weights); equal bit for bit to rows
+    ``lo .. hi`` of :class:`WideGraphNorm`.  Every degree is still counted (pass 0 reads the whole input); pass 1 scatters
+    only the edges into the window.  Device memory beyond the outputs: the ~4 N-byte workspace, plus the full int64
+    [N + 1] offsets until the window's are cut out, plus one chunk of a host edge list."""
+
+    def __init__(self, graph, world: int, rank: int, edge_index=None, chunk_edges: int = 1 << 27):
+        if not 0 <= rank < world:
+            raise GrapesError(f"rank {rank} outside a world of {world}")
+        dev = graph.device
+        N = graph.num_nodes
+        L, st = lib(), _stream()
+        self.graph, self.world, self.rank = graph, int(world), int(rank)
+        self.holder = _any_ctx(dev)
+        self.n = N
+        ws = torch.empty(max(int(L.cdll.grapes_graph_norm_workspace_bytes(N)), 1), dtype=torch.uint8, device=dev)
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        nnz = torch.zeros(1, dtype=torch.int64, device=dev)
+        full = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        self.dinv = torch.empty(N, dtype=torch.float32, device=dev)
+        L.grapes_graph_norm_begin(N, ptr(ws), ws.numel(), ptr(err), st)
+        if edge_index is None:
+            L.grapes_graph_norm_add_csr(0, N, ptr(graph.indptr), ptr(graph.indices), 0, N, None, None, ptr(ws), ptr(err), st)
+        else:
+            for src, dst in _edge_chunks(edge_index, chunk_edges, dev):
+                L.grapes_graph_norm_add_edges(0, N, ptr(src), ptr(dst), int(src.numel()), None, None, ptr(ws), ptr(err), st)
+        L.grapes_graph_norm_offsets(N, ptr(ws), ptr(full), ptr(self.dinv), ptr(nnz), st)
+        bounds = torch.empty(self.world + 1, dtype=torch.int64, device=dev)
+        L.grapes_graph_norm_window_bounds(N, ptr(full), self.world, ptr(bounds), st)
+        WideGraphNorm._check(err)
+        self.bounds = [int(b) for b in bounds.tolist()]                 # one-off read-back
+        self.lo, self.hi = self.bounds[rank], self.bounds[rank + 1]
+        self.rows = self.hi - self.lo
+        self.in_off = (full[self.lo:self.hi + 1] - full[self.lo]).contiguous()
+        del full
+        self.E = int(self.in_off[-1].item())
+        self.in_src = torch.empty(max(self.E, 1), dtype=torch.int32, device=dev)
+        if edge_index is None:
+            L.grapes_graph_norm_window_add_csr(N, ptr(graph.indptr), ptr(graph.indices), 0, N, self.lo, self.hi,
+                                               ptr(self.in_off), ptr(self.in_src), ptr(ws), st)
+        else:
+            for src, dst in _edge_chunks(edge_index, chunk_edges, dev):
+                L.grapes_graph_norm_window_add_edges(N, ptr(src), ptr(dst), int(src.numel()), self.lo, self.hi,
+                                                     ptr(self.in_off), ptr(self.in_src), ptr(ws), st)
+        if self.rows > 0:
+            L.grapes_graph_norm_finish(self.rows, ptr(self.in_off), ptr(self.in_src), ptr(ws), st)
+        del ws
+        self._src = self.in_src                    # non-null for the kernels even when the window has no in-edge
+        if self.E == 0:
+            self.in_src = self.in_src[:0]
+
+    @property
+    def in_off_base(self) -> int:
+        """Device address that makes ``in_off[r]`` of the row-slab kernels (r = graph row) land on local row r - lo: the
+        window's offsets shifted back by ``lo`` entries.  Only rows of the window are ever read through it."""
+        return self.in_off.data_ptr() - 8 * self.lo
+
+    def aggregate_rows(self, x: torch.Tensor, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None) -> torch.Tensor:
+        """:meth:`WideGraphNorm.aggregate_rows` for a slab {R, r0} inside the window (r0 a graph row): x holds ALL rows."""
+        F = x.shape[1]
+        lib().grapes_aggregate_rows64(self.holder.ctx, ptr(x), int(x.dtype == torch.bfloat16), F, x.stride(0), ptr(slab),
+                                      R, self.in_off_base, ptr(self._src), ptr(self.dinv), ptr(bias), ptr(out),
+                                      out.stride(0), _stream())
+        return out
+
+    def aggregate_rows_peer(self, z_table, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None) -> torch.Tensor:
+        """The same over Z partitioned by window: rank o's rows in ``z_table.ptrs[o]`` (pitch ``z_table.ld`` floats),
+        ``grapes_aggregate_rows64_peer``; bit-identical to :meth:`aggregate_rows` over the unpartitioned Z."""
+        import ctypes
+        F = z_table.ld
+        b = (ctypes.c_int64 * (self.world + 1))(*self.bounds)
+        lib().grapes_aggregate_rows64_peer(self.holder.ctx, z_table.ptrs, b, self.world, F, z_table.ld, ptr(slab), R,
+                                           self.in_off_base, ptr(self._src), ptr(self.dinv), ptr(bias), ptr(out),
+                                           out.stride(0), _stream())
         return out
 
 
@@ -297,71 +382,196 @@ def full_graph_forward_streamed(gcn: "GCN", x: torch.Tensor, gn: WideGraphNorm, 
     (and ``mask``, default all rows) the scores of ``eval._scores`` are reduced per slab on the device.  Returns
     (logits [N, C] or None when ``return_logits`` is False, (accuracy, f1) or None).  Other depths, a layer 2 that would
     aggregate first (D <= C), other table dtypes and dropout in training mode raise ``GrapesError``."""
-    layers = list(gcn.gcn_layers)
-    if len(layers) != 2:
-        raise GrapesError(f"streamed full-graph forward covers the two-layer classifier, not {len(layers)} layers")
-    if gcn.training and gcn.dropout > 0:
-        raise GrapesError("streamed full-graph forward is evaluation only: dropout in training mode")
-    if x.dtype not in (torch.float32, torch.bfloat16) or x.dim() != 2 or x.stride(1) != 1:
-        raise GrapesError("streamed full-graph forward reads fp32 or bf16 rows with a unit column stride")
+    w1, b1, w2, b2, D, C, C4 = _classifier_parts(gcn, x)
     dev = x.device
     N, F = x.shape                                    # (shadows torch.nn.functional inside this function)
+    agg_first = F <= D
+    resident = N * C4 * 4 + (0 if agg_first else N * D * 4) + (N * C4 * 4 if return_logits else 0)
+    R = int(slab_rows) if slab_rows else slab_rows_for(N, _slab_row_bytes(x, D, C4), resident, dev, mem_budget)
+    R = max(1, min(R, max(N, 1)))
+    starts, slabs = _slab_plan(0, N, R, dev)
+    Z = torch.zeros((N, C4), dtype=torch.float32, device=dev)
+    _layer1_into(x, gn, (w1, b1, w2, D, C, C4), starts, slabs, N, R, Z, 0)
+    logits, counts = _layer2(lambda s, n, o: gn.aggregate_rows(Z, s, n, o, bias=b2), starts, slabs, N, R, C, C4, dev,
+                             y, mask, return_logits)
+    scores = None if counts is None else _scores_from_counts(counts, y.dim() == 1)
+    return logits, scores
+
+
+def row_slab_refusal(gcn: "GCN", x: torch.Tensor):
+    """Why the row-slab forwards (:func:`full_graph_forward_streamed`, :func:`full_graph_forward_sharded`) do not cover
+    this classifier and feature table, or None when they do."""
+    layers = list(gcn.gcn_layers)
+    if len(layers) != 2:
+        return f"streamed full-graph forward covers the two-layer classifier, not {len(layers)} layers"
+    if gcn.training and gcn.dropout > 0:
+        return "streamed full-graph forward is evaluation only: dropout in training mode"
+    if x.dtype not in (torch.float32, torch.bfloat16) or x.dim() != 2 or x.stride(1) != 1:
+        return "streamed full-graph forward reads fp32 or bf16 rows with a unit column stride"
+    if layers[0].lin.weight.shape[0] <= layers[1].lin.weight.shape[0]:
+        return "streamed full-graph forward needs hidden width D > classes C (layer 2 transforms first)"
+    return None
+
+
+def _classifier_parts(gcn: "GCN", x: torch.Tensor):
+    """Checks of the row-slab forwards and the classifier's fp32 weights: (w1, b1, w2, b2 padded to C4, D, C, C4)."""
+    why = row_slab_refusal(gcn, x)
+    if why is not None:
+        raise GrapesError(why)
+    layers = list(gcn.gcn_layers)
     w1 = layers[0].lin.weight.detach().float().contiguous()
     b1 = layers[0].bias.detach().float().contiguous()
     w2 = layers[1].lin.weight.detach().float().contiguous()
     D, C = w1.shape[0], w2.shape[0]
-    if D <= C:
-        raise GrapesError("streamed full-graph forward needs hidden width D > classes C (layer 2 transforms first)")
     C4 = (C + 3) // 4 * 4
     b2 = F_pad(layers[1].bias.detach().float(), C4 - C).contiguous()
-    agg_first = F <= D
-    resident = N * C4 * 4 + (0 if agg_first else N * D * 4) + (N * C4 * 4 if return_logits else 0)
-    per_row = 4 * ((F if agg_first else 0) + (F if (not agg_first and x.dtype != torch.float32) else 0) + D + C4)
-    R = int(slab_rows) if slab_rows else slab_rows_for(N, per_row, resident, dev, mem_budget)
-    R = max(1, min(R, max(N, 1)))
-    starts = list(range(0, N, R))
-    slabs = torch.tensor([[min(R, N - r0), r0] for r0 in starts] or [[0, 0]], dtype=torch.int32, device=dev)
+    return w1, b1, w2, b2, D, C, C4
 
-    Z = torch.zeros((N, C4), dtype=torch.float32, device=dev)
+
+def _slab_row_bytes(x: torch.Tensor, D: int, C4: int) -> int:
+    F = x.shape[1]
+    agg_first = F <= D
+    return 4 * ((F if agg_first else 0) + (F if (not agg_first and x.dtype != torch.float32) else 0) + D + C4)
+
+
+def _slab_plan(lo: int, hi: int, R: int, dev):
+    """Slab starts over rows [lo, hi) and the device {rows, r0} pair of each."""
+    starts = list(range(lo, hi, R))
+    slabs = torch.tensor([[min(R, hi - r0), r0] for r0 in starts] or [[0, 0]], dtype=torch.int32, device=dev)
+    return starts, slabs
+
+
+def _layer1_into(x, gn, w, starts, slabs, hi, R, Z, z0):
+    """Z[r - z0] = relu(A_hat X W1^T + b1)[r] W2^T for the rows r of the slabs (ending at ``hi``), at the narrower width:
+    F <= D aggregates X per slab first; F > D forms P = X W1^T for ALL N rows (the sources of any row) first."""
+    w1, b1, w2, D, C, C4 = w
+    dev = x.device
+    N, F = x.shape
     H = torch.empty((R, D), dtype=torch.float32, device=dev)
-    if agg_first:
+    if F <= D:
         Y = torch.empty((R, F), dtype=torch.float32, device=dev)
         for i, r0 in enumerate(starts):
-            n = min(R, N - r0)
+            n = min(R, hi - r0)
             gn.aggregate_rows(x, slabs[i], n, Y)
             _gemm_into(Y, F, w1, F, H, D, n, D, F, bias=b1)
             torch.relu_(H[:n])
-            _gemm_into(H, D, w2, D, Z[r0:], C4, n, C, D)
+            _gemm_into(H, D, w2, D, Z[r0 - z0:], C4, n, C, D)
         del Y
     else:
         P = torch.empty((N, D), dtype=torch.float32, device=dev)
-        for r0 in starts:
+        for r0 in range(0, N, R):
             n = min(R, N - r0)
             xs = x[r0:r0 + n] if x.dtype == torch.float32 else x[r0:r0 + n].float()
             _gemm_into(xs, xs.stride(0), w1, F, P[r0:], D, n, D, F)
         for i, r0 in enumerate(starts):
-            n = min(R, N - r0)
+            n = min(R, hi - r0)
             gn.aggregate_rows(P, slabs[i], n, H, bias=b1)
             torch.relu_(H[:n])
-            _gemm_into(H, D, w2, D, Z[r0:], C4, n, C, D)
+            _gemm_into(H, D, w2, D, Z[r0 - z0:], C4, n, C, D)
         del P
     del H
 
-    logits = torch.empty((N, C4), dtype=torch.float32, device=dev) if return_logits else None
+
+def _layer2(agg, starts, slabs, hi, R, C, C4, dev, y, mask, return_logits):
+    """logits = A_hat Z + b2 per slab through ``agg(slab, n, out)``, with the masked counts of :func:`_slab_counts` reduced
+    on the device when ``y`` is given.  Returns (logits [hi - starts[0], C] or None, counts int64 [3] or None)."""
+    lo = starts[0] if starts else hi
+    logits = torch.empty((hi - lo, C4), dtype=torch.float32, device=dev) if return_logits else None
     out = None if return_logits else torch.empty((R, C4), dtype=torch.float32, device=dev)
     counts = torch.zeros(3, dtype=torch.int64, device=dev) if y is not None else None
     for i, r0 in enumerate(starts):
-        n = min(R, N - r0)
-        o = logits[r0:r0 + n] if return_logits else out
-        gn.aggregate_rows(Z, slabs[i], n, o, bias=b2)
+        n = min(R, hi - r0)
+        o = logits[r0 - lo:r0 - lo + n] if return_logits else out
+        agg(slabs[i], n, o)
         if counts is not None:
             lg, ys = o[:n, :C], y[r0:r0 + n]
             if mask is not None:
                 m = mask[r0:r0 + n]
                 lg, ys = lg[m], ys[m]
             counts += _slab_counts(lg, ys)
-    scores = None if counts is None else _scores_from_counts(counts, y.dim() == 1)
-    return (logits[:, :C] if return_logits else None), scores
+    return (logits[:, :C] if return_logits else None), counts
+
+
+class LocalRowTable:
+    """The layer-2 operand table of :func:`full_graph_forward_sharded` for one emulated rank of a single process: every
+    window's rows in its own allocation on this device (``tables[o]``, shared by the emulated ranks), a barrier that does
+    nothing.  Run :func:`sharded_layer1` for every emulated rank before :func:`sharded_layer2` for any of them.
+    :class:`grapes_b200.dist.PeerRowTable` is the same interface over the ranks' symmetric memory."""
+
+    def __init__(self, tables, rank: int):
+        import ctypes
+        self.tables, self.rank = tables, rank
+        self.rows = tables[rank]
+        self.ld = int(self.rows.shape[1])
+        self.ptrs = (ctypes.c_void_p * len(tables))(*[t.data_ptr() for t in tables])
+
+    @staticmethod
+    def make(world: int, rows: int, ld: int, device):
+        tables = [torch.zeros((max(rows, 1), ld), dtype=torch.float32, device=device) for _ in range(world)]
+        return [LocalRowTable(tables, r) for r in range(world)]
+
+    def barrier(self):
+        pass
+
+
+def _sharded_rows(sgn, R):
+    return max(1, min(int(R), max(sgn.rows, 1)))
+
+
+@torch.no_grad()
+def sharded_layer1(gcn: "GCN", x: torch.Tensor, sgn: ShardedGraphNorm, z_table, slab_rows=None, mem_budget=None):
+    """Phase 1 of :func:`full_graph_forward_sharded`: Z rows of this rank's window into ``z_table.rows`` (local row j =
+    graph row lo + j), on the calls and in the order of :func:`full_graph_forward_streamed`'s layer 1.  With F > D
+    every rank forms P = X W1^T for ALL N rows (the sources of its window may be any rows), so that product and its
+    [N, D] buffer do not shrink with the number of ranks; with F <= D (the products and papers shapes) nothing does."""
+    w1, b1, w2, b2, D, C, C4 = _classifier_parts(gcn, x)
+    if sgn.rows == 0:
+        return
+    if z_table.ld != C4 or z_table.rows.shape[0] < sgn.rows:
+        raise GrapesError(f"row table of pitch {z_table.ld} x {z_table.rows.shape[0]} rows; the window needs {C4} x {sgn.rows}")
+    N, F = x.shape
+    resident = 0 if F <= D else N * D * 4
+    R = int(slab_rows) if slab_rows else slab_rows_for(sgn.rows, _slab_row_bytes(x, D, C4), resident, x.device, mem_budget)
+    R = _sharded_rows(sgn, R)
+    starts, slabs = _slab_plan(sgn.lo, sgn.hi, R, x.device)
+    _layer1_into(x, sgn, (w1, b1, w2, D, C, C4), starts, slabs, sgn.hi, R, z_table.rows, sgn.lo)
+
+
+@torch.no_grad()
+def sharded_layer2(gcn: "GCN", sgn: ShardedGraphNorm, z_table, slab_rows=None, mem_budget=None, y=None, mask=None,
+                   return_logits: bool = False):
+    """Phase 2 of :func:`full_graph_forward_sharded`: logits of this rank's window = A_hat Z + b2 with Z read from the rows'
+    owners (``ShardedGraphNorm.aggregate_rows_peer``).  Every rank's phase 1 must have completed.  Returns (window logits
+    [rows, C] or None, int64 counts [3] of :func:`_slab_counts` or None)."""
+    layers = list(gcn.gcn_layers)
+    C = layers[1].lin.weight.shape[0]
+    C4 = (C + 3) // 4 * 4
+    b2 = F_pad(layers[1].bias.detach().float(), C4 - C).contiguous()
+    dev = sgn.dinv.device
+    resident = sgn.rows * C4 * 4 if return_logits else 0
+    R = int(slab_rows) if slab_rows else slab_rows_for(sgn.rows, 4 * C4, resident, dev, mem_budget)
+    R = _sharded_rows(sgn, R)
+    starts, slabs = _slab_plan(sgn.lo, sgn.hi, R, dev)
+    return _layer2(lambda s, n, o: sgn.aggregate_rows_peer(z_table, s, n, o, bias=b2), starts, slabs, sgn.hi, R, C, C4,
+                   dev, y, mask, return_logits)
+
+
+@torch.no_grad()
+def full_graph_forward_sharded(gcn: "GCN", x: torch.Tensor, sgn: ShardedGraphNorm, z_table, y=None, mask=None,
+                               return_logits: bool = False, slab_rows=None, mem_budget=None):
+    """The data-parallel form of :func:`full_graph_forward_streamed`: this rank computes the rows of its window only.
+    Layer 1 over the window's slabs (X replicated) writes Z for the window into this rank's slot of ``z_table``
+    (``rows``, ``ld`` = round_up(C, 4), ``ptrs`` = every rank's slot, ``barrier()``); after a barrier, layer 2 aggregates the
+    window reading each source row of Z from the rank that owns it; a second barrier keeps Z until every rank has read it.
+    The window's logits are bit-identical to the same rows of :func:`full_graph_forward_streamed` and of ``gcn(x,
+    GraphNorm)``.  Returns (window logits [rows, C] or None, int64 counts [3] of the window's masked rows or None); sum the
+    counts over the ranks and score them with :func:`_scores_from_counts`."""
+    sharded_layer1(gcn, x, sgn, z_table, slab_rows=slab_rows, mem_budget=mem_budget)
+    z_table.barrier()
+    res = sharded_layer2(gcn, sgn, z_table, slab_rows=slab_rows, mem_budget=mem_budget, y=y, mask=mask,
+                         return_logits=return_logits)
+    z_table.barrier()
+    return res
 
 
 def _slab_counts(logits_masked: torch.Tensor, y_masked: torch.Tensor) -> torch.Tensor:

@@ -19,9 +19,10 @@ from .graph import DeviceGraph
 from .utils import get_logger
 
 
-def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = True, args=None, graph=None):
+def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = True, args=None, graph=None, group=None):
     """The reference's two evaluation modes (/root/reference/eval.py:47-70 full-batch, :71-163 mini-batch) on the
-    device, with the engine's current weights loaded into drop-in ``GCN`` modules (grapes_b200/eval.py)."""
+    device, with the engine's current weights loaded into drop-in ``GCN`` modules (grapes_b200/eval.py); data parallel
+    over ``group`` when it has more than one rank."""
     from .eval import evaluate as _evaluate
     dev = engine.device
     sd = engine.state_dicts()
@@ -37,18 +38,20 @@ def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = 
     ns = args if args is not None else type("A", (), dict(sampling_hops=engine.H, num_samples=engine.k,
                                                           use_indicators=engine.use_ind))()
     return _evaluate(gcn_c, gcn_gf, data, ns, graph, None, engine.num_ind, dev, mask=mask, eval_on_cpu=False,
-                     loader=loader, full_batch=full_batch, engine=None if full_batch else engine)
+                     loader=loader, full_batch=full_batch, engine=None if full_batch else engine, group=group)
 
 
 def train(args: Arguments, data=None, device: Optional[torch.device] = None, use_cuda_graph: bool = True,
-          max_batches: Optional[int] = None, exchange: str = "peer", step_log=None):
+          max_batches: Optional[int] = None, exchange: str = "peer", step_log=None, shard_eval: bool = True):
     """``train(args)`` of the reference (main.py:57-364).  Under ``torchrun`` (WORLD_SIZE > 1, or an initialised
     ``torch.distributed`` group) it is data parallel: every rank holds a replica of the graph and features, batch ``i`` of
     the un-shuffled loader goes to rank ``i mod W`` (``dist.shard_batches``), and the engine exchanges the gradient and
     applies both optimisers inside its step, so all ranks hold the same weights (BASELINE.json north_star).
     ``step_log(dict)`` (optional) receives what main.py:293-311 sends to wandb for every batch -- batch losses, log_z,
     -log_probs and the per-hop sampler statistics ``{min_prob,max_prob,mean_entropy,std_entropy}_{hop}`` -- one step
-    behind, read from pinned host memory (no device stall)."""
+    behind, read from pinned host memory (no device stall).  ``shard_eval`` (data parallel only): every evaluation is
+    split between the ranks (``eval.evaluate(..., group=...)``, the same scores); False makes every rank evaluate the whole
+    mask, as one process does."""
     logger = get_logger()
     if not torch.cuda.is_available():
         raise GrapesError("grapes_b200 has no CPU fallback: a CUDA (sm_100a) device is required")
@@ -100,6 +103,7 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
                           dropout=args.dropout)                # gcn_c only (main.py:107-112); evaluation never drops
     if world > 1:
         engine.enable_data_parallel(exchange=exchange)
+    eval_group = dist.group.WORLD if world > 1 and shard_eval else None
     train_idx = data.train_mask.nonzero().squeeze(1).to(device)
     batches = [b.to(torch.int32).contiguous() for b in torch.split(train_idx, args.batch_size)]   # DataLoader(TensorDataset(train_idx), batch_size)
     if max_batches is not None:
@@ -157,10 +161,12 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
         collect()
         engine.check_overflow()
         if (epoch + 1) % args.eval_frequency == 0:                # main.py:319
-            accuracy, f1 = evaluate(engine, data, data.val_mask, full_batch=args.eval_full_batch, args=args)
+            accuracy, f1 = evaluate(engine, data, data.val_mask, full_batch=args.eval_full_batch, args=args,
+                                    group=eval_group)
             logger.info(f'loss_gfn={state["acc_gfn"]:.6f}, loss_c={state["acc_c"]:.6f}, '
                         f'valid_accuracy={accuracy:.3f}, valid_f1={f1:.3f}')
-    test_accuracy, test_f1 = evaluate(engine, data, data.test_mask, full_batch=args.eval_full_batch, args=args)
+    test_accuracy, test_f1 = evaluate(engine, data, data.test_mask, full_batch=args.eval_full_batch, args=args,
+                                      group=eval_group)
     logger.info(f'test_accuracy={test_accuracy:.3f}, test_f1={test_f1:.3f}')
     train.last_engine = engine
     train.last_log = state["last"]

@@ -122,6 +122,26 @@ int grapes_graph_norm_add_edges(int pass, int64_t num_nodes, const int64_t* src,
 int grapes_graph_norm_offsets(int64_t num_nodes, void* workspace, int64_t* in_off, float* dinv, int64_t* nnz_dev,
                               void* stream);
 int grapes_graph_norm_finish(int64_t num_nodes, const int64_t* in_off, int* in_src, void* workspace, void* stream);
+/* ---- one destination window [lo, hi) of that structure (the row partition of the data-parallel full-batch evaluation).
+ * window_bounds: from the full in_off of `offsets`, bounds_dev[0 .. world] (int64, on the device) = the least i with
+ * (in_off[i] + i) * world >= k * (in_off[N] + N): the rows cut into `world` contiguous windows balanced by the prefix of
+ * indeg + 1, each within one row's indeg + 1 of the mean; windows are empty when N < world.  Deterministic: every rank
+ * computes the same bounds.
+ * Sequence for the window of one rank: begin -> add_*(pass 0) over the WHOLE input (dinv and the bounds need every
+ * degree) -> offsets into a full [N+1] in_off -> window_bounds -> the caller forms win_off[j] = in_off[lo + j] - in_off[lo]
+ * (j <= hi - lo) and may free the full in_off -> window_add_* over the whole input (only edges into [lo, hi) are
+ * scattered, to in_src[win_off[c - lo] + k]) -> finish(hi - lo, win_off, in_src, workspace) (the per-row sorts of the
+ * window; skip it for an empty window).  The window equals rows [lo, hi) of the whole structure bit for bit.
+ * Peak device scratch beyond the outputs (win_off, the window's in_src, dinv [N]): the workspace (~4 N bytes) plus the
+ * full in_off (8 (N + 1) bytes), which is needed only until win_off is formed.                                        */
+int grapes_graph_norm_window_bounds(int64_t num_nodes, const int64_t* in_off, int world, int64_t* bounds_dev,
+                                    void* stream);
+int grapes_graph_norm_window_add_csr(int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0, int64_t r1,
+                                     int64_t lo, int64_t hi, const int64_t* win_off, int* in_src, void* workspace,
+                                     void* stream);
+int grapes_graph_norm_window_add_edges(int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                       int64_t lo, int64_t hi, const int64_t* win_off, int* in_src, void* workspace,
+                                       void* stream);
 
 /* ---- frontier expansion / dedup / relabel  (utils.py:74-82, main.py:183-195, utils.py:98-120) */
 /* rows[P] -> row_off[P+1] = exclusive scan of CSR degrees, *m_dev = total.  Sets the bit of every
@@ -223,6 +243,16 @@ int grapes_aggregate_bf16(grapes_ctx* ctx, const void* X_bf16, int F, int ldx, c
 int grapes_aggregate_rows64(grapes_ctx* ctx, const void* X, int x_bf16, int F, int ldx, const int* slab_dev, int cap_r,
                             const int64_t* in_off, const int* in_src, const float* dinv, const float* bias, float* out,
                             int ldo, void* stream);
+/* The same slab aggregation, fp32, over an operand whose rows are partitioned between `world` <= 8 owners (layer 2 of the
+ * data-parallel full-batch evaluation): row s of Z is z_rows[o][(s - bounds[o]) * ldz ...] for the owner o with
+ * bounds[o] <= s < bounds[o + 1].  z_rows: HOST array of `world` device pointers -- peer-mapped buffers of the ranks (own
+ * at its rank's index) or any allocations this device can read; bounds: HOST array of world + 1 row bounds, bounds[0] = 0.
+ * in_off is read at r0 + j (for a window structure pass its local offsets shifted back by the window's first row).  The
+ * summation order is grapes_aggregate_rows64's, so the rows are bit-identical to it over the unpartitioned Z.
+ * Register-staged; out[j, F:ldo) = 0.                                                                                  */
+int grapes_aggregate_rows64_peer(grapes_ctx* ctx, const void* const* z_rows, const int64_t* bounds, int world, int F,
+                                 int ldz, const int* slab_dev, int cap_r, const int64_t* in_off, const int* in_src,
+                                 const float* dinv, const float* bias, float* out, int ldo, void* stream);
 /* z may be given as `nparts` partial vectors `part_stride` floats apart (summed on the fly)           */
 int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int part_stride, const int* n_dev, int cap_n, const int* in_off,
                             const int* in_src, const float* dinv, const float* bias, float* out, float* zero_out,
