@@ -141,76 +141,116 @@ __global__ void __launch_bounds__(256) k_agg(const void* __restrict__ X, int F, 
 }
 
 // ---------------------------------------------------------------------------------------
-// k_agg_peer: k_agg<VEC, false, true> over an fp32 operand whose rows are partitioned between `world` owners (the layer 2
-// of the sharded whole-graph forward, grapes_aggregate_rows64_peer): row s lives at base[o] + (s - bound[o]) * ldx for the
-// owner o with bound[o] <= s < bound[o + 1], in this rank's memory or a peer's (NVLink).  The loading lane resolves the
-// owner and broadcasts the row address instead of the row id; the fma chain (self term, then sources ascending, bias last)
-// is k_agg's, so the rows are bit-identical to grapes_aggregate_rows64 over the unpartitioned operand.  A kernel of its own
-// rather than a template parameter of k_agg, which would rename every existing k_agg instantiation.
+// k_agg_px: k_agg over a table whose rows are partitioned between `world` owners: row s lives at
+// base[o] + (s - bound[o]) * ldx for the owner o with bound[o] <= s < bound[o + 1], in this rank's memory or a peer's
+// (NVLink).  Serves the hop / classifier gather of a feature table sharded across the data-parallel ranks
+// (grapes_aggregate_peer), the same over slabs of the int64 whole-graph structure (grapes_aggregate_rows64_peer_x) and
+// the layer 2 of the sharded whole-graph forward (grapes_aggregate_rows64_peer).  The loading lane resolves the owner and
+// broadcasts the row address instead of the row id; everything else (nodes indirection, indicator columns by local id,
+// bias / relu, out or the 3xTF32 split, ones_col, zero pad, W64 slabs) and the fma chain (self term, then sources
+// ascending, bias last) are k_agg's, so the rows are bit-identical to grapes_aggregate / grapes_aggregate_bf16 /
+// grapes_aggregate_rows64 over the unpartitioned table.  Register-staged: whether cp.async.bulk reads peer-mapped memory
+// is not established.  A kernel of its own rather than a template parameter of k_agg, which would rename every existing
+// k_agg instantiation.
 // ---------------------------------------------------------------------------------------
 #define GRAPES_PEER_MAX 8
 struct PeerRows {
-    const float* base[GRAPES_PEER_MAX];
-    int bound[GRAPES_PEER_MAX + 1];
-    int world;
+    const void* base[GRAPES_PEER_MAX];
+    int bound[GRAPES_PEER_MAX];                 // first row of each owner; INT_MAX past the last owner
 };
 
-__device__ __forceinline__ const float* peer_row(const PeerRows& P, int s, int ldx) {
+template <bool XB16>
+__device__ __forceinline__ const void* peer_row(const PeerRows& P, int s, int ldx) {
     // selects with constant indices (bounds do not decrease: the last window starting at or before s owns it); an index
     // computed at run time would copy the parameter struct to the stack
-    const float* b = P.base[0];
+    const void* b = P.base[0];
     int lo = 0;
 #pragma unroll
     for (int k = 1; k < GRAPES_PEER_MAX; ++k)
-        if (k < P.world && s >= P.bound[k]) { b = P.base[k]; lo = P.bound[k]; }
-    return b + (size_t)(s - lo) * ldx;
+        if (s >= P.bound[k]) { b = P.base[k]; lo = P.bound[k]; }
+    return reinterpret_cast<const char*>(b) + (size_t)(s - lo) * ldx * (XB16 ? 2 : 4);
 }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) k_agg_peer(const PeerRows P, int F, int ldx, const int* __restrict__ n_dev, int cap_n,
-                                                  const long long* __restrict__ in_off, const int* __restrict__ in_src,
-                                                  const float* __restrict__ dinv, const float* __restrict__ bias,
-                                                  float* __restrict__ out, int ldo) {
+// __maxnreg__ instead of __launch_bounds__(256): with the launch bound alone ptxas settles on 32-40 registers and spills
+// the owner select's live values (24-28 bytes); 48 registers hold them (k_agg: 40-48)
+template <int VEC, bool XB16, bool W64>
+__global__ void __maxnreg__(48) k_agg_px(const PeerRows P, int F, int ldx,
+                                                const int* __restrict__ nodes, const int* __restrict__ n_dev, int cap_n,
+                                                const typename GrapesOff<W64>::T* __restrict__ in_off,
+                                                const int* __restrict__ in_src,
+                                                const float* __restrict__ dinv, const uint32_t* __restrict__ ind_bits,
+                                                int num_ind, const float* __restrict__ bias, int relu,
+                                                float* __restrict__ out, int ldo, float* __restrict__ out_hi,
+                                                float* __restrict__ out_lo, int ones_col) {
+    typedef typename GrapesOff<W64>::T OffT;
     pdl_begin();
     const int n = min(*n_dev, cap_n);
-    const int r0 = n_dev[1];
+    const int r0 = W64 ? n_dev[1] : 0;
     const int lane = lane_id();
     const int warps = (gridDim.x * blockDim.x) >> 5;
     for (int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += warps) {
-        const int jr = r0 + j;
+        const int jr = r0 + j;                               // row of in_off / dinv
         const float dj = dinv[jr];
-        const long long beg = in_off[jr], end = in_off[jr + 1];
-        const float* xj = peer_row(P, jr, ldx);
-        float* oj = out + (size_t)j * ldo;
-        for (int cb = 0; cb < F; cb += 32 * VEC) {
+        const OffT beg = in_off[jr], end = in_off[jr + 1];
+        const void* xj = peer_row<XB16>(P, nodes ? nodes[j] : jr, ldx);
+        float* oj = out ? out + (size_t)j * ldo : nullptr;
+        float* ohj = out_hi ? out_hi + (size_t)j * ldo : nullptr;
+        float* olj = out_hi ? out_lo + (size_t)j * ldo : nullptr;
+        for (int cb = 0; cb < F; cb += 32 * VEC) {           // warp-uniform trip count
             const int c0 = cb + lane * VEC;
             const bool act = c0 < F;
             float acc[VEC];
 #pragma unroll
             for (int i = 0; i < VEC; ++i) acc[i] = 0.f;
-            if (act) vec_fma<VEC>(acc, dj * dj, xj + c0);
-            for (long long pb = beg; pb < end; pb += 32) {
-                const long long p = pb + lane;
+            if (act) vec_fma_x<VEC, XB16>(acc, dj * dj, xj, c0);
+            for (OffT pb = beg; pb < end; pb += 32) {
+                const OffT p = pb + lane;
                 float w = 0.f; unsigned long long sa = 0ull;
                 if (p < end) {
                     const int sl = in_src[p];
                     w = dinv[sl] * dj;
-                    sa = (unsigned long long)peer_row(P, sl, ldx);
+                    sa = (unsigned long long)peer_row<XB16>(P, nodes ? nodes[sl] : sl, ldx);
                 }
-                const int cnt = (int)min(32ll, end - pb);
+                const int cnt = (int)min((OffT)32, end - pb);
                 for (int t = 0; t < cnt; ++t) {
                     const float wt = __shfl_sync(GRAPES_FULL_MASK, w, t);
                     const unsigned long long st = __shfl_sync(GRAPES_FULL_MASK, sa, t);
-                    if (act) vec_fma<VEC>(acc, wt, reinterpret_cast<const float*>(st) + c0);
+                    if (act) vec_fma_x<VEC, XB16>(acc, wt, reinterpret_cast<const void*>(st), c0);
                 }
             }
             if (act) {
 #pragma unroll
-                for (int i = 0; i < VEC; ++i) if (bias) acc[i] += bias[c0 + i];
-                *reinterpret_cast<typename VecT<VEC>::T*>(oj + c0) = *reinterpret_cast<typename VecT<VEC>::T*>(acc);
+                for (int i = 0; i < VEC; ++i) {
+                    float v = acc[i];
+                    if (bias) v += bias[c0 + i];
+                    if (relu) v = fmaxf(v, 0.f);
+                    acc[i] = v;
+                }
+                if (oj) *reinterpret_cast<typename VecT<VEC>::T*>(oj + c0) = *reinterpret_cast<typename VecT<VEC>::T*>(acc);
+                if (ohj) {                                   // 3xTF32 operand split for the tcgen05 GEMM
+                    float h[VEC], l[VEC];
+#pragma unroll
+                    for (int i = 0; i < VEC; ++i) { h[i] = f32_to_tf32(acc[i]); l[i] = f32_to_tf32(acc[i] - h[i]); }
+                    *reinterpret_cast<typename VecT<VEC>::T*>(ohj + c0) = *reinterpret_cast<typename VecT<VEC>::T*>(h);
+                    *reinterpret_cast<typename VecT<VEC>::T*>(olj + c0) = *reinterpret_cast<typename VecT<VEC>::T*>(l);
+                }
             }
         }
-        for (int c = F + lane; c < ldo; c += 32) oj[c] = 0.f;
+        if (ldo > F) {
+            float a = 0.f;
+            if (lane < num_ind) {
+                a = dj * dj * (float)((ind_bits[j] >> lane) & 1u);
+                for (OffT p = beg; p < end; ++p) {
+                    const int sl = in_src[p];
+                    a = fmaf(dinv[sl] * dj, (float)((ind_bits[sl] >> lane) & 1u), a);
+                }
+            }
+            for (int c = F + lane; c < ldo; c += 32) {
+                const float v = (c < F + num_ind) ? a : (c == ones_col ? 1.f : 0.f);
+                if (oj) oj[c] = v;
+                if (ohj) { const float h = f32_to_tf32(v); ohj[c] = h; olj[c] = f32_to_tf32(v - h); }
+            }
+        }
     }
 }
 
@@ -1117,6 +1157,44 @@ static int launch_gemm_dropout(grapes_ctx* ctx, const float* A, int lda, const f
     return GRAPES_OK;
 }
 
+// the owner table of the peer aggregations: HOST arrays of `world` row bases and world + 1 bounds into the parameter struct
+static int peer_rows(const void* const* x_rows, const int64_t* bounds, int world, PeerRows& P, size_t& al) {
+    GRAPES_REQUIRE(x_rows && bounds, "null argument");
+    GRAPES_REQUIRE(world >= 1 && world <= GRAPES_PEER_MAX, "1 to 8 row owners");
+    GRAPES_REQUIRE(bounds[0] == 0 && bounds[world] < (1ll << 31), "bounds[0] must be 0 and bounds[world] fit int32");
+    P = PeerRows{};
+    for (int o = 0; o < GRAPES_PEER_MAX; ++o) P.bound[o] = INT_MAX;
+    for (int o = 0; o < world; ++o) {
+        GRAPES_REQUIRE(bounds[o] <= bounds[o + 1], "bounds must not decrease");
+        GRAPES_REQUIRE(x_rows[o] || bounds[o] == bounds[o + 1], "null row base of a non-empty window");
+        P.base[o] = x_rows[o];
+        P.bound[o] = (int)bounds[o];
+        al |= (size_t)x_rows[o];
+    }
+    return GRAPES_OK;
+}
+
+// one k_agg_px launch in the widest vector form the layout allows (the form k_agg would take)
+template <bool W64>
+static void launch_agg_px(grapes_ctx* ctx, const PeerRows& P, int x_bf16, int F, int ldx, const int* nodes,
+                          const int* n_dev, int cap_n, const typename GrapesOff<W64>::T* in_off, const int* in_src,
+                          const float* dinv, const uint32_t* ind_bits, int num_ind, const float* bias, int relu,
+                          float* out, int ldo, float* out_hi, float* out_lo, int ones_col, size_t al, cudaStream_t s) {
+    const int blocks = grid_for(ctx, (long long)cap_n * 32, 256, 8);
+    al |= ((size_t)out) | ((size_t)out_hi) | ((size_t)out_lo);
+    const bool v4 = (al & 15) == 0 && (F % 4 == 0) && (ldx % 4 == 0) && (ldo % 4 == 0);
+    const bool v2 = (al & 7) == 0 && (F % 2 == 0) && (ldx % 2 == 0) && (ldo % 2 == 0);
+#define AGGPX(VEC, XB) pdl((k_agg_px<VEC, XB, W64>), blocks, 256, 0, s)(P, F, ldx, nodes, n_dev, cap_n, in_off, in_src, \
+                                                                         dinv, ind_bits, num_ind, bias, relu, out, ldo, \
+                                                                         out_hi, out_lo, ones_col)
+    if (x_bf16) {
+        if (v4) AGGPX(4, true); else if (v2) AGGPX(2, true); else AGGPX(1, true);
+    } else {
+        if (v4) AGGPX(4, false); else if (v2) AGGPX(2, false); else AGGPX(1, false);
+    }
+#undef AGGPX
+}
+
 static int g_agg_variant = 0;
 #define AGG_MIN_ROWS 4096               // smallest row capacity that takes the multi-row / TMA-staged forms (aligned widths)
 
@@ -1276,37 +1354,52 @@ int grapes_aggregate_rows64(grapes_ctx* ctx, const void* X, int x_bf16, int F, i
     return GRAPES_OK;
 }
 
-int grapes_aggregate_rows64_peer(grapes_ctx* ctx, const void* const* z_rows, const int64_t* bounds, int world, int F,
-                                 int ldz, const int* slab_dev, int cap_r, const int64_t* in_off, const int* in_src,
-                                 const float* dinv, const float* bias, float* out, int ldo, void* stream) {
-    if (cap_r <= 0) return GRAPES_OK;                    // an empty window: nothing to read or write
-    GRAPES_REQUIRE(ctx && z_rows && bounds && slab_dev && in_off && in_src && dinv && out, "null argument");
-    GRAPES_REQUIRE(world >= 1 && world <= GRAPES_PEER_MAX, "1 to 8 row owners");
-    GRAPES_REQUIRE(F > 0 && ldz >= F && ldo >= F, "bad shape");
-    PeerRows P = {};
-    size_t al = (size_t)out;
-    GRAPES_REQUIRE(bounds[0] == 0 && bounds[world] < (1ll << 31), "bounds[0] must be 0 and bounds[world] fit int32");
-    for (int o = 0; o < world; ++o) {
-        GRAPES_REQUIRE(bounds[o] <= bounds[o + 1], "bounds must not decrease");
-        GRAPES_REQUIRE(z_rows[o] || bounds[o] == bounds[o + 1], "null row base of a non-empty window");
-        P.base[o] = reinterpret_cast<const float*>(z_rows[o]);
-        P.bound[o] = (int)bounds[o];
-        al |= (size_t)z_rows[o];
-    }
-    P.bound[world] = (int)bounds[world];
-    P.world = world;
-    cudaStream_t s = (cudaStream_t)stream;
-    const long long* off = reinterpret_cast<const long long*>(in_off);
-    const int blocks = grid_for(ctx, (long long)cap_r * 32, 256, 8);
-    if ((al & 15) == 0 && F % 4 == 0 && ldz % 4 == 0 && ldo % 4 == 0)
-        pdl((k_agg_peer<4>), blocks, 256, 0, s)(P, F, ldz, slab_dev, cap_r, off, in_src, dinv, bias, out, ldo);
-    else if ((al & 7) == 0 && F % 2 == 0 && ldz % 2 == 0 && ldo % 2 == 0)
-        pdl((k_agg_peer<2>), blocks, 256, 0, s)(P, F, ldz, slab_dev, cap_r, off, in_src, dinv, bias, out, ldo);
-    else
-        pdl((k_agg_peer<1>), blocks, 256, 0, s)(P, F, ldz, slab_dev, cap_r, off, in_src, dinv, bias, out, ldo);
+int grapes_aggregate_peer(grapes_ctx* ctx, const void* const* x_rows, const int64_t* bounds, int world, int x_bf16, int F,
+                          int ldx, const int* nodes, const int* n_dev, int cap_n, const int* in_off, const int* in_src,
+                          const float* dinv, const uint32_t* ind_bits, int num_ind, const float* bias, int relu,
+                          float* out, int ldo, float* out_hi, float* out_lo, int ones_col, void* stream) {
+    GRAPES_REQUIRE(ctx && n_dev && in_off && in_src && dinv && (out || out_hi), "null argument");
+    GRAPES_REQUIRE((out_hi == nullptr) == (out_lo == nullptr), "out_hi and out_lo go together");
+    GRAPES_REQUIRE(F > 0 && ldx >= F, "bad shape");
+    GRAPES_REQUIRE(ones_col < 0 || (ones_col >= F + num_ind && ones_col < ldo), "ones_col must lie in the pad columns");
+    GRAPES_REQUIRE(ldo >= F + num_ind, "ldo too small");
+    GRAPES_REQUIRE(num_ind == 0 || ind_bits, "indicator columns need ind_bits");
+    GRAPES_REQUIRE(num_ind <= 8, "at most 8 indicator columns");
+    PeerRows P;
+    size_t al = 0;
+    const int rc = peer_rows(x_rows, bounds, world, P, al);
+    if (rc != GRAPES_OK) return rc;
+    if (cap_n > 0)
+        launch_agg_px<false>(ctx, P, x_bf16, F, ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, bias,
+                             relu, out, ldo, out_hi, out_lo, ones_col, al, (cudaStream_t)stream);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
+}
+
+int grapes_aggregate_rows64_peer_x(grapes_ctx* ctx, const void* const* x_rows, const int64_t* bounds, int world,
+                                   int x_bf16, int F, int ldx, const int* slab_dev, int cap_r, const int64_t* in_off,
+                                   const int* in_src, const float* dinv, const float* bias, float* out, int ldo,
+                                   void* stream) {
+    if (cap_r <= 0) return GRAPES_OK;                    // an empty window: nothing to read or write
+    GRAPES_REQUIRE(ctx && slab_dev && in_off && in_src && dinv && out, "null argument");
+    GRAPES_REQUIRE(F > 0 && ldx >= F && ldo >= F, "bad shape");
+    PeerRows P;
+    size_t al = 0;
+    const int rc = peer_rows(x_rows, bounds, world, P, al);
+    if (rc != GRAPES_OK) return rc;
+    launch_agg_px<true>(ctx, P, x_bf16, F, ldx, nullptr, slab_dev, cap_r, reinterpret_cast<const long long*>(in_off),
+                        in_src, dinv, nullptr, 0, bias, 0, out, ldo, nullptr, nullptr, -1, al, (cudaStream_t)stream);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_aggregate_rows64_peer(grapes_ctx* ctx, const void* const* z_rows, const int64_t* bounds, int world, int F,
+                                 int ldz, const int* slab_dev, int cap_r, const int64_t* in_off, const int* in_src,
+                                 const float* dinv, const float* bias, float* out, int ldo, void* stream) {
+    return grapes_aggregate_rows64_peer_x(ctx, z_rows, bounds, world, 0, F, ldz, slab_dev, cap_r, in_off, in_src, dinv,
+                                          bias, out, ldo, stream);
 }
 
 int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int part_stride, const int* n_dev, int cap_n, const int* in_off,

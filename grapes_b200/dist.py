@@ -7,7 +7,7 @@ The trajectory-balance loss is the square of a per-batch scalar, so W-rank data 
 W per-batch gradients -- not one W x B batch (SURVEY.md section 7.2)."""
 from __future__ import annotations
 
-from typing import List
+from typing import List, Tuple
 
 import torch
 import torch.distributed as dist
@@ -116,21 +116,22 @@ def gather_batch_predictions(local: torch.Tensor, batch_sizes: List[int], group=
 
 
 class PeerRowTable:
-    """The layer-2 operand table of :func:`grapes_b200.gcn.full_graph_forward_sharded` across the ranks of ``group``: one
-    ``torch.distributed._symmetric_memory`` buffer of ``rows`` x ``ld`` floats per rank (this rank's window of Z, zero pad
-    columns), ``ptrs`` = the HOST array of every rank's buffer address (own at ``rank``), and ``barrier()`` = the
+    """A row table partitioned across the ranks of ``group`` -- the layer-2 operand of
+    :func:`grapes_b200.gcn.full_graph_forward_sharded`, or a shard of the feature table (:class:`ShardedFeatures`): one
+    ``torch.distributed._symmetric_memory`` buffer of ``rows`` x ``ld`` elements of ``dtype`` (fp32 or bf16) per rank (this
+    rank's rows, zero pad columns), ``ptrs`` = the HOST array of every rank's buffer address (own at ``rank``), and ``barrier()`` = the
     stream-ordered barrier of the symmetric-memory handle (no host synchronisation).  Construction only allocates (rank
     local); :meth:`rendezvous` maps the peers and is collective.  Built once per graph and classifier width and cached
     with the window structure (``eval._sharded_eval``)."""
 
-    def __init__(self, rows: int, ld: int, device: torch.device, group=None):
+    def __init__(self, rows: int, ld: int, device: torch.device, group=None, dtype: torch.dtype = torch.float32):
         import torch.distributed._symmetric_memory as symm_mem
         self.group = group or dist.group.WORLD
         self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
         if self.world > 8:
             raise RuntimeError("the peer row table is built for one NVSwitch box (<= 8 ranks)")
         self.ld = int(ld)
-        self.buf = symm_mem.empty(max(int(rows), 1) * self.ld, dtype=torch.float32, device=device)
+        self.buf = symm_mem.empty(max(int(rows), 1) * self.ld, dtype=dtype, device=device)
         self.buf.zero_()
         self.rows = self.buf.view(max(int(rows), 1), self.ld)
         self.hdl, self.ptrs = None, None
@@ -148,3 +149,123 @@ class PeerRowTable:
 
     def barrier(self):
         self.hdl.barrier(channel=0)
+
+
+def feature_bounds(num_nodes: int, world: int) -> List[int]:
+    """Row bounds of a feature table sharded between ``world`` ranks: equal contiguous ranges, bounds[r] = min(N, r *
+    ceil(N / W)).  The table is sharded because it does not fit one device, so memory balance is the goal; the last
+    ranges are short or empty when W does not divide N (N < W included)."""
+    per = -(-int(num_nodes) // int(world))
+    return [min(int(num_nodes), r * per) for r in range(int(world) + 1)]
+
+
+def feature_pitch(num_features: int) -> int:
+    """Row pitch (elements) of a feature shard: F rounded up to 4, the pitch the engine gives a replicated fp32 table;
+    for bf16 it keeps every row 8-byte aligned.  The pad columns are zero."""
+    return (int(num_features) + 3) // 4 * 4
+
+
+def fill_plan(lo: int, hi: int, row_bytes: int, chunk_bytes: int = 1 << 30) -> List[Tuple[int, int]]:
+    """Row ranges [a, b) covering [lo, hi) with at most ``chunk_bytes`` of source rows each (at least one row): the copies
+    that fill one shard, so a host table is staged through at most that much device memory at a time."""
+    step = max(1, int(chunk_bytes) // max(int(row_bytes), 1))
+    return [(a, min(a + step, hi)) for a in range(int(lo), int(hi), step)]
+
+
+class ShardedFeatures:
+    """A feature table [N, F] sharded by rows across the data-parallel ranks (``train(..., shard_features=True)``): rank r
+    holds rows ``bounds[r] .. bounds[r + 1]`` (:func:`feature_bounds`) in a :class:`PeerRowTable` of pitch ``ldx``
+    (:func:`feature_pitch`, zero pad columns) and reads the other rows from their owners over NVLink peer memory.  Pass it
+    as ``x`` to :class:`grapes_b200.engine.GrapesEngine` and as ``features`` to :func:`grapes_b200.eval.evaluate`; the
+    results are bit-identical to those over the replicated table.
+
+    Attributes: ``N``, ``F``, ``ldx``, ``dtype`` (fp32 or bf16, as ``x``), ``world``, ``rank``, ``bounds`` (W + 1 ints),
+    ``table`` (``rows`` [max rows, ldx], ``ptrs`` = HOST array of every rank's shard), ``local`` = this rank's [rows, F]
+    view, ``bounds_c`` = the bounds as a HOST int64 array for the C ABI.
+
+    The constructor is collective over ``group`` (default: the world).  It fills this rank's rows from ``x[lo:hi]`` in
+    chunks of at most ``chunk_bytes``; ``x`` may be a host tensor (memory-mapped or not) or a device tensor, and the whole
+    table never goes to one device.  When the symmetric allocation or mapping fails on any rank, every rank raises
+    ``GrapesError`` (agreed through :func:`ranks_agree`): there is no replicated fall-back, since the table may not fit.
+    The shards are read-only once built; construction ends with a collective, so every shard is filled before any rank
+    reads a peer's."""
+
+    def __init__(self, x: torch.Tensor, device, group=None, chunk_bytes: int = 1 << 30):
+        from ._lib import GrapesError
+        device = torch.device(device)
+        self.group = group or dist.group.WORLD
+        world, rank = dist.get_world_size(self.group), dist.get_rank(self.group)
+        self._shape(x, world, rank)
+        rows = max(self.bounds[r + 1] - self.bounds[r] for r in range(world))
+        table, why = None, ""
+        try:
+            table = PeerRowTable(rows, self.ldx, device, self.group, dtype=self.dtype)
+        except Exception as exc:                        # noqa: BLE001 -- agreed below and raised on every rank
+            why = f"{type(exc).__name__}: {exc}"
+        if ranks_agree(table is not None, device, self.group):
+            try:
+                table.rendezvous()
+            except Exception as exc:                    # noqa: BLE001
+                why, table = f"{type(exc).__name__}: {exc}", None
+            if not ranks_agree(table is not None, device, self.group):
+                table = None
+        else:
+            table = None
+        if table is None:
+            raise GrapesError("sharded feature table: symmetric allocation or peer mapping failed " +
+                              (f"on this rank ({why})" if why else "on another rank"))
+        self.table = table
+        self._fill(x, chunk_bytes)
+        torch.cuda.synchronize(device)
+        ranks_agree(True, device, self.group)           # every shard is filled before any rank reads a peer's
+
+    def _shape(self, x, world: int, rank: int):
+        from ._lib import GrapesError
+        if x.dim() != 2 or x.dtype not in (torch.float32, torch.bfloat16):
+            raise GrapesError("a sharded feature table is a 2-D fp32 or bf16 tensor")
+        if not 1 <= world <= 8:
+            raise GrapesError(f"a sharded feature table spans 1 to 8 ranks (one NVSwitch box), not {world}")
+        self.N, self.F = int(x.shape[0]), int(x.shape[1])
+        self.dtype, self.world, self.rank = x.dtype, int(world), int(rank)
+        self.ldx = feature_pitch(self.F)
+        self.bounds = feature_bounds(self.N, world)
+        self.lo, self.hi = self.bounds[rank], self.bounds[rank + 1]
+
+    def _fill(self, x: torch.Tensor, chunk_bytes: int):
+        import ctypes
+        self.local = self.table.rows[:self.hi - self.lo, :self.F]
+        for a, b in fill_plan(self.lo, self.hi, self.F * x.element_size(), chunk_bytes):
+            self.local[a - self.lo:b - self.lo].copy_(x[a:b])
+        self.bounds_c = (ctypes.c_int64 * (self.world + 1))(*self.bounds)
+
+    @property
+    def ptrs(self):
+        return self.table.ptrs
+
+    @property
+    def x_bf16(self) -> bool:
+        return self.dtype == torch.bfloat16
+
+    @property
+    def table_bytes(self) -> int:
+        """Device bytes of this rank's shard (pad columns included)."""
+        return self.table.rows.numel() * self.table.rows.element_size()
+
+    @classmethod
+    def emulate(cls, x: torch.Tensor, world: int, device=None, chunk_bytes: int = 1 << 30) -> List["ShardedFeatures"]:
+        """One-process stand-in: the W shards in W allocations of one device (:class:`grapes_b200.gcn.LocalRowTable`), one
+        holder per emulated rank, all sharing them; any one of them serves an engine, which then reads all W."""
+        from .gcn import LocalRowTable
+        device = torch.device(device) if device is not None else x.device
+        out = []
+        for r in range(int(world)):
+            s = cls.__new__(cls)
+            s.group = None
+            s._shape(x, int(world), r)
+            out.append(s)
+        rows = max(out[0].bounds[r + 1] - out[0].bounds[r] for r in range(int(world)))
+        tables = LocalRowTable.make(int(world), rows, out[0].ldx, device, dtype=x.dtype)
+        for s, t in zip(out, tables):
+            s.table = t
+            s._fill(x, chunk_bytes)
+        return out

@@ -94,15 +94,26 @@ class GrapesEngine:
         dropout = float(dropout)
         if not 0. <= dropout <= 1.:
             raise ValueError(f"dropout probability has to be between 0 and 1, but got {dropout}")
+        from .dist import ShardedFeatures
+        # a feature table sharded across the data-parallel ranks: both feature gathers read each row from its owner
+        # (grapes_aggregate_peer); nothing else of the step changes
+        self.features = x if isinstance(x, ShardedFeatures) else None
+        if self.features is not None:
+            if embed_nodes:
+                raise GrapesError("learned node features (embed_nodes) with a sharded feature table: the table optimiser "
+                                  "is not sharded; replicate the table")
+            if x.N != graph.num_nodes:
+                raise GrapesError(f"sharded feature table of {x.N} rows for a graph of {graph.num_nodes} nodes")
         self.g = graph
         self.L = lib()
         dev = graph.device
         self.device = dev
-        assert x.is_cuda and x.dtype in (torch.float32, torch.bfloat16) and x.is_contiguous()
+        if self.features is None:
+            assert x.is_cuda and x.dtype in (torch.float32, torch.bfloat16) and x.is_contiguous()
         # bf16 feature table (papers100M-shaped config): rows are gathered as stored and widened to fp32 in the aggregation
         self.x_bf16 = x.dtype == torch.bfloat16
         assert sampling_hops <= 7, "indicator bits are packed in 8 columns"
-        self.x, self.y = x, y.contiguous()
+        self.x, self.y = (None if self.features is not None else x), y.contiguous()
         # main.py:89-100,116: `x` is a learned table (nn.Parameter inside optimizer_c); it is updated IN PLACE by every
         # optimiser step (dense Adam from the sparse classifier gradient, grapes_adam_embed)
         self.embed_nodes = bool(embed_nodes)
@@ -113,11 +124,11 @@ class GrapesEngine:
             self.y = self.y.to(torch.float32)
         else:
             self.y = self.y.to(torch.int64)
-        N, F = graph.num_nodes, x.shape[1]
+        N, F = graph.num_nodes, int(x.shape[1]) if self.features is None else x.F
         # TMA row copies need 16-byte rows: a table whose width is not a multiple of 4 floats (Reddit 602, Cora 1433) is
         # re-pitched once to ldx = round_up(F, 4); self.x stays the [N, F] view, the kernels get (F, ldx)
-        self.ldx = F
-        if x.dtype == torch.float32 and F % 4 != 0 and not embed_nodes:
+        self.ldx = F if self.features is None else x.ldx
+        if self.features is None and x.dtype == torch.float32 and F % 4 != 0 and not embed_nodes:
             self.ldx = _round_up(F, 4)
             xp = torch.zeros((N, self.ldx), dtype=torch.float32, device=x.device)
             xp[:, :F].copy_(x)
@@ -577,7 +588,6 @@ class GrapesEngine:
         L = self.L
         H, F, D, C, B = self.H, self.F, self.D, self.C, self.bsz
         ovf = ptr(self.overflow)
-        X = ptr(self.x)
         # ---- classifier on the sampled subgraph (main.py:252-269) ----
         L.tag = "[cls]"
         L.grapes_rank_nodes(ctx, ptr(self.bm_all), None, ptr(self.pref_all), None, ptr(self.all_nodes), None, None,
@@ -617,9 +627,8 @@ class GrapesEngine:
             L.grapes_build_csr(ctx, ptr(self.cl_src[0]), ptr(self.cl_dst[0]), self._hc(H - 1, "blk"), self.cap_blk,
                                A_dev, cap_A, ptr(self.cnt_scratch), 0, ptr(self.cl_out_off0), ptr(self.cl_out_dst0),
                                ptr(self.cl_tmp), None, self._cnt("cl_nnz", 3), ovf, st)
-        (L.grapes_aggregate_bf16 if self.x_bf16 else L.grapes_aggregate)(
-                           ctx, X, F, self.ldx, ptr(self.all_nodes), A_dev, cap_A, ptr(self.cl_in_off[0]),
-                           ptr(self.cl_in_src[0]), ptr(self.cl_dinv[0]), None, 0, None, 0, ptr(self.Yc), ldYc, None, None, -1, st)
+        self._aggregate_x(ctx, ptr(self.all_nodes), A_dev, cap_A, ptr(self.cl_in_off[0]), ptr(self.cl_in_src[0]),
+                          ptr(self.cl_dinv[0]), None, 0, ptr(self.Yc), ldYc, None, None, -1, st)
         if training and self.dropout > 0:
             L.grapes_gemm_bias_relu_dropout(ctx, ptr(self.Yc), ldYc, self._par(nc.W1), F, ptr(self.out1), D, A_dev, cap_A,
                                             D, F, self._par(nc.b1), ptr(self.drop_state), self._drop_tag(0),
@@ -746,12 +755,25 @@ class GrapesEngine:
                            self._hc(h, "nnz"), ovf, st)
         if not self.random_sampling:
             tc = self.use_tc
-            agg_x = L.grapes_aggregate_bf16 if self.x_bf16 else L.grapes_aggregate
-            agg_x(ctx, ptr(self.x), self.F, self.ldx, ptr(hw.batch_nodes), n_dev, cap_n, ptr(hw.in_off),
-                               ptr(hw.in_src), ptr(hw.dinv), ptr(hw.ind_bits) if self.use_ind else None, self.num_ind,
-                               None, 0, None if (tc and not self.y_single) else ptr(hw.Y), self.ldY,
-                               ptr(hw.Y) if (tc and not self.y_single) else None, ptr(hw.Y_lo),
-                               self.Fp if self.use_tc_bwd else -1, st)
+            self._aggregate_x(ctx, ptr(hw.batch_nodes), n_dev, cap_n, ptr(hw.in_off), ptr(hw.in_src), ptr(hw.dinv),
+                              ptr(hw.ind_bits) if self.use_ind else None, self.num_ind,
+                              None if (tc and not self.y_single) else ptr(hw.Y), self.ldY,
+                              ptr(hw.Y) if (tc and not self.y_single) else None, ptr(hw.Y_lo),
+                              self.Fp if self.use_tc_bwd else -1, st)
+
+    def _aggregate_x(self, ctx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, out, ldo, out_hi, out_lo,
+                     ones_col, st):
+        """The two reads of the feature table (hop aggregation, classifier layer 1): Y = A_hat x[nodes] (| indicators),
+        one launch over the replicated table, or over the shards of a sharded one (bit-identical)."""
+        L, fs = self.L, self.features
+        if fs is not None:
+            L.grapes_aggregate_peer(ctx, fs.ptrs, fs.bounds_c, fs.world, int(self.x_bf16), self.F, self.ldx, nodes, n_dev,
+                                    cap_n, in_off, in_src, dinv, ind_bits, num_ind, None, 0, out, ldo, out_hi, out_lo,
+                                    ones_col, st)
+        else:
+            (L.grapes_aggregate_bf16 if self.x_bf16 else L.grapes_aggregate)(
+                ctx, ptr(self.x), self.F, self.ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, None, 0,
+                out, ldo, out_hi, out_lo, ones_col, st)
 
     def _enqueue_front0(self, ctx, st):
         """Per-batch reset (main.py:161-176: one memset + one kernel) and the whole hop-0 front end of the ACTIVE step

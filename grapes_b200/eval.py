@@ -31,7 +31,7 @@ import torch.distributed as dist
 
 from ._lib import GrapesError
 from .gcn import (GCN, GraphNorm, ShardedGraphNorm, WideGraphNorm, _scores_from_counts, full_graph_forward,
-                  full_graph_forward_sharded, full_graph_forward_streamed, row_slab_refusal)
+                  full_graph_forward_sharded, full_graph_forward_streamed, needs_p_table, row_slab_refusal)
 from .graph import DeviceGraph
 from .utils import TensorMap, get_logger
 
@@ -83,18 +83,30 @@ def evaluate(gcn_c: GCN,
              return_predictions: bool = False,
              engine=None,
              group=None,
+             *,
+             features=None,
              ):
     """``group``: a ``torch.distributed`` process group of more than one rank makes the evaluation data parallel, with
-    the scores of one process (see :func:`_evaluate_sharded`); None or a one-rank group runs the single-process code."""
+    the scores of one process (see :func:`_evaluate_sharded`); None or a one-rank group runs the single-process code.
+
+    ``features``: the feature table sharded across the ranks of ``group`` (:class:`grapes_b200.dist.ShardedFeatures`),
+    read instead of ``data.x``, which is then never moved to the device.  Mini batch runs on the engine (built over the
+    sharded table when ``engine`` is None).  Full batch needs ``group`` and runs the sharded forward only: a classifier the
+    row-slab forward does not cover, or a Z / P table that could not be mapped, raises ``GrapesError`` on every rank,
+    since there is no replicated table to fall back to."""
     get_logger().info('Evaluating')
     device = torch.device(device)
+    sharded_group = group is not None and dist.is_initialized() and dist.get_world_size(group) > 1
+    if features is not None and full_batch and not sharded_group:
+        raise GrapesError("full-batch evaluation of a sharded feature table runs over the process group that holds the "
+                          "shards (pass group=); evaluate mini-batch (full_batch=False) otherwise")
     if device.type != "cuda":
         raise GrapesError("grapes_b200 has no CPU fallback: evaluation runs on the CUDA device (eval_on_cpu is ignored)")
-    x = data.x.to(device)
+    x = features if features is not None else data.x.to(device)
     y = data.y.to(device)
     gcn_c = gcn_c.to(device).eval()
     mask_d = mask.to(device) if mask is not None else torch.ones(data.num_nodes, dtype=torch.bool, device=device)
-    if group is not None and dist.is_initialized() and dist.get_world_size(group) > 1:
+    if sharded_group:
         res = _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, device, x, y, mask_d, loader,
                                 full_batch, return_predictions, engine, group)
         if res is not None:
@@ -120,7 +132,7 @@ def evaluate(gcn_c: GCN,
     assert loader is not None, 'loader must be provided if full_batch is False'
     batches = [b[0] if isinstance(b, (tuple, list)) else b for b in loader]
     eng = engine if engine is not None else _eval_engine(adjacency, data, args, gcn_c, gcn_gf, num_indicators, device,
-                                                         max([int(b.numel()) for b in batches] + [1]))
+                                                         max([int(b.numel()) for b in batches] + [1]), x)
     total = sum(int(b.numel()) for b in batches)
     preds = torch.zeros(max(total, 1), dtype=torch.int32, device=device)
     off = 0
@@ -144,26 +156,32 @@ def _mean_of_hits(hits: int, rows: int) -> float:
         return float(np.float32(hits) * (np.float32(1) / np.float32(rows)))
 
 
-def _sharded_eval(adjacency: DeviceGraph, data, group, C4: int, device):
-    """(window structure, peer row table or None) of this rank, cached on the graph object like ``_graph_norm``.  The
-    table is None when the symmetric mapping failed on any rank (every rank agrees, so none of them waits on a peer)."""
+def _sharded_eval(adjacency: DeviceGraph, data, group, C4: int, device, p_shape=None, fallback: bool = True):
+    """(window structure, peer row table or None, P table or None) of this rank, cached on the graph object like
+    ``_graph_norm``.  The tables are None when the symmetric mapping failed on any rank (every rank agrees, so none of
+    them waits on a peer).  ``p_shape`` = (rows, D): also the P table of a sharded feature table with F > D.
+    ``fallback``: the caller runs the replicated evaluation when they are None (warned here)."""
     from .dist import PeerRowTable, ranks_agree
     ei = getattr(data, "edge_index", None)
     world, rank = dist.get_world_size(group), dist.get_rank(group)
-    key = (None if ei is None else (ei.data_ptr(), tuple(ei.shape)), world, rank, C4)
+    key = (None if ei is None else (ei.data_ptr(), tuple(ei.shape)), world, rank, C4, p_shape)
     cached = getattr(adjacency, "_sharded_eval", None)
     if cached is None or cached[0] != key:
-        adjacency._sharded_eval = None
-        sgn, table, why = None, None, ""
+        adjacency._sharded_eval, adjacency._sharded_eval_p = None, None
+        sgn, table, ptab, why = None, None, None, ""
         try:                                           # rank-local failures (memory, ids, mapping) become the fall-back
             sgn = ShardedGraphNorm(adjacency, world, rank, edge_index=ei)
             rows = max(sgn.bounds[r + 1] - sgn.bounds[r] for r in range(world))
             table = PeerRowTable(rows, C4, device, group)
+            if p_shape is not None:
+                ptab = PeerRowTable(p_shape[0], p_shape[1], device, group)
         except Exception as exc:                       # noqa: BLE001 -- reported below, never silent
-            why = f"{type(exc).__name__}: {exc}"
+            why, table = f"{type(exc).__name__}: {exc}", None
         if ranks_agree(table is not None, device, group):
             try:
                 table.rendezvous()
+                if ptab is not None:
+                    ptab.rendezvous()
             except Exception as exc:                   # noqa: BLE001
                 why, table = f"{type(exc).__name__}: {exc}", None
             if not ranks_agree(table is not None, device, group):
@@ -171,13 +189,15 @@ def _sharded_eval(adjacency: DeviceGraph, data, group, C4: int, device):
         else:
             table = None
         if table is None:
-            sgn = None                                 # the replicated evaluation builds the whole structure instead
-            warnings.warn("grapes_b200: sharded full-batch structure or peer-mapped row table unavailable" +
-                          (f" ({why})" if why else
-                          " on another rank") + "; every rank runs the replicated full-batch evaluation")
+            sgn, ptab = None, None                     # the replicated evaluation builds the whole structure instead
+            adjacency._sharded_eval_failure = why or "on another rank"
+            if fallback:
+                warnings.warn("grapes_b200: sharded full-batch structure or peer-mapped row table unavailable" +
+                              (f" ({why})" if why else
+                              " on another rank") + "; every rank runs the replicated full-batch evaluation")
         cached = (key, sgn, table)
-        adjacency._sharded_eval = cached
-    return cached[1], cached[2]
+        adjacency._sharded_eval, adjacency._sharded_eval_p = cached, ptab
+    return cached[1], cached[2], adjacency._sharded_eval_p
 
 
 def _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, device, x, y, mask_d, loader, full_batch,
@@ -192,19 +212,36 @@ def _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, devi
       replicated, so every rank decides alike) or when the window structure or the peer mapping failed on any rank.
     * mini batch: rank r runs the batches i = r mod W of the split, all of them; hits and rows are summed as integers, and
       ``return_predictions`` gathers every rank's predictions back into batch order."""
-    from .dist import allreduce_counts_, eval_batches, gather_batch_predictions, ranks_agree
+    from .dist import ShardedFeatures, allreduce_counts_, eval_batches, gather_batch_predictions, ranks_agree
     world, rank = dist.get_world_size(group), dist.get_rank(group)
+    sharded_x = isinstance(x, ShardedFeatures)
     if full_batch:
         if return_predictions:
             raise GrapesError("data-parallel full-batch evaluation returns scores only: gathering the [N, C] logits on "
                               "every rank is the memory it avoids (evaluate without a group for the logits)")
-        if row_slab_refusal(gcn_c, x) is not None:
+        why = row_slab_refusal(gcn_c, x)
+        if why is not None:
+            if sharded_x:             # no replicated table to fall back to; the same decision on every rank
+                raise GrapesError(f"full-batch evaluation of a sharded feature table: {why}; evaluate mini-batch "
+                                  "(full_batch=False) instead")
             return None               # a classifier the row-slab forward does not cover: the same on every rank
+        if sharded_x and (x.world != world or x.N != adjacency.num_nodes):
+            raise GrapesError(f"sharded feature table of {x.N} rows over {x.world} ranks; the group has {world} ranks "
+                              f"and the graph {adjacency.num_nodes} nodes")
         C = int(gcn_c.gcn_layers[-1].lin.weight.shape[0])
-        sgn, table = _sharded_eval(adjacency, data, group, (C + 3) // 4 * 4, device)
+        p_shape = None
+        if needs_p_table(gcn_c, x):
+            p_shape = (max(x.bounds[r + 1] - x.bounds[r] for r in range(world)),
+                       int(gcn_c.gcn_layers[0].lin.weight.shape[0]))
+        sgn, table, ptab = _sharded_eval(adjacency, data, group, (C + 3) // 4 * 4, device, p_shape,
+                                         fallback=not sharded_x)
         if table is None:
+            if sharded_x:
+                raise GrapesError("full-batch evaluation of a sharded feature table: window structure or peer-mapped "
+                                  f"Z / P table unavailable ({adjacency._sharded_eval_failure}); evaluate mini-batch "
+                                  "(full_batch=False) instead")
             return None
-        _, counts = full_graph_forward_sharded(gcn_c, x, sgn, table, y=y, mask=mask_d)
+        _, counts = full_graph_forward_sharded(gcn_c, x, sgn, table, y=y, mask=mask_d, p_table=ptab)
         allreduce_counts_(counts, group)
         ei = getattr(data, "edge_index", None)
         if y.dim() == 1 and (int(ei.shape[1]) if ei is not None else adjacency.nnz) < WIDE_MIN_EDGES:
@@ -217,7 +254,7 @@ def _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, devi
     sizes = [int(b.numel()) for b in batches]
     mine = eval_batches(len(batches), rank, world)
     eng = engine if engine is not None else _eval_engine(adjacency, data, args, gcn_c, gcn_gf, num_indicators, device,
-                                                         max(sizes + [1]))
+                                                         max(sizes + [1]), x)
     total = sum(sizes[i] for i in mine)
     preds = torch.zeros(max(total, 1), dtype=torch.int32, device=device)
     off = 0
@@ -241,15 +278,21 @@ def _evaluate_sharded(gcn_c, gcn_gf, data, args, adjacency, num_indicators, devi
     return acc, acc
 
 
-def _eval_engine(adjacency: DeviceGraph, data, args, gcn_c: GCN, gcn_gf: GCN, num_indicators: int, device, batch_size: int):
+def _eval_engine(adjacency: DeviceGraph, data, args, gcn_c: GCN, gcn_gf: GCN, num_indicators: int, device, batch_size: int,
+                 x=None):
     """Engine for a stand-alone ``evaluate(..., full_batch=False)`` call (the training loop passes its own): built once
-    per (graph, features, shape) and cached on the graph object; the modules' weights are loaded on every call."""
+    per (graph, features, shape) and cached on the graph object; the modules' weights are loaded on every call.  ``x``: the
+    device table or a sharded one (default ``data.x``)."""
+    from .dist import ShardedFeatures
     from .engine import GrapesEngine
     D = int(gcn_c.gcn_layers[0].lin.weight.shape[0])
     C = int(gcn_c.gcn_layers[-1].lin.weight.shape[0])
-    x = data.x.to(device).contiguous()
-    key = (x.data_ptr(), tuple(x.shape), D, C, int(batch_size), int(args.num_samples), int(args.sampling_hops),
-           bool(num_indicators))
+    if not isinstance(x, ShardedFeatures):
+        x = data.x.to(device).contiguous()
+        xkey = (x.data_ptr(), tuple(x.shape))
+    else:
+        xkey = (id(x), x.N, x.F)
+    key = (xkey, D, C, int(batch_size), int(args.num_samples), int(args.sampling_hops), bool(num_indicators))
     cached = getattr(adjacency, "_eval_engine", None)
     if cached is None or cached[0] != key:
         eng = GrapesEngine(adjacency, x, data.y.to(device), num_classes=C, batch_size=int(batch_size),

@@ -342,6 +342,16 @@ class ShardedGraphNorm:
                                            out.stride(0), _stream())
         return out
 
+    def aggregate_rows_sharded(self, ptrs, bounds_c, world: int, x_bf16: bool, F: int, ld: int, slab: torch.Tensor,
+                               R: int, out: torch.Tensor, bias=None) -> torch.Tensor:
+        """:meth:`aggregate_rows` over a table sharded by the feature bounds (``bounds_c``, HOST int64 [world + 1]):
+        owner o's rows at ``ptrs[o]`` with pitch ``ld`` elements, fp32 or bf16 (``grapes_aggregate_rows64_peer_x``);
+        bit-identical to :meth:`aggregate_rows` over the unpartitioned table."""
+        lib().grapes_aggregate_rows64_peer_x(self.holder.ctx, ptrs, bounds_c, int(world), int(bool(x_bf16)), F, ld,
+                                             ptr(slab), R, self.in_off_base, ptr(self._src), ptr(self.dinv), ptr(bias),
+                                             ptr(out), out.stride(0), _stream())
+        return out
+
 
 def _gemm_into(A, lda, W, ldw, C, ldc, M, N, K, bias=None):
     """C[:M, :N] = A W^T (+ bias) on the same SIMT ``grapes_gemm`` call as :func:`_gemm` (layout 3), into a caller view."""
@@ -398,9 +408,16 @@ def full_graph_forward_streamed(gcn: "GCN", x: torch.Tensor, gn: WideGraphNorm, 
     return logits, scores
 
 
-def row_slab_refusal(gcn: "GCN", x: torch.Tensor):
+def _is_sharded(x) -> bool:
+    from .dist import ShardedFeatures
+    return isinstance(x, ShardedFeatures)
+
+
+def row_slab_refusal(gcn: "GCN", x):
     """Why the row-slab forwards (:func:`full_graph_forward_streamed`, :func:`full_graph_forward_sharded`) do not cover
-    this classifier and feature table, or None when they do."""
+    this classifier and feature table (a tensor or a :class:`grapes_b200.dist.ShardedFeatures`), or None when they do."""
+    if _is_sharded(x):
+        x = x.local
     layers = list(gcn.gcn_layers)
     if len(layers) != 2:
         return f"streamed full-graph forward covers the two-layer classifier, not {len(layers)} layers"
@@ -428,7 +445,8 @@ def _classifier_parts(gcn: "GCN", x: torch.Tensor):
     return w1, b1, w2, b2, D, C, C4
 
 
-def _slab_row_bytes(x: torch.Tensor, D: int, C4: int) -> int:
+def _slab_row_bytes(x, D: int, C4: int) -> int:
+    x = x.local if _is_sharded(x) else x
     F = x.shape[1]
     agg_first = F <= D
     return 4 * ((F if agg_first else 0) + (F if (not agg_first and x.dtype != torch.float32) else 0) + D + C4)
@@ -441,22 +459,34 @@ def _slab_plan(lo: int, hi: int, R: int, dev):
     return starts, slabs
 
 
-def _layer1_into(x, gn, w, starts, slabs, hi, R, Z, z0):
+def _layer1_into(x, gn, w, starts, slabs, hi, R, Z, z0, p_table=None):
     """Z[r - z0] = relu(A_hat X W1^T + b1)[r] W2^T for the rows r of the slabs (ending at ``hi``), at the narrower width:
-    F <= D aggregates X per slab first; F > D forms P = X W1^T for ALL N rows (the sources of any row) first."""
+    F <= D aggregates X per slab first; F > D forms P = X W1^T for ALL N rows (the sources of any row) first.  A sharded
+    table ``x`` (:class:`grapes_b200.dist.ShardedFeatures`) is read from its owners; with F > D, P is then the sharded
+    ``p_table`` (:func:`sharded_layer1_p`), already formed by every rank."""
     w1, b1, w2, D, C, C4 = w
-    dev = x.device
-    N, F = x.shape
+    sharded = _is_sharded(x)
+    dev = gn.dinv.device
+    N, F = (x.N, x.F) if sharded else x.shape
     H = torch.empty((R, D), dtype=torch.float32, device=dev)
     if F <= D:
         Y = torch.empty((R, F), dtype=torch.float32, device=dev)
         for i, r0 in enumerate(starts):
             n = min(R, hi - r0)
-            gn.aggregate_rows(x, slabs[i], n, Y)
+            if sharded:
+                gn.aggregate_rows_sharded(x.ptrs, x.bounds_c, x.world, x.x_bf16, F, x.ldx, slabs[i], n, Y)
+            else:
+                gn.aggregate_rows(x, slabs[i], n, Y)
             _gemm_into(Y, F, w1, F, H, D, n, D, F, bias=b1)
             torch.relu_(H[:n])
             _gemm_into(H, D, w2, D, Z[r0 - z0:], C4, n, C, D)
         del Y
+    elif sharded:
+        for i, r0 in enumerate(starts):
+            n = min(R, hi - r0)
+            gn.aggregate_rows_sharded(p_table.ptrs, x.bounds_c, x.world, False, D, p_table.ld, slabs[i], n, H, bias=b1)
+            torch.relu_(H[:n])
+            _gemm_into(H, D, w2, D, Z[r0 - z0:], C4, n, C, D)
     else:
         P = torch.empty((N, D), dtype=torch.float32, device=dev)
         for r0 in range(0, N, R):
@@ -493,7 +523,8 @@ def _layer2(agg, starts, slabs, hi, R, C, C4, dev, y, mask, return_logits):
 
 
 class LocalRowTable:
-    """The layer-2 operand table of :func:`full_graph_forward_sharded` for one emulated rank of a single process: every
+    """A partitioned row table (the layer-2 operand of :func:`full_graph_forward_sharded`, or the shards of
+    :class:`grapes_b200.dist.ShardedFeatures`) for one emulated rank of a single process: every
     window's rows in its own allocation on this device (``tables[o]``, shared by the emulated ranks), a barrier that does
     nothing.  Run :func:`sharded_layer1` for every emulated rank before :func:`sharded_layer2` for any of them.
     :class:`grapes_b200.dist.PeerRowTable` is the same interface over the ranks' symmetric memory."""
@@ -506,8 +537,8 @@ class LocalRowTable:
         self.ptrs = (ctypes.c_void_p * len(tables))(*[t.data_ptr() for t in tables])
 
     @staticmethod
-    def make(world: int, rows: int, ld: int, device):
-        tables = [torch.zeros((max(rows, 1), ld), dtype=torch.float32, device=device) for _ in range(world)]
+    def make(world: int, rows: int, ld: int, device, dtype: torch.dtype = torch.float32):
+        tables = [torch.zeros((max(rows, 1), ld), dtype=dtype, device=device) for _ in range(world)]
         return [LocalRowTable(tables, r) for r in range(world)]
 
     def barrier(self):
@@ -518,23 +549,56 @@ def _sharded_rows(sgn, R):
     return max(1, min(int(R), max(sgn.rows, 1)))
 
 
+def needs_p_table(gcn: "GCN", x) -> bool:
+    """True when :func:`full_graph_forward_sharded` over the sharded table ``x`` needs a P table (F > D): a row table of
+    ``x``'s bounds, [max rows, D] fp32 per rank, for :func:`sharded_layer1_p`."""
+    return _is_sharded(x) and x.F > int(list(gcn.gcn_layers)[0].lin.weight.shape[0])
+
+
 @torch.no_grad()
-def sharded_layer1(gcn: "GCN", x: torch.Tensor, sgn: ShardedGraphNorm, z_table, slab_rows=None, mem_budget=None):
-    """Phase 1 of :func:`full_graph_forward_sharded`: Z rows of this rank's window into ``z_table.rows`` (local row j =
-    graph row lo + j), on the calls and in the order of :func:`full_graph_forward_streamed`'s layer 1.  With F > D
-    every rank forms P = X W1^T for ALL N rows (the sources of its window may be any rows), so that product and its
-    [N, D] buffer do not shrink with the number of ranks; with F <= D (the products and papers shapes) nothing does."""
+def sharded_layer1_p(gcn: "GCN", x, p_table, slab_rows=None, mem_budget=None):
+    """Phase 0 of :func:`full_graph_forward_sharded` over a sharded feature table with F > D: P = X W1^T for this rank's
+    table rows (``x.local``) into ``p_table.rows`` (pitch D), on the SIMT GEMM of the streamed forward, so P is
+    bit-identical to its [N, D] P; layer 1 then aggregates P read from its owners.  Every rank's phase 0 must complete
+    before any rank's phase 1."""
     w1, b1, w2, b2, D, C, C4 = _classifier_parts(gcn, x)
+    rows, F = x.hi - x.lo, x.F
+    if p_table.ld != D or p_table.rows.shape[0] < rows:
+        raise GrapesError(f"P table of pitch {p_table.ld} x {p_table.rows.shape[0]} rows; the shard needs {D} x {rows}")
+    dev = p_table.rows.device
+    R = int(slab_rows) if slab_rows else slab_rows_for(rows, 4 * (F + D), 0, dev, mem_budget)
+    R = max(1, min(R, max(rows, 1)))
+    for a in range(0, rows, R):
+        n = min(R, rows - a)
+        xs = x.local[a:a + n] if x.dtype == torch.float32 else x.local[a:a + n].float()
+        _gemm_into(xs, xs.stride(0), w1, F, p_table.rows[a:], D, n, D, F)
+
+
+@torch.no_grad()
+def sharded_layer1(gcn: "GCN", x, sgn: ShardedGraphNorm, z_table, slab_rows=None, mem_budget=None, p_table=None):
+    """Phase 1 of :func:`full_graph_forward_sharded`: Z rows of this rank's window into ``z_table.rows`` (local row j =
+    graph row lo + j), on the calls and in the order of :func:`full_graph_forward_streamed`'s layer 1.  ``x`` is the
+    replicated table or a :class:`grapes_b200.dist.ShardedFeatures` (rows read from their owners,
+    ``grapes_aggregate_rows64_peer_x``).  With F > D and a replicated table every rank forms P = X W1^T for ALL N rows
+    (the sources of its window may be any rows), so that product and its [N, D] buffer do not shrink with the number of
+    ranks; with a sharded table each rank forms P for its own table rows only (``p_table``, :func:`sharded_layer1_p`)."""
+    w1, b1, w2, b2, D, C, C4 = _classifier_parts(gcn, x)
+    if needs_p_table(gcn, x) and p_table is None:
+        raise GrapesError("sharded feature table with F > D: layer 1 aggregates the sharded P = X W1^T (p_table)")
     if sgn.rows == 0:
         return
     if z_table.ld != C4 or z_table.rows.shape[0] < sgn.rows:
         raise GrapesError(f"row table of pitch {z_table.ld} x {z_table.rows.shape[0]} rows; the window needs {C4} x {sgn.rows}")
-    N, F = x.shape
-    resident = 0 if F <= D else N * D * 4
-    R = int(slab_rows) if slab_rows else slab_rows_for(sgn.rows, _slab_row_bytes(x, D, C4), resident, x.device, mem_budget)
+    sharded = _is_sharded(x)
+    N, F = (x.N, x.F) if sharded else x.shape
+    if sharded and (x.N != sgn.n or x.world != sgn.world):
+        raise GrapesError(f"sharded table of {x.N} rows over {x.world} ranks; the structure has {sgn.n} over {sgn.world}")
+    dev = sgn.dinv.device
+    resident = 0 if (F <= D or sharded) else N * D * 4
+    R = int(slab_rows) if slab_rows else slab_rows_for(sgn.rows, _slab_row_bytes(x, D, C4), resident, dev, mem_budget)
     R = _sharded_rows(sgn, R)
-    starts, slabs = _slab_plan(sgn.lo, sgn.hi, R, x.device)
-    _layer1_into(x, sgn, (w1, b1, w2, D, C, C4), starts, slabs, sgn.hi, R, z_table.rows, sgn.lo)
+    starts, slabs = _slab_plan(sgn.lo, sgn.hi, R, dev)
+    _layer1_into(x, sgn, (w1, b1, w2, D, C, C4), starts, slabs, sgn.hi, R, z_table.rows, sgn.lo, p_table)
 
 
 @torch.no_grad()
@@ -557,16 +621,21 @@ def sharded_layer2(gcn: "GCN", sgn: ShardedGraphNorm, z_table, slab_rows=None, m
 
 
 @torch.no_grad()
-def full_graph_forward_sharded(gcn: "GCN", x: torch.Tensor, sgn: ShardedGraphNorm, z_table, y=None, mask=None,
-                               return_logits: bool = False, slab_rows=None, mem_budget=None):
+def full_graph_forward_sharded(gcn: "GCN", x, sgn: ShardedGraphNorm, z_table, y=None, mask=None,
+                               return_logits: bool = False, slab_rows=None, mem_budget=None, p_table=None):
     """The data-parallel form of :func:`full_graph_forward_streamed`: this rank computes the rows of its window only.
     Layer 1 over the window's slabs (X replicated) writes Z for the window into this rank's slot of ``z_table``
     (``rows``, ``ld`` = round_up(C, 4), ``ptrs`` = every rank's slot, ``barrier()``); after a barrier, layer 2 aggregates the
     window reading each source row of Z from the rank that owns it; a second barrier keeps Z until every rank has read it.
     The window's logits are bit-identical to the same rows of :func:`full_graph_forward_streamed` and of ``gcn(x,
     GraphNorm)``.  Returns (window logits [rows, C] or None, int64 counts [3] of the window's masked rows or None); sum the
-    counts over the ranks and score them with :func:`_scores_from_counts`."""
-    sharded_layer1(gcn, x, sgn, z_table, slab_rows=slab_rows, mem_budget=mem_budget)
+    counts over the ranks and score them with :func:`_scores_from_counts`.  ``x`` may be a sharded feature table
+    (:class:`grapes_b200.dist.ShardedFeatures`, the same bounds on every rank); with F > D it needs ``p_table``
+    (:func:`needs_p_table`), formed first by :func:`sharded_layer1_p` and followed by a barrier."""
+    if needs_p_table(gcn, x):
+        sharded_layer1_p(gcn, x, p_table, slab_rows=slab_rows, mem_budget=mem_budget)
+        p_table.barrier()
+    sharded_layer1(gcn, x, sgn, z_table, slab_rows=slab_rows, mem_budget=mem_budget, p_table=p_table)
     z_table.barrier()
     res = sharded_layer2(gcn, sgn, z_table, slab_rows=slab_rows, mem_budget=mem_budget, y=y, mask=mask,
                          return_logits=return_logits)

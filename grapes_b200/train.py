@@ -22,7 +22,7 @@ from .utils import get_logger
 def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = True, args=None, graph=None, group=None):
     """The reference's two evaluation modes (/root/reference/eval.py:47-70 full-batch, :71-163 mini-batch) on the
     device, with the engine's current weights loaded into drop-in ``GCN`` modules (grapes_b200/eval.py); data parallel
-    over ``group`` when it has more than one rank."""
+    over ``group`` when it has more than one rank.  Reads the engine's feature table when it is sharded."""
     from .eval import evaluate as _evaluate
     dev = engine.device
     sd = engine.state_dicts()
@@ -38,11 +38,13 @@ def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = 
     ns = args if args is not None else type("A", (), dict(sampling_hops=engine.H, num_samples=engine.k,
                                                           use_indicators=engine.use_ind))()
     return _evaluate(gcn_c, gcn_gf, data, ns, graph, None, engine.num_ind, dev, mask=mask, eval_on_cpu=False,
-                     loader=loader, full_batch=full_batch, engine=None if full_batch else engine, group=group)
+                     loader=loader, full_batch=full_batch, engine=None if full_batch else engine, group=group,
+                     features=engine.features)
 
 
 def train(args: Arguments, data=None, device: Optional[torch.device] = None, use_cuda_graph: bool = True,
-          max_batches: Optional[int] = None, exchange: str = "peer", step_log=None, shard_eval: bool = True):
+          max_batches: Optional[int] = None, exchange: str = "peer", step_log=None, shard_eval: bool = True, *,
+          shard_features: bool = False):
     """``train(args)`` of the reference (main.py:57-364).  Under ``torchrun`` (WORLD_SIZE > 1, or an initialised
     ``torch.distributed`` group) it is data parallel: every rank holds a replica of the graph and features, batch ``i`` of
     the un-shuffled loader goes to rank ``i mod W`` (``dist.shard_batches``), and the engine exchanges the gradient and
@@ -51,8 +53,20 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
     -log_probs and the per-hop sampler statistics ``{min_prob,max_prob,mean_entropy,std_entropy}_{hop}`` -- one step
     behind, read from pinned host memory (no device stall).  ``shard_eval`` (data parallel only): every evaluation is
     split between the ranks (``eval.evaluate(..., group=...)``, the same scores); False makes every rank evaluate the whole
-    mask, as one process does."""
+    mask, as one process does.
+
+    ``shard_features`` (data parallel only; no effect with one process): the feature table is sharded by rows across the
+    ranks (:class:`grapes_b200.dist.ShardedFeatures`) instead of replicated, each rank holding 1/W of it and gathering
+    the other rows over NVLink peer memory, with bit-identical results.  For tables that do not fit one GPU: ``data.x``
+    may stay on the host (memory-mapped or not) and is never moved to one device whole.  Not with ``--embed_nodes``, and
+    full-batch evaluation needs ``shard_eval``."""
     logger = get_logger()
+    if shard_features and args.embed_nodes:
+        raise GrapesError("shard_features with --embed_nodes: the learned table's optimiser is not sharded; "
+                          "replicate the table (shard_features=False)")
+    if shard_features and args.eval_full_batch and not shard_eval:
+        raise GrapesError("shard_features with full-batch evaluation needs shard_eval=True: no rank holds the whole "
+                          "table to evaluate alone")
     if not torch.cuda.is_available():
         raise GrapesError("grapes_b200 has no CPU fallback: a CUDA (sm_100a) device is required")
     import torch.distributed as dist
@@ -91,7 +105,11 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
     if need + args.batch_size + args.num_samples > graph.max_frontier:
         graph = DeviceGraph(graph.indptr, graph.indices, data.num_nodes,
                             max_frontier=need + args.batch_size + args.num_samples)
-    x_dev = data.x.to(device).contiguous()
+    if shard_features and world > 1:
+        from .dist import ShardedFeatures
+        x_dev = ShardedFeatures(data.x, device)      # collective; raises on every rank when any rank cannot map it
+    else:
+        x_dev = data.x.to(device).contiguous()
     if args.embed_nodes:
         data.x = x_dev                       # evaluation reads the table the optimiser updates
     engine = GrapesEngine(graph, x_dev, data.y.to(device), num_classes=num_classes, embed_nodes=args.embed_nodes,

@@ -249,10 +249,28 @@ int grapes_aggregate_rows64(grapes_ctx* ctx, const void* X, int x_bf16, int F, i
  * at its rank's index) or any allocations this device can read; bounds: HOST array of world + 1 row bounds, bounds[0] = 0.
  * in_off is read at r0 + j (for a window structure pass its local offsets shifted back by the window's first row).  The
  * summation order is grapes_aggregate_rows64's, so the rows are bit-identical to it over the unpartitioned Z.
- * Register-staged; out[j, F:ldo) = 0.                                                                                  */
+ * Register-staged; out[j, F:ldo) = 0.  grapes_aggregate_rows64_peer_x with x_bf16 = 0.                               */
 int grapes_aggregate_rows64_peer(grapes_ctx* ctx, const void* const* z_rows, const int64_t* bounds, int world, int F,
                                  int ldz, const int* slab_dev, int cap_r, const int64_t* in_off, const int* in_src,
                                  const float* dinv, const float* bias, float* out, int ldo, void* stream);
+/* grapes_aggregate_rows64 over a table whose rows are partitioned between `world` <= 8 owners, fp32 or bf16 (x_bf16 = 1,
+ * widened on read): row s is x_rows[o] + (s - bounds[o]) * ldx elements for the owner o with bounds[o] <= s <
+ * bounds[o + 1].  x_rows / bounds as for grapes_aggregate_rows64_peer (empty windows allowed, their base may be NULL).
+ * Bit-identical to grapes_aggregate_rows64 over the unpartitioned table; register-staged.                            */
+int grapes_aggregate_rows64_peer_x(grapes_ctx* ctx, const void* const* x_rows, const int64_t* bounds, int world,
+                                   int x_bf16, int F, int ldx, const int* slab_dev, int cap_r, const int64_t* in_off,
+                                   const int* in_src, const float* dinv, const float* bias, float* out, int ldo,
+                                   void* stream);
+/* grapes_aggregate / grapes_aggregate_bf16 (x_bf16 = 1) over a feature table sharded by rows between `world` <= 8 owners:
+ * the feature row of node g = nodes[j] (or j when nodes is NULL) is x_rows[o] + (g - bounds[o]) * ldx elements for the
+ * owner o with bounds[o] <= g < bounds[o + 1] -- this rank's shard or a peer's over NVLink.  x_rows: HOST array of `world`
+ * device pointers; bounds: HOST array of world + 1 non-decreasing bounds, bounds[0] = 0, bounds[world] < 2^31.  Indicator
+ * columns, bias / relu, out or out_hi / out_lo, ones_col and the zero pad as grapes_aggregate; the summation order is
+ * theirs, so the rows are bit-identical to them over the unpartitioned table.  Register-staged, one launch.          */
+int grapes_aggregate_peer(grapes_ctx* ctx, const void* const* x_rows, const int64_t* bounds, int world, int x_bf16, int F,
+                          int ldx, const int* nodes, const int* n_dev, int cap_n, const int* in_off, const int* in_src,
+                          const float* dinv, const uint32_t* ind_bits, int num_ind, const float* bias, int relu,
+                          float* out, int ldo, float* out_hi, float* out_lo, int ones_col, void* stream);
 /* z may be given as `nparts` partial vectors `part_stride` floats apart (summed on the fly)           */
 int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int part_stride, const int* n_dev, int cap_n, const int* in_off,
                             const int* in_src, const float* dinv, const float* bias, float* out, float* zero_out,
