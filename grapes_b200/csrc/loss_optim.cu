@@ -505,9 +505,11 @@ __global__ void __launch_bounds__(256) k_gfn_finalize_scale(float* scal, float l
 // were never touched (m = v = 0, no gradient) are left alone: their update is exactly 0.  The bias correction uses
 // t = *step + t_add: t_add = 1 when `step` is optimizer_c's count BEFORE this update (grapes_adam_embed: the parameter
 // Adam launched afterwards increments it), 0 when that launch already ran (grapes_embed_merge_adam).  go != NULL: the
-// go word of a data-parallel exchange; a failed exchange (GO_FAIL) makes the launch a no-op.
+// go word of a data-parallel exchange; a failed exchange (GO_FAIL) makes the launch a no-op.  The walk covers the N
+// rows [row0, row0 + N) of the table: x, m and v point at row row0 (a shard of a table sharded by rows), while the
+// gradient bitmap and its rank are those of the whole table, tested at row0 + the local row.
 __global__ void __launch_bounds__(256) k_adam_embed(float* __restrict__ x, float* __restrict__ m, float* __restrict__ v,
-                                                    int64_t N, int F4, const uint32_t* __restrict__ bm,
+                                                    int row0, int64_t N, int F4, const uint32_t* __restrict__ bm,
                                                     const int* __restrict__ pref, const float* __restrict__ grows,
                                                     int ldg4, float lr, float beta1, float beta2, float eps,
                                                     const float* __restrict__ step, const unsigned int* go, float t_add) {
@@ -528,7 +530,7 @@ __global__ void __launch_bounds__(256) k_adam_embed(float* __restrict__ x, float
     float4* v4 = reinterpret_cast<float4*>(v);
     const float4* g4 = reinterpret_cast<const float4*>(grows);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int node = (int)(i / F4), c = (int)(i - (int64_t)node * F4);
+        const int local = (int)(i / F4), c = (int)(i - (int64_t)local * F4), node = row0 + local;
         const bool hit = bitmap_test(bm, node);
         float4 mi = m4[i], vi = v4[i];
         if (!hit && mi.x == 0.f && mi.y == 0.f && mi.z == 0.f && mi.w == 0.f && vi.x == 0.f && vi.y == 0.f &&
@@ -844,20 +846,69 @@ int grapes_adam_step2(grapes_ctx* ctx, float* params, const float* grads, float*
     return GRAPES_OK;
 }
 
+// the walk of k_adam_embed over rows [row0, row0 + rows) (0 rows: no launch); go: see k_adam_embed
+static void launch_adam_embed(grapes_ctx* ctx, float* table, float* exp_avg, float* exp_avg_sq, int64_t row0,
+                              int64_t rows, int F, const uint32_t* bm, const int* pref, const float* grad_rows, int ldg,
+                              float lr, float beta1, float beta2, float eps, const float* step_dev, const unsigned int* go,
+                              float t_add, cudaStream_t s) {
+    if (rows == 0) return;
+    const long long total = (long long)rows * (F / 4);
+    long long blocks = (total + 255) / 256;
+    const long long cap = (long long)ctx->sm_count * 8;
+    if (blocks > cap) blocks = cap;
+    pdl((k_adam_embed), (int)blocks, 256, 0, s)(table, exp_avg, exp_avg_sq, (int)row0, rows, F / 4, bm, pref, grad_rows,
+                                               ldg / 4, lr, beta1, beta2, eps, step_dev, go, t_add);
+    grapes_count_launches(1);
+}
+
 int grapes_adam_embed(grapes_ctx* ctx, float* table, float* exp_avg, float* exp_avg_sq, int64_t num_nodes, int F,
                       const uint32_t* bm_rows, const int* pref_rows, const float* grad_rows, int ldg, float lr,
                       float beta1, float beta2, float eps, const float* step_dev, void* stream) {
     GRAPES_REQUIRE(ctx && table && exp_avg && exp_avg_sq && bm_rows && pref_rows && grad_rows && step_dev, "null argument");
     GRAPES_REQUIRE(F > 0 && F % 4 == 0 && ldg % 4 == 0 && ldg >= F, "embedding width and gradient pitch must be multiples of 4");
     GRAPES_REQUIRE(num_nodes == ctx->num_nodes, "table rows != graph nodes");
-    const long long total = (long long)num_nodes * (F / 4);
-    long long blocks = (total + 255) / 256;
-    const long long cap = (long long)ctx->sm_count * 8;
-    if (blocks > cap) blocks = cap;
-    pdl((k_adam_embed), (int)blocks, 256, 0, (cudaStream_t)stream)(table, exp_avg, exp_avg_sq, num_nodes, F / 4, bm_rows,
-                                                                  pref_rows, grad_rows, ldg / 4, lr, beta1, beta2, eps,
-                                                                  step_dev, nullptr, 1.0f);
+    launch_adam_embed(ctx, table, exp_avg, exp_avg_sq, 0, num_nodes, F, bm_rows, pref_rows, grad_rows, ldg, lr, beta1,
+                      beta2, eps, step_dev, nullptr, 1.0f, (cudaStream_t)stream);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_adam_embed_rows(grapes_ctx* ctx, float* table, float* exp_avg, float* exp_avg_sq, int64_t num_nodes,
+                           int64_t row0, int64_t rows, int F, const uint32_t* bm_rows, const int* pref_rows,
+                           const float* grad_rows, int ldg, float lr, float beta1, float beta2, float eps,
+                           const float* step_dev, void* stream) {
+    GRAPES_REQUIRE(ctx && bm_rows && pref_rows && grad_rows && step_dev, "null argument");
+    GRAPES_REQUIRE(rows == 0 || (table && exp_avg && exp_avg_sq), "null shard");
+    GRAPES_REQUIRE(F > 0 && F % 4 == 0 && ldg % 4 == 0 && ldg >= F, "embedding width and gradient pitch must be multiples of 4");
+    GRAPES_REQUIRE(0 <= row0 && rows >= 0 && row0 + rows <= num_nodes, "row range outside the table");
+    GRAPES_REQUIRE(num_nodes <= ctx->num_nodes, "table rows > graph nodes");
+    launch_adam_embed(ctx, table, exp_avg, exp_avg_sq, row0, rows, F, bm_rows, pref_rows, grad_rows, ldg, lr, beta1,
+                      beta2, eps, step_dev, nullptr, 1.0f, (cudaStream_t)stream);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+// union, rank and mean rows of the world slots, then the table walk over [row0, row0 + rows)
+static int embed_merge_adam(grapes_ctx* ctx, const float* slots, int world, int cap_rows, int F,
+                            const unsigned int* state, uint32_t* bm_union, int* pref_union, int* union_ids, int cap_union,
+                            int* union_count, float* mean_rows, float* table, float* exp_avg, float* exp_avg_sq,
+                            int64_t row0, int64_t rows, float lr, float beta1, float beta2, float eps,
+                            const float* step_dev, int* overflow, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    const long long slot = grapes_embed_slot_floats(cap_rows, F);
+    pdl((k_embed_union), grid_for(ctx, (long long)cap_rows, 256), 256, 0, s)(slots, slot, world, cap_rows, state, bm_union);
     grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    // popcount-prefix rank of the union bitmap: ascending union ids and the local row of every id
+    const int rc = grapes_rank_nodes(ctx, bm_union, nullptr, pref_union, nullptr, union_ids, nullptr, nullptr, nullptr,
+                                     nullptr, nullptr, 0, 0, cap_union, union_count, nullptr, overflow, stream);
+    if (rc != GRAPES_OK) return rc;
+    pdl((k_embed_mean_rows), grid_for(ctx, (long long)cap_union * 32, 256), 256, 0, s)(
+        slots, slot, world, cap_rows, F / 4, state, union_ids, union_count, cap_union, mean_rows, 1.0f / (float)world);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    launch_adam_embed(ctx, table, exp_avg, exp_avg_sq, row0, rows, F, bm_union, pref_union, mean_rows, F, lr, beta1,
+                      beta2, eps, step_dev, state ? state + PS_GO : nullptr, 0.0f, s);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
 }
@@ -872,29 +923,26 @@ int grapes_embed_merge_adam(grapes_ctx* ctx, const float* slots, int world, int 
     GRAPES_REQUIRE(world >= 1 && world <= EMBED_MAX_WORLD, "1 <= world <= 8");
     GRAPES_REQUIRE(F > 0 && F % 4 == 0 && cap_rows > 0 && cap_union > 0, "table width must be a multiple of 4");
     GRAPES_REQUIRE(num_nodes == ctx->num_nodes, "table rows != graph nodes");
-    cudaStream_t s = (cudaStream_t)stream;
-    const long long slot = grapes_embed_slot_floats(cap_rows, F);
-    pdl((k_embed_union), grid_for(ctx, (long long)cap_rows, 256), 256, 0, s)(slots, slot, world, cap_rows, state, bm_union);
-    grapes_count_launches(1);
-    GRAPES_LAUNCH_OK();
-    // popcount-prefix rank of the union bitmap: ascending union ids and the local row of every id
-    const int rc = grapes_rank_nodes(ctx, bm_union, nullptr, pref_union, nullptr, union_ids, nullptr, nullptr, nullptr,
-                                     nullptr, nullptr, 0, 0, cap_union, union_count, nullptr, overflow, stream);
-    if (rc != GRAPES_OK) return rc;
-    pdl((k_embed_mean_rows), grid_for(ctx, (long long)cap_union * 32, 256), 256, 0, s)(
-        slots, slot, world, cap_rows, F / 4, state, union_ids, union_count, cap_union, mean_rows, 1.0f / (float)world);
-    grapes_count_launches(1);
-    GRAPES_LAUNCH_OK();
-    const long long total = (long long)num_nodes * (F / 4);
-    long long blocks = (total + 255) / 256;
-    const long long bcap = (long long)ctx->sm_count * 8;
-    if (blocks > bcap) blocks = bcap;
-    pdl((k_adam_embed), (int)blocks, 256, 0, s)(table, exp_avg, exp_avg_sq, num_nodes, F / 4, bm_union, pref_union,
-                                               mean_rows, F / 4, lr, beta1, beta2, eps, step_dev,
-                                               state ? state + PS_GO : nullptr, 0.0f);
-    grapes_count_launches(1);
-    GRAPES_LAUNCH_OK();
-    return GRAPES_OK;
+    return embed_merge_adam(ctx, slots, world, cap_rows, F, state, bm_union, pref_union, union_ids, cap_union,
+                            union_count, mean_rows, table, exp_avg, exp_avg_sq, 0, num_nodes, lr, beta1, beta2, eps,
+                            step_dev, overflow, stream);
+}
+
+int grapes_embed_merge_adam_rows(grapes_ctx* ctx, const float* slots, int world, int cap_rows, int F,
+                                 const unsigned int* state, uint32_t* bm_union, int* pref_union, int* union_ids,
+                                 int cap_union, int* union_count, float* mean_rows, float* table, float* exp_avg,
+                                 float* exp_avg_sq, int64_t num_nodes, int64_t row0, int64_t rows, float lr, float beta1,
+                                 float beta2, float eps, const float* step_dev, int* overflow, void* stream) {
+    GRAPES_REQUIRE(ctx && slots && bm_union && pref_union && union_ids && union_count && mean_rows && step_dev &&
+                       overflow, "null argument");
+    GRAPES_REQUIRE(rows == 0 || (table && exp_avg && exp_avg_sq), "null shard");
+    GRAPES_REQUIRE(world >= 1 && world <= EMBED_MAX_WORLD, "1 <= world <= 8");
+    GRAPES_REQUIRE(F > 0 && F % 4 == 0 && cap_rows > 0 && cap_union > 0, "table width must be a multiple of 4");
+    GRAPES_REQUIRE(0 <= row0 && rows >= 0 && row0 + rows <= num_nodes, "row range outside the table");
+    GRAPES_REQUIRE(num_nodes <= ctx->num_nodes, "table rows > graph nodes");
+    return embed_merge_adam(ctx, slots, world, cap_rows, F, state, bm_union, pref_union, union_ids, cap_union,
+                            union_count, mean_rows, table, exp_avg, exp_avg_sq, row0, rows, lr, beta1, beta2, eps,
+                            step_dev, overflow, stream);
 }
 
 int grapes_argmax_rows(grapes_ctx* ctx, const float* logits, int ldl, int C, const int* row_ids, const int* B_dev,

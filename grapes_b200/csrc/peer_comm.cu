@@ -26,6 +26,24 @@
 // suffice, but only because that merge launch sits between this rank's tails of steps s and s + 1 on one stream: a rank
 // can push step s + 2 into slot parity s & 1 of peer p only after its tail of s + 1 saw p's flag of s + 1, which p's
 // tail of s + 1 releases after (stream order) p's merge of step s has finished reading parity s & 1.
+//
+// Learned table sharded by rows (grapes_embed_merge_adam_rows over rank r's rows [lo_r, hi_r) only): rank r's step
+// s + 1 gathers rows of every shard o (hop aggregations, classifier layer 1, predict), so those reads must follow o's
+// table walk of step s.  The exchange's flag of step s does not order them: o releases it in its tail, BEFORE its merge.
+// Every rank therefore owns a small symmetric epoch buffer [world words | own count] (grapes_embed_epoch_words):
+//   post     after this rank's shard walk, same stream: count += 1, then st.release.sys of the count into word[rank] of
+//            every rank's epoch buffer.  Skipped when the step's exchange failed (go word GO_FAIL): nothing was applied.
+//   wait     before the first read of the table of a step or of predict, same stream: ld.acquire.sys spin until word[p]
+//            of this rank's own buffer has reached the own count for every p -- every peer has applied as many table
+//            steps as this rank -- bounded like the tail's wait.  A timeout raises GRAPES_OVF_PEER_TIMEOUT and sets the
+//            exchange's sticky failure, so that step's tail and merge are no-ops on this rank (as for a missing flag).
+// The count lives in device memory, so a replayed graph advances it; a step enqueued without the optimiser (the graph
+// warm-up) waits but never posts.  No deadlock: r's wait before step s + 1 needs o's post of s, which follows o's merge and
+// tail of s, which needed only the flags of step s -- released by every rank's tail of s, which precedes that rank's
+// wait of s + 1 in its stream.  Writes after reads are ordered already: o's walk of step s + 1 follows o's tail of s + 1,
+// which waited for r's flag of s + 1, released after all of r's reads of step s + 1 (with the NCCL exchange the
+// all-gather of s + 1 orders them the same way).  The two-parity argument above is unchanged: the merge still sits
+// between this rank's tails on one stream, and the post after it changes no slot.
 #define GRAPES_PDL_GROUP 8
 #include "common.cuh"
 
@@ -252,6 +270,46 @@ __global__ void __launch_bounds__(256) k_step_tail_embed(const TailArgs a, const
     step_tail<true, true>(a, &e);
 }
 
+// ---- epoch of a learned table sharded by rows (grapes_embed_epoch_post / _wait); epoch: [world words | own count] ----
+struct EpochBufs {
+    unsigned int* buf[PEER_MAX];       // every rank's epoch buffer (peer-mapped)
+};
+
+__global__ void __launch_bounds__(32) k_embed_epoch_post(const EpochBufs e, unsigned int* own, int rank, int world,
+                                                          const unsigned int* state) {
+    pdl_begin();
+    if (state && (*(volatile const unsigned int*)(state + PS_GO) & GO_FAIL)) return;    // the step was not applied
+    const unsigned int c = *(volatile unsigned int*)(own + world) + 1u;
+    __syncwarp();
+    if (threadIdx.x == 0) own[world] = c;
+    __threadfence_system();                           // this rank's walk (earlier launches of the stream) before the words
+#pragma unroll
+    for (int r = 0; r < PEER_MAX; ++r)                // lane r -> rank r; constant indices keep the table in parameters
+        if (r == (int)threadIdx.x && r < world) st_release_sys_u32(e.buf[r] + rank, c);
+}
+
+__global__ void __launch_bounds__(32) k_embed_epoch_wait(const unsigned int* epoch, int world, unsigned int* state,
+                                                          int* err_flag, unsigned int spin_limit) {
+    pdl_begin();
+    const int tid = threadIdx.x;
+    const bool failed = state && *(volatile const unsigned int*)(state + PS_FAILED) != 0u;
+    const unsigned int c = *(volatile const unsigned int*)(epoch + world);
+    int arrived = 1;
+    if (tid < world && !failed) {
+        unsigned int it = 0;
+        while ((int)(ld_acquire_sys_u32(epoch + tid) - c) < 0) {
+            if (++it > spin_limit) { arrived = 0; break; }                       // never hang the GPU
+            __nanosleep(32);
+        }
+    }
+    const bool ok = __all_sync(0xffffffffu, arrived) && !failed;
+    if (tid == 0 && !ok) {
+        atomicOr(err_flag, GRAPES_OVF_PEER_TIMEOUT);
+        if (state) state[PS_FAILED] = 1u;
+        __threadfence();
+    }
+}
+
 static int launch_tail(grapes_ctx* ctx, TailArgs& a, void* const* peer_bufs, void* stream,
                        const EmbedPush* embed = nullptr) {
     for (int r = 0; r < PEER_MAX; ++r)
@@ -367,6 +425,38 @@ int grapes_step_tail_embed(grapes_ctx* ctx, float* scal, int do_scale, float los
     e.count = count_dev; e.ids = ids; e.rows = rows; e.ldg = ldg; e.F = F; e.cap = cap_rows;
     e.slot = grapes_embed_slot_floats(cap_rows, F);
     return launch_tail(ctx, a, peer_bufs, stream, &e);
+}
+
+int grapes_embed_epoch_words(int world) {
+    return (world < 1 ? 1 : world) + 1;
+}
+
+int grapes_embed_epoch_post(grapes_ctx* ctx, void* const* epoch_bufs, int rank, int world, const unsigned int* state,
+                            void* stream) {
+    GRAPES_REQUIRE(ctx && epoch_bufs, "null argument");
+    GRAPES_REQUIRE(world >= 1 && world <= PEER_MAX && rank >= 0 && rank < world, "1 <= world <= 8");
+    EpochBufs e;
+    memset(&e, 0, sizeof(e));
+    for (int r = 0; r < world; ++r) {
+        GRAPES_REQUIRE(epoch_bufs[r], "null epoch buffer");
+        e.buf[r] = reinterpret_cast<unsigned int*>(epoch_bufs[r]);
+    }
+    pdl((k_embed_epoch_post), 1, 32, 0, (cudaStream_t)stream)(e, e.buf[rank], rank, world, state);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_embed_epoch_wait(grapes_ctx* ctx, const unsigned int* epoch, int world, unsigned int* state, int* err_flag,
+                            uint32_t spin_limit, void* stream) {
+    GRAPES_REQUIRE(ctx && epoch && err_flag, "null argument");
+    GRAPES_REQUIRE(world >= 1 && world <= PEER_MAX, "1 <= world <= 8");
+    // 0: the tail's bound (a few seconds of polling, about 1 us per try)
+    pdl((k_embed_epoch_wait), 1, 32, 0, (cudaStream_t)stream)(epoch, world, state, err_flag,
+                                                             spin_limit ? spin_limit : 3000000u);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
 }
 
 }  // extern "C"

@@ -269,3 +269,86 @@ class ShardedFeatures:
             s.table = t
             s._fill(x, chunk_bytes)
         return out
+
+
+class ShardedEmbedding(ShardedFeatures):
+    """A LEARNED node-feature table [N, F] (``--embed_nodes``; fp32, F % 4 == 0) sharded by rows across the data-parallel
+    ranks (``train(..., shard_embeddings=True)``): rank r holds rows ``bounds[r] .. bounds[r + 1]`` as
+    :class:`ShardedFeatures` does, plus the two Adam moments of those rows (``exp_avg``, ``exp_avg_sq``: [rows, F], zero at
+    the start, ordinary device memory) and updates only those rows (``grapes_embed_merge_adam_rows``).  Every step posts
+    a table epoch into a small symmetric buffer (``epoch``; ``epoch_ptrs`` = the HOST array of every rank's), and every
+    read of the table waits for every peer's post of the previous step (``grapes_embed_epoch_post`` / ``_wait``; the
+    ordering argument is in csrc/peer_comm.cu).  Results are bit-identical to the replicated learned table.
+
+    The constructor is collective, with :class:`ShardedFeatures`' fill and its rule of agreeing on failure (every rank
+    raises ``GrapesError`` when any rank cannot allocate or map).  :meth:`to_dense` returns the [N, F] table (collective
+    under a group).  :meth:`emulate` is the one-process stand-in: W shards with their moments on one device, no epoch."""
+
+    def __init__(self, x: torch.Tensor, device, group=None, chunk_bytes: int = 1 << 30):
+        import ctypes
+        from ._lib import GrapesError, lib
+        self._check(x)
+        super().__init__(x, device, group, chunk_bytes)
+        device = torch.device(device)
+        self._moments(device)
+        self.shards = None
+        buf, why = None, ""
+        try:
+            import torch.distributed._symmetric_memory as symm_mem
+            buf = symm_mem.empty(int(lib().cdll.grapes_embed_epoch_words(self.world)), dtype=torch.int32, device=device)
+            buf.zero_()
+            hdl = symm_mem.rendezvous(buf, self.group.group_name if hasattr(self.group, "group_name") else self.group)
+            ptrs = [int(p) for p in hdl.buffer_ptrs]
+            assert ptrs[self.rank] == buf.data_ptr()
+        except Exception as exc:                        # noqa: BLE001 -- agreed below and raised on every rank
+            why, buf = f"{type(exc).__name__}: {exc}", None
+        torch.cuda.synchronize(device)
+        if not ranks_agree(buf is not None, device, self.group):   # also: every epoch buffer is zero before any post
+            raise GrapesError("sharded learned table: symmetric epoch buffer could not be mapped " +
+                              (f"on this rank ({why})" if why else "on another rank"))
+        self.epoch, self._epoch_hdl = buf, hdl
+        self.epoch_ptrs = (ctypes.c_void_p * self.world)(*ptrs)
+
+    @staticmethod
+    def _check(x):
+        from ._lib import GrapesError
+        if x.dim() != 2 or x.dtype != torch.float32 or int(x.shape[1]) % 4 != 0:
+            raise GrapesError("a sharded learned table is a 2-D fp32 tensor whose width is a multiple of 4")
+
+    def _moments(self, device):
+        rows = max(self.hi - self.lo, 1)
+        self.exp_avg = torch.zeros((rows, self.F), dtype=torch.float32, device=device)
+        self.exp_avg_sq = torch.zeros((rows, self.F), dtype=torch.float32, device=device)
+
+    @property
+    def moment_bytes(self) -> int:
+        """Device bytes of this rank's two moment arrays."""
+        return 2 * self.exp_avg.numel() * self.exp_avg.element_size()
+
+    @classmethod
+    def emulate(cls, x: torch.Tensor, world: int, device=None, chunk_bytes: int = 1 << 30) -> List["ShardedEmbedding"]:
+        cls._check(x)
+        out = super().emulate(x, world, device, chunk_bytes)
+        for s in out:
+            s._moments(s.table.rows.device)
+            s.shards, s.epoch, s.epoch_ptrs = out, None, None
+        return out
+
+    def _dense(self, local_of) -> torch.Tensor:
+        """[N, F] from every rank's [rows, F] array ``local_of(holder)`` (all-gather under a group)."""
+        if self.shards is not None:
+            return torch.cat([local_of(s)[:s.hi - s.lo] for s in self.shards])
+        rows = max(self.bounds[r + 1] - self.bounds[r] for r in range(self.world))
+        mine = torch.zeros((max(rows, 1), self.F), dtype=torch.float32, device=self.exp_avg.device)
+        mine[:self.hi - self.lo].copy_(local_of(self)[:self.hi - self.lo])
+        parts = [torch.empty_like(mine) for _ in range(self.world)]
+        dist.all_gather(parts, mine, group=self.group)
+        return torch.cat([parts[r][:self.bounds[r + 1] - self.bounds[r]] for r in range(self.world)])
+
+    def to_dense(self) -> torch.Tensor:
+        """The whole [N, F] table (a new tensor on this device); collective under a group."""
+        return self._dense(lambda s: s.table.rows[:, :s.F])
+
+    def moments_dense(self) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Both Adam moments of the whole table, [N, F] each; collective under a group."""
+        return self._dense(lambda s: s.exp_avg), self._dense(lambda s: s.exp_avg_sq)

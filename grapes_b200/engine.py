@@ -94,12 +94,14 @@ class GrapesEngine:
         dropout = float(dropout)
         if not 0. <= dropout <= 1.:
             raise ValueError(f"dropout probability has to be between 0 and 1, but got {dropout}")
-        from .dist import ShardedFeatures
+        from .dist import ShardedEmbedding, ShardedFeatures
         # a feature table sharded across the data-parallel ranks: both feature gathers read each row from its owner
-        # (grapes_aggregate_peer); nothing else of the step changes
+        # (grapes_aggregate_peer); nothing else of the step changes.  A learned table sharded with its Adam moments
+        # (ShardedEmbedding) is also updated shard by shard: each rank walks only its own rows.
         self.features = x if isinstance(x, ShardedFeatures) else None
+        self.embed_shards = x if (embed_nodes and isinstance(x, ShardedEmbedding)) else None
         if self.features is not None:
-            if embed_nodes:
+            if embed_nodes and self.embed_shards is None:
                 raise GrapesError("learned node features (embed_nodes) with a sharded feature table: the table optimiser "
                                   "is not sharded; replicate the table")
             if x.N != graph.num_nodes:
@@ -118,7 +120,8 @@ class GrapesEngine:
         # optimiser step (dense Adam from the sparse classifier gradient, grapes_adam_embed)
         self.embed_nodes = bool(embed_nodes)
         if self.embed_nodes:
-            assert x.dtype == torch.float32 and x.shape[1] % 4 == 0, "learned node features: fp32, width a multiple of 4"
+            assert x.dtype == torch.float32 and (x.F if self.features is not None else x.shape[1]) % 4 == 0, \
+                "learned node features: fp32, width a multiple of 4"
         self.multilabel = (y.dim() == 2)
         if self.multilabel:
             self.y = self.y.to(torch.float32)
@@ -271,7 +274,8 @@ class GrapesEngine:
             self.cl_out_dst0 = e(self.cap_blk, **i32)
             self.dYc = z((A, _round_up(F, 4)), **f32)
             self.dXc = z((A, _round_up(F, 4)), **f32)
-            self.emb_exp_avg, self.emb_exp_avg_sq = torch.zeros_like(x), torch.zeros_like(x)
+            if self.embed_shards is None:                 # a sharded table keeps the moments of its rows itself
+                self.emb_exp_avg, self.emb_exp_avg_sq = torch.zeros_like(x), torch.zeros_like(x)
 
         self.params = z(n_par, **f32)
         self.grads = z(n_par, **f32)
@@ -287,6 +291,7 @@ class GrapesEngine:
         self.peer = None                         # PeerGradExchange when the exchange runs over NVLink peer memory
         self.dp_group = None                     # process group of the NCCL exchange
         self.dp_world, self.dp_rank = 1, 0
+        self.epoch_spin_limit = 0                # tries of grapes_embed_epoch_wait (0: the step tail's bound)
         self.tail_state = torch.zeros(int(self.L.cdll.grapes_peer_state_words()), dtype=torch.int32, device=dev)
         self._graph_launches: Dict[tuple, int] = {}
         self.launches_per_graph = 0
@@ -449,6 +454,7 @@ class GrapesEngine:
         tc = self.use_tc
         gf, nz = self.net_gf, self.net_z
 
+        self._enqueue_epoch_wait(ctx, st)
         # ---- per-batch reset + hop-0 front end: already enqueued next to the previous step's classifier tail when this
         # state was prefetched (step(..., next_targets=...)), else inline ----
         if self._front_ready[self.par]:
@@ -658,6 +664,7 @@ class GrapesEngine:
         ovf = ptr(self.overflow)
         gf = self.net_gf
         self._front_ready = [False, False]
+        self._enqueue_epoch_wait(ctx, st)
         self._enqueue_front0(ctx, st)
         for h in range(H):
             hw = self.hops[h]
@@ -775,6 +782,19 @@ class GrapesEngine:
                 ctx, ptr(self.x), self.F, self.ldx, nodes, n_dev, cap_n, in_off, in_src, dinv, ind_bits, num_ind, None, 0,
                 out, ldo, out_hi, out_lo, ones_col, st)
 
+    def _sharded_dp(self) -> bool:
+        """The learned table is sharded across the ranks of this engine's data-parallel group."""
+        return self.embed_shards is not None and self.dp_world > 1
+
+    def _enqueue_epoch_wait(self, ctx, st):
+        """Sharded learned table under data parallelism: before the first read of the table, wait until every rank has
+        applied as many table steps to its shard as this one (grapes_embed_epoch_wait; csrc/peer_comm.cu)."""
+        if not self._sharded_dp():
+            return
+        es, pe = self.embed_shards, self.peer
+        self.L.grapes_embed_epoch_wait(ctx, ptr(es.epoch), es.world, ptr(pe.state) if pe is not None else None,
+                                       ptr(self.overflow), self.epoch_spin_limit, st)
+
     def _enqueue_front0(self, ctx, st):
         """Per-batch reset (main.py:161-176: one memset + one kernel) and the whole hop-0 front end of the ACTIVE step
         state on stream `st`: everything of a batch that can be computed before the previous batch's optimiser step."""
@@ -871,7 +891,11 @@ class GrapesEngine:
         With learned node features (``embed_nodes``) the table is replicated like ``x``: rank 0's table is broadcast once
         here (the moments start at zero), every step ships its row-sparse table gradient (at most cap_A rows) to every
         rank -- inside the peer tail, or by one ``all_gather`` -- and every rank applies the same dense Adam to the mean
-        of the ranks' gradients (``grapes_embed_merge_adam``), so the tables stay bit-identical."""
+        of the ranks' gradients (``grapes_embed_merge_adam``), so the tables stay bit-identical.  A learned table
+        sharded across ``group`` (``x`` a :class:`grapes_b200.dist.ShardedEmbedding`) is not broadcast (every rank
+        filled its rows from the same draw); each rank applies that Adam to its own rows only and posts a table epoch
+        (``grapes_embed_merge_adam_rows`` + ``grapes_embed_epoch_post``), and every read of the table waits for the
+        peers' posts."""
         import torch.distributed as dist
         if exchange not in ("peer", "nccl"):
             raise ValueError("exchange must be 'peer' or 'nccl'")
@@ -880,6 +904,10 @@ class GrapesEngine:
         self.peer, self.dp_group = None, None
         if self.embed_nodes and self.dp_world > 8:
             raise GrapesError("learned node features are exchanged among at most 8 ranks (one NVLink box)")
+        es = self.embed_shards
+        if es is not None and self.dp_world > 1 and (es.group is None or es.world != self.dp_world or
+                                                     es.rank != self.dp_rank):
+            raise GrapesError("the sharded learned table must be sharded across the data-parallel group itself")
         embed_floats = 0
         if self.embed_nodes and self.dp_world > 1:
             self.emb_slot = int(self.L.cdll.grapes_embed_slot_floats(self.cap_A, self.F))
@@ -889,9 +917,13 @@ class GrapesEngine:
             self.pref_union = torch.zeros(self.W + 1, dtype=torch.int32, device=self.device)
             self.union_ids = torch.zeros(self.cap_U, dtype=torch.int32, device=self.device)
             self.mean_rows = torch.zeros((self.cap_U, self.F), dtype=torch.float32, device=self.device)
-            dist.broadcast(self.x, src=dist.get_global_rank(group, 0), group=group)
-            self.emb_exp_avg.zero_()
-            self.emb_exp_avg_sq.zero_()
+            if es is None:
+                dist.broadcast(self.x, src=dist.get_global_rank(group, 0), group=group)
+                self.emb_exp_avg.zero_()
+                self.emb_exp_avg_sq.zero_()
+            else:
+                es.exp_avg.zero_()
+                es.exp_avg_sq.zero_()
         if self.dp_world > 1:
             if exchange == "peer":
                 # symmetric (peer-mapped) buffers need P2P access between every pair of GPUs of the group.  Every rank tries,
@@ -937,7 +969,15 @@ class GrapesEngine:
         n_z = 0 if self.reinforce else nz.size                       # gcn_z has no grad under REINFORCE (main.py:279)
         n1 = (gf.size + n_z) if scale else 0
         embed_dp = self.embed_nodes and self.dp_world > 1
-        if self.embed_nodes and not embed_dp:
+        if self.embed_nodes and not embed_dp and self.embed_shards is not None:
+            # emulated ranks (one process): every shard's walk over its own rows, in rank order
+            if self.embed_shards.shards is None:
+                raise GrapesError("a learned table sharded across a process group needs enable_data_parallel(group)")
+            for sh in self.embed_shards.shards:
+                L.grapes_adam_embed_rows(ctx, ptr(sh.table.rows), ptr(sh.exp_avg), ptr(sh.exp_avg_sq), self.N, sh.lo,
+                                         sh.hi - sh.lo, self.F, ptr(self.bm_all), ptr(self.pref_all), ptr(self.dXc),
+                                         self.dXc.shape[1], self.lr_gc, 0.9, 0.999, 1e-8, ptr(self.adam_steps), st)
+        elif self.embed_nodes and not embed_dp:
             L.grapes_adam_embed(ctx, ptr(self.x), ptr(self.emb_exp_avg), ptr(self.emb_exp_avg_sq), self.N, self.F,
                                 ptr(self.bm_all), ptr(self.pref_all), ptr(self.dXc), self.dXc.shape[1], self.lr_gc,
                                 0.9, 0.999, 1e-8, ptr(self.adam_steps), st)
@@ -983,7 +1023,17 @@ class GrapesEngine:
 
     def _enqueue_embed_merge(self, slots, state, st):
         """optimizer_c's step of the table on the mean of the ranks' row-sparse gradients (after the parameter Adam, so
-        the step count it reads already includes this step)."""
+        the step count it reads already includes this step).  A sharded table: the walk covers this rank's rows only,
+        then this rank posts its table epoch."""
+        es = self.embed_shards
+        if es is not None:
+            self.L.grapes_embed_merge_adam_rows(
+                self.g.ctx, slots, self.dp_world, self.cap_A, self.F, state, ptr(self.bm_union), ptr(self.pref_union),
+                ptr(self.union_ids), self.cap_U, self._cnt("U"), ptr(self.mean_rows), ptr(es.table.rows),
+                ptr(es.exp_avg), ptr(es.exp_avg_sq), self.N, es.lo, es.hi - es.lo, self.lr_gc, 0.9, 0.999, 1e-8,
+                ptr(self.adam_steps), ptr(self.overflow), st)
+            self.L.grapes_embed_epoch_post(self.g.ctx, es.epoch_ptrs, es.rank, es.world, state, st)
+            return
         self.L.grapes_embed_merge_adam(self.g.ctx, slots, self.dp_world, self.cap_A, self.F, state, ptr(self.bm_union),
                                        ptr(self.pref_union), ptr(self.union_ids), self.cap_U, self._cnt("U"),
                                        ptr(self.mean_rows), ptr(self.x), ptr(self.emb_exp_avg), ptr(self.emb_exp_avg_sq),

@@ -44,7 +44,7 @@ def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = 
 
 def train(args: Arguments, data=None, device: Optional[torch.device] = None, use_cuda_graph: bool = True,
           max_batches: Optional[int] = None, exchange: str = "peer", step_log=None, shard_eval: bool = True, *,
-          shard_features: bool = False):
+          shard_features: bool = False, shard_embeddings: bool = False):
     """``train(args)`` of the reference (main.py:57-364).  Under ``torchrun`` (WORLD_SIZE > 1, or an initialised
     ``torch.distributed`` group) it is data parallel: every rank holds a replica of the graph and features, batch ``i`` of
     the un-shuffled loader goes to rank ``i mod W`` (``dist.shard_batches``), and the engine exchanges the gradient and
@@ -59,11 +59,23 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
     ranks (:class:`grapes_b200.dist.ShardedFeatures`) instead of replicated, each rank holding 1/W of it and gathering
     the other rows over NVLink peer memory, with bit-identical results.  For tables that do not fit one GPU: ``data.x``
     may stay on the host (memory-mapped or not) and is never moved to one device whole.  Not with ``--embed_nodes``, and
-    full-batch evaluation needs ``shard_eval``."""
+    full-batch evaluation needs ``shard_eval``.
+
+    ``shard_embeddings`` (data parallel with ``--embed_nodes`` only; no effect with one process): the learned table and
+    its two Adam moments are sharded by rows across the ranks (:class:`grapes_b200.dist.ShardedEmbedding`); each rank
+    updates only its rows and reads the others from their owners, with results bit-identical to the replicated learned
+    table.  Full-batch evaluation needs ``shard_eval``.  The initial table is still drawn whole on the host of every
+    process (N x node_emb_dim floats) before each rank keeps its rows."""
     logger = get_logger()
     if shard_features and args.embed_nodes:
         raise GrapesError("shard_features with --embed_nodes: the learned table's optimiser is not sharded; "
                           "replicate the table (shard_features=False)")
+    if shard_embeddings and not args.embed_nodes:
+        raise GrapesError("shard_embeddings shards the learned table of --embed_nodes; to shard a given feature table "
+                          "use shard_features=True")
+    if shard_embeddings and args.eval_full_batch and not shard_eval:
+        raise GrapesError("shard_embeddings with full-batch evaluation needs shard_eval=True: no rank holds the whole "
+                          "table to evaluate alone")
     if shard_features and args.eval_full_batch and not shard_eval:
         raise GrapesError("shard_features with full-batch evaluation needs shard_eval=True: no rank holds the whole "
                           "table to evaluate alone")
@@ -93,7 +105,9 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
         # torchrun it is replicated and every rank applies the mean of the ranks' row-sparse gradients.
         logger.info('Using learned node embeddings for features')
         gen = torch.Generator().manual_seed(0 if args.seed is None else args.seed)
-        data.x = torch.empty(data.num_nodes, args.node_emb_dim).normal_(generator=gen).to(device)
+        data.x = torch.empty(data.num_nodes, args.node_emb_dim).normal_(generator=gen)
+        if not (shard_embeddings and world > 1):
+            data.x = data.x.to(device)       # a sharded table is filled rank by rank from the host draw
         data.num_features = num_features = args.node_emb_dim
     if args.model_type != 'gcn':
         raise ValueError("only model_type='gcn' is wired in the reference's train() (main.py:109)")
@@ -105,7 +119,11 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
     if need + args.batch_size + args.num_samples > graph.max_frontier:
         graph = DeviceGraph(graph.indptr, graph.indices, data.num_nodes,
                             max_frontier=need + args.batch_size + args.num_samples)
-    if shard_features and world > 1:
+    sharded_table = shard_embeddings and world > 1
+    if sharded_table:
+        from .dist import ShardedEmbedding
+        x_dev = ShardedEmbedding(data.x, device)     # collective; every rank fills its rows from the same draw
+    elif shard_features and world > 1:
         from .dist import ShardedFeatures
         x_dev = ShardedFeatures(data.x, device)      # collective; raises on every rank when any rank cannot map it
     else:
@@ -156,6 +174,13 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
             step_log(log)
         state["pending"] = None
 
+    def sync_ranks():
+        # a sharded learned table: every rank's last table step is applied before any rank's evaluation reads its rows
+        if sharded_table:
+            from .dist import ranks_agree
+            torch.cuda.synchronize(device)
+            ranks_agree(True, device)
+
     mem1, mem2, mem3 = [], [], []
     logger.info('Training')
     test_f1 = 0.0
@@ -179,10 +204,12 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
         collect()
         engine.check_overflow()
         if (epoch + 1) % args.eval_frequency == 0:                # main.py:319
+            sync_ranks()
             accuracy, f1 = evaluate(engine, data, data.val_mask, full_batch=args.eval_full_batch, args=args,
                                     group=eval_group)
             logger.info(f'loss_gfn={state["acc_gfn"]:.6f}, loss_c={state["acc_c"]:.6f}, '
                         f'valid_accuracy={accuracy:.3f}, valid_f1={f1:.3f}')
+    sync_ranks()
     test_accuracy, test_f1 = evaluate(engine, data, data.test_mask, full_batch=args.eval_full_batch, args=args,
                                       group=eval_group)
     logger.info(f'test_accuracy={test_accuracy:.3f}, test_f1={test_f1:.3f}')

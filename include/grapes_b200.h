@@ -423,6 +423,14 @@ int grapes_adam_step2(grapes_ctx* ctx, float* params, const float* grads, float*
 int grapes_adam_embed(grapes_ctx* ctx, float* table, float* exp_avg, float* exp_avg_sq, int64_t num_nodes, int F,
                       const uint32_t* bm_rows, const int* pref_rows, const float* grad_rows, int ldg, float lr,
                       float beta1, float beta2, float eps, const float* step_dev, void* stream);
+/* grapes_adam_embed over the rows [row0, row0 + rows) of a table of num_nodes rows (0 <= row0 <= row0 + rows <= num_nodes):
+ * table, exp_avg and exp_avg_sq point at row row0 (one rank's shard of a table sharded by rows, pitch F), while bm_rows /
+ * pref_rows / grad_rows are those of the whole table (bit row0 + i).  Per element the arithmetic of grapes_adam_embed, so
+ * a shard's rows equal the same rows of the whole-table walk bit for bit.  rows == 0: no launch.                     */
+int grapes_adam_embed_rows(grapes_ctx* ctx, float* table, float* exp_avg, float* exp_avg_sq, int64_t num_nodes,
+                           int64_t row0, int64_t rows, int F, const uint32_t* bm_rows, const int* pref_rows,
+                           const float* grad_rows, int ldg, float lr, float beta1, float beta2, float eps,
+                           const float* step_dev, void* stream);
 int grapes_fill_f32(grapes_ctx* ctx, float* p, float value, int n, void* stream);
 
 /* ---- step tail: gradient scale + data-parallel exchange + both Adam groups in ONE launch -------------------------- */
@@ -486,6 +494,27 @@ int grapes_embed_merge_adam(grapes_ctx* ctx, const float* slots, int world, int 
                             int* union_count, float* mean_rows, float* table, float* exp_avg, float* exp_avg_sq,
                             int64_t num_nodes, float lr, float beta1, float beta2, float eps, const float* step_dev,
                             int* overflow, void* stream);
+/* grapes_embed_merge_adam whose table walk covers only the rows [row0, row0 + rows) (this rank's shard of a table
+ * sharded by rows; table / exp_avg / exp_avg_sq point at row row0, pitch F).  Union, rank and mean rows are unchanged;
+ * the go word of `state` is honoured as there.  Follow it on the same stream with grapes_embed_epoch_post.         */
+int grapes_embed_merge_adam_rows(grapes_ctx* ctx, const float* slots, int world, int cap_rows, int F,
+                                 const unsigned int* state, uint32_t* bm_union, int* pref_union, int* union_ids,
+                                 int cap_union, int* union_count, float* mean_rows, float* table, float* exp_avg,
+                                 float* exp_avg_sq, int64_t num_nodes, int64_t row0, int64_t rows, float lr, float beta1,
+                                 float beta2, float eps, const float* step_dev, int* overflow, void* stream);
+/* Table epoch of a learned table sharded by rows (ordering argument: csrc/peer_comm.cu).  Every rank owns one symmetric
+ * buffer of grapes_embed_epoch_words(world) uint32, zeroed once: word[r] = table steps rank r has applied, then this
+ * rank's own count.  post: after this rank's shard walk, count += 1 and a system-scope release of it into word[rank] of
+ * every rank's buffer (epoch_bufs: HOST array of `world` peer-mapped pointers); no-op when state != NULL and the step's
+ * go word carries GO_FAIL.  wait (epoch = this rank's own buffer): before any read of the table, a bounded acquire spin
+ * until every word[p] has reached the own count.  spin_limit tries (0: the step tail's bound, a few seconds); on timeout
+ * GRAPES_OVF_PEER_TIMEOUT is ORed into *err_flag and, state != NULL, the exchange's sticky failure is set, so that
+ * step's tail and merge are no-ops.  Both launches read everything from device memory (graph-capturable).          */
+int grapes_embed_epoch_words(int world);
+int grapes_embed_epoch_post(grapes_ctx* ctx, void* const* epoch_bufs, int rank, int world, const unsigned int* state,
+                            void* stream);
+int grapes_embed_epoch_wait(grapes_ctx* ctx, const unsigned int* epoch, int world, unsigned int* state, int* err_flag,
+                            uint32_t spin_limit, void* stream);
 
 #ifdef __cplusplus
 }
