@@ -320,6 +320,14 @@ class ShardedEmbedding(ShardedFeatures):
         self.exp_avg = torch.zeros((rows, self.F), dtype=torch.float32, device=device)
         self.exp_avg_sq = torch.zeros((rows, self.F), dtype=torch.float32, device=device)
 
+    def load_rows(self, x: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor, chunk_bytes: int = 1 << 30):
+        """Overwrites this rank's rows of the table and of both moments in place from [N, F] sources (host,
+        memory-mapped or device; a checkpoint's ``table_source``), in chunks of at most ``chunk_bytes``."""
+        n = self.hi - self.lo
+        for a, b in fill_plan(self.lo, self.hi, self.F * 4, chunk_bytes):
+            for dst, src in ((self.table.rows[:n, :self.F], x), (self.exp_avg, exp_avg), (self.exp_avg_sq, exp_avg_sq)):
+                dst[a - self.lo:b - self.lo].copy_(src[a:b])
+
     @property
     def moment_bytes(self) -> int:
         """Device bytes of this rank's two moment arrays."""

@@ -1,5 +1,10 @@
 """CLI with the reference's behaviour (/root/reference/main.py:367-390):
-``python -m grapes_b200.main --config_file configs/gflownet/cora.txt [--flag value ...]``."""
+``python -m grapes_b200.main --config_file configs/gflownet/cora.txt [--flag value ...]``.
+
+``GRAPES_CHECKPOINT_DIR=<dir>`` (the ``Arguments`` stay the reference's): run r of ``--runs`` writes a checkpoint into
+``<dir>/run<r>`` at the end of every epoch and, when that directory holds a complete checkpoint, resumes from it."""
+import os
+
 import numpy as np
 import torch
 
@@ -11,8 +16,10 @@ def main(argv=None):
     args = parse_cli(argv)
     results = torch.empty(args.runs)
     mem1, mem2, mem3 = [], [], []
+    ckpt = os.environ.get("GRAPES_CHECKPOINT_DIR")
     for r in range(args.runs):
-        test_f1, m1, m2, m3 = train(args)
+        kw = dict(checkpoint_dir=os.path.join(ckpt, f"run{r}"), resume=True) if ckpt else {}
+        test_f1, m1, m2, m3 = train(args, **kw)
         results[r] = test_f1
         mem1.extend(m1); mem2.extend(m2); mem3.extend(m3)
     print(f'Memory point 1: {np.mean(mem1)} MB ± {np.std(mem1):.2f}')

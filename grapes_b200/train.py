@@ -44,7 +44,8 @@ def evaluate(engine: GrapesEngine, data, mask: torch.Tensor, full_batch: bool = 
 
 def train(args: Arguments, data=None, device: Optional[torch.device] = None, use_cuda_graph: bool = True,
           max_batches: Optional[int] = None, exchange: str = "peer", step_log=None, shard_eval: bool = True, *,
-          shard_features: bool = False, shard_embeddings: bool = False):
+          shard_features: bool = False, shard_embeddings: bool = False, checkpoint_dir: Optional[str] = None,
+          checkpoint_every: int = 0, resume: bool = False):
     """``train(args)`` of the reference (main.py:57-364).  Under ``torchrun`` (WORLD_SIZE > 1, or an initialised
     ``torch.distributed`` group) it is data parallel: every rank holds a replica of the graph and features, batch ``i`` of
     the un-shuffled loader goes to rank ``i mod W`` (``dist.shard_batches``), and the engine exchanges the gradient and
@@ -65,8 +66,17 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
     its two Adam moments are sharded by rows across the ranks (:class:`grapes_b200.dist.ShardedEmbedding`); each rank
     updates only its rows and reads the others from their owners, with results bit-identical to the replicated learned
     table.  Full-batch evaluation needs ``shard_eval``.  The initial table is still drawn whole on the host of every
-    process (N x node_emb_dim floats) before each rank keeps its rows."""
+    process (N x node_emb_dim floats) before each rank keeps its rows, unless the run resumes from a checkpoint.
+
+    ``checkpoint_dir``: a checkpoint (:mod:`grapes_b200.checkpoint`) is written there at the end of every epoch, after
+    that epoch's evaluation, and with ``checkpoint_every = n > 0`` also after every n steps of the rank.  ``resume``:
+    the run continues from the directory's latest checkpoint (its epoch, batch, loss accumulators and every device
+    state), bit-identical to a run that never stopped; without one it starts fresh.  A resumed ``--embed_nodes`` run
+    reads the learned table from the checkpoint and draws no initial table.  The memory points returned cover only
+    the steps this process ran."""
     logger = get_logger()
+    if checkpoint_every < 0 or (checkpoint_every and checkpoint_dir is None) or (resume and checkpoint_dir is None):
+        raise GrapesError("checkpoint_every > 0 and resume need checkpoint_dir")
     if shard_features and args.embed_nodes:
         raise GrapesError("shard_features with --embed_nodes: the learned table's optimiser is not sharded; "
                           "replicate the table (shard_features=False)")
@@ -96,18 +106,29 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
         data, num_features, num_classes = get_data(root=path, name=args.dataset, seed=args.seed, split_id=args.split_id)
     else:
         num_features, num_classes = data.num_features, data.num_classes
+    from .checkpoint import latest, load, save, table_source
+    resume_from = latest(checkpoint_dir) if resume else None
+    if resume and resume_from is None:
+        logger.info(f'No checkpoint in {checkpoint_dir}: starting fresh')
     if args.embed_nodes or data.x is None:
         if not args.embed_nodes:
             raise ValueError('Dataset does not contain node features, and embed_nodes is False. '
                              'Did you mean to run with --embed_nodes=True?')          # main.py:91-94
-        # main.py:95-100: embeddings = nn.Parameter(FloatTensor(N, node_emb_dim).normal_()), appended to optimizer_c.
-        # Here the table lives in HBM and the engine's optimiser launch updates it in place (grapes_adam_embed); under
-        # torchrun it is replicated and every rank applies the mean of the ranks' row-sparse gradients.
         logger.info('Using learned node embeddings for features')
-        gen = torch.Generator().manual_seed(0 if args.seed is None else args.seed)
-        data.x = torch.empty(data.num_nodes, args.node_emb_dim).normal_(generator=gen)
-        if not (shard_embeddings and world > 1):
-            data.x = data.x.to(device)       # a sharded table is filled rank by rank from the host draw
+        if resume_from is not None:
+            # the table and its moments come from the checkpoint (load() below): no initial draw
+            if shard_embeddings and world > 1:
+                data.x = table_source(resume_from)[0]    # memory-mapped [N, F]: each rank fills its rows from it
+            else:
+                data.x = torch.empty(data.num_nodes, args.node_emb_dim, device=device)
+        else:
+            # main.py:95-100: embeddings = nn.Parameter(FloatTensor(N, node_emb_dim).normal_()), appended to optimizer_c.
+            # Here the table lives in HBM and the engine's optimiser launch updates it in place (grapes_adam_embed); under
+            # torchrun it is replicated and every rank applies the mean of the ranks' row-sparse gradients.
+            gen = torch.Generator().manual_seed(0 if args.seed is None else args.seed)
+            data.x = torch.empty(data.num_nodes, args.node_emb_dim).normal_(generator=gen)
+            if not (shard_embeddings and world > 1):
+                data.x = data.x.to(device)       # a sharded table is filled rank by rank from the host draw
         data.num_features = num_features = args.node_emb_dim
     if args.model_type != 'gcn':
         raise ValueError("only model_type='gcn' is wired in the reference's train() (main.py:109)")
@@ -153,6 +174,14 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
     host = [torch.zeros(nread, dtype=torch.float32).pin_memory() for _ in range(2)]
     ready = [torch.cuda.Event(), torch.cuda.Event()]
     state = {"pending": None, "acc_c": 0.0, "acc_gfn": 0.0, "last": None}
+    start_epoch, start_batch, step_no = 1, 0, 0
+    if resume_from is not None:
+        loop = load(engine, resume_from, args=args)
+        state.update(acc_c=loop["acc_c"], acc_gfn=loop["acc_gfn"], last=loop["last"])
+        start_epoch, start_batch, step_no = loop["epoch"], loop["batch"], loop["step"]
+        if start_batch >= len(batches):                  # saved at the end of its epoch
+            start_epoch, start_batch = start_epoch + 1, 0
+        logger.info(f'Resuming from {resume_from}: epoch {start_epoch}, batch {start_batch}, step {step_no}')
 
     def collect():
         j = state["pending"]
@@ -181,13 +210,20 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
             torch.cuda.synchronize(device)
             ranks_agree(True, device)
 
+    def checkpoint(epoch, done):
+        collect()                                         # the step log is complete up to the checkpoint
+        save(engine, checkpoint_dir, dict(epoch=epoch, batch=done, step=step_no, acc_c=state["acc_c"],
+                                          acc_gfn=state["acc_gfn"], last=state["last"]), args=args)
+
     mem1, mem2, mem3 = [], [], []
     logger.info('Training')
     test_f1 = 0.0
-    step_no = 0
-    for epoch in range(1, args.max_epochs + 1):
-        state["acc_c"] = state["acc_gfn"] = 0.0
-        for bi, batch in enumerate(batches):
+    for epoch in range(start_epoch, args.max_epochs + 1):
+        first = start_batch if epoch == start_epoch else 0
+        if first == 0:
+            state["acc_c"] = state["acc_gfn"] = 0.0
+        for bi in range(first, len(batches)):
+            batch = batches[bi]
             # the next batch's reset + hop-0 front end is enqueued next to this step's classifier tail
             engine.step(batch, use_graph=use_cuda_graph, next_targets=batches[bi + 1] if bi + 1 < len(batches) else None)
             host[step_no % 2].copy_(engine.scal_stats, non_blocking=True)
@@ -201,6 +237,9 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
             if not args.random_sampling:
                 mem1.append(torch.cuda.max_memory_allocated() / (1024 * 1024)); mem2.append(mb)
             mem3.append(mb)
+            # the last batch of an epoch is checkpointed after the epoch's evaluation instead
+            if checkpoint_every and step_no % checkpoint_every == 0 and bi + 1 < len(batches):
+                checkpoint(epoch, bi + 1)
         collect()
         engine.check_overflow()
         if (epoch + 1) % args.eval_frequency == 0:                # main.py:319
@@ -209,6 +248,8 @@ def train(args: Arguments, data=None, device: Optional[torch.device] = None, use
                                     group=eval_group)
             logger.info(f'loss_gfn={state["acc_gfn"]:.6f}, loss_c={state["acc_c"]:.6f}, '
                         f'valid_accuracy={accuracy:.3f}, valid_f1={f1:.3f}')
+        if checkpoint_dir is not None:
+            checkpoint(epoch, len(batches))
     sync_ranks()
     test_accuracy, test_f1 = evaluate(engine, data, data.test_mask, full_batch=args.eval_full_batch, args=args,
                                       group=eval_group)
