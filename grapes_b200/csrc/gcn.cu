@@ -475,20 +475,25 @@ __global__ void __launch_bounds__(256) k_fill_inv_count(float* __restrict__ v, c
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) v[j] = inv;
 }
 
-// both parts in one launch: blocks [0, nbA) do the self term for rows that are NOT expanded rows (tested in the
-// prev bitmap), blocks [nbA, ..) own the expanded rows completely (self term + their out-edges) -> no write race.
+// both parts in one launch: blocks [0, nbA) do the self term for rows that are NOT expanded rows with an out-edge
+// (the prev bitmap and the graph's CSR degree tell), blocks [nbA, ..) own the expanded rows with out-edges completely
+// (self term + their out-edges) -> every row written once, no write race.  An expanded row without out-edges is a
+// frontier node only when another row points to it (directed graphs); blocks B skip it, so blocks A take it.
 __global__ void __launch_bounds__(256) k_dz_fused(const float* __restrict__ dl, const int* __restrict__ n_dev, int cap_n,
                                                   const int* __restrict__ P_dev, int cap_P,
                                                   const int* __restrict__ row_off, const int* __restrict__ e_src,
                                                   const int* __restrict__ e_dst, const float* __restrict__ dinv,
                                                   const uint32_t* __restrict__ bm_prev,
-                                                  const int* __restrict__ batch_nodes, int nbA,
+                                                  const int* __restrict__ batch_nodes,
+                                                  const long long* __restrict__ indptr, int nbA,
                                                   float* __restrict__ dz) {
     pdl_begin();
     if ((int)blockIdx.x < nbA) {
         const int n = min(*n_dev, cap_n);
-        for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += nbA * blockDim.x)
-            if (!bitmap_test(bm_prev, batch_nodes[j])) dz[j] = dinv[j] * dinv[j] * dl[j];
+        for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += nbA * blockDim.x) {
+            const int g = batch_nodes[j];
+            if (!bitmap_test(bm_prev, g) || indptr[g + 1] == indptr[g]) dz[j] = dinv[j] * dinv[j] * dl[j];
+        }
         return;
     }
     const int P = min(*P_dev, cap_P);
@@ -1416,13 +1421,15 @@ int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int par
 
 int grapes_aggregate_scalar_T(grapes_ctx* ctx, const float* dl, const int* n_dev, int cap_n, const int* P_dev,
                               int cap_P, const int* row_off, const int* e_src, const int* e_dst, const float* dinv,
-                              const uint32_t* bm_prev, const int* batch_nodes, float* dz, void* stream) {
+                              const uint32_t* bm_prev, const int* batch_nodes, const int64_t* indptr, float* dz,
+                              void* stream) {
     GRAPES_REQUIRE(ctx && dl && n_dev && P_dev && row_off && e_src && e_dst && dinv && dz, "null argument");
+    GRAPES_REQUIRE(!bm_prev == !batch_nodes && !bm_prev == !indptr, "bm_prev, batch_nodes and indptr go together");
     cudaStream_t s = (cudaStream_t)stream;
-    if (bm_prev && batch_nodes) {
+    if (bm_prev) {
         const int nbA = grid_for(ctx, cap_n, 256), nbB = grid_for(ctx, (long long)cap_P * 32, 256);
         pdl((k_dz_fused), nbA + nbB, 256, 0, s)(dl, n_dev, cap_n, P_dev, cap_P, row_off, e_src, e_dst, dinv, bm_prev,
-                                             batch_nodes, nbA, dz);
+                                             batch_nodes, reinterpret_cast<const long long*>(indptr), nbA, dz);
         grapes_count_launches(1);
         GRAPES_LAUNCH_OK();
         return GRAPES_OK;

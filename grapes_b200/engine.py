@@ -820,7 +820,7 @@ class GrapesEngine:
         n_dev, P_dev = self._hc(h, "n"), self._hc(h, "P")
         L.grapes_aggregate_scalar_T(ctx, ptr(hw.dl_all), n_dev, cap_n, P_dev, cap_P, ptr(hw.row_off), ptr(hw.e_src),
                                     ptr(hw.e_dst), ptr(hw.dinv), ptr(self.bm_prev[h]), ptr(hw.batch_nodes),
-                                    ptr(hw.dz), st)
+                                    ptr(self.g.indptr), ptr(hw.dz), st)
         if self.use_tc_bwd:
             L.grapes_sampler_l1_bwd_tc(ctx, ptr(hw.Y), ptr(hw.Y_lo), self.ldY, Fp + 1, n_dev, cap_n, Fp, Fp,
                                        ptr(hw.mask_gf), self._par(gf.W1), Fp, D, self._par(gf.b1), self._par(gf.W2),
@@ -860,7 +860,7 @@ class GrapesEngine:
         L.grapes_fill_inv_count(ctx, ptr(self.zlogits), n_dev, cap_n, st)
         L.grapes_aggregate_scalar_T(ctx, ptr(self.zlogits), n_dev, cap_n, P_dev, cap_P, ptr(hw.row_off),
                                     ptr(hw.e_src), ptr(hw.e_dst), ptr(hw.dinv), ptr(self.bm_prev[h]),
-                                    ptr(hw.batch_nodes), ptr(self.dz_z), st)
+                                    ptr(hw.batch_nodes), ptr(self.g.indptr), ptr(self.dz_z), st)
         if self.use_tc_bwd:
             L.grapes_sampler_l1_bwd_tc(ctx, ptr(hw.Y), ptr(hw.Y_lo), self.ldY, Fp + 1, n_dev, cap_n, F, Fp,
                                        ptr(self.mask_z), self._par(nz.W1), F, D, self._par(nz.b1), self._par(nz.W2),

@@ -275,10 +275,15 @@ int grapes_aggregate_peer(grapes_ctx* ctx, const void* const* x_rows, const int6
 int grapes_aggregate_scalar(grapes_ctx* ctx, const float* z, int nparts, int part_stride, const int* n_dev, int cap_n, const int* in_off,
                             const int* in_src, const float* dinv, const float* bias, float* out, float* zero_out,
                             void* stream);
-/* transposed scalar aggregation on the hop graph (backward of the above), row-major edge list.       */
+/* transposed scalar aggregation on the hop graph (backward of the above) from the row-major edge list of the expansion
+ * (rows[P] of the graph's CSR -> row_off, e_src, e_dst in local ids): writes dz[j] for every j < *n_dev,
+ *   dz[j] = dinv[j]^2 dl[j] + sum over edges j -> d of the hop graph, d != j, of dinv[j] dinv[d] dl[d].
+ * bm_prev (the expanded rows' bitmap), batch_nodes (local -> graph id) and indptr (the CSR the rows were expanded from)
+ * given together: one launch; all three NULL: two launches.  Same bits either way; no atomics.                       */
 int grapes_aggregate_scalar_T(grapes_ctx* ctx, const float* dl, const int* n_dev, int cap_n, const int* P_dev,
                               int cap_P, const int* row_off, const int* e_src, const int* e_dst, const float* dinv,
-                              const uint32_t* bm_prev, const int* batch_nodes, float* dz, void* stream);
+                              const uint32_t* bm_prev, const int* batch_nodes, const int64_t* indptr, float* dz,
+                              void* stream);
 /* v[j] = 1/n: gradient of log_z = mean(gcn_z logits) w.r.t. those logits (main.py:227-228)          */
 int grapes_fill_inv_count(grapes_ctx* ctx, float* v, const int* n_dev, int cap_n, void* stream);
 int grapes_vec_sum(grapes_ctx* ctx, const float* v, const int* n_dev, int cap_n, float scale, int divide_by_n,
