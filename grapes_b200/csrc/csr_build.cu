@@ -498,6 +498,36 @@ __global__ void __launch_bounds__(CB_THREADS) k_gnw_edges(const int64_t* __restr
         gnw_edge(src[e], dst[e], N, lo, hi, cnt, win_off, in_src);
 }
 
+// Transposed structure (grapes_graph_norm_t_*, the backward of the whole-graph aggregation): row s lists the destinations
+// d of the edges s -> d, stored self-loops dropped.  From the graph's CSR, whose row s already holds its destinations
+// sorted and unique, that is row s without s itself: a count (pass 0) and an order-keeping warp compaction (pass 1) at
+// out_off[s], no cursor and no sort.  From an edge list it is k_gn_edges with the roles of source and destination swapped.
+template <bool FILL>
+__global__ void __launch_bounds__(CB_THREADS) k_gnt_csr(const long long* __restrict__ indptr, const int* __restrict__ indices,
+                                                         int64_t r0, int64_t r1, int64_t N, int* __restrict__ cnt,
+                                                         const long long* __restrict__ out_off, int* __restrict__ out_dst,
+                                                         int* __restrict__ err) {
+    const int lane = lane_id();
+    const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t r = r0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); r < r1; r += warps) {
+        const long long e0 = indptr[r], e1 = indptr[r + 1];
+        long long base = FILL ? out_off[r] : 0;
+        for (long long c0 = e0; c0 < e1; c0 += 32) {
+            const long long e = c0 + lane;
+            const int64_t v = e < e1 ? (int64_t)indices[e] : (int64_t)r;
+            const bool bad = v < 0 || v >= N;
+            if (!FILL && bad) atomicOr(err, GN_ERR_ID);
+            const unsigned m = __ballot_sync(GRAPES_FULL_MASK, !bad && v != r);
+            if (FILL && !bad && v != r) out_dst[base + __popc(m & ((1u << lane) - 1u))] = (int)v;
+            base += __popc(m);
+        }
+        if (!FILL && lane == 0) {
+            if (base >= 0x7fffffff) { atomicOr(err, GN_ERR_DEG); base = 0x7ffffffe; }
+            cnt[r] = (int)base;
+        }
+    }
+}
+
 // bounds[k] = the least i in [0, N] with (in_off[i] + i) * W >= k * T, T = in_off[N] + N: the prefix of indeg + 1 cut into
 // W parts, so every window holds T / W of it to within one row's indeg + 1.  bounds[0] = 0, bounds[W] = N.
 __global__ void k_gn_bounds(int64_t N, const long long* __restrict__ in_off, int W, long long* __restrict__ bounds) {
@@ -838,6 +868,47 @@ int grapes_graph_norm_finish(int64_t num_nodes, const int64_t* in_off, int* in_s
     pdl((k_gn_sort_rows<CB_LONG_THREADS, CB_LONG_SMEM, true>), sms, CB_LONG_THREADS, CB_LONG_SMEM * 4, s)(
         num_nodes, off, in_src, worklist, flags);
     grapes_count_launches(3);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_t_add_csr(int pass, int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0,
+                                int64_t r1, int64_t* out_off, int* out_dst, void* workspace, int* err_dev, void* stream) {
+    GRAPES_REQUIRE(pass == 0 || pass == 1, "pass is 0 (count) or 1 (compaction)");
+    GRAPES_REQUIRE(indptr && workspace && err_dev && (pass == 0 || (out_off && out_dst)), "null argument");
+    GRAPES_REQUIRE(0 <= r0 && r0 <= r1 && r1 <= num_nodes, "row range outside [0, N]");
+    if (r1 == r0) return GRAPES_OK;
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    int* cnt = (int*)((unsigned char*)workspace + gn_layout(num_nodes).cnt);
+    const int64_t ctas = ((r1 - r0) * 32 + CB_THREADS - 1) / CB_THREADS;
+    const int grid = (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (pass == 0)
+        pdl(k_gnt_csr<false>, grid, CB_THREADS, 0, s)((const long long*)indptr, indices, r0, r1, num_nodes, cnt, nullptr,
+                                                       nullptr, err_dev);
+    else
+        pdl(k_gnt_csr<true>, grid, CB_THREADS, 0, s)((const long long*)indptr, indices, r0, r1, num_nodes, cnt,
+                                                      (const long long*)out_off, out_dst, err_dev);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_t_add_edges(int pass, int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                  int64_t* out_off, int* out_dst, void* workspace, int* err_dev, void* stream) {
+    // the forward's counting sort keyed by the source: row = src[e], entry = dst[e]
+    return grapes_graph_norm_add_edges(pass, num_nodes, dst, src, num_edges, out_off, out_dst, workspace, err_dev, stream);
+}
+
+int grapes_graph_norm_t_offsets(int64_t num_nodes, void* workspace, int64_t* out_off, int64_t* nnz_dev, void* stream) {
+    GRAPES_REQUIRE(workspace && out_off && nnz_dev, "null argument");
+    const GnLayout L = gn_layout(num_nodes);
+    unsigned char* ws = (unsigned char*)workspace;
+    int* cnt = (int*)(ws + L.cnt);
+    cudaStream_t s = (cudaStream_t)stream;
+    cb_scan64(cnt, num_nodes, (long long*)(ws + L.tile_sum), (long long*)out_off, (long long*)nnz_dev, s);
+    GRAPES_CUDA_OK(cudaMemsetAsync(cnt, 0, sizeof(int) * (size_t)num_nodes, s));    // cnt becomes the scatter cursor
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
 }

@@ -83,6 +83,7 @@ class GraphNorm(NormAdj):
         builder = builder or os.environ.get("GRAPES_GRAPHNORM_BUILDER", "torch")
         self._own_ctx = None
         self.graph = graph
+        self._edge_index = edge_index            # the transposed structure is built from the same input, on demand
         if builder == "lib":
             self._build_lib(graph, edge_index)
         else:
@@ -190,9 +191,17 @@ class GraphNorm(NormAdj):
             pass
 
     def aggregate(self, x, transpose=False, bias=None):
+        """A_hat x (+ bias); ``transpose``: A_hat^T x (+ bias), the backward, on the transposed arrays built on the first
+        call (:func:`transposed_structure`) with int32 offsets, through the same ``grapes_aggregate``."""
         if transpose:
-            raise GrapesError("GraphNorm is forward-only (evaluation); training uses the sampled blocks")
-        return super().aggregate(x, False, bias)
+            self.build_transposed()
+        return super().aggregate(x, transpose, bias)
+
+    def build_transposed(self):
+        """The transposed arrays ``out_off`` (int32) / ``out_dst``, once."""
+        if self.out_off is None:
+            off, self.out_dst = transposed_structure(self.n, self.dinv.device, self.graph, self._edge_index)
+            self.out_off = off.to(torch.int32)
 
 
 class WideGraphNorm:
@@ -200,16 +209,24 @@ class WideGraphNorm:
     (``grapes_graph_norm_*``): ``in_off`` int64 [N+1], ``in_src`` int32 [nnz'], ``dinv`` fp32 [N], equal bit for bit to
     the torch-sort builder.  Built on the device by a counting sort by destination that reads the input where it lies:
     the graph's CSR, or ``edge_index`` (host or device, int64 [2, E]; duplicates kept and counted) in chunks of
-    ``chunk_edges`` columns, so a host edge list never has to be on the device at once.  Device memory beyond the
-    outputs: ``grapes_graph_norm_workspace_bytes(N)`` (~4 N bytes) plus one chunk of a host edge list (16 bytes per edge).
-    Forward only: its aggregation is ``aggregate_rows`` over row slabs (:func:`full_graph_forward_streamed`)."""
+    ``chunk_edges`` columns, so a host edge list never has to be on the device at once.  Without a graph (``graph=None``)
+    the structure is that of ``edge_index`` on ``num_nodes`` nodes of ``device``.  Device memory beyond the outputs:
+    ``grapes_graph_norm_workspace_bytes(N)`` (~4 N bytes) plus one chunk of a host edge list (16 bytes per edge).
+    :meth:`aggregate_rows` aggregates one row slab (:func:`full_graph_forward_streamed`); :meth:`aggregate` all rows,
+    forward or transposed (the backward of the drop-in module), the transposed arrays ``out_off`` / ``out_dst`` built
+    from the same input on the first transposed call."""
 
-    def __init__(self, graph, edge_index=None, chunk_edges: int = 1 << 27):
-        dev = graph.device
-        N = graph.num_nodes
+    def __init__(self, graph, edge_index=None, chunk_edges: int = 1 << 27, *, num_nodes=None, device=None):
+        if graph is None and (edge_index is None or num_nodes is None or device is None):
+            raise GrapesError("WideGraphNorm without a graph needs edge_index, num_nodes and device")
+        dev = graph.device if graph is not None else torch.device(device)
+        N = graph.num_nodes if graph is not None else int(num_nodes)
         L, st = lib(), _stream()
         self.graph = graph
         self.holder = _any_ctx(dev)
+        self._input = (edge_index, chunk_edges)
+        self.out_off = self.out_dst = None
+        self._slabs = None
         ws = torch.empty(max(int(L.cdll.grapes_graph_norm_workspace_bytes(N)), 1), dtype=torch.uint8, device=dev)
         err = torch.zeros(1, dtype=torch.int32, device=dev)
         nnz = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -238,21 +255,80 @@ class WideGraphNorm:
             self.in_src = self.in_src[:0]
 
     @staticmethod
-    def _check(err):
+    def _check(err, edges: str = "in-edges"):
         e = int(err.item())
         if e & 1:
             raise GrapesError("edge_index holds node ids outside [0, num_nodes)")
         if e & 2:
-            raise GrapesError("a node has 2^31 - 1 or more in-edges")
+            raise GrapesError(f"a node has 2^31 - 1 or more {edges}")
 
-    def aggregate_rows(self, x: torch.Tensor, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None) -> torch.Tensor:
+    def aggregate_rows(self, x: torch.Tensor, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None,
+                       transpose: bool = False) -> torch.Tensor:
         """out[j] = (A_hat x)[r0 + j] (+ bias) for j < R, slab = int32 {R, r0} on the device; x fp32 or bf16 rows
-        (widened on read), out fp32 [>= R, >= F] with a unit column stride."""
+        (widened on read), out fp32 [>= R, >= F] with a unit column stride.  ``transpose``: rows of A_hat^T x."""
         F = x.shape[1]
+        if transpose:
+            self.build_transposed()
+        off, idx = (self.out_off, self.out_dst) if transpose else (self.in_off, self.in_src)
         lib().grapes_aggregate_rows64(self.holder.ctx, ptr(x), int(x.dtype == torch.bfloat16), F, x.stride(0), ptr(slab),
-                                      R, ptr(self.in_off), ptr(self.in_src), ptr(self.dinv), ptr(bias), ptr(out),
-                                      out.stride(0), _stream())
+                                      R, ptr(off), ptr(idx), ptr(self.dinv), ptr(bias), ptr(out), out.stride(0),
+                                      _stream())
         return out
+
+    def aggregate(self, x: torch.Tensor, transpose: bool = False, bias=None) -> torch.Tensor:
+        """A_hat x (+ bias) over all N rows, or A_hat^T x (+ bias) with ``transpose``: fp32 [N, F], one
+        ``grapes_aggregate_rows64`` launch per slab of ``SLAB_ROWS`` rows (bit-identical to ``grapes_aggregate`` on the
+        int32 structure of the same graph, see :class:`GraphNorm`)."""
+        x = x.contiguous()
+        out = torch.empty((self.n, x.shape[1]), dtype=torch.float32, device=x.device)
+        if self._slabs is None:
+            self._slabs = _slab_plan(0, self.n, self.SLAB_ROWS, x.device)
+        for i, r0 in enumerate(self._slabs[0]):
+            self.aggregate_rows(x, self._slabs[1][i], min(self.SLAB_ROWS, self.n - r0), out[r0:], bias, transpose)
+        return out
+
+    #: rows per launch of :meth:`aggregate`: 2^20 rows take the whole-graph launch shape of the row-slab kernels
+    SLAB_ROWS = 1 << 20
+
+    def build_transposed(self):
+        """The transposed arrays ``out_off`` (int64) / ``out_dst``, once."""
+        if self.out_off is None:
+            edge_index, chunk_edges = self._input
+            self.out_off, self.out_dst = transposed_structure(self.n, self.dinv.device, self.graph, edge_index,
+                                                              chunk_edges)
+
+
+def transposed_structure(N: int, dev, graph=None, edge_index=None, chunk_edges: int = 1 << 27):
+    """(out_off int64 [N + 1], out_dst int32 [nnz']) of the transposed gcn_norm structure (``grapes_graph_norm_t_*``):
+    row s lists the destinations of the edges s -> d, ascending, stored self-loops dropped, duplicates of ``edge_index``
+    kept.  Read from ``edge_index`` (host or device int64 [2, E], in chunks of ``chunk_edges`` columns) when given,
+    otherwise from ``graph``'s canonical CSR.  With the forward's ``dinv`` it is A_hat^T."""
+    L, st = lib(), _stream()
+    ws = torch.empty(max(int(L.cdll.grapes_graph_norm_workspace_bytes(N)), 1), dtype=torch.uint8, device=dev)
+    err = torch.zeros(1, dtype=torch.int32, device=dev)
+    nnz = torch.zeros(1, dtype=torch.int64, device=dev)
+    out_off = torch.empty(N + 1, dtype=torch.int64, device=dev)
+
+    def run(pass_, out_dst):
+        if edge_index is None:
+            L.grapes_graph_norm_t_add_csr(pass_, N, ptr(graph.indptr), ptr(graph.indices), 0, N, ptr(out_off),
+                                          ptr(out_dst), ptr(ws), ptr(err), st)
+            return
+        for src, dst in _edge_chunks(edge_index, chunk_edges, dev):
+            L.grapes_graph_norm_t_add_edges(pass_, N, ptr(src), ptr(dst), int(src.numel()), ptr(out_off), ptr(out_dst),
+                                            ptr(ws), ptr(err), st)
+
+    L.grapes_graph_norm_begin(N, ptr(ws), ws.numel(), ptr(err), st)
+    run(0, None)
+    L.grapes_graph_norm_t_offsets(N, ptr(ws), ptr(out_off), ptr(nnz), st)
+    WideGraphNorm._check(err, "out-edges")
+    E = int(nnz.item())                                          # one-off read-back: the size of out_dst
+    out_dst = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+    run(1, out_dst)
+    if edge_index is not None:
+        L.grapes_graph_norm_finish(N, ptr(out_off), ptr(out_dst), ptr(ws), st)
+    del ws
+    return out_off, (out_dst if E > 0 else out_dst[:0])
 
 
 def _edge_chunks(edge_index, chunk_edges, dev):
@@ -740,6 +816,28 @@ def _gemm_tn(A, B, R, M, N):
     return out
 
 
+def _colsum(M):
+    """sum over the rows of M [R, C] (fp32, contiguous): ``grapes_colsum``, fixed-order slabs."""
+    R, C = M.shape
+    out = torch.zeros(C, dtype=torch.float32, device=M.device)
+    if R > 0:
+        n = torch.tensor([R], dtype=torch.int32, device=M.device)
+        lib().grapes_colsum(_any_ctx(M.device).ctx, ptr(M), n.data_ptr(), R, C, C, 1.0, 0, ptr(out), _stream())
+    return out
+
+
+def gcn_structure(edge_index, num_nodes: int, device):
+    """The gcn_norm structure GCNConv aggregates over for a raw ``edge_index`` [2, E] on ``num_nodes`` nodes (PyG
+    semantics: duplicates counted, stored self-loops replaced by one per node).  Edge lists within the library's small
+    context take :class:`NormAdj`; larger ones (the whole graph) :class:`WideGraphNorm`, built from the edge list in
+    chunks (host or device).  Structures (:class:`NormAdj`, :class:`GraphNorm`, :class:`WideGraphNorm`) pass through."""
+    if isinstance(edge_index, (NormAdj, WideGraphNorm)):
+        return edge_index
+    if max(int(edge_index.shape[1]), int(num_nodes), 1) > _any_ctx(device).max_frontier:
+        return WideGraphNorm(None, edge_index=edge_index, num_nodes=num_nodes, device=device)
+    return NormAdj(edge_index, num_nodes)
+
+
 class _GCNConvFn(torch.autograd.Function):
     """out = A_hat (x W^T) + b, computed at the narrower width: (A_hat x) W^T when in <= out."""
 
@@ -774,7 +872,7 @@ class _GCNConvFn(torch.autograd.Function):
         n, O = dout.shape
         I = w.shape[1]
         need_dx = ctx_.needs_input_grad[0]
-        db = dout.sum(0) if ctx_.needs_input_grad[2] else None
+        db = _colsum(dout) if ctx_.needs_input_grad[2] else None
         dx = None
         if ctx_.agg_first:
             dW = _gemm_tn(dout, saved, n, O, I)                       # dout^T (A_hat x)
@@ -813,8 +911,9 @@ class GCNConv(nn.Module):
             self.bias.zero_()
 
     def forward(self, x, edge_index):
-        adj = edge_index if isinstance(edge_index, NormAdj) else NormAdj(edge_index, x.shape[0])
-        return _GCNConvFn.apply(x, self.lin.weight, self.bias, adj)
+        """``edge_index``: a raw [2, E] edge list (see :func:`gcn_structure`) or a prebuilt structure; forward and
+        backward (weights, bias and ``x`` when it requires grad) run on the library's kernels either way."""
+        return _GCNConvFn.apply(x, self.lin.weight, self.bias, gcn_structure(edge_index, x.shape[0], x.device))
 
 
 class GCN(nn.Module):
@@ -830,6 +929,8 @@ class GCN(nn.Module):
 
     def forward(self, x: torch.Tensor, edge_index: Union[torch.Tensor, List[torch.Tensor]]):
         layerwise_adjacency = type(edge_index) == list
+        if not layerwise_adjacency:
+            edge_index = gcn_structure(edge_index, x.shape[0], x.device)      # built once, shared by the layers
         for i, layer in enumerate(self.gcn_layers[:-1], start=1):
             edges = edge_index[-i] if layerwise_adjacency else edge_index
             x = torch.relu(layer(x, edges))

@@ -22,6 +22,11 @@ def main(argv=None):
         test_f1, m1, m2, m3 = train(args, **kw)
         results[r] = test_f1
         mem1.extend(m1); mem2.extend(m2); mem3.extend(m3)
+    report(results, mem1, mem2, mem3)
+
+
+def report(results, mem1, mem2, mem3):
+    """main.py:386-390: the memory points and ``Acc: mean ± std`` over the runs."""
     print(f'Memory point 1: {np.mean(mem1)} MB ± {np.std(mem1):.2f}')
     print(f'Memory point 2: {np.mean(mem2)} MB ± {np.std(mem2):.2f}')
     print(f'Memory point 2: {np.mean(mem3)} MB ± {np.std(mem3):.2f}')

@@ -122,6 +122,23 @@ int grapes_graph_norm_add_edges(int pass, int64_t num_nodes, const int64_t* src,
 int grapes_graph_norm_offsets(int64_t num_nodes, void* workspace, int64_t* in_off, float* dinv, int64_t* nnz_dev,
                               void* stream);
 int grapes_graph_norm_finish(int64_t num_nodes, const int64_t* in_off, int* in_src, void* workspace, void* stream);
+/* ---- the transposed structure (the backward dh = A_hat^T dout of the whole-graph aggregation): out_off int64 [N+1],
+ * out_dst int32 [nnz'] -- row s lists the destinations d of the edges s -> d, ascending, stored self-loops dropped,
+ * duplicates of an edge list kept and counted.  The weights stay dinv[s] dinv[d] and the self term dinv[s]^2 with the
+ * FORWARD's dinv (in-degree + 1), so grapes_aggregate / grapes_aggregate_rows64 handed (out_off, out_dst, dinv) compute
+ * A_hat^T G.  nnz' is the forward's.  Sequence, all on `stream`, no host synchronisation inside, in a workspace of
+ * grapes_graph_norm_workspace_bytes(N) (it may be the forward's once that build has finished):
+ *   begin -> t_add_*(pass 0) over the whole input -> t_offsets (out_off, *nnz_dev = nnz'; dinv is not touched) ->
+ *   t_add_*(pass 1) over the same input -> for an edge list only: finish(N, out_off, out_dst, workspace) (row sorts).
+ * t_add_csr reads rows [r0, r1) of a canonical CSR (rows sorted, unique, e.g. a DeviceGraph's): pass 1 is an
+ * order-keeping compaction, already ascending, so it needs no finish.  t_add_edges reads int64 chunks src[e] -> dst[e]
+ * as grapes_graph_norm_add_edges does.  *err_dev |= 1: an id outside [0, N) (skipped), |= 2: a node with 2^31 - 1 or more
+ * out-edges.                                                                                                          */
+int grapes_graph_norm_t_add_csr(int pass, int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0,
+                                int64_t r1, int64_t* out_off, int* out_dst, void* workspace, int* err_dev, void* stream);
+int grapes_graph_norm_t_add_edges(int pass, int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                  int64_t* out_off, int* out_dst, void* workspace, int* err_dev, void* stream);
+int grapes_graph_norm_t_offsets(int64_t num_nodes, void* workspace, int64_t* out_off, int64_t* nnz_dev, void* stream);
 /* ---- one destination window [lo, hi) of that structure (the row partition of the data-parallel full-batch evaluation).
  * window_bounds: from the full in_off of `offsets`, bounds_dev[0 .. world] (int64, on the device) = the least i with
  * (in_off[i] + i) * world >= k * (in_off[N] + N): the rows cut into `world` contiguous windows balanced by the prefix of
