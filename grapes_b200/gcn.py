@@ -67,18 +67,18 @@ class GraphNorm(NormAdj):
     stored self-loops are dropped, one self-loop per node is added, deg = in-degree + 1; the in-neighbour lists are
     the CSR of the transposed adjacency (edge_index[0] = source row, edge_index[1] = destination column),
     ascending source inside a row.  Two builders of the same arrays (see ``__init__``): the default sorts the
-    (destination, source) keys with ``torch.sort`` (one-off set-up, GPU-verified); the opt-in "lib" builder uses the
+    (destination, source) keys with ``torch.sort`` (one-off set-up); the opt-in "lib" builder uses the
     library's own kernels -- ``grapes_row_offsets`` + ``grapes_expand_rows`` turn the CSR back into its edge list,
     ``grapes_build_csr`` (counting sort by destination, per-row sort, self-loops dropped, deg^-1/2) is the routine that
     builds every hop's structure.  One-off, cached on the graph; the aggregation itself is ``grapes_aggregate``
     (TMA-staged SpMM) straight on these arrays.  nnz must fit int32 offsets; larger graphs use :class:`WideGraphNorm`."""
 
     def __init__(self, graph, edge_index=None, builder=None):
-        """``builder``: "torch" (default; GPU-verified in round 1 and 2) sorts the (destination, source) keys with
+        """``builder``: "torch" (default) sorts the (destination, source) keys with
         ``torch.sort``; "lib" (``GRAPES_GRAPHNORM_BUILDER=lib``) builds the same arrays with the library's own kernels
-        (``grapes_row_offsets`` / ``grapes_expand_rows`` / ``grapes_build_csr``).  The "lib" builder was written after this
-        round's GPU budget was spent: it is exercised by ``bench.py --full-eval`` (a process of its own) and by
-        the opt-in test ``tests/test_gpu_eval.py::test_full_graph_forward_tensor_core_path`` (GRAPES_TEST_UNVERIFIED=1)."""
+        (``grapes_row_offsets`` / ``grapes_expand_rows`` / ``grapes_build_csr``), equal to the torch builder bit for bit
+        (``tests/test_gpu_eval.py::test_lib_builder_equals_torch_builder``); it raises when ``grapes_build_csr`` flags an
+        overflow.  ``bench.py --full-eval`` measures it in a process of its own."""
         import os
         builder = builder or os.environ.get("GRAPES_GRAPHNORM_BUILDER", "torch")
         self._own_ctx = None
