@@ -694,6 +694,12 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_l1_fwd_ts(
 #pragma unroll
                 for (int i = 0; i < 8; ++i)                            // SWIZZLE_128B: 16-byte chunk index ^ (row % 8)
                     cur[i] = *reinterpret_cast<const float4*>(tile + ((i ^ (r_in & 7)) << 4));
+                // The TMA refills the slot through the async proxy as soon as yempty completes, so these generic-proxy
+                // reads must be performed first: the proxy fence (MEMBAR + FENCE.VIEW.ASYNC in SASS) holds the arrive
+                // until they have returned.  Without it the arrive waited on no load: when the TMA was parked on yempty
+                // (W resident, the Y ring full behind a slow epilogue) and the loads queued behind the epilogue's global
+                // stores, some 16-byte chunks were read from the NEXT fill of the slot, the k-block `ystages` later.
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&yempty_bar[ys]);          // the tile is in registers: the slot may be refilled
                 uint32_t hi[32], lo[32];
@@ -1300,12 +1306,12 @@ static int launch_fwd_ts(grapes_ctx* ctx, const float* Y, int ldy, const int* n_
         const int m_tiles_cap = (cap_n + TC_BM - 1) / TC_BM;
         if ((rc = make_map(&ma, Y, cap_n, K, ldy)) != GRAPES_OK) return rc;
         const int tail_b = 1024 /*align slack*/ + 1536 /*barriers, bias + output weights of the half*/;
-        // W half resident when it leaves room for >= 4 raw Y tiles; otherwise W streams through a 4-stage ring.  The dense
-        // layer (hout != NULL) always streams W: with W resident it wrote wrong rows, differently from run to run, once
-        // several CTAs each walked more row tiles than the Y ring holds k-blocks (tests/test_gpu_dense_tc.py: every
-        // products-shaped row count, K <= 160); the cause is not found yet, and the streamed form passes every case
-        const int wres = (!hout && nkb * 2 * TC_TILE_BYTES + 4 * TC_TILE_BYTES + tail_b <= 227 * 1024 && ctx->sm_count >= NH)
-                             ? 1 : 0;
+        // W half resident when it leaves room for >= 4 raw Y tiles; otherwise W streams through a 4-stage ring (and with
+        // grapes_tc_debug bit 1: both forms sum in the same order, so they give the same bits).  Both instantiations take
+        // the same policy.  (The dense layer once had to stream W: with W resident its CTAs read Y chunks from the next
+        // fill of a ring slot; see the proxy fence in the converters of k_l1_fwd_ts.)
+        const int wres = (nkb * 2 * TC_TILE_BYTES + 4 * TC_TILE_BYTES + tail_b <= 227 * 1024 && ctx->sm_count >= NH &&
+                          !(g_tc_debug & 2)) ? 1 : 0;
         const int bstages = 4;
         const int nbt = wres ? nkb : bstages;
         int ystages = (227 * 1024 - tail_b - nbt * 2 * TC_TILE_BYTES) / TC_TILE_BYTES;

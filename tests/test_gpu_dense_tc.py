@@ -1,15 +1,19 @@
 """grapes_gemm_bias_relu_tc -- H = relu(Y W^T + b) on the tcgen05 kernels, the hidden layer of the whole-graph evaluation
-forward -- against float64, through the C ABI.
+forward -- against float64, element by element, through the C ABI.
 
 It is the DENSE instantiation of k_l1_fwd_ts: the sampler head's kernel with the hidden activations stored instead of
-reduced against w2; it streams W through a ring of shared-memory stages (the sampler form keeps W resident when it fits:
-at most 5 k-blocks of 32, K <= 160; the dense form gave wrong rows that way, which the products-shaped cases here catch).
-The cases straddle the k-block counts of those forms (K <= 160, 6 to 8 k-blocks, and LONGK: more than 8 k-blocks, the
-accumulator drained into an fp32 master every 8), and include a context limited to one SM, on which every CTA walks
-hundreds of row tiles.  H starts as NaN: rows at or past the device count and the pitch columns [D, ldh) must keep it.  Y
-carries NaN in its rows past the device count and in its pitch columns past K, which the kernel must not let into a
-stored row.  The relu mask H > 0 equals, bit for bit, the maskT bits of grapes_sampler_l1_fwd_tc on the same inputs:
-both instantiations compute the same pre-activation, so any difference is a bug in one epilogue."""
+reduced against w2, and the same policy for W: resident in shared memory up to 5 k-blocks of 32 (K <= 160), streamed through
+a ring of shared-memory stages above.  The cases straddle the k-block counts of those forms (K <= 160, 6 to 8 k-blocks, and
+LONGK: more than 8 k-blocks, the accumulator drained into an fp32 master every 8), and include a context limited to one SM,
+on which every CTA walks hundreds of row tiles.  The row counts up to 200 003 make every resident CTA walk more row tiles
+than its Y ring holds: there the converters used to hand a ring slot back to the TMA before their reads of it had been
+performed, and behind this instantiation's store-heavy epilogue some of those reads returned the slot's next fill (wrong rows,
+different from run to run; the proxy fence before the release in k_l1_fwd_ts fixed it).  Every element must be within 1e-5
+of the sum of the magnitudes of its terms, sum_k |Y_rk W_dk| + |b_d|.  H starts as NaN: rows at or past the device count
+and the pitch columns [D, ldh) must keep it.  Y carries NaN in its rows past the device count and in its pitch columns past
+K, which the kernel must not let into a stored row.  The relu mask H > 0 equals, bit for bit, the maskT bits of
+grapes_sampler_l1_fwd_tc on the same inputs: both instantiations compute the same pre-activation, so any difference is a
+bug in one epilogue."""
 import ctypes
 
 import pytest
@@ -110,16 +114,22 @@ def _mask_bits(ctx, Y, n, cap_n, K, W, b):
 
 
 def _ref(Y, W, b, rows):
-    """float64 relu(Y W^T + b) of the given rows (a slice or an index tensor), on the device"""
+    """float64 relu(Y W^T + b) of the given rows (a slice or an index tensor), on the device, and the scale of each
+    element: sum_k |Y_rk W_dk| + |b_d|"""
     K = W.shape[1]
-    return torch.relu(Y[rows, :K].double() @ W.double().t() + b.double())
+    Yr = Y[rows, :K].double()
+    return (torch.relu(Yr @ W.double().t() + b.double()),
+            Yr.abs() @ W.double().abs().t() + b.double().abs())
 
 
-def _check(H, ref, rows, D, what=""):
+def _check(H, ref_scale, rows, D, what=""):
+    ref, scale = ref_scale
     got = H[rows, :D]
     assert bool(torch.isfinite(got).all()), f"{what}: non-finite entries in rows < n"
-    err = ((got.double() - ref).abs().max() / ref.abs().max().clamp_min(1e-30)).item()
-    assert err < TOL, f"{what}: relative error {err:.3e}"
+    err = (got.double() - ref).abs() / scale
+    worst = int(err.max(1).values.argmax())
+    assert bool((err <= TOL).all()), (f"{what}: {int((err > TOL).any(1).sum())} rows off float64, worst error "
+                                      f"{err.max().item():.3e} of the element scale (row {worst} of the checked rows)")
 
 
 def _run_case(ctx, dev, n, cap_n, K, D, seed, ldy=None, ldh=None, n_dev=None, h_rows=None, mask=True):
@@ -149,10 +159,12 @@ def test_dense_matches_fp64(cuda_device, ctxs, K, D):
     _run_case(ctxs["full"], cuda_device, 5000, 5200, K, D, seed=K * 7 + D)
 
 
-@pytest.mark.parametrize("n", [1, 127, 128, 129, 5000, 64943])
-@pytest.mark.parametrize("K,D", [(100, 256), (192, 128), (602, 512)])
+@pytest.mark.parametrize("n", [1, 127, 128, 129, 5000, 64943, 200_003])
+@pytest.mark.parametrize("K,D", [(100, 256), (192, 128), (602, 512), (15, 512), (33, 128), (131, 384)])
 def test_dense_row_counts(cuda_device, ctxs, n, K, D):
-    """a partial first / last row tile, exact tile multiples and a Reddit-sized row count"""
+    """a partial first / last row tile, exact tile multiples and a Reddit-sized row count; at 200 003 rows every CTA of
+    the resident forms (K = 15, 33, 100, 131) walks more row tiles than its Y ring holds k-blocks (10 to 11 tiles per CTA
+    at D = 128 on 148 SMs)"""
     _run_case(ctxs["full"], cuda_device, n, n + 300, K, D, seed=n + K)
 
 
