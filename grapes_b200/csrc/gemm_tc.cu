@@ -768,11 +768,21 @@ __device__ __forceinline__ float tf32_rna(float x) { return grapes_tf32_rna(x); 
 //   N = 2 * NB * 32 columns this is ONE tcgen05.mma per 8-row slice and 128-unit half (instead of three), reading
 //   12 KB of operands instead of 24 KB (the kernel is fed at the shared-memory read limit).  The two accumulator halves
 //   are added in the epilogue.  Columns [col0, col0 + NB*32) of Y per CTA (NB <= 4): wider Y = several column chunks (blockIdx.y).
+// The tensor core adds into its fp32 accumulator with truncation, so a long chain drifts when the terms do not cancel
+// (nonnegative features, dz of one sign: 1.9e-4 of the magnitude after 1563 groups in one chain; B200 at 1000 W).
+// Both backward kernels therefore cut every CTA's chain each TCBS_FLUSH groups (4 MMAs per group and accumulator; 96
+// groups drift 4.5e-6 in the same test): the epilogue stores each interval to its own partial slab
+// part[flush][cta][D][N], zero-fills the slabs past the CTA's last interval (the host sizes nflush for cap_n), and
+// k_l1_bwd_finalize adds the slabs rounding to nearest.
+#define TCBS_FLUSH 96
 #define TCB_THREADS 320          // TMA, MMA, 4 mask-expander (+ epilogue) warps, 4 operand-scaling warps
-__global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
+// (register cap: with the interval epilogue inside the expanders' loop ptxas takes 126 registers instead of 85, which
+//  leaves less of the register file to the kernels that share the SM in the training step: the Cora-shaped step measured
+//  2 % slower on a B200 at 1000 W, with this kernel's own time unchanged.  Launched with TCB_THREADS threads.)
+__global__ void __maxnreg__(88) k_l1_bwd_tc(
     const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmY_lo, int presplit, int col0,
     const int* __restrict__ n_dev, int cap_n, int NH, int NB, int stages, const uint32_t* __restrict__ maskT, int D,
-    const float* __restrict__ dz, float* __restrict__ part, int debug, int ncols, long long chunk_stride) {
+    const float* __restrict__ dz, float* __restrict__ part, int debug, int ncols, long long chunk_stride, int nflush) {
     pdl_begin();
     // blockIdx.y = column chunk of Y (128 columns each): all chunks of a wide Y (Cora 1437, Reddit 606 columns) run in ONE
     // launch next to each other instead of one launch per chunk; every chunk has its own slab of the partial buffer
@@ -788,21 +798,23 @@ __global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
     uint64_t* full_bar = bars;                       // [stages] 4 mask-expander + 4 scaling warps -> MMA
     uint64_t* empty_bar = bars + 4;                  // [stages] MMA -> TMA + expanders
     uint64_t* tma_bar = bars + 8;                    // [stages] TMA (Y tile) -> expanders
-    uint64_t* done_bar = bars + 12;                  // all MMAs retired -> epilogue
+    uint64_t* done_bar = bars + 12;                  // MMAs of a flush interval retired -> epilogue
     uint32_t* tmem_slot = (uint32_t*)(bars + 13);
-    float* s_dz = (float*)(bars + 16);               // [stages][32] dz of the group's rows
+    uint64_t* drained_bar = bars + 14;               // epilogue -> MMA: accumulators may be overwritten
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n = min(*n_dev, cap_n);
     const int groups = (n + TCB_ROWS - 1) / TCB_ROWS;
     const int N = NB * 32;                           // S columns of this launch; accumulator holds 2N per half
     const int my_groups = (groups > (int)blockIdx.x) ? (groups - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+    const int my_flushes = (my_groups + TCBS_FLUSH - 1) / TCBS_FLUSH;     // <= nflush (sized for cap_n on the host)
 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tmY);
         if (presplit) tma_prefetch_desc(&tmY_lo);
         for (int s = 0; s < stages; ++s) { mbar_init(&full_bar[s], 8); mbar_init(&empty_bar[s], 1); mbar_init(&tma_bar[s], 1); }
         mbar_init(done_bar, 1);
+        mbar_init(drained_bar, 4);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) tmem_alloc(tmem_slot, 512);
@@ -831,8 +843,13 @@ __global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
             const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 16) | ((uint32_t)((2 * N) >> 3) << 17) |
                                    ((uint32_t)(128 >> 4) << 24);
             int stage = 0; uint32_t phase = 0;
-            bool first = true;
-            for (int g = blockIdx.x; g < groups; g += gridDim.x) {
+            for (int it = 0; it < my_groups; ++it) {
+                const int in_flush = it % TCBS_FLUSH;
+                if (in_flush == 0 && it > 0) {
+                    umma_commit(done_bar);                      // interval done: the epilogue stores it to its slab
+                    mbar_wait(drained_bar, (uint32_t)((it / TCBS_FLUSH - 1) & 1));
+                    tc_fence_after();
+                }
                 mbar_wait(&full_bar[stage], phase);
                 tc_fence_after();
                 const uint32_t sa = smem_u32(smem + stage * stage_bytes);
@@ -844,10 +861,9 @@ __global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
                     for (int ks = 0; ks < TCB_ROWS / 8; ++ks) {
                         const uint64_t adv_a = (uint64_t)((ks * 32) >> 4);       // 8 r = 32 bytes along the swizzle row
                         const uint64_t adv_b = (uint64_t)((ks * 1024) >> 4);     // 8 rows of 128 bytes
-                        umma_tf32(d_tmem, ad + adv_a, bd + adv_b, idesc, (first && ks == 0) ? 0u : 1u);
+                        umma_tf32(d_tmem, ad + adv_a, bd + adv_b, idesc, (in_flush == 0 && ks == 0) ? 0u : 1u);
                     }
                 }
-                first = false;
                 umma_commit(&empty_bar[stage]);
                 if (++stage == stages) { stage = 0; phase ^= 1; }
             }
@@ -897,7 +913,37 @@ __global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
 #pragma unroll
             for (int h = 0; h < 4; ++h) if (h < NH) words_nx[h] = maskT[(size_t)blockIdx.x * D + h * 128 + e];
         }
-        for (int g = blockIdx.x; g < groups; g += gridDim.x) {
+        // epilogue of flush interval fl: its partial S -> part[fl][cta][NH*128][N]  (hi-part + lo-part accumulators)
+        const int q = warp & 3;
+        auto slab_row = [&](int fl, int h) {
+            return part + (((size_t)fl * gridDim.x + blockIdx.x) * NH * 128 + (size_t)(h * 128 + q * 32 + lane)) * N;
+        };
+        auto drain = [&](int fl) {
+            mbar_wait(done_bar, (uint32_t)(fl & 1));
+            tc_fence_after();
+            for (int h = 0; h < NH; ++h) {
+                float* row = slab_row(fl, h);
+                for (int ch = 0; ch < NB; ++ch) {
+                    uint32_t v[32], v2[32];
+                    tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(h * 2 * N + ch * 32), v);
+                    tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(h * 2 * N + N + ch * 32), v2);
+#pragma unroll
+                    for (int c = 0; c < 32; c += 4)
+                        *reinterpret_cast<float4*>(row + ch * 32 + c) =
+                            make_float4(__uint_as_float(v[c]) + __uint_as_float(v2[c]),
+                                        __uint_as_float(v[c + 1]) + __uint_as_float(v2[c + 1]),
+                                        __uint_as_float(v[c + 2]) + __uint_as_float(v2[c + 2]),
+                                        __uint_as_float(v[c + 3]) + __uint_as_float(v2[c + 3]));
+                }
+            }
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(drained_bar);
+        };
+        int g = blockIdx.x;
+        for (int fl = 0; fl < my_flushes; ++fl) {
+          const int g_end = min(groups, g + TCBS_FLUSH * (int)gridDim.x);   // the groups of interval fl
+          for (; g < g_end; g += gridDim.x) {
             uint32_t words[4];
 #pragma unroll
             for (int h = 0; h < 4; ++h) words[h] = words_nx[h];
@@ -926,34 +972,15 @@ __global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
             __syncwarp();
             if (lane == 0) mbar_arrive(&full_bar[stage]);
             if (++stage == stages) { stage = 0; phase ^= 1; }
+          }
+          drain(fl);
         }
-        // epilogue: this CTA's partial S -> part[cta][NH*128][N]  (hi-part + lo-part accumulators)
-        const int q = warp & 3;
-        float* dst = part + (size_t)blockIdx.x * NH * 128 * N;
-        if (my_groups > 0) {
-            mbar_wait(done_bar, 0);
-            tc_fence_after();
+        // flush slabs this CTA did not reach (fewer rows than the capacity the host sized for): zeros
+        for (int fl = my_flushes; fl < nflush; ++fl)
             for (int h = 0; h < NH; ++h) {
-                float* row = dst + (size_t)(h * 128 + q * 32 + lane) * N;
-                for (int ch = 0; ch < NB; ++ch) {
-                    uint32_t v[32], v2[32];
-                    tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(h * 2 * N + ch * 32), v);
-                    tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(h * 2 * N + N + ch * 32), v2);
-#pragma unroll
-                    for (int c = 0; c < 32; c += 4)
-                        *reinterpret_cast<float4*>(row + ch * 32 + c) =
-                            make_float4(__uint_as_float(v[c]) + __uint_as_float(v2[c]),
-                                        __uint_as_float(v[c + 1]) + __uint_as_float(v2[c + 1]),
-                                        __uint_as_float(v[c + 2]) + __uint_as_float(v2[c + 2]),
-                                        __uint_as_float(v[c + 3]) + __uint_as_float(v2[c + 3]));
-                }
-            }
-        } else {
-            for (int h = 0; h < NH; ++h) {
-                float* row = dst + (size_t)(h * 128 + q * 32 + lane) * N;
+                float* row = slab_row(fl, h);
                 for (int c = 0; c < N; c += 4) *reinterpret_cast<float4*>(row + c) = make_float4(0.f, 0.f, 0.f, 0.f);
             }
-        }
     }
     tc_fence_before();
     __syncthreads();
@@ -983,7 +1010,6 @@ __global__ void __launch_bounds__(TCB_THREADS, 1) k_l1_bwd_tc(
 // ------------------------------------------------------------------------------------------------
 #define TCBS_THREADS 448            // TMA, MMA, 4 mask-expander (+ epilogue) warps, 8 converter warps (two groups)
 #define TCBS_STAGES 4
-#define TCBS_FLUSH 96               // groups (x 4 MMAs per accumulator) between two flushes of the accumulators
 __global__ void __launch_bounds__(TCBS_THREADS, 1) k_l1_bwd_ts(
     const __grid_constant__ CUtensorMap tmY, int ncols, const int* __restrict__ n_dev, int cap_n, int NH,
     const uint32_t* __restrict__ maskT, int D, const float* __restrict__ dz, float* __restrict__ part,
@@ -1055,8 +1081,8 @@ __global__ void __launch_bounds__(TCBS_THREADS, 1) k_l1_bwd_ts(
             for (int it = 0; it < my_groups; ++it) {
                 const int in_flush = it % TCBS_FLUSH;
                 if (in_flush == 0 && it > 0) {
-                    // the tensor core adds into its fp32 accumulator with truncation: chains are kept short.  The epilogue
-                    // stores the interval's sums to their own partial slab; the finalize adds the slabs (round to nearest)
+                    // the tensor core adds into its fp32 accumulator with truncation: chains are kept short (TCBS_FLUSH).
+                    // The epilogue stores the interval's sums to their own partial slab; the finalize adds the slabs
                     umma_commit(done_bar);
                     mbar_wait(drained_bar, (uint32_t)((it / TCBS_FLUSH - 1) & 1));
                     tc_fence_after();
@@ -1504,14 +1530,18 @@ int grapes_sampler_l1_bwd_tc(grapes_ctx* ctx, const float* Y, const float* Y_lo,
     const int max_groups = (cap_n + TCB_ROWS - 1) / TCB_ROWS;
     int blocks = grapes_max_i(1, ctx->sm_count / nchunks);           // CTAs per chunk
     if (blocks > max_groups) blocks = max_groups;
-    while (blocks > 1 && (size_t)nchunks * blocks * D * 128 * sizeof(float) > ctx->partials_bytes) --blocks;
-    GRAPES_REQUIRE((size_t)nchunks * blocks * D * 128 * sizeof(float) <= ctx->partials_bytes, "split partial buffer too small");
-    const long long chunk_stride = (long long)blocks * D * 128;
+    // one partial slab per CTA and flush interval, as in k_l1_bwd_ts
+    auto slabs = [&](int b) { return (size_t)b * grapes_div_up(grapes_div_up(max_groups, b), TCBS_FLUSH); };
+    while (blocks > 1 && nchunks * slabs(blocks) * D * 128 * sizeof(float) > ctx->partials_bytes) --blocks;
+    GRAPES_REQUIRE(nchunks * slabs(blocks) * D * 128 * sizeof(float) <= ctx->partials_bytes, "split partial buffer too small");
+    const int nflush = (int)(slabs(blocks) / blocks);
+    const long long chunk_stride = (long long)slabs(blocks) * D * 128;
     pdl((k_l1_bwd_tc), dim3(blocks, nchunks), TCB_THREADS, smem_bytes, s)(my, my_lo, Y_lo ? 1 : 0, 0, n_dev, cap_n, NH, NB, stages,
-                                                                      maskT, D, dz, ctx->partials, g_tc_debug, ncols, chunk_stride);
+                                                                      maskT, D, dz, ctx->partials, g_tc_debug, ncols, chunk_stride,
+                                                                      nflush);
     grapes_count_launches(1);
-    pdl((k_l1_bwd_finalize), D, FIN_THREADS, 0, s)(ctx->partials, blocks, D, ncols, nchunks, chunk_stride, K, W1, ldw, b1, w2,
-                                                ones_col, scale, gW1, gb1, gw2);
+    pdl((k_l1_bwd_finalize), D, FIN_THREADS, 0, s)(ctx->partials, blocks * nflush, D, ncols, nchunks, chunk_stride, K, W1, ldw, b1,
+                                                w2, ones_col, scale, gW1, gb1, gw2);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;

@@ -365,7 +365,13 @@ int grapes_gemm_bias_relu_tc(grapes_ctx* ctx, const float* Y, int ldy, const int
                              const float* W_lo, int ldw, int D, const float* b, float* H, int ldh, void* stream);
 
 /* backward on tensor cores: S = mask^T (dz * Y) from the relu mask bits; Y must hold a column of ones at
- * `ones_col` (K <= ones_col < ncols <= ldy).  Accumulates scale * d(sum dz.z)/d(W1,b1,w2).               */
+ * `ones_col` (K <= ones_col < ncols <= ldy).  Accumulates scale * d(sum dz.z)/d(W1,b1,w2).
+ * n = min(*n_dev, cap_n).  The kernels read Y in groups of 32 rows: rows [n, round_up(n, 32)) within cap_n are read
+ * and multiplied by a dz of 0, so they must hold FINITE values (0 * inf or 0 * NaN would reach the gradients); dz past
+ * n is not read, the mask bits of rows >= n do not matter, and rows past cap_n are never read.  A zero-initialised Y
+ * buffer meets this.
+ * The split partial buffer of the ctx (partials_bytes) must hold one D x 128 slab per CTA, 128-column chunk and flush
+ * interval of 96 row groups; a call it cannot hold returns an error and writes nothing.                           */
 int grapes_sampler_l1_bwd_tc(grapes_ctx* ctx, const float* Y, const float* Y_lo, int ldy, int ncols, const int* n_dev,
                              int cap_n, int K, int ones_col, const uint32_t* maskT, const float* W1, int ldw, int D,
                              const float* b1, const float* w2, const float* dz, float scale, float* gW1, float* gb1,
