@@ -502,16 +502,17 @@ __global__ void __launch_bounds__(CB_THREADS) k_gnw_edges(const int64_t* __restr
 // d of the edges s -> d, stored self-loops dropped.  From the graph's CSR, whose row s already holds its destinations
 // sorted and unique, that is row s without s itself: a count (pass 0) and an order-keeping warp compaction (pass 1) at
 // out_off[s], no cursor and no sort.  From an edge list it is k_gn_edges with the roles of source and destination swapped.
+// out_off is read at r - off0: 0 for the whole structure, lo for the offsets of a source window [lo, hi).
 template <bool FILL>
 __global__ void __launch_bounds__(CB_THREADS) k_gnt_csr(const long long* __restrict__ indptr, const int* __restrict__ indices,
                                                          int64_t r0, int64_t r1, int64_t N, int* __restrict__ cnt,
-                                                         const long long* __restrict__ out_off, int* __restrict__ out_dst,
-                                                         int* __restrict__ err) {
+                                                         const long long* __restrict__ out_off, int64_t off0,
+                                                         int* __restrict__ out_dst, int* __restrict__ err) {
     const int lane = lane_id();
     const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t r = r0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); r < r1; r += warps) {
         const long long e0 = indptr[r], e1 = indptr[r + 1];
-        long long base = FILL ? out_off[r] : 0;
+        long long base = FILL ? out_off[r - off0] : 0;
         for (long long c0 = e0; c0 < e1; c0 += 32) {
             const long long e = c0 + lane;
             const int64_t v = e < e1 ? (int64_t)indices[e] : (int64_t)r;
@@ -886,10 +887,10 @@ int grapes_graph_norm_t_add_csr(int pass, int64_t num_nodes, const int64_t* indp
     cudaStream_t s = (cudaStream_t)stream;
     if (pass == 0)
         pdl(k_gnt_csr<false>, grid, CB_THREADS, 0, s)((const long long*)indptr, indices, r0, r1, num_nodes, cnt, nullptr,
-                                                       nullptr, err_dev);
+                                                       (int64_t)0, nullptr, err_dev);
     else
         pdl(k_gnt_csr<true>, grid, CB_THREADS, 0, s)((const long long*)indptr, indices, r0, r1, num_nodes, cnt,
-                                                      (const long long*)out_off, out_dst, err_dev);
+                                                      (const long long*)out_off, (int64_t)0, out_dst, err_dev);
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
@@ -959,6 +960,32 @@ int grapes_graph_norm_window_add_edges(int64_t num_nodes, const int64_t* src, co
     grapes_count_launches(1);
     GRAPES_LAUNCH_OK();
     return GRAPES_OK;
+}
+
+int grapes_graph_norm_t_window_add_csr(int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0,
+                                       int64_t r1, int64_t lo, int64_t hi, const int64_t* win_off, int* out_dst,
+                                       void* workspace, void* stream) {
+    GRAPES_REQUIRE(indptr && workspace && win_off && out_dst, "null argument");
+    GRAPES_REQUIRE(0 <= r0 && r0 <= r1 && r1 <= num_nodes, "row range outside [0, N]");
+    GRAPES_REQUIRE(0 <= lo && lo <= hi && hi <= num_nodes, "window outside [0, N]");
+    // CSR row s is transposed row s: only the input rows inside the window are read
+    const int64_t a = r0 > lo ? r0 : lo, b = r1 < hi ? r1 : hi;
+    if (b <= a) return GRAPES_OK;
+    int sms = 0;
+    if (gn_sms(&sms) != GRAPES_OK) return GRAPES_ERR_CUDA;
+    const int64_t ctas = ((b - a) * 32 + CB_THREADS - 1) / CB_THREADS;
+    pdl(k_gnt_csr<true>, (int)(ctas < (int64_t)sms * 16 ? ctas : (int64_t)sms * 16), CB_THREADS, 0, (cudaStream_t)stream)(
+        (const long long*)indptr, indices, a, b, num_nodes, nullptr, (const long long*)win_off, lo, out_dst, nullptr);
+    grapes_count_launches(1);
+    GRAPES_LAUNCH_OK();
+    return GRAPES_OK;
+}
+
+int grapes_graph_norm_t_window_add_edges(int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                         int64_t lo, int64_t hi, const int64_t* win_off, int* out_dst, void* workspace,
+                                         void* stream) {
+    // the forward window's scatter keyed by the source: row = src[e] in [lo, hi), entry = dst[e]
+    return grapes_graph_norm_window_add_edges(num_nodes, dst, src, num_edges, lo, hi, win_off, out_dst, workspace, stream);
 }
 
 }  // extern "C"

@@ -357,6 +357,8 @@ class ShardedGraphNorm:
         self.graph, self.world, self.rank = graph, int(world), int(rank)
         self.holder = _any_ctx(dev)
         self.n = N
+        self._input = (edge_index, chunk_edges)
+        self.out_off = self.out_dst = None
         ws = torch.empty(max(int(L.cdll.grapes_graph_norm_workspace_bytes(N)), 1), dtype=torch.uint8, device=dev)
         err = torch.zeros(1, dtype=torch.int32, device=dev)
         nnz = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -393,6 +395,48 @@ class ShardedGraphNorm:
         if self.E == 0:
             self.in_src = self.in_src[:0]
 
+    def build_transposed(self):
+        """The source window ``lo .. hi`` of the transposed structure, once, from the constructor's input: ``out_off``
+        int64 [rows + 1] local to the window and ``out_dst`` int32 (``grapes_graph_norm_t_window_*``), equal bit for bit
+        to rows ``lo .. hi`` of :func:`transposed_structure`.  The same bounds as the forward window, so a rank owns the
+        same rows in both directions; ``dinv`` is not touched.  Device memory beyond the outputs: the ~4 N-byte workspace
+        plus the full int64 [N + 1] offsets until the window's are cut out, plus one chunk of a host edge list."""
+        if self.out_off is not None:
+            return
+        edge_index, chunk_edges = self._input
+        graph, N, dev = self.graph, self.n, self.dinv.device
+        L, st = lib(), _stream()
+        ws = torch.empty(max(int(L.cdll.grapes_graph_norm_workspace_bytes(N)), 1), dtype=torch.uint8, device=dev)
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        nnz = torch.zeros(1, dtype=torch.int64, device=dev)
+        full = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        L.grapes_graph_norm_begin(N, ptr(ws), ws.numel(), ptr(err), st)
+        if edge_index is None:
+            L.grapes_graph_norm_t_add_csr(0, N, ptr(graph.indptr), ptr(graph.indices), 0, N, None, None, ptr(ws), ptr(err),
+                                          st)
+        else:
+            for src, dst in _edge_chunks(edge_index, chunk_edges, dev):
+                L.grapes_graph_norm_t_add_edges(0, N, ptr(src), ptr(dst), int(src.numel()), None, None, ptr(ws), ptr(err),
+                                                st)
+        L.grapes_graph_norm_t_offsets(N, ptr(ws), ptr(full), ptr(nnz), st)
+        WideGraphNorm._check(err, "out-edges")
+        out_off = (full[self.lo:self.hi + 1] - full[self.lo]).contiguous()
+        del full
+        E = int(out_off[-1].item())                                   # one-off read-back: the size of out_dst
+        out_dst = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+        if edge_index is None:
+            L.grapes_graph_norm_t_window_add_csr(N, ptr(graph.indptr), ptr(graph.indices), 0, N, self.lo, self.hi,
+                                                 ptr(out_off), ptr(out_dst), ptr(ws), st)
+        else:
+            for src, dst in _edge_chunks(edge_index, chunk_edges, dev):
+                L.grapes_graph_norm_t_window_add_edges(N, ptr(src), ptr(dst), int(src.numel()), self.lo, self.hi,
+                                                       ptr(out_off), ptr(out_dst), ptr(ws), st)
+            if self.rows > 0:
+                L.grapes_graph_norm_finish(self.rows, ptr(out_off), ptr(out_dst), ptr(ws), st)
+        del ws
+        self._dst = out_dst                        # non-null for the kernels even when the window has no out-edge
+        self.out_off, self.out_dst = out_off, (out_dst if E > 0 else out_dst[:0])
+
     @property
     def in_off_base(self) -> int:
         """Device address that makes ``in_off[r]`` of the row-slab kernels (r = graph row) land on local row r - lo: the
@@ -407,14 +451,20 @@ class ShardedGraphNorm:
                                       out.stride(0), _stream())
         return out
 
-    def aggregate_rows_peer(self, z_table, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None) -> torch.Tensor:
-        """The same over Z partitioned by window: rank o's rows in ``z_table.ptrs[o]`` (pitch ``z_table.ld`` floats),
-        ``grapes_aggregate_rows64_peer``; bit-identical to :meth:`aggregate_rows` over the unpartitioned Z."""
+    def aggregate_rows_peer(self, z_table, slab: torch.Tensor, R: int, out: torch.Tensor, bias=None,
+                            transpose: bool = False, F=None) -> torch.Tensor:
+        """The same over Z partitioned by window: rank o's rows in ``z_table.ptrs[o]`` (pitch ``z_table.ld`` floats, the
+        first ``F`` of them read, default all), ``grapes_aggregate_rows64_peer``; bit-identical to :meth:`aggregate_rows`
+        over the unpartitioned Z.  ``transpose``: rows of A_hat^T Z on the transposed window (:meth:`build_transposed`,
+        built here on first use), bit-identical to ``WideGraphNorm.aggregate(Z, transpose=True)``."""
         import ctypes
-        F = z_table.ld
+        F = z_table.ld if F is None else int(F)
+        if transpose:
+            self.build_transposed()
+        off, idx = (self.out_off, self._dst) if transpose else (self.in_off, self._src)
         b = (ctypes.c_int64 * (self.world + 1))(*self.bounds)
         lib().grapes_aggregate_rows64_peer(self.holder.ctx, z_table.ptrs, b, self.world, F, z_table.ld, ptr(slab), R,
-                                           self.in_off_base, ptr(self._src), ptr(self.dinv), ptr(bias), ptr(out),
+                                           off.data_ptr() - 8 * self.lo, ptr(idx), ptr(self.dinv), ptr(bias), ptr(out),
                                            out.stride(0), _stream())
         return out
 

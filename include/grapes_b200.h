@@ -159,6 +159,26 @@ int grapes_graph_norm_window_add_csr(int64_t num_nodes, const int64_t* indptr, c
 int grapes_graph_norm_window_add_edges(int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
                                        int64_t lo, int64_t hi, const int64_t* win_off, int* in_src, void* workspace,
                                        void* stream);
+/* ---- one source window [lo, hi) of the transposed structure (the backward of the data-parallel full-graph training):
+ * row s in [lo, hi) lists the destinations d of the edges s -> d, ascending, stored self-loops dropped, duplicates of an
+ * edge list kept and counted -- rows lo .. hi of grapes_graph_norm_t_*, bit for bit.  Use the bounds of the forward
+ * window (grapes_graph_norm_window_bounds), so a rank owns the same rows in both directions.
+ * Sequence for the window of one rank, all on `stream`, no host synchronisation inside: begin -> t_add_*(pass 0) over the
+ * WHOLE input (every out-degree is counted) -> t_offsets into a full [N+1] out_off -> the caller forms
+ * win_off[j] = out_off[lo + j] - out_off[lo] (j <= hi - lo) and may free the full out_off -> t_window_add_* over the
+ * whole input (only edges out of [lo, hi) are written, at out_dst[win_off[s - lo] ...]) -> for an edge list only:
+ * finish(hi - lo, win_off, out_dst, workspace) (the per-row sorts of the window; skip it for an empty window).
+ * t_window_add_csr reads rows [r0, r1) of a canonical CSR and, of those, touches only the rows inside the window: an
+ * order-keeping compaction that needs no cursor and no sort.  t_window_add_edges is grapes_graph_norm_window_add_edges
+ * with the roles of source and destination swapped (the cursor that t_offsets zeroed).  Ids were checked by pass 0.
+ * Peak device scratch beyond the outputs (win_off, the window's out_dst): the workspace (~4 N bytes) plus the full
+ * out_off (8 (N + 1) bytes) until win_off is formed.  dinv is not touched: the forward's serves both directions.   */
+int grapes_graph_norm_t_window_add_csr(int64_t num_nodes, const int64_t* indptr, const int* indices, int64_t r0,
+                                       int64_t r1, int64_t lo, int64_t hi, const int64_t* win_off, int* out_dst,
+                                       void* workspace, void* stream);
+int grapes_graph_norm_t_window_add_edges(int64_t num_nodes, const int64_t* src, const int64_t* dst, int64_t num_edges,
+                                         int64_t lo, int64_t hi, const int64_t* win_off, int* out_dst, void* workspace,
+                                         void* stream);
 
 /* ---- frontier expansion / dedup / relabel  (utils.py:74-82, main.py:183-195, utils.py:98-120) */
 /* rows[P] -> row_off[P+1] = exclusive scan of CSR degrees, *m_dev = total.  Sets the bit of every
